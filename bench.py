@@ -9,6 +9,7 @@ output activations at batch 256 through PytorchActivationQuantizationHolder(Acti
 
     python bench.py --gpus N --steps K --warmup W                 (N > 1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W (the reference's CPU torch path, rank 0 only)
+    python bench.py ... --dump-outputs DIR                         (also write the last timed step's outputs to DIR/*.npy)
 
 Prints ONE JSON line (rank 0).  metric = algorithmic GB/s (8 B per f32 element), whole job.
 Multi-GPU: activations shard by batch (every rank owns 256 images: weak scaling), weights shard by layer; there is
@@ -70,6 +71,8 @@ def parse_args():
     ap.add_argument("--ref-batch", type=int, default=64, help="images per step of the cpu_baseline sample inside the B200 arm's line "
                     "(--impl reference itself runs the full --batch)")
     ap.add_argument("--no-per-config", action="store_true", help="skip the C1 / C3 / C4 / C5 rows (per_config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned as "
+                    "DIR/<name>.npy (float32): every quantized weight tensor and a fixed sample of every activation site")
     return ap.parse_args()
 
 
@@ -317,6 +320,25 @@ def verify_against_oracle(torch, wplan, weights, wq, holders, acts, last, aplan)
             "what": "3 windows of <= 65536 elements of 4 activation sites (incl. the last timed output and the largest site) + 3 weight tensors"}
 
 
+DUMP_SAMPLE = 1 << 17      # elements written per activation site: 53 sites -> at most 27.8 MB, + 13.9 MB of weights
+
+
+def dump_outputs(out_dir, layer_ids, weights_out, acts_out):
+    """Writes the outputs of one step so that two builds can be compared array for array: weight_<layer>.npy, every
+    quantized weight tensor whole; act_<site>.npy, the site's output whole if it has at most DUMP_SAMPLE elements, else
+    DUMP_SAMPLE of its flat elements at indices drawn without replacement by numpy's default_rng(<site>), increasing."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for k, y in zip(layer_ids, weights_out):
+        np.save(os.path.join(out_dir, f"weight_{k:02d}.npy"), y.to(torch.float32).cpu().numpy())
+    for i, y in enumerate(acts_out):
+        if y.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(i).choice(y.numel(), DUMP_SAMPLE, replace=False))
+            y = y.reshape(-1)[torch.from_numpy(idx).to(y.device)]
+        np.save(os.path.join(out_dir, f"act_{i:02d}.npy"), y.to(torch.float32).cpu().numpy())
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -374,11 +396,13 @@ def run_b200(args):
     assert not aplan.other and len(aplan._plans) == 1
 
     ev = lambda: torch.cuda.Event(enable_timing=True)  # noqa: E731
+    step_outputs = {"weights": [], "acts": []}        # what the latest step() returned (plan-owned buffers, no copies)
 
     def step():
         if wplan is not None:
-            wplan.run()
-        return aplan.run()[-1]
+            step_outputs["weights"] = wplan.run()
+        step_outputs["acts"] = aplan.run()
+        return step_outputs["acts"][-1]
 
     def step_per_call():
         if wplan is not None:
@@ -470,6 +494,8 @@ def run_b200(args):
     ms_step = t.item() / args.steps
     value = tot_bytes.item() / (ms_step * 1e-3) / 1e9
     clocks = sampler.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, my_layers, step_outputs["weights"], step_outputs["acts"])
 
     # ---- the same step as per-holder calls (53 + 1 launches), same timing rules
     torch.cuda.synchronize()

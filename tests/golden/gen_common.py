@@ -5,6 +5,7 @@ import json
 import os
 import sys
 import warnings
+import zlib
 
 import numpy as np
 
@@ -90,7 +91,9 @@ def all_finite_half_patterns(dtype):
     return t[keep]
 
 
-def add_case(name, cls_name, args, x, extra_params=None, lut_info=None):
+def add_case(name, cls_name, args, x, extra_params=None, lut_info=None, x_gen=None):
+    """`x_gen`: name of the generator in tests/golden_util.py that reproduces `x` exactly (e.g. "all_finite_half_patterns");
+    the input is then not stored, only what the reference computed from it."""
     cls = getattr(Q, cls_name)
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
@@ -100,7 +103,10 @@ def add_case(name, cls_name, args, x, extra_params=None, lut_info=None):
     case = {"name": name, "cls": cls_name, "args": args, "shape": list(x.shape),
             "x_dtype": str(x.dtype).replace("torch.", ""), "y_dtype": str(y.dtype).replace("torch.", ""),
             "params": {}}
-    arrays[f"{name}/x"] = store(x)
+    if x_gen is None:
+        arrays[f"{name}/x"] = store(x)
+    else:
+        case["x_gen"] = x_gen
     arrays[f"{name}/y"] = store(y)
     # constructor-derived parameters (what the host side of the replacement must reproduce bit-for-bit)
     for attr in ("scales", "zero_points", "min_range", "max_range", "scale", "zero_point",
@@ -152,10 +158,26 @@ def lut_channel_input(rng, lut, thr, bw, signed, L, eps=1e-8):
     return v
 
 
+MAX_ARCHIVE_BYTES = 900_000     # keeps every fixture file below 1 MB
+
+
 def save(stem):
-    np.savez_compressed(os.path.join(HERE, stem + ".npz"), **arrays)
+    """arrays -> stem.npz, stem_2.npz, ... (a new archive whenever the compressed size would pass MAX_ARCHIVE_BYTES; the
+    manifest lists them under "archives"), manifest -> stem.json."""
+    parts, part, size = [], {}, 0
+    for key, a in arrays.items():
+        n = len(zlib.compress(np.ascontiguousarray(a).tobytes())) + 256       # + npy header and zip entry
+        if part and size + n > MAX_ARCHIVE_BYTES:
+            parts.append(part)
+            part, size = {}, 0
+        part[key] = a
+        size += n
+    parts.append(part)
+    manifest["archives"] = [stem + ".npz"] + [f"{stem}_{k}.npz" for k in range(2, len(parts) + 1)]
+    for name, part in zip(manifest["archives"], parts):
+        np.savez_compressed(os.path.join(HERE, name), **part)
     with open(os.path.join(HERE, stem + ".json"), "w") as f:
         json.dump(manifest, f, indent=1)
     tot = sum(a.nbytes for a in arrays.values())
     print(f"{len(manifest['cases'])} cases, {len(arrays)} arrays, {tot / 1e6:.1f} MB raw ->",
-          os.path.getsize(os.path.join(HERE, stem + '.npz')) / 1e6, "MB")
+          [os.path.getsize(os.path.join(HERE, name)) / 1e6 for name in manifest["archives"]], "MB")

@@ -12,8 +12,9 @@ mid-point +- {0..3} ulp, all 2^16 bit patterns for half-precision per-tensor cas
 inputs, outputs and the constructor-derived parameters.  The reference has no golden vectors of its
 own (SURVEY.md 8c), so these fixtures are what pins the oracle and the CUDA path.
 
-Outputs: golden_v1.npz (arrays) + golden_v1.json (manifest).  Half-precision tensors are stored as
-uint16 bit patterns.  The reference cannot travel to the GPU box; the fixtures do.
+Outputs: golden_v1.npz, golden_v1_2.npz, ... (arrays, each file below 1 MB) + golden_v1.json (manifest,
+which lists the archives).  Half-precision tensors are stored as uint16 bit patterns; the all-bit-pattern
+inputs are not stored, tests/golden_util.py regenerates them.  The reference cannot travel to the GPU box; the fixtures do.
 """
 import os
 import sys
@@ -70,7 +71,7 @@ for dt in ("bfloat16", "float16"):
              dict(num_bits=bits, threshold=thr, per_channel=True, channel_axis=axis), x)
     x = all_finite_half_patterns(dt)
     add_case(f"w_sym_b4_pt_{dt}_allbits", "WeightsSymmetricInferableQuantizer",
-             dict(num_bits=4, threshold=[1.7], per_channel=False), x)
+             dict(num_bits=4, threshold=[1.7], per_channel=False), x, x_gen="all_finite_half_patterns")
 
 # uniform weights: straddling, strictly positive, strictly negative ranges (range fixing) + zp truncation
 for bits in (2, 4, 8):
@@ -110,9 +111,12 @@ for cls_name, thr_list in (("ActivationSymmetricInferableQuantizer", [3.7, 0.61]
                          torch.from_numpy(v.reshape(2, 3, 10, 100)))
 for dt in ("bfloat16", "float16"):
     x = all_finite_half_patterns(dt)
-    add_case(f"a_sym_b8_s_{dt}_allbits", "ActivationSymmetricInferableQuantizer", dict(num_bits=8, threshold=[3.7], signed=True), x)
-    add_case(f"a_pot_b8_u_{dt}_allbits", "ActivationPOTInferableQuantizer", dict(num_bits=8, threshold=[4.0], signed=False), x)
-    add_case(f"a_uni_b8_{dt}_allbits", "ActivationUniformInferableQuantizer", dict(num_bits=8, min_range=[-1.0], max_range=[2.3]), x)
+    add_case(f"a_sym_b8_s_{dt}_allbits", "ActivationSymmetricInferableQuantizer", dict(num_bits=8, threshold=[3.7], signed=True), x,
+             x_gen="all_finite_half_patterns")
+    add_case(f"a_pot_b8_u_{dt}_allbits", "ActivationPOTInferableQuantizer", dict(num_bits=8, threshold=[4.0], signed=False), x,
+             x_gen="all_finite_half_patterns")
+    add_case(f"a_uni_b8_{dt}_allbits", "ActivationUniformInferableQuantizer", dict(num_bits=8, min_range=[-1.0], max_range=[2.3]), x,
+             x_gen="all_finite_half_patterns")
 
 for bits in (2, 4, 7, 8):
     for tag, (a, b) in {"straddle": (-1.0, 2.3), "sym4": (-4.0, 4.0), "pos": (0.25, 6.0), "neg": (-3.0, -0.7)}.items():
@@ -182,7 +186,7 @@ for dt in ("bfloat16", "float16"):
         for thr in (4.0, 0.0625):
             add_case(f"al_{'s' if signed else 'u'}_t{thr}_{dt}_allbits", "ActivationLutPOTInferableQuantizer",
                      dict(num_bits=4, lut_values=lut, threshold=[thr], signed=signed), x,
-                     lut_info=dict(threshold=thr, bw=8, signed=signed, eps=1e-8))
+                     lut_info=dict(threshold=thr, bw=8, signed=signed, eps=1e-8), x_gen="all_finite_half_patterns")
 
 # range-fix constants asserted by the reference's own tests (test_fln_activation_quantizer_holder.py:42-45)
 q = Q.ActivationUniformInferableQuantizer(7, [-4.0], [4.0])

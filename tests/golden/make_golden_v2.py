@@ -58,7 +58,8 @@ for dt in ("bfloat16", "float16"):
         add_case(f"w_uni_b8_pc_{'x'.join(map(str, shape))}_ax{axis}_{dt}", "WeightsUniformInferableQuantizer",
                  dict(num_bits=8, min_range=lo, max_range=hi, per_channel=True, channel_axis=axis), x)
     add_case(f"w_uni_b4_pt_{dt}_allbits", "WeightsUniformInferableQuantizer",
-             dict(num_bits=4, min_range=[-0.7], max_range=[1.9], per_channel=False), all_finite_half_patterns(dt))
+             dict(num_bits=4, min_range=[-0.7], max_range=[1.9], per_channel=False), all_finite_half_patterns(dt),
+             x_gen="all_finite_half_patterns")
 
 # ---- 16-bit quantizers
 thr = thresholds(5)

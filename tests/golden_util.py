@@ -39,7 +39,7 @@ def _load():
             manifest = m
         else:
             manifest["cases"] = manifest["cases"] + m["cases"]
-        files.append(np.load(os.path.join(HERE, "golden", stem + ".npz")))
+        files += [np.load(os.path.join(HERE, "golden", a)) for a in m.get("archives", [stem + ".npz"])]
     names = [c["name"] for c in manifest["cases"]]
     assert len(names) == len(set(names)), "duplicate golden case names"
     return manifest, _Arrays(files)
@@ -53,12 +53,21 @@ def case_names():
     return [c["name"] for c in manifest()["cases"]]
 
 
+def all_finite_half_patterns(dtype_name):
+    """Every finite bfloat16 / float16 value as uint16 bit patterns, in increasing bit order: the input of the `_allbits`
+    cases, which the fixtures do not store (tests/golden/gen_common.py, `x_gen`)."""
+    bits = np.arange(1 << 16, dtype=np.uint32).astype(np.uint16)
+    exponent = np.uint16(0x7F80 if dtype_name == "bfloat16" else 0x7C00)
+    return bits[(bits & exponent) != exponent]
+
+
 def get_case(name):
     m, arrays = _load()
     for c in m["cases"]:
         if c["name"] == name:
             out = dict(c)
-            out["x"] = arrays[f"{name}/x"]
+            gen = c.get("x_gen")
+            out["x"] = all_finite_half_patterns(c["x_dtype"]) if gen == "all_finite_half_patterns" else arrays[f"{name}/x"]
             out["y"] = arrays[f"{name}/y"]
             out["idx"] = arrays[f"{name}/idx"] if c.get("has_idx") else None
             out["p"] = {k: arrays[f"{name}/p/{k}"] for k, v in c["params"].items() if v["kind"] in ("tensor", "ndarray")}

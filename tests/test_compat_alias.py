@@ -15,8 +15,9 @@ PICKLES = os.path.join(ROOT, "tests", "golden", "ref_pickles")
 NAMES = sorted(os.path.basename(p)[:-3] for p in glob.glob(os.path.join(PICKLES, "*.pt")))
 
 
-def test_alias_serves_the_reference_module_paths():
-    """Run in a fresh interpreter so that the alias cannot collide with anything already imported."""
+def test_alias_serves_the_reference_module_paths(tmp_path):
+    """Run in a fresh interpreter, from an empty directory, so that the alias cannot collide with anything already
+    imported or lying in the working directory."""
     code = r'''
 import sys
 sys.path.insert(0, %r)
@@ -47,7 +48,7 @@ for missing in ("mct_quantizers.keras", "mct_quantizers.pytorch.onnxruntime_sess
         raise AssertionError(missing + " should not resolve")
 print("ok")
 ''' % ROOT
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path)
     assert out.returncode == 0 and out.stdout.strip().endswith("ok"), out.stderr[-2000:]
 
 
