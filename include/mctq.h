@@ -122,6 +122,36 @@ int mctq_dequant_affine(const void* codes, int code_mode, int is_signed, float* 
                         const float* scale, const int32_t* zp, int64_t C, int64_t inner, int64_t elem_offset,
                         void* stream);
 
+/* Rebuild weights from packed codes, many tensors per launch (packed models: mct_quantizers_b200/pytorch/packed_weights.py).
+ * No reference call site: the result is bit-identical to what the weight quantizer returns for the float weight the codes were
+ * taken from (mctq_fq_affine* with code_mode / mctq_fq_lut* with idx_mode), so a packed model computes the float model's
+ * outputs.  Per tensor, elements are [outer][C][inner] in memory order and
+ *   affine: y = (T)((float)(q - zp[c]) * scale[c])      T = y_dtype (one f32 rounding, then one rounding to T)
+ *   LUT:    y = lut_quotients[idx] * thr[c]             f32 out; lut_quotients[k] = lut_k / 2^(bw - signed) in f32, idx is the
+ *                                                       index into the ORIGINAL centroid list (what mctq_fq_lut* emit)
+ * mctq_unpack_plan compiles the HOST descriptor array into a HOST plan blob of mctq_unpack_plan_bytes(descs, n_desc) bytes
+ * (returns the total number of tiles, or < 0: MCTQ_E_BADARG for a malformed descriptor or a code / output buffer that is not
+ * 16-byte aligned, MCTQ_E_DTYPE, MCTQ_E_LUT for K outside 1..256 (1..16 for MCTQ_PACK_LUT_I4)).  Tensors are grouped by kernel
+ * variant (kind, output dtype, channel mode, vector width); every group runs as launches of <= 64 tensors whose argument
+ * blocks travel as kernel parameters.  Tensors with n == 0 are accepted and skipped.  codes, y and the parameter arrays
+ * (device memory) must stay valid while the plan is in use; mctq_unpack_multi enqueues the launches on `stream`. */
+#define MCTQ_PACK_AFFINE_I8 1 /* one byte per element, int8 if is_signed else uint8 */
+#define MCTQ_PACK_AFFINE_I4 2 /* two per byte, element 2j in the low nibble (the MCTQ_CODES_INT4 layout) */
+#define MCTQ_PACK_LUT_U8 3    /* one LUT index per byte, K <= 256 */
+#define MCTQ_PACK_LUT_I4 4    /* two LUT indices per byte, K <= 16 */
+typedef struct MctqPackedDesc {
+    const void* codes;
+    void* y;
+    int64_t n, C, inner;
+    int32_t kind, is_signed, y_dtype, K;
+    const float* scale;         /* affine: scale[C];   LUT: thr[C] */
+    const int32_t* zp;          /* affine: zp[C];      LUT: NULL */
+    const float* lut_quotients; /* LUT: K entries;     affine: NULL */
+} MctqPackedDesc;
+size_t mctq_unpack_plan_bytes(const MctqPackedDesc* descs_host, int n_desc);     /* 0: some tensor is not plannable */
+int64_t mctq_unpack_plan(const MctqPackedDesc* descs_host, int n_desc, void* plan_host_out, size_t plan_bytes);
+int mctq_unpack_multi(const void* plan_host, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Whole-model weight quantisation: one launch over a table of tensors (SURVEY 8f rank 1).
  * Replaces the per-layer loop  for name, w, quantizer in self._weights_vars: quantizer(w)

@@ -17,6 +17,7 @@ from mct_quantizers_b200.pytorch.load_model import pytorch_load_quantized_model
 from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
 from mct_quantizers_b200.pytorch.model_quantization import quantize_model_weights, plan_model_weights, ModelWeightPlan, \
     ActivationPlan, quantize_activations
+from mct_quantizers_b200.pytorch.packed_weights import pack_model_weights
 from mct_quantizers_b200.pytorch import quantizers as pytorch_quantizers
 from mct_quantizers_b200.pytorch.fused_activation_holder import PytorchFusedActivationQuantizationHolder, \
     fuse_activation_producers

@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libmctq_sm100.so")
 F32, BF16, F16 = 0, 1, 2
 CODES_NONE, CODES_INT8, CODES_INT4 = 0, 1, 2
 PRE_RELU, PRE_RELU6, PRE_ADD, PRE_ADD_RELU = 1, 2, 3, 4
+PACK_AFFINE_I8, PACK_AFFINE_I4, PACK_LUT_U8, PACK_LUT_I4 = 1, 2, 3, 4
 
 _lock = threading.Lock()
 _lib = None
@@ -41,6 +42,13 @@ class MctqSiteDesc(ctypes.Structure):
                 ("qmin", c_i32), ("qmax", c_i32), ("reserved", c_i32)]
 
 
+class MctqPackedDesc(ctypes.Structure):
+    """Mirror of `struct MctqPackedDesc` (include/mctq.h)."""
+    _fields_ = [("codes", c_vp), ("y", c_vp), ("n", c_i64), ("C", c_i64), ("inner", c_i64),
+                ("kind", c_i32), ("is_signed", c_i32), ("y_dtype", c_i32), ("K", c_i32),
+                ("scale", c_vp), ("zp", c_vp), ("lut_quotients", c_vp)]
+
+
 # name -> (restype, argtypes): every symbol include/mctq.h declares
 SIGNATURES = {
     "mctq_abi_version": (c_int, []),
@@ -52,6 +60,9 @@ SIGNATURES = {
     "mctq_fq_affine_prepared": (c_int, [c_vp, c_vp, c_vp, c_i64, c_int, c_vp, c_i64, c_i64, c_i64, c_i32, c_i32, c_int, c_vp]),
     "mctq_fq_affine_scalar_pre": (c_int, [c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_f32, c_i32, c_i32, c_i32, c_vp]),
     "mctq_dequant_affine": (c_int, [c_vp, c_int, c_int, c_vp, c_i64, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp]),
+    "mctq_unpack_plan_bytes": (c_sz, [c_vp, c_int]),
+    "mctq_unpack_plan": (c_i64, [c_vp, c_int, c_vp, c_sz]),
+    "mctq_unpack_multi": (c_int, [c_vp, c_vp]),
     "mctq_multi_tile_elems": (c_i64, []),
     "mctq_multi_plan": (c_i64, [c_vp, c_int, c_vp]),
     "mctq_fq_affine_multi": (c_int, [c_vp, c_vp, c_int, c_i64, c_vp]),

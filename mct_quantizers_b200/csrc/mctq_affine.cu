@@ -3,7 +3,6 @@
 
 namespace mctq {
 
-constexpr float kMagic = 12582912.0f;      // 1.5 * 2^23: (t + kMagic) - kMagic == rint(t) for |t| < 2^22
 constexpr int32_t kFastRangeLimit = 1 << 21;
 
 struct AffineArgs {
@@ -37,9 +36,6 @@ struct AffineArgs {
 
 constexpr size_t kPrepHeaderBytes = 16;
 inline size_t prep_bytes(int64_t C) { int64_t C4 = (C + 3) & ~(int64_t)3; return kPrepHeaderBytes + (size_t)C * 16 + (size_t)C4 * 12; }
-
-// (float)k for |k| < 2^22 without I2F (a quarter-rate conversion): the mantissa of 1.5 * 2^23 + k holds k
-__device__ __forceinline__ float small_int_to_float(int k) { return __fsub_rn(__int_as_float(0x4B400000 + k), kMagic); }
 
 template <bool RINT> struct AffineOp {
     using Args = AffineArgs;
@@ -410,16 +406,10 @@ __global__ void __launch_bounds__(kThreads) dequant_affine_kernel(const void* co
     }
 }
 
-// Streaming consumer of the code wire format: tile = 256 threads x 4 vectors x 4 elements; a vector is 4 codes (one 32-bit
-// load for int8, 16 bits for packed int4) and one 16-byte f32 store.  5 (int8) / 4.5 (int4) algorithmic bytes per element.
-//   MODE 0  per-tensor: parameters loaded once per thread
-//   MODE 1  per-channel, rows a multiple of 4: one channel (one division, two parameter loads) per vector
-//   MODE 2  per-channel, any row length below 2^32: the vector's first channel from one 32-bit division, the following
-//           elements walk (rem, c) forward
-// (q - zp) -> float goes through the magic-number trick (integer add into the mantissa of 1.5 * 2^23, one FADD) instead of
-// a quarter-rate I2F: exact for |q - zp| < 2^22.
-// V: codes per vector.  4 (one 32-bit / 16-bit load, one 16-byte store) or 8 (64-bit / 32-bit load, ONE 32-byte store:
-// STG.256) when the whole vector lies in one channel -- half the loads, stores and channel look-ups per element.
+// Streaming consumer of the code wire format: tile = 256 threads x 4 vectors x V codes, one f32 store per vector; 5 (int8) /
+// 4.5 (int4) algorithmic bytes per element.  Code loading, channel walk (MODE 0 / 1 / 2) and stores: codes_tile in
+// mctq_common.cuh.  V = 8 (ONE 32-byte store: STG.256) when the whole vector lies in one channel -- half the loads, stores
+// and channel look-ups per element.
 template <int CODE, int MODE, int V>
 __global__ void __launch_bounds__(kThreads) dequant_affine_vec_kernel(const void* codes, int is_signed, float* y, int64_t n,
                                                                       const float* __restrict__ scale, const int32_t* __restrict__ zp,
@@ -427,103 +417,10 @@ __global__ void __launch_bounds__(kThreads) dequant_affine_vec_kernel(const void
                                                                       const FastDiv div_inner, const FastDiv div_C) {
     constexpr int UNROLL = 4;
     constexpr int64_t TILE = (int64_t)kThreads * UNROLL * V;
-    constexpr int RAW = (CODE == MCTQ_CODES_INT8 && V == 8) ? 2 : 1;           // 32-bit words of codes per vector
-    static_assert(V == 4 || (V == 8 && MODE != 2), "vector width");
-    const int64_t t0 = (int64_t)blockIdx.x * TILE;
     pdl_wait();
     pdl_launch_dependents();
-    uint32_t raw[UNROLL][RAW];
-    const uint8_t* cb = reinterpret_cast<const uint8_t*>(codes);
-#pragma unroll
-    for (int j = 0; j < UNROLL; ++j) {
-        const int64_t e = t0 + (int64_t)(j * kThreads + threadIdx.x) * V;
-#pragma unroll
-        for (int r = 0; r < RAW; ++r) raw[j][r] = 0;
-        if (e + V <= n) {
-            if (CODE == MCTQ_CODES_INT8) {
-                if (V == 8) { const uint2 v = __ldg(reinterpret_cast<const uint2*>(cb + e)); raw[j][0] = v.x; raw[j][RAW - 1] = v.y; }
-                else raw[j][0] = __ldg(reinterpret_cast<const uint32_t*>(cb + e));
-            } else {
-                if (V == 8) raw[j][0] = __ldg(reinterpret_cast<const uint32_t*>(cb + (e >> 1)));
-                else raw[j][0] = __ldg(reinterpret_cast<const uint16_t*>(cb + (e >> 1)));
-            }
-        } else {
-            for (int k = 0; k < V && e + k < n; ++k) {
-                const int64_t i = e + k;
-                if (CODE == MCTQ_CODES_INT8) raw[j][(k >> 2) % RAW] |= (uint32_t)cb[i] << (8 * (k & 3));
-                else raw[j][0] |= (uint32_t)((cb[i >> 1] >> ((i & 1) * 4)) & 0xf) << (4 * k);
-            }
-        }
-    }
-    float s0 = 0.0f;
-    int z0 = 0;
-    if (MODE == 0) { s0 = __ldg(scale); z0 = __ldg(zp); }
-    const bool small = (uint64_t)(elem_offset + n) < (1ull << 31);
-#pragma unroll
-    for (int j = 0; j < UNROLL; ++j) {
-        const int64_t e = t0 + (int64_t)(j * kThreads + threadIdx.x) * V;
-        if (e >= n) continue;
-        uint32_t c = 0, rem = 0;
-        float sv = s0;
-        int zv = z0;
-        if (MODE != 0) {
-            const uint64_t g = (uint64_t)(elem_offset + e);
-            if (small) {                                        // the usual case (< 2^31 elements): multiply-shift division
-                const uint32_t g32 = (uint32_t)g, r = fdiv_u32(g32, div_inner);
-                rem = g32 - r * inner;
-                c = r - fdiv_u32(r, div_C) * C;
-            } else {
-                const uint64_t r = g / inner;
-                rem = (uint32_t)(g - r * inner);
-                c = (uint32_t)(r % C);
-            }
-            sv = __ldg(scale + c);
-            zv = __ldg(zp + c);
-        }
-        // MODE 2, rows of at least one vector: the vector crosses at most one row boundary, so the parameters of the next
-        // channel are fetched up front and selected per element (no divergent reloads inside the element loop)
-        const bool two_rows = MODE == 2 && inner >= (uint32_t)V;
-        uint32_t first_cnt = V;
-        float sv1 = sv;
-        int zv1 = zv;
-        if (two_rows) {
-            first_cnt = inner - rem;
-            const uint32_t c1 = (c + 1 == C) ? 0 : c + 1;
-            sv1 = __ldg(scale + c1);
-            zv1 = __ldg(zp + c1);
-        }
-        uint32_t out[V];
-#pragma unroll
-        for (int k = 0; k < V; ++k) {
-            int q;
-            if (CODE == MCTQ_CODES_INT8) {
-                const uint32_t word = raw[j][(k >> 2) % RAW];
-                q = is_signed ? (int)(int8_t)(word >> (8 * (k & 3))) : (int)((word >> (8 * (k & 3))) & 0xffu);
-            } else {
-                const int nib = (int)((raw[j][0] >> (4 * k)) & 0xfu);
-                q = is_signed ? ((nib ^ 8) - 8) : nib;
-            }
-            float se = sv;
-            int ze = zv;
-            if (two_rows && (uint32_t)k >= first_cnt) { se = sv1; ze = zv1; }
-            const float d = __fsub_rn(__int_as_float(0x4B400000 + (q - ze)), kMagic);        // (float)(q - zp), exact
-            out[k] = __float_as_uint(__fmul_rn(d, se));
-            if (MODE == 2 && !two_rows) {
-                if (++rem == inner) {
-                    rem = 0;
-                    c = (c + 1 == C) ? 0 : c + 1;
-                    sv = __ldg(scale + c);
-                    zv = __ldg(zp + c);
-                }
-            }
-        }
-        if (e + V <= n) {
-            if (V == 8) st_stream256(y + e, out);
-            else st_stream(reinterpret_cast<uint4*>(y + e), make_uint4(out[0], out[1], out[2], out[3]));
-        } else {
-            for (int k = 0; k < V && e + k < n; ++k) y[e + k] = __uint_as_float(out[k]);
-        }
-    }
+    codes_tile<CODE, MODE, V, UNROLL>(reinterpret_cast<const uint8_t*>(codes), y, (int64_t)blockIdx.x * TILE, n, is_signed, C, inner,
+                                      elem_offset, div_inner, div_C, AffineCodeOp{scale, zp});
 }
 
 // ------------------------------------------------------------------------------------------ multi-tensor

@@ -198,6 +198,147 @@ template <int V, int CODE> __device__ __forceinline__ void st_codes(void* codes,
         else st_stream(reinterpret_cast<uint32_t*>(p), w);
     }
 }
+constexpr float kMagic = 12582912.0f;      // 1.5 * 2^23: (t + kMagic) - kMagic == rint(t) for |t| < 2^22
+
+// (float)k for |k| < 2^22 without I2F (a quarter-rate conversion): the mantissa of 1.5 * 2^23 + k holds k
+__device__ __forceinline__ float small_int_to_float(int k) { return __fsub_rn(__int_as_float(0x4B400000 + k), kMagic); }
+
+// ------------------------------------------------------------------------------------------ consumers of codes
+// The read side of the code wire format (MCTQ_CODES_INT8: one byte per element; MCTQ_CODES_INT4: two per byte, element 2j
+// in the low nibble), shared by mctq_dequant_affine and the multi-tensor unpack kernels (mctq_unpack.cu).  A tile is
+// kThreads x UNROLL vectors of V codes; a vector is one 32-bit / 16-bit load (V = 4) or 64-bit / 32-bit load (V = 8).
+//   MODE 0  per-tensor: parameters loaded once per thread
+//   MODE 1  per-channel, rows a multiple of V: one channel (one division, one parameter load) per vector
+//   MODE 2  per-channel, any row length below 2^32: the vector's first channel from one 32-bit division, the following
+//           elements walk (rem, c) forward
+// Op turns (code, channel parameters) into the f32 value: `Param load(uint32_t c)` and `float value(int q, const Param&)`.
+template <int CODE, int V> struct CodeVec {
+    static constexpr int kWords = (CODE == MCTQ_CODES_INT8 && V == 8) ? 2 : 1;   // 32-bit words of codes per vector
+};
+
+// codes of elements [e, e + V) into raw (a vector that crosses n reads only the elements below n)
+template <int CODE, int V>
+__device__ __forceinline__ void load_code_vec(const uint8_t* cb, int64_t e, int64_t n, uint32_t* raw) {
+    constexpr int RAW = CodeVec<CODE, V>::kWords;
+#pragma unroll
+    for (int r = 0; r < RAW; ++r) raw[r] = 0;
+    if (e + V <= n) {
+        if (CODE == MCTQ_CODES_INT8) {
+            if (V == 8) { const uint2 v = __ldg(reinterpret_cast<const uint2*>(cb + e)); raw[0] = v.x; raw[RAW - 1] = v.y; }
+            else raw[0] = __ldg(reinterpret_cast<const uint32_t*>(cb + e));
+        } else {
+            if (V == 8) raw[0] = __ldg(reinterpret_cast<const uint32_t*>(cb + (e >> 1)));
+            else raw[0] = __ldg(reinterpret_cast<const uint16_t*>(cb + (e >> 1)));
+        }
+    } else {
+        for (int k = 0; k < V && e + k < n; ++k) {
+            const int64_t i = e + k;
+            if (CODE == MCTQ_CODES_INT8) raw[(k >> 2) % RAW] |= (uint32_t)cb[i] << (8 * (k & 3));
+            else raw[0] |= (uint32_t)((cb[i >> 1] >> ((i & 1) * 4)) & 0xf) << (4 * k);
+        }
+    }
+}
+
+// code k of a loaded vector, sign-extended when is_signed
+template <int CODE, int V>
+__device__ __forceinline__ int code_at(const uint32_t* raw, int k, int is_signed) {
+    if (CODE == MCTQ_CODES_INT8) {
+        const uint32_t word = raw[(k >> 2) % CodeVec<CODE, V>::kWords];
+        return is_signed ? (int)(int8_t)(word >> (8 * (k & 3))) : (int)((word >> (8 * (k & 3))) & 0xffu);
+    }
+    const int nib = (int)((raw[0] >> (4 * k)) & 0xfu);
+    return is_signed ? ((nib ^ 8) - 8) : nib;
+}
+
+// V values to y[e, e + V) as T: one 32-byte (f32, V = 8), 16-byte or 8-byte store; element stores for a vector crossing n
+template <typename T, int V>
+__device__ __forceinline__ void store_vec(T* y, int64_t e, int64_t n, const float* v) {
+    if (e + V <= n) {
+        if constexpr (sizeof(T) == 4) {
+            uint32_t w[V];
+#pragma unroll
+            for (int k = 0; k < V; ++k) w[k] = __float_as_uint(v[k]);
+            if (V == 8) st_stream256(y + e, w);
+            else st_stream(reinterpret_cast<uint4*>(y + e), make_uint4(w[0], w[1], w[2], w[3]));
+        } else {
+            uint32_t w[V / 2];
+            Pack<T, V>::pack(v, w);
+            st_words<V / 2>(y + e, w);
+        }
+    } else {
+        for (int k = 0; k < V && e + k < n; ++k) y[e + k] = from_f32<T>(v[k]);
+    }
+}
+
+// one tile of a code consumer: every load of the tile is issued before the first use
+template <int CODE, int MODE, int V, int UNROLL, typename T, class Op>
+__device__ __forceinline__ void codes_tile(const uint8_t* cb, T* y, int64_t t0, int64_t n, int is_signed, uint32_t C,
+                                           uint32_t inner, int64_t elem_offset, const FastDiv& div_inner,
+                                           const FastDiv& div_C, const Op& op) {
+    constexpr int RAW = CodeVec<CODE, V>::kWords;
+    static_assert(V == 4 || (V == 8 && MODE != 2), "vector width");
+    using Param = typename Op::Param;
+    uint32_t raw[UNROLL][RAW];
+#pragma unroll
+    for (int j = 0; j < UNROLL; ++j)
+        load_code_vec<CODE, V>(cb, t0 + (int64_t)(j * kThreads + threadIdx.x) * V, n, raw[j]);
+    Param p0 = {};
+    if (MODE == 0) p0 = op.load(0);
+    const bool small = (uint64_t)(elem_offset + n) < (1ull << 31);
+#pragma unroll
+    for (int j = 0; j < UNROLL; ++j) {
+        const int64_t e = t0 + (int64_t)(j * kThreads + threadIdx.x) * V;
+        if (e >= n) continue;
+        uint32_t c = 0, rem = 0;
+        Param p = p0;
+        if (MODE != 0) {
+            const uint64_t g = (uint64_t)(elem_offset + e);
+            if (small) {                                        // the usual case (< 2^31 elements): multiply-shift division
+                const uint32_t g32 = (uint32_t)g, r = fdiv_u32(g32, div_inner);
+                rem = g32 - r * inner;
+                c = r - fdiv_u32(r, div_C) * C;
+            } else {
+                const uint64_t r = g / inner;
+                rem = (uint32_t)(g - r * inner);
+                c = (uint32_t)(r % C);
+            }
+            p = op.load(c);
+        }
+        // MODE 2, rows of at least one vector: the vector crosses at most one row boundary, so the parameters of the next
+        // channel are fetched up front and selected per element (no divergent reloads inside the element loop)
+        const bool two_rows = MODE == 2 && inner >= (uint32_t)V;
+        uint32_t first_cnt = V;
+        Param p1 = p;
+        if (two_rows) {
+            first_cnt = inner - rem;
+            p1 = op.load((c + 1 == C) ? 0 : c + 1);
+        }
+        float out[V];
+#pragma unroll
+        for (int k = 0; k < V; ++k) {
+            const int q = code_at<CODE, V>(raw[j], k, is_signed);
+            out[k] = op.value(q, (two_rows && (uint32_t)k >= first_cnt) ? p1 : p);
+            if (MODE == 2 && !two_rows) {
+                if (++rem == inner) {
+                    rem = 0;
+                    c = (c + 1 == C) ? 0 : c + 1;
+                    p = op.load(c);
+                }
+            }
+        }
+        store_vec<T, V>(y, e, n, out);
+    }
+}
+
+// affine codes: y = (q - zp_c) * s_c, one f32 rounding; exact (q - zp) for |q - zp| < 2^22
+struct AffineCodeOp {
+    struct Param { float s; int zp; };
+    const float* __restrict__ scale;
+    const int32_t* __restrict__ zp;
+    __device__ __forceinline__ Param load(uint32_t c) const { return {__ldg(scale + c), __ldg(zp + c)}; }
+    __device__ __forceinline__ float value(int q, const Param& p) const { return __fmul_rn(small_int_to_float(q - p.zp), p.s); }
+};
+
 // ------------------------------------------------------------------------------------------ channel window
 // A tile covers logical elements [g0, g0 + tile) of the [outer][C][inner] view.  It touches rows
 // r0 .. r0 + nr - 1 (row = g / inner, channel = row % C).  Slot jj of the window holds channel (r0 + jj) % C,

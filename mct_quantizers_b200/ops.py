@@ -7,6 +7,7 @@ sm_100a kernels.
     torch.ops.mctq.fq_lut_tensor      <- lut_quantizer(..., threshold=Tensor, per_channel, channel_axis, input_rank)
     torch.ops.mctq.fq_lut_scalar      <- lut_quantizer(..., threshold=float)            (activations)
     torch.ops.mctq.quantize_affine_*  -> integer codes (+ optional fake-quant values); mctq.dequantize_affine
+    torch.ops.mctq.lut_indices        -> LUT indices;                                    mctq.dequantize_lut
 
 (reference call sites: see include/mctq.h).  Each op has a CUDA implementation (device pointers + the
 caller's current stream into the C ABI, no synchronisation), a CPU-tensor implementation that streams the
@@ -36,6 +37,8 @@ _LIB.define("dequantize_affine(Tensor codes, int code_mode, bool is_signed, int[
             "int axis) -> Tensor")
 _LIB.define("lut_indices(Tensor x, Tensor table, int K, Tensor threshold, bool per_channel, int axis, float eps, "
             "int idx_mode) -> Tensor")
+_LIB.define("dequantize_lut(Tensor idx, int idx_mode, int[] shape, Tensor lut, int lut_values_bitwidth, bool is_signed, "
+            "Tensor threshold, bool per_channel, int axis) -> Tensor")
 
 
 # --------------------------------------------------------------------------------------------- helpers
@@ -376,6 +379,25 @@ def contiguous_layout(shape, axis):
     return shape[axis], inner
 
 
+def affine_codes(xd, scale, zero_point, C, inner, quant_min, quant_max, code_mode):
+    """Integer codes of a dense CUDA tensor (no values) over its [outer][C][inner] memory-order view: int8 / uint8 [n] for
+    CODES_INT8, packed nibbles uint8 [(n + 1) // 2] for CODES_INT4.  Same kernels and arithmetic as the fake-quant ops."""
+    _check_range(quant_min, quant_max)
+    n = xd.numel()
+    if code_mode == _native.CODES_INT8:
+        codes = torch.empty(n, dtype=torch.int8 if quant_min < 0 else torch.uint8, device=xd.device)
+    else:
+        codes = torch.empty((n + 1) // 2, dtype=torch.uint8, device=xd.device)
+    if n:
+        lib = _native.load()
+        s, z = _param_on(scale, xd.device), _param_on(zero_point, xd.device)
+        with _on_device(xd.device) as cur:
+            rc, what = _launch_affine_params(lib, xd.data_ptr(), None, codes.data_ptr(), n, _dtype_tag(xd), s, z, C, inner,
+                                             int(quant_min), int(quant_max), int(code_mode), cur.idx)
+        _native.check(rc, what)
+    return codes
+
+
 def _affine_tensor_cuda(x, scale, zero_point, quant_min, quant_max):
     tag = _dtype_tag(x)
     _check_range(quant_min, quant_max)
@@ -634,6 +656,46 @@ def _lut_indices_cuda(x, table, K, threshold, per_channel, axis, eps, idx_mode):
     return _lut_tensor_launch(x, table, K, threshold, per_channel, axis, eps, idx_mode, False)[1]
 
 
+def lut_quotients(lut, lut_values_bitwidth, is_signed):
+    """q_k = lut_k / 2^(bw - signed) as a host f32 tensor: the division the reference performs before it multiplies by the
+    threshold (quantizer_utils.py: `lut_values / 2 ** (lut_values_bitwidth - int(signed))`, CPU f32)."""
+    return lut.detach().to("cpu", torch.float32).reshape(-1) / 2 ** (int(lut_values_bitwidth) - int(bool(is_signed)))
+
+
+def _dequantize_lut_cuda(idx, idx_mode, shape, lut, lut_values_bitwidth, is_signed, threshold, per_channel, axis):
+    """y[i] = q[idx[i]] * thr[c(i)] (f32) over the row-major `shape`: the consumer of mctq::lut_indices.  Like fq_lut_tensor,
+    a 0-dim `shape` comes back 1-D."""
+    if idx_mode == _native.CODES_INT8:
+        kind = _native.PACK_LUT_U8
+    elif idx_mode == _native.CODES_INT4:
+        kind = _native.PACK_LUT_I4
+    else:
+        raise RuntimeError("idx_mode must be 1 (uint8) or 2 (packed 4-bit)")
+    shape = [int(s) for s in shape]
+    n = 1
+    for s in shape:
+        n *= s
+    if threshold.dtype != torch.float32:
+        raise RuntimeError(f"threshold must be Float, found {threshold.dtype}")
+    if per_channel:
+        nd = len(shape)
+        if not -nd <= axis < nd:
+            raise IndexError(f"Dimension out of range (expected to be in range of [{-nd}, {nd - 1}], but got {axis})")
+        C, inner = contiguous_layout(shape, axis % nd)
+        if threshold.numel() != C:
+            raise RuntimeError(f"threshold has {threshold.numel()} entries for {C} channels on axis {axis}")
+    else:
+        C, inner = 1, 1
+        if threshold.numel() != 1:
+            raise RuntimeError("per-tensor LUT dequantization needs a single threshold")
+    need = n if kind == _native.PACK_LUT_U8 else (n + 1) // 2
+    if idx.numel() != need or idx.dtype not in (torch.uint8, torch.int8):
+        raise RuntimeError(f"idx must hold {need} bytes for shape {shape} and idx_mode {idx_mode}")
+    q = lut_quotients(lut, lut_values_bitwidth, is_signed)
+    item = (idx, kind, False, torch.float32, shape if shape else [1], None, C, inner, threshold.reshape(-1), None, q)
+    return UnpackPlan([item]).run()[0]
+
+
 def _lut_scalar_cuda(x, table, K, divisor, threshold, round_to_input_dtype, multiply=False):
     """`multiply`: normalise with x * (float)(1.0 / divisor) -- the reference's CUDA flavour of `tensor / python_number`
     (quantizer_utils.reference_arithmetic) -- instead of the true division x / (float)divisor."""
@@ -828,6 +890,7 @@ _LIB.impl("fq_lut_scalar", _lut_scalar_cuda, "CUDA")
 _LIB.impl("quantize_affine_channel", _quantize_affine_channel_cuda, "CUDA")
 _LIB.impl("dequantize_affine", _dequantize_affine_cuda, "CUDA")
 _LIB.impl("lut_indices", _lut_indices_cuda, "CUDA")
+_LIB.impl("dequantize_lut", _dequantize_lut_cuda, "CUDA")
 
 _LIB.impl("fq_affine_scalar_pre", _affine_scalar_pre_cuda, "CUDA")
 _LIB.impl("fq_affine_scalar_pre", _via_device(_affine_scalar_pre_cuda), "CPU")
@@ -839,6 +902,7 @@ _LIB.impl("fq_lut_scalar", _lut_scalar_cpu, "CPU")
 _LIB.impl("quantize_affine_channel", _via_device(_quantize_affine_channel_cuda), "CPU")
 _LIB.impl("dequantize_affine", _via_device(_dequantize_affine_cuda), "CPU")
 _LIB.impl("lut_indices", _via_device(_lut_indices_cuda, keep=(1,)), "CPU")
+_LIB.impl("dequantize_lut", _via_device(_dequantize_lut_cuda, keep=(3,)), "CPU")
 
 
 # --------------------------------------------------------------------------------------------- fake / meta impls
@@ -891,6 +955,11 @@ def _(x, table, K, threshold, per_channel, axis, eps, idx_mode):
     if idx_mode == _native.CODES_INT4:
         return x.new_empty(((x.numel() + 1) // 2,), dtype=torch.uint8)
     return torch.empty_like(x, dtype=torch.uint8)
+
+
+@torch.library.register_fake("mctq::dequantize_lut")
+def _(idx, idx_mode, shape, lut, lut_values_bitwidth, is_signed, threshold, per_channel, axis):
+    return idx.new_empty(list(shape) if len(shape) else [1], dtype=torch.float32)
 
 
 # --------------------------------------------------------------------------------------------- whole-model launch
@@ -1110,3 +1179,105 @@ class LutMultiPlan:
         _native.check(rc, "mctq_fq_lut_prepared_multi")
         return self.outputs
 
+
+
+class UnpackPlan:
+    """Rebuild many packed tensors in one launch per kernel variant and 64 tensors (C ABI: mctq_unpack_plan +
+    mctq_unpack_multi).  The result of each tensor is bit-identical to the fake-quant output its codes were taken from.
+
+    Build once from items (all on one CUDA device)
+        (codes, kind, is_signed, dtype, shape, stride, C, inner, scale, zero_point, lut_quotients)
+    codes      uint8 / int8 tensor in the layout of `kind` (_native.PACK_*), elements in the output's memory order
+    dtype      output dtype (f32 for the LUT kinds); shape / stride of the output (stride None: row-major)
+    C, inner   [outer][C][inner] view of the output's memory (C = 1: per tensor)
+    scale      f32 [C] (affine scale, or LUT threshold); zero_point int32 [C] (affine) or None
+    lut_quotients  f32 [K] (LUT kinds, see lut_quotients()) or None
+    `outputs` (optional): tensors to write into instead of plan-owned buffers.
+    `fresh=True`: every run() writes into newly allocated tensors (re-planned on the host) and the plan keeps no reference
+    to them, so that a caller can drop the rebuilt tensors after use and keep only the codes resident.
+
+    run() enqueues the launches on the current stream and returns the outputs."""
+
+    def __init__(self, items, outputs=None, fresh=False):
+        if not items:
+            raise ValueError("UnpackPlan needs at least one tensor")
+        lib = _native.load()
+        self.device = items[0][0].device
+        if self.device.type != "cuda":
+            raise ValueError("UnpackPlan needs CUDA tensors")
+        self.n_desc = len(items)
+        self._descs = (_native.MctqPackedDesc * self.n_desc)()
+        self._keep, self._out_specs = [], []
+        for k, (codes, kind, is_signed, dtype, shape, stride, C, inner, scale, zp, quot) in enumerate(items):
+            if codes.device != self.device:
+                raise ValueError("all tensors of an UnpackPlan must live on one CUDA device")
+            if codes.dtype not in (torch.uint8, torch.int8):
+                raise ValueError(f"tensor {k}: codes must be uint8 / int8, found {codes.dtype}")
+            n = 1
+            for s_ in shape:
+                n *= int(s_)
+            need = n if kind in (_native.PACK_AFFINE_I8, _native.PACK_LUT_U8) else (n + 1) // 2
+            if codes.numel() != need:
+                raise ValueError(f"tensor {k}: {codes.numel()} code bytes for {n} elements of kind {kind}")
+            if not codes.is_contiguous() or codes.data_ptr() % 16:      # the kernels load codes in 16-byte aligned vectors
+                codes = codes.clone(memory_format=torch.contiguous_format)
+            s = _param_on(scale.detach().reshape(-1).contiguous(), self.device)
+            z = _param_on(zp.detach().reshape(-1).contiguous(), self.device) if zp is not None else None
+            q = _param_on(quot.detach().reshape(-1).contiguous(), self.device) if quot is not None else None
+            if s.dtype != torch.float32 or (z is not None and z.dtype != torch.int32) or (q is not None and q.dtype != torch.float32):
+                raise ValueError(f"tensor {k}: scale / threshold and quotients must be float32, zero points int32")
+            self._keep.append((codes, s, z, q))
+            d = self._descs[k]
+            d.codes, d.n, d.C, d.inner = codes.data_ptr(), n, int(C), int(inner)
+            d.kind, d.is_signed, d.y_dtype = int(kind), int(bool(is_signed)), _DT[dtype]
+            d.K = q.numel() if q is not None else 0
+            d.scale, d.zp, d.lut_quotients = s.data_ptr(), _ptr(z), _ptr(q)
+            self._out_specs.append((tuple(int(v) for v in shape), None if stride is None else tuple(int(v) for v in stride), dtype))
+        self._plan_host, self._plan_nb, self.fresh = None, 0, fresh
+        if fresh:
+            if outputs is not None:
+                raise ValueError("a fresh UnpackPlan allocates its outputs on every run")
+            self._install(self._new_outputs(), lib)       # validates the descriptors once
+            self.outputs = None
+        elif outputs is not None:
+            outputs = list(outputs)
+            for k, (y, (shape, stride, dtype)) in enumerate(zip(outputs, self._out_specs)):
+                if y.device != self.device or y.dtype != dtype or tuple(y.shape) != shape or \
+                        (stride is not None and tuple(y.stride()) != stride) or (stride is None and not y.is_contiguous()):
+                    raise ValueError(f"output {k} does not match the packed tensor's device, dtype, shape or strides")
+            self._install(outputs, lib)
+        else:
+            self._install(self._new_outputs(), lib)
+
+    def _new_outputs(self):
+        return [torch.empty(shape, dtype=dtype, device=self.device) if stride is None else
+                torch.empty_strided(shape, stride, dtype=dtype, device=self.device)
+                for shape, stride, dtype in self._out_specs]
+
+    def _install(self, outputs, lib):
+        for d, y in zip(self._descs, outputs):
+            d.y = y.data_ptr() if y.numel() else None
+        descs = ctypes.cast(self._descs, c_vp)
+        nb = lib.mctq_unpack_plan_bytes(descs, self.n_desc)
+        if nb == 0:
+            raise MctqError(f"mctq_unpack_plan: {_native.ERRORS.get(lib.mctq_unpack_plan(descs, self.n_desc, None, 0), 'rejected')}")
+        if nb > self._plan_nb:
+            self._plan_host, self._plan_nb = (ctypes.c_uint8 * nb)(), nb
+        total = lib.mctq_unpack_plan(descs, self.n_desc, ctypes.cast(self._plan_host, c_vp), self._plan_nb)
+        if total < 0:
+            raise MctqError(f"mctq_unpack_plan: {_native.ERRORS.get(total, total)}")
+        self.total_tiles = int(total)
+        self.n_launches = ctypes.c_int32.from_buffer(self._plan_host, 8).value      # one per kernel variant and 64 tensors
+        self.outputs = outputs
+
+    def run(self):
+        lib = _native._lib or _native.load()
+        if self.fresh:
+            self._install(self._new_outputs(), lib)
+        with _on_device(self.device):
+            rc = lib.mctq_unpack_multi(ctypes.cast(self._plan_host, c_vp), _stream(self.device))
+        _native.check(rc, "mctq_unpack_multi")
+        outputs = self.outputs
+        if self.fresh:
+            self.outputs = None
+        return outputs

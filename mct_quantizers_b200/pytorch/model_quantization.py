@@ -3,13 +3,15 @@
 The reference re-quantizes each wrapped weight with its own kernel(s) on every forward
 (mct_quantizers/pytorch/quantize_wrapper.py:228-240): 53 launches (+ 106 host syncs) for MobileNetV2.  Here all
 affine weight quantizers of a model are gathered into one descriptor table and run as ONE kernel
-(mctq_fq_affine_multi), all LUT weight quantizers as a second one (mctq_fq_lut_prepared_multi); user-defined quantizers
-and tensors outside the prepared paths keep their own call."""
+(mctq_fq_affine_multi), all LUT weight quantizers as a second one (mctq_fq_lut_prepared_multi) and all packed weights
+(packed_weights.py) as a third (mctq_unpack_multi); user-defined quantizers and tensors outside the prepared paths keep
+their own call."""
 from typing import Dict, List
 
 import torch
 
-from mct_quantizers_b200.ops import MultiTensorPlan, LutMultiPlan, ScalarSitesPlan
+from mct_quantizers_b200.ops import MultiTensorPlan, LutMultiPlan, ScalarSitesPlan, UnpackPlan
+from mct_quantizers_b200.pytorch.packed_weights import PackedWeight
 
 
 def _is_affine_weight_quantizer(q) -> bool:
@@ -75,7 +77,11 @@ class WeightPlan:
     `.half()` or a re-assigned parameter the stale storage is never quantized.  Tensors a multi-tensor launch cannot take
     (non-dense views, CPU tensors, user-defined quantizers, uniform quantizers whose zero point leaves the range: the
     per-layer call raises the reference's error) go through their quantizer's own `__call__`, which also owns the
-    reuse contract (`enable_reuse` / `resue_outputs`)."""
+    reuse contract (`enable_reuse` / `resue_outputs`).
+
+    Packed weights (a PackedWeight in the weight slot) are the third family: all of a device are rebuilt by one UnpackPlan
+    into plan-owned outputs, so a plan holds every rebuilt weight at once -- one launch instead of one per wrapper, at the
+    cost of the memory saving that packing gives a per-wrapper forward."""
 
     def __init__(self, weight_vars):
         self.vars = [(name, w, q) for name, w, q in weight_vars]
@@ -84,10 +90,16 @@ class WeightPlan:
         self._build()
 
     def _build(self):
-        self.fused_idx, self.lut_idx, self.other = [], [], []
-        self._plans, self._lut_plans = [], []                     # [(indices, plan)] per device
-        by_dev, lut_by_dev = {}, {}
+        self.fused_idx, self.lut_idx, self.packed_idx, self.other = [], [], [], []
+        self._plans, self._lut_plans, self._unpack_plans = [], [], []     # [(indices, plan)] per device
+        by_dev, lut_by_dev, packed_by_dev = {}, {}, {}
         for k, (name, w, q) in enumerate(self.vars):
+            if isinstance(w, PackedWeight):
+                idx, items = packed_by_dev.setdefault(w.device, ([], []))
+                idx.append(k)
+                items.append(w.plan_item())
+                self.packed_idx.append(k)
+                continue
             ok_dtype = w.is_cuda and w.dtype in (torch.float32, torch.bfloat16, torch.float16) and w.numel() > 0
             reuse = bool(q.__dict__.get('enable_reuse', False))
             item = None
@@ -115,6 +127,8 @@ class WeightPlan:
             self._plans.append((idx, MultiTensorPlan(items)))
         for dev, (idx, items) in lut_by_dev.items():
             self._lut_plans.append((idx, LutMultiPlan(items)))
+        for dev, (idx, items) in packed_by_dev.items():
+            self._unpack_plans.append((idx, UnpackPlan(items)))
         self._ws = [w for _, w, _ in self.vars]
         self._qs = [q for _, _, q in self.vars]
         self._attrs, self._versioned = _plan_watch(self._qs)
@@ -141,6 +155,9 @@ class WeightPlan:
             for k, y in zip(idx, plan.run()):
                 out[k] = y
         for idx, plan in self._lut_plans:
+            for k, y in zip(idx, plan.run()):
+                out[k] = y
+        for idx, plan in self._unpack_plans:
             for k, y in zip(idx, plan.run()):
                 out[k] = y
         for k, w, q in self.other:
@@ -216,6 +233,12 @@ def quantize_activations(pairs) -> List[torch.Tensor]:
     return ActivationPlan(pairs).run()
 
 
+def _wrapper_weight_vars(mod):
+    """(name, weight, quantizer) of a wrapper's float weights, then (name, PackedWeight, quantizer) of its packed ones."""
+    packed = mod.__dict__.get('_packed')
+    return list(mod.get_weights_vars()) + (packed.weight_vars(mod) if packed is not None else [])
+
+
 def quantize_weight_vars(weight_vars) -> Dict[str, torch.Tensor]:
     plan = WeightPlan(weight_vars)
     return dict(zip(plan.names, plan.run()))
@@ -228,7 +251,7 @@ def quantize_model_weights(model: torch.nn.Module) -> Dict[str, Dict[str, torch.
     triples, owners = [], []
     for mod_name, mod in model.named_modules():
         if isinstance(mod, PytorchQuantizationWrapper):
-            for name, w, q in mod.get_weights_vars():
+            for name, w, q in _wrapper_weight_vars(mod):
                 triples.append((name, w, q))
                 owners.append(mod_name)
     result: Dict[str, Dict[str, torch.Tensor]] = {}
@@ -253,7 +276,9 @@ class ModelWeightPlan:
             y = model(x)                      # wrappers run their layers on the installed weights, no per-layer launches
 
     or, for inference with constant weights, `plan.enable()` once (and `plan.refresh()` again only if the float weights
-    change).  Results are identical to the per-layer path (same kernels' arithmetic, checked by tests)."""
+    change).  Results are identical to the per-layer path (same kernels' arithmetic, checked by tests).  Packed weights
+    (packed_weights.py) are rebuilt by one unpack launch per device and stay installed while the plan is enabled: the
+    plan holds every rebuilt weight of the model at once."""
 
     def __init__(self, model: torch.nn.Module):
         from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
@@ -267,7 +292,7 @@ class ModelWeightPlan:
         """(Re)build the plan from the wrappers' CURRENT weight variables."""
         triples, self._owner = [], []
         for mod in self.wrappers:
-            for name, w, q in mod.get_weights_vars():
+            for name, w, q in _wrapper_weight_vars(mod):
                 triples.append((name, w, q))
                 self._owner.append(mod)
         self._ids = [(id(w), id(q)) for _, w, q in triples]
@@ -279,7 +304,7 @@ class ModelWeightPlan:
         / converted storage (`model.to()`, `.half()`) is caught by WeightPlan's signature check."""
         if self.plan is None:
             return
-        live = [(id(w), id(q)) for mod in self.wrappers for _, w, q in mod.get_weights_vars()]
+        live = [(id(w), id(q)) for mod in self.wrappers for _, w, q in _wrapper_weight_vars(mod)]
         if live != self._ids:
             self._collect()
         per_wrapper = {}

@@ -130,11 +130,14 @@ class PytorchQuantizationWrapper(nn.Module):
         return flags
 
     def forward(self, *args: List[Any], **kwargs: Dict[str, Any]) -> Union[torch.Tensor, List[torch.Tensor]]:
+        d = self.__dict__
+        packed = d.get('_packed')
+        if packed is not None:              # packed weights (pack_weights): rebuilt from their codes, see packed_weights.py
+            return packed.forward(self, args, kwargs)
         # Lean path for the usual case -- an nn.Module layer with named weights and no extra call arguments: same effects as
         # the general path below (every weight quantized, the result installed as the layer's attribute, the layer called)
         # without nn.Module's __getattr__ / __setattr__ detours, which cost more than the launch of a small weight
         # (13 -> 7 us of Python per wrapped layer and forward).
-        d = self.__dict__
         layer = d['_modules'].get(LAYER)
         if layer is not None and d['is_str_attr'] and not d['op_call_args'] and not d['op_call_kwargs'] \
                 and not d['is_inputs_as_list'] and type(self).set_quantize_weights is PytorchQuantizationWrapper.set_quantize_weights:
@@ -161,11 +164,14 @@ class PytorchQuantizationWrapper(nn.Module):
                 else:
                     quantized_weights[name] = quantizer(unquantized_weight)
             self.set_quantize_weights(quantized_weights)
+        return self._run_layer(args, kwargs)
 
+    def _run_layer(self, args, kwargs):
+        """Call the layer on the installed (quantized) weights."""
         if not self.is_str_attr:
             # splice the (quantized) constants back into the positional inputs at their recorded positions
             args = list(args)
-            for pos in sorted(w[0] for w in self._weights_vars):
+            for pos in sorted(self.weights_quantizers):
                 args.insert(pos, getattr(self, f'{QUANTIZED_POSITIONAL_WEIGHT}_{pos}'))
 
         _kwargs = {**self.op_call_kwargs, **kwargs}
@@ -174,8 +180,19 @@ class PytorchQuantizationWrapper(nn.Module):
         return self.layer(*args, *self.op_call_args, **_kwargs)
 
     def get_quantized_weights(self) -> Dict[str, torch.Tensor]:
-        """weight name / position -> quantized weight (the quantizers run; the layer does not)."""
-        return {name: quantizer(w) for name, w, quantizer in self.get_weights_vars()}
+        """weight name / position -> quantized weight (the quantizers run; the layer does not).  Packed weights are rebuilt
+        from their codes."""
+        out = {name: quantizer(w) for name, w, quantizer in self.get_weights_vars()}
+        packed = self.__dict__.get('_packed')
+        if packed is not None:
+            out.update(zip((e.name for e in packed.entries), packed.rebuild(self)))
+        return out
+
+    def pack_weights(self) -> Dict[str, Dict]:
+        """Keep the weights of this wrapper as int8 / int4 codes or LUT indices instead of floats (inference only, one-way;
+        see mct_quantizers_b200.pytorch.packed_weights).  Returns, per weight, whether it was packed and why not."""
+        from mct_quantizers_b200.pytorch.packed_weights import pack_wrapper_weights
+        return pack_wrapper_weights(self)
 
     def quantize_weights_batched(self) -> Dict[str, torch.Tensor]:
         """get_quantized_weights() with every affine weight quantizer of this wrapper fused into one launch."""
