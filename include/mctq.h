@@ -152,6 +152,21 @@ size_t mctq_unpack_plan_bytes(const MctqPackedDesc* descs_host, int n_desc);    
 int64_t mctq_unpack_plan(const MctqPackedDesc* descs_host, int n_desc, void* plan_host_out, size_t plan_bytes);
 int mctq_unpack_multi(const void* plan_host, void* stream);
 
+/* Fused packed linear: y[M][out] = x[M][in] @ W^T + bias, reading the packed codes of W directly (W is never built in memory).
+ * Replaces the pair  mctq_unpack_multi(W) -> F.linear(x, W, bias)  of a packed nn.Linear wrapper's forward at small M, where
+ * the product is bound by the bytes of W: the codes are read once instead of being expanded to a float W in HBM and read back.
+ *   w          HOST descriptor of the packed weight, row-major [out][in]: n = out * in, C = 1 (per tensor) or C = out with
+ *              inner = in (per output row); w->y is unused.  Any kind; codes at any alignment (any `in`, int4 rows may start
+ *              in a high nibble)
+ *   x, y       device, M rows of x_dtype, contiguous; x_dtype must equal w->y_dtype (the rebuilt weight's dtype, f32 for LUT)
+ *   bias       device, out entries of x_dtype, or NULL
+ * W means exactly the weight mctq_unpack_multi rebuilds.  Accumulation is in f32 (a per-row scale or threshold may be applied
+ * once per row for f32 outputs), y is rounded once to x_dtype, and the summation order is fixed: two calls on the same inputs
+ * give the same bits.  Not bit-identical to a cuBLAS product.  M == 0 is a no-op.  Returns MCTQ_E_BADARG (shape, null or
+ * parameter-layout errors), MCTQ_E_DTYPE, MCTQ_E_LUT (K outside 1..16 / 1..256) before any CUDA call. */
+int mctq_packed_linear(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x, int x_dtype,
+                       int64_t M, const void* bias, void* y, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Whole-model weight quantisation: one launch over a table of tensors (SURVEY 8f rank 1).
  * Replaces the per-layer loop  for name, w, quantizer in self._weights_vars: quantizer(w)

@@ -216,6 +216,18 @@ template <int CODE, int V> struct CodeVec {
     static constexpr int kWords = (CODE == MCTQ_CODES_INT8 && V == 8) ? 2 : 1;   // 32-bit words of codes per vector
 };
 
+// the first cnt (<= V) codes of elements [e, e + V), one byte load each: any e, including an int4 element in a high nibble;
+// raw must be zeroed by the caller
+template <int CODE, int V>
+__device__ __forceinline__ void load_code_elems(const uint8_t* cb, int64_t e, int cnt, uint32_t* raw) {
+    constexpr int RAW = CodeVec<CODE, V>::kWords;
+    for (int k = 0; k < cnt; ++k) {
+        const int64_t i = e + k;
+        if (CODE == MCTQ_CODES_INT8) raw[(k >> 2) % RAW] |= (uint32_t)cb[i] << (8 * (k & 3));
+        else raw[0] |= (uint32_t)((cb[i >> 1] >> ((i & 1) * 4)) & 0xf) << (4 * k);
+    }
+}
+
 // codes of elements [e, e + V) into raw (a vector that crosses n reads only the elements below n)
 template <int CODE, int V>
 __device__ __forceinline__ void load_code_vec(const uint8_t* cb, int64_t e, int64_t n, uint32_t* raw) {
@@ -231,11 +243,7 @@ __device__ __forceinline__ void load_code_vec(const uint8_t* cb, int64_t e, int6
             else raw[0] = __ldg(reinterpret_cast<const uint16_t*>(cb + (e >> 1)));
         }
     } else {
-        for (int k = 0; k < V && e + k < n; ++k) {
-            const int64_t i = e + k;
-            if (CODE == MCTQ_CODES_INT8) raw[(k >> 2) % RAW] |= (uint32_t)cb[i] << (8 * (k & 3));
-            else raw[0] |= (uint32_t)((cb[i >> 1] >> ((i & 1) * 4)) & 0xf) << (4 * k);
-        }
+        load_code_elems<CODE, V>(cb, e, n - e < V ? (int)(n - e) : V, raw);
     }
 }
 
@@ -330,13 +338,26 @@ __device__ __forceinline__ void codes_tile(const uint8_t* cb, T* y, int64_t t0, 
     }
 }
 
-// affine codes: y = (q - zp_c) * s_c, one f32 rounding; exact (q - zp) for |q - zp| < 2^22
+// affine codes: y = (q - zp_c) * s_c, one f32 rounding; exact (q - zp) for |q - zp| < 2^22.  level() is the value before the
+// per-channel factor, which a consumer that sums over a row (mctq_packed_linear.cu) may apply once per row instead
 struct AffineCodeOp {
     struct Param { float s; int zp; };
     const float* __restrict__ scale;
     const int32_t* __restrict__ zp;
     __device__ __forceinline__ Param load(uint32_t c) const { return {__ldg(scale + c), __ldg(zp + c)}; }
-    __device__ __forceinline__ float value(int q, const Param& p) const { return __fmul_rn(small_int_to_float(q - p.zp), p.s); }
+    __device__ static __forceinline__ float level(int q, const Param& p) { return small_int_to_float(q - p.zp); }
+    __device__ static __forceinline__ float value(int q, const Param& p) { return __fmul_rn(level(q, p), p.s); }
+};
+
+// LUT indices: y = q_idx * thr_c with the quotients q_k of the tensor's centroid list in shared memory (staged once per CTA;
+// entries past K are 0, so no index of the code width can read outside the table)
+struct LutCodeOp {
+    using Param = float;
+    const float* __restrict__ thr;
+    const float* sm_q;
+    __device__ __forceinline__ float load(uint32_t c) const { return __ldg(thr + c); }
+    __device__ __forceinline__ float level(int q) const { return sm_q[q]; }
+    __device__ __forceinline__ float value(int q, float t) const { return __fmul_rn(level(q), t); }
 };
 
 // ------------------------------------------------------------------------------------------ channel window

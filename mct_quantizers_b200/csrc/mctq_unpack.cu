@@ -36,16 +36,6 @@ struct UnpackParamsT {
 using UnpackParams = UnpackParamsT<kUnpackMaxDesc>;
 static_assert(sizeof(UnpackParams) <= 32764, "kernel parameter space");
 
-// LUT indices: the quotients of the tensor's centroid list live in shared memory (staged once per CTA; entries past K are 0,
-// so no index of the code width can read outside the table)
-struct LutCodeOp {
-    using Param = float;
-    const float* __restrict__ thr;
-    const float* sm_q;
-    __device__ __forceinline__ float load(uint32_t c) const { return __ldg(thr + c); }
-    __device__ __forceinline__ float value(int q, float t) const { return __fmul_rn(sm_q[q], t); }
-};
-
 constexpr int kUnpackUnroll = 4;
 
 template <int KIND, typename T, int MODE, int V, int CAP>

@@ -8,6 +8,7 @@ sm_100a kernels.
     torch.ops.mctq.fq_lut_scalar      <- lut_quantizer(..., threshold=float)            (activations)
     torch.ops.mctq.quantize_affine_*  -> integer codes (+ optional fake-quant values); mctq.dequantize_affine
     torch.ops.mctq.lut_indices        -> LUT indices;                                    mctq.dequantize_lut
+    torch.ops.mctq.packed_linear      <- F.linear(x, <weight rebuilt from packed codes>, bias)   (small row counts)
 
 (reference call sites: see include/mctq.h).  Each op has a CUDA implementation (device pointers + the
 caller's current stream into the C ABI, no synchronisation), a CPU-tensor implementation that streams the
@@ -39,6 +40,8 @@ _LIB.define("lut_indices(Tensor x, Tensor table, int K, Tensor threshold, bool p
             "int idx_mode) -> Tensor")
 _LIB.define("dequantize_lut(Tensor idx, int idx_mode, int[] shape, Tensor lut, int lut_values_bitwidth, bool is_signed, "
             "Tensor threshold, bool per_channel, int axis) -> Tensor")
+_LIB.define("packed_linear(Tensor x, Tensor codes, int kind, bool is_signed, int out_features, Tensor scale, "
+            "Tensor? zero_point, Tensor? lut_quotients, Tensor? bias) -> Tensor")
 
 
 # --------------------------------------------------------------------------------------------- helpers
@@ -696,6 +699,72 @@ def _dequantize_lut_cuda(idx, idx_mode, shape, lut, lut_values_bitwidth, is_sign
     return UnpackPlan([item]).run()[0]
 
 
+class PackedLinear:
+    """Launch state of one packed [out_features, in_features] weight for mctq_packed_linear: the descriptor is built once, and
+    a call is one C-ABI call with pointers and the row count.
+        codes, kind, is_signed   the packed weight (kind: _native.PACK_*), row-major [out][in]
+        dtype                    the rebuilt weight's dtype (f32 for the LUT kinds): x, bias and y have it
+        scale                    f32, 1 (per tensor) or out_features entries (affine scale or LUT threshold)
+        zero_point               int32 like scale (affine) or None; lut_quotients f32 [K] (LUT kinds) or None
+    `__call__(x, bias)` returns x @ W^T + bias for a contiguous x of `dtype` on the codes' device, enqueued on the current
+    stream; W is exactly the weight UnpackPlan rebuilds, the sum is accumulated in f32 in a fixed order."""
+
+    def __init__(self, codes, kind, is_signed, dtype, out_features, in_features, scale, zero_point, lut_quotients):
+        self.device = codes.device
+        if self.device.type != "cuda":
+            raise ValueError("PackedLinear needs CUDA tensors")
+        self.out_features, self.in_features, self.dtype = int(out_features), int(in_features), dtype
+        n = self.out_features * self.in_features
+        if codes.dtype not in (torch.uint8, torch.int8) or codes.numel() != (n if kind in (_native.PACK_AFFINE_I8, _native.PACK_LUT_U8) else (n + 1) // 2):
+            raise ValueError(f"codes ({codes.dtype}, {codes.numel()} bytes) do not hold a packed {out_features}x{in_features} weight of kind {kind}")
+        codes = codes.contiguous()
+        s = _param_on(scale.detach().reshape(-1).contiguous(), self.device)
+        z = _param_on(zero_point.detach().reshape(-1).contiguous(), self.device) if zero_point is not None else None
+        q = _param_on(lut_quotients.detach().reshape(-1).contiguous(), self.device) if lut_quotients is not None else None
+        if s.dtype != torch.float32 or (z is not None and z.dtype != torch.int32) or (q is not None and q.dtype != torch.float32):
+            raise ValueError("scale / threshold and quotients must be float32, zero points int32")
+        if s.numel() not in (1, self.out_features) or (z is not None and z.numel() != s.numel()):
+            raise ValueError(f"{s.numel()} parameters for {out_features} output channels (per tensor or per output channel)")
+        self._keep = (codes, s, z, q)
+        d = self._desc = _native.MctqPackedDesc()
+        d.codes, d.y, d.n = codes.data_ptr(), None, n
+        d.C, d.inner = (s.numel(), self.in_features) if s.numel() > 1 else (1, 1)
+        d.kind, d.is_signed, d.y_dtype = int(kind), int(bool(is_signed)), _DT.get(dtype, -1)
+        d.K = q.numel() if q is not None else 0
+        d.scale, d.zp, d.lut_quotients = s.data_ptr(), _ptr(z), _ptr(q)
+        self._desc_ptr = ctypes.addressof(d)
+
+    def __call__(self, x, bias=None):
+        if x.dtype != self.dtype or (bias is not None and bias.dtype != self.dtype):
+            raise RuntimeError(f"packed_linear: x and bias must have the weight's dtype {self.dtype}")
+        if x.dim() == 0 or x.shape[-1] != self.in_features:
+            raise RuntimeError(f"packed_linear: x of shape {list(x.shape)} does not end in in_features = {self.in_features}")
+        if x.device != self.device or (bias is not None and bias.device != self.device):
+            raise RuntimeError(f"packed_linear: x and bias must live on {self.device}")
+        if bias is not None and bias.numel() != self.out_features:
+            raise RuntimeError(f"packed_linear: bias has {bias.numel()} entries for {self.out_features} outputs")
+        x = x.contiguous()
+        y = torch.empty(tuple(x.shape[:-1]) + (self.out_features,), dtype=self.dtype, device=self.device)
+        M = x.numel() // self.in_features
+        if M:
+            b = bias.contiguous() if bias is not None else None
+            fast = _native.fast
+            with _on_device(self.device):
+                args = (self._desc_ptr, self.out_features, self.in_features, x.data_ptr(), _DT[self.dtype], M, _ptr(b),
+                        y.data_ptr(), _stream(self.device))
+                rc = fast.packed_linear(*args) if fast is not None else _native.load().mctq_packed_linear(*args)
+            _native.check(rc, "mctq_packed_linear")
+        return y
+
+
+def _packed_linear_cuda(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
+    _dtype_tag(x)
+    if x.dim() == 0:
+        raise RuntimeError("packed_linear: x must have at least one dimension")
+    _native.load()
+    return PackedLinear(codes, kind, is_signed, x.dtype, out_features, x.shape[-1], scale, zero_point, lut_quotients)(x, bias)
+
+
 def _lut_scalar_cuda(x, table, K, divisor, threshold, round_to_input_dtype, multiply=False):
     """`multiply`: normalise with x * (float)(1.0 / divisor) -- the reference's CUDA flavour of `tensor / python_number`
     (quantizer_utils.reference_arithmetic) -- instead of the true division x / (float)divisor."""
@@ -891,6 +960,7 @@ _LIB.impl("quantize_affine_channel", _quantize_affine_channel_cuda, "CUDA")
 _LIB.impl("dequantize_affine", _dequantize_affine_cuda, "CUDA")
 _LIB.impl("lut_indices", _lut_indices_cuda, "CUDA")
 _LIB.impl("dequantize_lut", _dequantize_lut_cuda, "CUDA")
+_LIB.impl("packed_linear", _packed_linear_cuda, "CUDA")
 
 _LIB.impl("fq_affine_scalar_pre", _affine_scalar_pre_cuda, "CUDA")
 _LIB.impl("fq_affine_scalar_pre", _via_device(_affine_scalar_pre_cuda), "CPU")
@@ -903,6 +973,7 @@ _LIB.impl("quantize_affine_channel", _via_device(_quantize_affine_channel_cuda),
 _LIB.impl("dequantize_affine", _via_device(_dequantize_affine_cuda), "CPU")
 _LIB.impl("lut_indices", _via_device(_lut_indices_cuda, keep=(1,)), "CPU")
 _LIB.impl("dequantize_lut", _via_device(_dequantize_lut_cuda, keep=(3,)), "CPU")
+_LIB.impl("packed_linear", _via_device(_packed_linear_cuda), "CPU")
 
 
 # --------------------------------------------------------------------------------------------- fake / meta impls
@@ -960,6 +1031,11 @@ def _(x, table, K, threshold, per_channel, axis, eps, idx_mode):
 @torch.library.register_fake("mctq::dequantize_lut")
 def _(idx, idx_mode, shape, lut, lut_values_bitwidth, is_signed, threshold, per_channel, axis):
     return idx.new_empty(list(shape) if len(shape) else [1], dtype=torch.float32)
+
+
+@torch.library.register_fake("mctq::packed_linear")
+def _(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
+    return x.new_empty(tuple(x.shape[:-1]) + (out_features,))
 
 
 # --------------------------------------------------------------------------------------------- whole-model launch

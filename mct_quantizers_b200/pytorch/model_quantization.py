@@ -278,12 +278,14 @@ class ModelWeightPlan:
     or, for inference with constant weights, `plan.enable()` once (and `plan.refresh()` again only if the float weights
     change).  Results are identical to the per-layer path (same kernels' arithmetic, checked by tests).  Packed weights
     (packed_weights.py) are rebuilt by one unpack launch per device and stay installed while the plan is enabled: the
-    plan holds every rebuilt weight of the model at once."""
+    plan holds every rebuilt weight of the model at once.  Wrappers in fused linear mode are not part of the plan."""
 
     def __init__(self, model: torch.nn.Module):
         from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
+        # wrappers in fused linear mode (packed_weights.py) are left out: rebuilding their weights is what the mode avoids
         self.wrappers = [mod for mod in model.modules()
-                         if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization]
+                         if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization
+                         and not getattr(mod.__dict__.get('_packed'), 'fused', False)]
         self.plan = None
         self._collect()
         self.active = False

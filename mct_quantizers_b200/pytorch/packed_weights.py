@@ -15,6 +15,12 @@ device whose codes fit 8 bits -- affine ranges of at most 256 levels (int4 codes
 256 centroids (4-bit indices for at most 16).  Everything else keeps its float weight and its current path; the report says
 why for each weight.
 
+Fused linear mode (`pack_model_weights(model, fused_linear=True)`, opt-in): a packed `torch.nn.Linear` wrapper computes
+`x @ W^T + b` straight from its codes (csrc/mctq_packed_linear.cu) when the input has at most FUSED_LINEAR_MAX_ROWS rows, so
+W is never rebuilt in memory.  W is exactly the rebuilt weight, the sum is accumulated in f32 in a fixed order and rounded
+once to x's dtype: deterministic and within f32 rounding of the exact product, but not bit-identical to the float model.
+Larger inputs, and every input the fused kernel does not take (see PackedState.fused_forward), run the exact packed path.
+
 Packing is one-way and for inference only:
   * the rebuild dtype is the weight's dtype at packing time; `.half()` does not change it (the codes are integer buffers);
   * the packed state travels with the module: `state_dict` / `load_state_dict` between packed models of the same structure,
@@ -25,9 +31,17 @@ import weakref
 from typing import Dict, List, Optional, Tuple
 
 import torch
+from torch.nn.modules import module as _nn_module
 
 from mct_quantizers_b200 import _native, ops
-from mct_quantizers_b200.common.constants import POSITIONAL_WEIGHT, QUANTIZED_POSITIONAL_WEIGHT
+from mct_quantizers_b200.common.constants import LAYER, POSITIONAL_WEIGHT, QUANTIZED_POSITIONAL_WEIGHT
+
+# Largest number of input rows (the product of x's leading dimensions) a fused-mode wrapper computes with the fused kernel,
+# per dtype of the rebuilt weight: above it, rebuilding W and calling F.linear is faster.  The largest M at which the fused
+# kernel beat the rebuild in every benchmarked format of the dtype (tools/packed_linear_bench.py, Llama-7B's MLP shapes,
+# one B200 at 1000 W, profiles/r04_packed_linear_bench.txt): f32 8 (4-bit LUT; 16 loses), bf16 4 (int4 and int8; 8 loses).
+# f16 runs the bf16 code path and takes its value.
+FUSED_LINEAR_MAX_ROWS = {torch.float32: 8, torch.bfloat16: 4, torch.float16: 4}
 
 _KIND_NAMES = {_native.PACK_AFFINE_I8: "affine_i8", _native.PACK_AFFINE_I4: "affine_i4",
                _native.PACK_LUT_U8: "lut_u8", _native.PACK_LUT_I4: "lut_i4"}
@@ -174,16 +188,44 @@ def _emit_codes(q, w, kind):
     return codes, qmin < 0, int(C), int(inner)
 
 
+def fused_linear_eligibility(wrapper) -> Tuple[bool, str]:
+    """(True, '') when `wrapper` can run in fused linear mode, else (False, reason).  Host-only: looks at the wrapper's
+    layer, weights and packed layout, never at device memory."""
+    d = wrapper.__dict__
+    if not d.get('is_str_attr', False):
+        return False, "the weights are positional inputs of a functional op"
+    layer = d['_modules'].get(LAYER)
+    if type(layer) is not torch.nn.Linear:
+        return False, f"the layer is {type(layer).__name__}, not torch.nn.Linear"
+    if d.get('op_call_args') or d.get('op_call_kwargs') or d.get('is_inputs_as_list'):
+        return False, "the wrapper passes extra call arguments to the layer"
+    if list(wrapper.weights_quantizers) != ['weight']:
+        return False, "the wrapper quantizes weights other than 'weight'"
+    state = d.get('_packed')
+    e = next((e for e in state.entries if e.name == 'weight'), None) if state is not None else None
+    if e is None:
+        return False, "the weight is not packed"
+    out_f, in_f = layer.out_features, layer.in_features
+    if e.shape_out != (out_f, in_f) or e.stride_out != (in_f, 1):
+        return False, "the rebuilt weight is not a row-major [out_features, in_features] matrix"
+    if not (e.C == 1 or (e.C == out_f and e.inner == in_f)):
+        return False, "the parameters are not per tensor or per output channel (channel_axis 0)"
+    return True, ""
+
+
 class PackedState:
-    """Per-wrapper packed state (the wrapper's `_packed` attribute): its PackedWeight entries and the unpack plan of its
-    forward (built on first use, rebuilt when the codes move; not pickled)."""
+    """Per-wrapper packed state (the wrapper's `_packed` attribute): its PackedWeight entries, whether the wrapper runs in
+    fused linear mode, and the launch state of its forward (the unpack plan / the fused-linear descriptor, built on first use
+    and rebuilt when the codes move; not pickled)."""
+    fused = False
 
     def __init__(self, entries: List[PackedWeight]):
         self.entries = entries
-        self._plan, self._sig = None, None
+        self.fused = False
+        self._plan, self._sig, self._lin = None, None, None
 
     def __getstate__(self):
-        return {'entries': self.entries, '_plan': None, '_sig': None}
+        return {'entries': self.entries, 'fused': self.fused, '_plan': None, '_sig': None, '_lin': None}
 
     def bind(self, wrapper):
         """Point the entries at `wrapper` (after a copy or unpickling they point nowhere)."""
@@ -207,11 +249,47 @@ class PackedState:
             self._sig = sig
         return self._plan.run()
 
+    def fused_forward(self, wrapper, x):
+        """x @ W^T + b from the codes (mctq_packed_linear), or None when this call must take the exact packed path: x is not
+        a plain CUDA tensor on the codes' device with the rebuilt weight's dtype (and the bias's), autograd would record the
+        call, the layer has forward hooks, a compiler is tracing, or x has more than FUSED_LINEAR_MAX_ROWS rows."""
+        e = self.entries[0]
+        if e._owner is None or e._owner() is not wrapper:
+            self.bind(wrapper)
+        if type(x) not in ops._PLAIN_TENSOR_TYPES or not x.is_cuda or x.dtype != e.dtype_out or x.dim() == 0:
+            return None
+        layer = wrapper.__dict__['_modules'][LAYER]
+        in_f = layer.in_features
+        if x.shape[-1] != in_f or x.numel() > FUSED_LINEAR_MAX_ROWS.get(x.dtype, 0) * in_f:
+            return None
+        bias = layer.bias
+        if bias is not None and (bias.dtype != x.dtype or bias.device != x.device):
+            return None
+        if torch.is_grad_enabled() and (x.requires_grad or (bias is not None and bias.requires_grad)):
+            return None
+        if layer._forward_hooks or layer._forward_pre_hooks or _nn_module._global_forward_hooks or \
+                _nn_module._global_forward_pre_hooks or torch.compiler.is_compiling():
+            return None
+        codes = e.codes
+        if x.device != codes.device:
+            return None
+        lin = self.__dict__.get('_lin')
+        if lin is None or lin[0] != codes.data_ptr():
+            item = e.plan_item()
+            lin = (codes.data_ptr(), ops.PackedLinear(codes, e.kind, e.is_signed, e.dtype_out, layer.out_features, in_f,
+                                                      item[8], item[9], item[10]))
+            self._lin = lin
+        return lin[1](x, bias)
+
     def forward(self, wrapper, args, kwargs):
         if torch.jit.is_tracing():
             raise RuntimeError("this PytorchQuantizationWrapper holds packed weights (pack_weights / pack_model_weights): "
                                "they cannot be traced or exported to ONNX, which needs the float weights; export the "
                                "model before packing it")
+        if self.fused and len(args) == 1 and not kwargs:
+            y = self.fused_forward(wrapper, args[0])
+            if y is not None:
+                return y
         d = wrapper.__dict__
         if d.get('_prequantized', False):              # a ModelWeightPlan has installed this forward's weights
             return wrapper._run_layer(args, kwargs)
@@ -225,9 +303,11 @@ class PackedState:
             wrapper.set_quantize_weights({})               # drop the rebuilt weights: only the codes stay resident
 
 
-def pack_wrapper_weights(wrapper) -> Dict:
+def pack_wrapper_weights(wrapper, fused_linear: bool = False) -> Dict:
     """Pack every weight of `wrapper` that can be packed (see the module docstring).  Returns
-    {name: {'packed': bool, 'kind': str | None, 'reason': str, 'code_bytes': int, 'float_bytes': int}}."""
+    {name: {'packed': bool, 'kind': str | None, 'reason': str, 'code_bytes': int, 'float_bytes': int}}.
+    `fused_linear=True` also switches the wrapper to fused linear mode when fused_linear_eligibility allows it (on a wrapper
+    packed earlier it only switches the mode), and every report entry gains 'fused': bool and 'fused_reason': str."""
     report = {}
     state = wrapper.__dict__.get('_packed')
     entries = list(state.entries) if state is not None else []
@@ -252,8 +332,14 @@ def pack_wrapper_weights(wrapper) -> Dict:
         new.append((e, w))
         report[name] = dict(packed=True, kind=_KIND_NAMES[kind], reason="", code_bytes=codes.numel() * codes.element_size(),
                             float_bytes=w.numel() * w.element_size())
-    if not new:
-        return report
+    if new:
+        _drop_float_weights(wrapper, new, entries, keep)
+    if fused_linear:
+        _switch_to_fused(wrapper, report)
+    return report
+
+
+def _drop_float_weights(wrapper, new, entries, keep):
     # drop every reference to the float weights: the wrapper's parameter, the layer attribute (or the positional constant)
     for e, w in new:
         if wrapper.is_str_attr:
@@ -267,16 +353,31 @@ def pack_wrapper_weights(wrapper) -> Dict:
         e.quantizer.__dict__.pop('_direct_cache', None)      # launch constants of the float weight's path (pin its tables)
     wrapper._weights_vars = keep
     wrapper._training_arg = None
+    state = wrapper.__dict__.get('_packed')
     wrapper._packed = PackedState(entries)
-    return report
+    wrapper._packed.fused = state is not None and state.fused
+
+
+def _switch_to_fused(wrapper, report):
+    ok, reason = fused_linear_eligibility(wrapper)
+    state = wrapper.__dict__.get('_packed')
+    if ok:
+        state.fused, state._lin = True, None
+    for e in (state.entries if state is not None else []):
+        if e.name not in report:                      # packed by an earlier call
+            report[e.name] = dict(packed=True, kind=_KIND_NAMES[e.kind], reason="already packed",
+                                  code_bytes=e.codes.numel() * e.codes.element_size(), float_bytes=0)
+    for r in report.values():
+        r['fused'], r['fused_reason'] = ok, reason
 
 
 def _bits(t):
     return t.view(torch.int32) if t.element_size() == 4 else t.view(torch.int16)
 
 
-def pack_model_weights(model: torch.nn.Module) -> Dict[str, Dict]:
-    """pack_weights() on every PytorchQuantizationWrapper of `model`: {wrapper module name: {weight name: report entry}}."""
+def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False) -> Dict[str, Dict]:
+    """pack_weights(fused_linear) on every PytorchQuantizationWrapper of `model`: {wrapper module name: {weight name: report
+    entry}}."""
     from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
-    return {mod_name: pack_wrapper_weights(mod) for mod_name, mod in model.named_modules()
+    return {mod_name: pack_wrapper_weights(mod, fused_linear) for mod_name, mod in model.named_modules()
             if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization}
