@@ -162,7 +162,12 @@ int mctq_unpack_multi(const void* plan_host, void* stream);
  *   bias       device, out entries of x_dtype, or NULL
  * W means exactly the weight mctq_unpack_multi rebuilds.  Accumulation is in f32 (a per-row scale or threshold may be applied
  * once per row for f32 outputs), y is rounded once to x_dtype, and the summation order is fixed: two calls on the same inputs
- * give the same bits.  Not bit-identical to a cuBLAS product.  M == 0 is a no-op.  Returns MCTQ_E_BADARG (shape, null or
+ * give the same bits.  Not bit-identical to a cuBLAS product.  Envelope of the per-row factoring: for f32 affine weights the
+ * row sum is sum_k x_k * (q_k - zp_c), scaled afterwards, so the result is "W is exactly the rebuilt weight" (within the error
+ * of f32 accumulation) only while every partial sum of x * (q - zp) stays below FLT_MAX; max|x| * max|q - zp| * in_features
+ * < FLT_MAX suffices (|q - zp| <= 255: max|x| < 1.3e36 / in_features).  Beyond it the result may be +-inf or NaN where
+ * x @ W^T is finite.  Nothing checks this (a host-side check would need a synchronisation).
+ * M == 0 is a no-op.  Returns MCTQ_E_BADARG (shape, null or
  * parameter-layout errors), MCTQ_E_DTYPE, MCTQ_E_LUT (K outside 1..16 / 1..256) before any CUDA call. */
 int mctq_packed_linear(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x, int x_dtype,
                        int64_t M, const void* bias, void* y, void* stream);

@@ -13,6 +13,7 @@ from mct_quantizers_b200 import _native, ops
 from mct_quantizers_b200.pytorch import quantizers as Q
 from mct_quantizers_b200.pytorch.packed_weights import (FUSED_LINEAR_MAX_ROWS, PackedState, PackedWeight,
                                                         fused_linear_eligibility, pack_model_weights)
+from test_packed_variants import decoded_f64
 
 LUT_KINDS = (_native.PACK_LUT_U8, _native.PACK_LUT_I4)
 U_OUT = {torch.float32: 2.0 ** -24, torch.bfloat16: 2.0 ** -8, torch.float16: 2.0 ** -11}
@@ -152,9 +153,13 @@ def _exact_items(kind, dtype, out_f, in_f, per_channel, seed):
 
 
 def _rebuilt(codes, kind, is_signed, dtype, out_f, in_f, scale, zp, quot):
+    """The weight as the host decoder of the wire format rebuilds it (test_packed_variants.decoded_f64): a reference that
+    shares no decode code with the kernel under test."""
     C = scale.numel()
-    item = (codes, kind, is_signed, dtype, (out_f, in_f), None, C, in_f if C > 1 else 1, scale, zp, quot)
-    return ops.UnpackPlan([item]).run()[0]
+    host = lambda t: None if t is None else t.cpu().numpy()                     # noqa: E731
+    w = decoded_f64(host(codes), kind, is_signed, dtype, C, in_f if C > 1 else 1, host(scale), host(zp), host(quot),
+                    count=out_f * in_f)
+    return torch.from_numpy(w.reshape(out_f, in_f)).to(dtype)
 
 
 def _reference(x, w, bias):
@@ -171,7 +176,7 @@ def _reference(x, w, bias):
 
 CROSS = {dt: FUSED_LINEAR_MAX_ROWS[dt] for dt in (torch.float32, torch.bfloat16, torch.float16)}
 EXACT_SHAPES = [(1, 1, (1,)), (10, 33, (3,)), (4096, 4095, (2,)), (10, 4096, ("X",)), (1, 4095, (5,)), (4096, 64, (2, 3)),
-                (10, 33, ("X",)), (10, 1, (4,)), (4096, 33, (1,))]
+                (10, 33, ("X",)), (10, 1, (4,)), (4096, 33, (1,)), (17, 1040, (9,)), (7, 16, (2, 5))]
 KIND_DTYPES = [(k, dt) for k in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4) for dt in (torch.float32, torch.bfloat16, torch.float16)] \
     + [(k, torch.float32) for k in LUT_KINDS]
 
