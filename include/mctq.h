@@ -172,6 +172,27 @@ int mctq_unpack_multi(const void* plan_host, void* stream);
 int mctq_packed_linear(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x, int x_dtype,
                        int64_t M, const void* bias, void* y, void* stream);
 
+/* Batched packed linear: the product of mctq_packed_linear on the tensor cores (tcgen05.mma), for the row counts of batched
+ * decode and short prefills (tens to hundreds of rows), where the CUDA-core kernel's time grows with M.  Same descriptor,
+ * arguments and checks as mctq_packed_linear, plus
+ *   lut_quotients_host  LUT kinds: a HOST copy of the w->K quotients of w->lut_quotients (affine kinds: ignored, may be NULL).
+ *                       The kernel takes the quotients from it (by value); MCTQ_E_LUT when one is not exact in bf16.
+ * Contract: every operand the tensor cores multiply is exact -- the bf16 / f16 rebuilt weight itself; for f32 weights
+ * q - zp (needs |q - zp| <= 256, which packed weights satisfy) or the LUT quotient, with the per-row scale / threshold
+ * applied once per row after the sum (the factoring and the envelope of mctq_packed_linear); for f32 x, three bf16 terms
+ * x0 + x1 + x2 = x (exact for finite x; inf / NaN x enter as x0 alone, so a non-finite x gives the exact product's inf / NaN).
+ * Products are accumulated in f32 by the tensor cores and rounded once to x_dtype after the scale and the bias.
+ * Error bound (the tests enforce it): |y - y_exact| <= 2^-22 * (in_features / 16 + 8) * sum_k |x_k * W_jk| + u_T * |y_exact|
+ * + 2^-126 * sum_k |W_jk| (+ the output dtype's subnormal grain), u_T the unit roundoff of x_dtype.  The first term covers
+ * the f32 accumulation of the tensor cores (16 products per step, alignment that may truncate: a few units of 2^-24 per step)
+ * and the epilogue roundings; the third the f32 x below the normal range, whose low split terms bf16 cannot hold.  On data
+ * whose products and partial sums are exact in f32 the result is exact (the tests check this bit for bit).
+ * Deterministic: the split of the row length over the CTAs of a cluster and the order of the partial sums are fixed by the
+ * shape, so two calls on the same inputs give the same bits.  M == 0 is a no-op.  Returns MCTQ_E_BADARG, MCTQ_E_DTYPE,
+ * MCTQ_E_LUT before any CUDA call. */
+int mctq_packed_linear_batched(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x, int x_dtype,
+                               int64_t M, const void* bias, void* y, const float* lut_quotients_host, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Whole-model weight quantisation: one launch over a table of tensors (SURVEY 8f rank 1).
  * Replaces the per-layer loop  for name, w, quantizer in self._weights_vars: quantizer(w)

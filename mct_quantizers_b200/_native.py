@@ -64,6 +64,7 @@ SIGNATURES = {
     "mctq_unpack_plan": (c_i64, [c_vp, c_int, c_vp, c_sz]),
     "mctq_unpack_multi": (c_int, [c_vp, c_vp]),
     "mctq_packed_linear": (c_int, [c_vp, c_i64, c_i64, c_vp, c_int, c_i64, c_vp, c_vp, c_vp]),
+    "mctq_packed_linear_batched": (c_int, [c_vp, c_i64, c_i64, c_vp, c_int, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "mctq_multi_tile_elems": (c_i64, []),
     "mctq_multi_plan": (c_i64, [c_vp, c_int, c_vp]),
     "mctq_fq_affine_multi": (c_int, [c_vp, c_vp, c_int, c_i64, c_vp]),

@@ -492,22 +492,36 @@ struct NvtxRange {
 #define MCTQ_NVTX(name) mctq::NvtxRange mctq_nvtx_range_(name)
 inline int cuda_rc(cudaError_t e) { return e == cudaSuccess ? 0 : (int)e; }
 
-// launch with the programmatic-serialization attribute; the caller has already declared the launch to pdl_plan_launch
+// launch with the programmatic-serialization attribute, in thread-block clusters of cluster_x CTAs along x when
+// cluster_x > 1; the caller has already declared the launch to pdl_plan_launch
 template <typename... KArgs, typename... Args>
-inline int launch_planned(void (*kernel)(KArgs...), dim3 grid, size_t smem, cudaStream_t st, Args&&... args) {
+inline int launch_planned_cluster(void (*kernel)(KArgs...), dim3 grid, unsigned cluster_x, size_t smem, cudaStream_t st,
+                                  Args&&... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = dim3(kThreads);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
+    cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = g_pdl ? 1 : 0;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
+    if (cluster_x > 1) {
+        attr[1].id = cudaLaunchAttributeClusterDimension;
+        attr[1].val.clusterDim.x = cluster_x;
+        attr[1].val.clusterDim.y = 1;
+        attr[1].val.clusterDim.z = 1;
+        cfg.numAttrs = 2;
+    }
     cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cuda_rc(e);
+}
+
+template <typename... KArgs, typename... Args>
+inline int launch_planned(void (*kernel)(KArgs...), dim3 grid, size_t smem, cudaStream_t st, Args&&... args) {
+    return launch_planned_cluster(kernel, grid, 1u, smem, st, std::forward<Args>(args)...);
 }
 
 // same, for kernels that always use the late order: their outputs are recorded as "unknown"

@@ -99,6 +99,15 @@ static PyObject* py_packed_linear(PyObject* self, PyObject* const* a, Py_ssize_t
     FINISH(rc)
 }
 
+/* (desc_host_ptr, out_features, in_features, x, x_dtype, M, bias, y, lut_quotients_host, stream) */
+static PyObject* py_packed_linear_batched(PyObject* self, PyObject* const* a, Py_ssize_t nargs) {
+    NEED(10)
+    int rc = mctq_packed_linear_batched((const MctqPackedDesc*)as_ptr(a[0]), as_i64(a[1]), as_i64(a[2]), as_ptr(a[3]),
+                                        as_int(a[4]), as_i64(a[5]), as_ptr(a[6]), as_ptr(a[7]), (const float*)as_ptr(a[8]),
+                                        as_ptr(a[9]));
+    FINISH(rc)
+}
+
 static PyMethodDef methods[] = {
     {"fq_affine_scalar", (PyCFunction)(void (*)(void))py_fq_affine_scalar, METH_FASTCALL, "mctq_fq_affine_scalar"},
     {"fq_affine_scalar_pre", (PyCFunction)(void (*)(void))py_fq_affine_scalar_pre, METH_FASTCALL, "mctq_fq_affine_scalar_pre"},
@@ -107,6 +116,7 @@ static PyMethodDef methods[] = {
     {"fq_lut_prepared", (PyCFunction)(void (*)(void))py_fq_lut_prepared, METH_FASTCALL, "mctq_fq_lut_prepared"},
     {"fq_affine_scalar_multi", (PyCFunction)(void (*)(void))py_fq_affine_scalar_multi, METH_FASTCALL, "mctq_fq_affine_scalar_multi"},
     {"packed_linear", (PyCFunction)(void (*)(void))py_packed_linear, METH_FASTCALL, "mctq_packed_linear"},
+    {"packed_linear_batched", (PyCFunction)(void (*)(void))py_packed_linear_batched, METH_FASTCALL, "mctq_packed_linear_batched"},
     {NULL, NULL, 0, NULL}};
 
 static struct PyModuleDef moddef = {PyModuleDef_HEAD_INIT, "_mctq_fast", "CPython front door to libmctq_sm100.so", -1, methods};

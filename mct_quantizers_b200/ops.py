@@ -9,6 +9,7 @@ sm_100a kernels.
     torch.ops.mctq.quantize_affine_*  -> integer codes (+ optional fake-quant values); mctq.dequantize_affine
     torch.ops.mctq.lut_indices        -> LUT indices;                                    mctq.dequantize_lut
     torch.ops.mctq.packed_linear      <- F.linear(x, <weight rebuilt from packed codes>, bias)   (small row counts)
+    torch.ops.mctq.packed_linear_batched   the same product on the tensor cores                  (batched row counts)
 
 (reference call sites: see include/mctq.h).  Each op has a CUDA implementation (device pointers + the
 caller's current stream into the C ABI, no synchronisation), a CPU-tensor implementation that streams the
@@ -41,6 +42,8 @@ _LIB.define("lut_indices(Tensor x, Tensor table, int K, Tensor threshold, bool p
 _LIB.define("dequantize_lut(Tensor idx, int idx_mode, int[] shape, Tensor lut, int lut_values_bitwidth, bool is_signed, "
             "Tensor threshold, bool per_channel, int axis) -> Tensor")
 _LIB.define("packed_linear(Tensor x, Tensor codes, int kind, bool is_signed, int out_features, Tensor scale, "
+            "Tensor? zero_point, Tensor? lut_quotients, Tensor? bias) -> Tensor")
+_LIB.define("packed_linear_batched(Tensor x, Tensor codes, int kind, bool is_signed, int out_features, Tensor scale, "
             "Tensor? zero_point, Tensor? lut_quotients, Tensor? bias) -> Tensor")
 
 
@@ -707,7 +710,10 @@ class PackedLinear:
         scale                    f32, 1 (per tensor) or out_features entries (affine scale or LUT threshold)
         zero_point               int32 like scale (affine) or None; lut_quotients f32 [K] (LUT kinds) or None
     `__call__(x, bias)` returns x @ W^T + bias for a contiguous x of `dtype` on the codes' device, enqueued on the current
-    stream; W is exactly the weight UnpackPlan rebuilds, the sum is accumulated in f32 in a fixed order."""
+    stream; W is exactly the weight UnpackPlan rebuilds, the sum is accumulated in f32 in a fixed order.  `batched(x, bias)`
+    computes the same product with mctq_packed_linear_batched (tensor cores, for tens to hundreds of rows); for the LUT kinds
+    it reads the quotients on the host (_quotients_host: one synchronising copy per table contents, none when they are on
+    the CPU), so capture a batched LUT call in a CUDA graph after one eager call."""
 
     def __init__(self, codes, kind, is_signed, dtype, out_features, in_features, scale, zero_point, lut_quotients):
         self.device = codes.device
@@ -725,6 +731,7 @@ class PackedLinear:
             raise ValueError("scale / threshold and quotients must be float32, zero points int32")
         if s.numel() not in (1, self.out_features) or (z is not None and z.numel() != s.numel()):
             raise ValueError(f"{s.numel()} parameters for {out_features} output channels (per tensor or per output channel)")
+        self._quot_src = lut_quotients.detach().reshape(-1) if lut_quotients is not None else None
         self._keep = (codes, s, z, q)
         d = self._desc = _native.MctqPackedDesc()
         d.codes, d.y, d.n = codes.data_ptr(), None, n
@@ -735,6 +742,12 @@ class PackedLinear:
         self._desc_ptr = ctypes.addressof(d)
 
     def __call__(self, x, bias=None):
+        return self._run(x, bias, False)
+
+    def batched(self, x, bias=None):
+        return self._run(x, bias, True)
+
+    def _run(self, x, bias, batched):
         if x.dtype != self.dtype or (bias is not None and bias.dtype != self.dtype):
             raise RuntimeError(f"packed_linear: x and bias must have the weight's dtype {self.dtype}")
         if x.dim() == 0 or x.shape[-1] != self.in_features:
@@ -751,10 +764,36 @@ class PackedLinear:
             fast = _native.fast
             with _on_device(self.device):
                 args = (self._desc_ptr, self.out_features, self.in_features, x.data_ptr(), _DT[self.dtype], M, _ptr(b),
-                        y.data_ptr(), _stream(self.device))
-                rc = fast.packed_linear(*args) if fast is not None else _native.load().mctq_packed_linear(*args)
-            _native.check(rc, "mctq_packed_linear")
+                        y.data_ptr())
+                if batched:
+                    qh = _quotients_host(self._quot_src)
+                    args += (qh.ctypes.data if qh is not None else None, _stream(self.device))
+                    rc = fast.packed_linear_batched(*args) if fast is not None else \
+                        _native.load().mctq_packed_linear_batched(*args)
+                else:
+                    args += (_stream(self.device),)
+                    rc = fast.packed_linear(*args) if fast is not None else _native.load().mctq_packed_linear(*args)
+            _native.check(rc, "mctq_packed_linear_batched" if batched else "mctq_packed_linear")
         return y
+
+
+_QUOT_HOST = {}
+
+
+def _quotients_host(q):
+    """The f32 LUT quotients `q` as a host numpy array for mctq_packed_linear_batched, cached by storage and version like
+    _param_on: a device tensor is copied (and synchronised) once per contents, so that later calls, CUDA-graph capture
+    included, need no copy; an in-place update (load_state_dict) bumps the version and is read again."""
+    if q is None:
+        return None
+    key = (q.data_ptr(), _ver(q), q.numel(), q.dtype, str(q.device))
+    hit = _QUOT_HOST.get(key)
+    if hit is None:
+        if len(_QUOT_HOST) >= 1024:
+            _QUOT_HOST.clear()
+        hit = (q, np.ascontiguousarray(q.to("cpu", torch.float32).numpy()))
+        _QUOT_HOST[key] = hit
+    return hit[1]
 
 
 def _packed_linear_cuda(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
@@ -763,6 +802,15 @@ def _packed_linear_cuda(x, codes, kind, is_signed, out_features, scale, zero_poi
         raise RuntimeError("packed_linear: x must have at least one dimension")
     _native.load()
     return PackedLinear(codes, kind, is_signed, x.dtype, out_features, x.shape[-1], scale, zero_point, lut_quotients)(x, bias)
+
+
+def _packed_linear_batched_cuda(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
+    _dtype_tag(x)
+    if x.dim() == 0:
+        raise RuntimeError("packed_linear_batched: x must have at least one dimension")
+    _native.load()
+    lin = PackedLinear(codes, kind, is_signed, x.dtype, out_features, x.shape[-1], scale, zero_point, lut_quotients)
+    return lin.batched(x, bias)
 
 
 def _lut_scalar_cuda(x, table, K, divisor, threshold, round_to_input_dtype, multiply=False):
@@ -961,6 +1009,7 @@ _LIB.impl("dequantize_affine", _dequantize_affine_cuda, "CUDA")
 _LIB.impl("lut_indices", _lut_indices_cuda, "CUDA")
 _LIB.impl("dequantize_lut", _dequantize_lut_cuda, "CUDA")
 _LIB.impl("packed_linear", _packed_linear_cuda, "CUDA")
+_LIB.impl("packed_linear_batched", _packed_linear_batched_cuda, "CUDA")
 
 _LIB.impl("fq_affine_scalar_pre", _affine_scalar_pre_cuda, "CUDA")
 _LIB.impl("fq_affine_scalar_pre", _via_device(_affine_scalar_pre_cuda), "CPU")
@@ -974,6 +1023,7 @@ _LIB.impl("dequantize_affine", _via_device(_dequantize_affine_cuda), "CPU")
 _LIB.impl("lut_indices", _via_device(_lut_indices_cuda, keep=(1,)), "CPU")
 _LIB.impl("dequantize_lut", _via_device(_dequantize_lut_cuda, keep=(3,)), "CPU")
 _LIB.impl("packed_linear", _via_device(_packed_linear_cuda), "CPU")
+_LIB.impl("packed_linear_batched", _via_device(_packed_linear_batched_cuda), "CPU")
 
 
 # --------------------------------------------------------------------------------------------- fake / meta impls
@@ -1034,6 +1084,11 @@ def _(idx, idx_mode, shape, lut, lut_values_bitwidth, is_signed, threshold, per_
 
 
 @torch.library.register_fake("mctq::packed_linear")
+def _(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
+    return x.new_empty(tuple(x.shape[:-1]) + (out_features,))
+
+
+@torch.library.register_fake("mctq::packed_linear_batched")
 def _(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
     return x.new_empty(tuple(x.shape[:-1]) + (out_features,))
 

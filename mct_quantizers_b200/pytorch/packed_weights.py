@@ -21,6 +21,12 @@ W is never rebuilt in memory.  W is exactly the rebuilt weight, the sum is accum
 once to x's dtype: deterministic and within f32 rounding of the exact product, but not bit-identical to the float model.
 Larger inputs, and every input the fused kernel does not take (see PackedState.fused_forward), run the exact packed path.
 
+Batched linear mode (`pack_model_weights(model, fused_linear=True, batched_linear=True)`, opt-in on top of the fused mode):
+inputs of more than FUSED_LINEAR_MAX_ROWS and at most FUSED_BATCHED_MAX_ROWS rows take the tensor-core kernel
+(csrc/mctq_packed_gemm.cu) instead of the exact path; smaller inputs keep the fused kernel.  Same contract: W is exactly the
+rebuilt weight, f32 accumulation, one rounding to x's dtype, deterministic.  LUT weights qualify when every quotient of the
+table is exact in bf16 (integer centroids on grids of up to 8 bits).
+
 Packing is one-way and for inference only:
   * the rebuild dtype is the weight's dtype at packing time; `.half()` does not change it (the codes are integer buffers);
   * the packed state travels with the module: `state_dict` / `load_state_dict` between packed models of the same structure,
@@ -42,6 +48,14 @@ from mct_quantizers_b200.common.constants import LAYER, POSITIONAL_WEIGHT, QUANT
 # one B200 at 1000 W, profiles/r04_packed_linear_bench.txt): f32 8 (4-bit LUT; 16 loses), bf16 4 (int4 and int8; 8 loses).
 # f16 runs the bf16 code path and takes its value.
 FUSED_LINEAR_MAX_ROWS = {torch.float32: 8, torch.bfloat16: 4, torch.float16: 4}
+
+# Largest number of input rows a batched-mode wrapper computes with the tensor-core kernel (above FUSED_LINEAR_MAX_ROWS),
+# per dtype of the rebuilt weight: the largest M up to which the kernel beat rebuild + F.linear at every measured M in
+# every format of the dtype (tools/packed_batched_bench.py, Llama-7B's MLP shapes, one B200 at 1000 W,
+# profiles/r05_packed_batched_bench.txt).  f32: 256 (4-bit LUT, int4 and int8 affine; every M from 8 to 256 wins).  bf16: the kernel lost at
+# every M (int4 and int8), so the limit equals FUSED_LINEAR_MAX_ROWS and batched mode leaves bf16 wrappers as they are;
+# f16 runs the bf16 code path and takes its value.
+FUSED_BATCHED_MAX_ROWS = {torch.float32: 256, torch.bfloat16: 4, torch.float16: 4}
 
 _KIND_NAMES = {_native.PACK_AFFINE_I8: "affine_i8", _native.PACK_AFFINE_I4: "affine_i4",
                _native.PACK_LUT_U8: "lut_u8", _native.PACK_LUT_I4: "lut_i4"}
@@ -213,19 +227,41 @@ def fused_linear_eligibility(wrapper) -> Tuple[bool, str]:
     return True, ""
 
 
+def _lut_quotients_host(q):
+    """The f32 quotients of LUT quantizer q, computed on the host (no device synchronisation)."""
+    return ops.lut_quotients(torch.as_tensor(q._lut_values_np), q.lut_values_bitwidth, True)
+
+
+def batched_linear_eligibility(wrapper) -> Tuple[bool, str]:
+    """(True, '') when `wrapper` can run in batched linear mode: fused_linear_eligibility, and for LUT weights every quotient
+    of the table exact in bf16 (the tensor cores multiply it as a bf16 operand).  Host-only."""
+    ok, reason = fused_linear_eligibility(wrapper)
+    if not ok:
+        return ok, reason
+    e = next(e for e in wrapper.__dict__['_packed'].entries if e.name == 'weight')
+    if e.kind in (_native.PACK_LUT_U8, _native.PACK_LUT_I4):
+        bits = _lut_quotients_host(e.quantizer).view(torch.int32)
+        if bool(((bits & 0xFFFF) != 0).any()):
+            return False, "a LUT quotient is not exact in bfloat16 (the tensor cores take the quotients as bf16 operands)"
+    return True, ""
+
+
 class PackedState:
     """Per-wrapper packed state (the wrapper's `_packed` attribute): its PackedWeight entries, whether the wrapper runs in
-    fused linear mode, and the launch state of its forward (the unpack plan / the fused-linear descriptor, built on first use
+    fused linear mode (and batched linear mode), and the launch state of its forward (the unpack plan / the fused-linear descriptor, built on first use
     and rebuilt when the codes move; not pickled)."""
     fused = False
+    batched = False             # class default: states pickled before batched mode existed load with it off
 
     def __init__(self, entries: List[PackedWeight]):
         self.entries = entries
         self.fused = False
+        self.batched = False
         self._plan, self._sig, self._lin = None, None, None
 
     def __getstate__(self):
-        return {'entries': self.entries, 'fused': self.fused, '_plan': None, '_sig': None, '_lin': None}
+        return {'entries': self.entries, 'fused': self.fused, 'batched': self.batched, '_plan': None, '_sig': None,
+                '_lin': None}
 
     def bind(self, wrapper):
         """Point the entries at `wrapper` (after a copy or unpickling they point nowhere)."""
@@ -252,7 +288,8 @@ class PackedState:
     def fused_forward(self, wrapper, x):
         """x @ W^T + b from the codes (mctq_packed_linear), or None when this call must take the exact packed path: x is not
         a plain CUDA tensor on the codes' device with the rebuilt weight's dtype (and the bias's), autograd would record the
-        call, the layer has forward hooks, a compiler is tracing, or x has more than FUSED_LINEAR_MAX_ROWS rows."""
+        call, the layer has forward hooks, a compiler is tracing, or x has more than FUSED_LINEAR_MAX_ROWS rows (batched
+        mode: more than FUSED_BATCHED_MAX_ROWS rows; rows above FUSED_LINEAR_MAX_ROWS take mctq_packed_linear_batched)."""
         e = self.entries[0]
         if e._owner is None or e._owner() is not wrapper:
             self.bind(wrapper)
@@ -260,7 +297,8 @@ class PackedState:
             return None
         layer = wrapper.__dict__['_modules'][LAYER]
         in_f = layer.in_features
-        if x.shape[-1] != in_f or x.numel() > FUSED_LINEAR_MAX_ROWS.get(x.dtype, 0) * in_f:
+        limit = (FUSED_BATCHED_MAX_ROWS if self.__dict__.get('batched', False) else FUSED_LINEAR_MAX_ROWS).get(x.dtype, 0)
+        if x.shape[-1] != in_f or x.numel() > limit * in_f:
             return None
         bias = layer.bias
         if bias is not None and (bias.dtype != x.dtype or bias.device != x.device):
@@ -279,6 +317,8 @@ class PackedState:
             lin = (codes.data_ptr(), ops.PackedLinear(codes, e.kind, e.is_signed, e.dtype_out, layer.out_features, in_f,
                                                       item[8], item[9], item[10]))
             self._lin = lin
+        if x.numel() > FUSED_LINEAR_MAX_ROWS.get(x.dtype, 0) * in_f:
+            return lin[1].batched(x, bias)
         return lin[1](x, bias)
 
     def forward(self, wrapper, args, kwargs):
@@ -303,11 +343,15 @@ class PackedState:
             wrapper.set_quantize_weights({})               # drop the rebuilt weights: only the codes stay resident
 
 
-def pack_wrapper_weights(wrapper, fused_linear: bool = False) -> Dict:
+def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bool = False) -> Dict:
     """Pack every weight of `wrapper` that can be packed (see the module docstring).  Returns
     {name: {'packed': bool, 'kind': str | None, 'reason': str, 'code_bytes': int, 'float_bytes': int}}.
     `fused_linear=True` also switches the wrapper to fused linear mode when fused_linear_eligibility allows it (on a wrapper
-    packed earlier it only switches the mode), and every report entry gains 'fused': bool and 'fused_reason': str."""
+    packed earlier it only switches the mode), and every report entry gains 'fused': bool and 'fused_reason': str.
+    `batched_linear=True` (needs fused_linear=True) also switches it to batched linear mode when batched_linear_eligibility
+    allows it, and every report entry gains 'batched': bool and 'batched_reason': str."""
+    if batched_linear and not fused_linear:
+        raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     report = {}
     state = wrapper.__dict__.get('_packed')
     entries = list(state.entries) if state is not None else []
@@ -336,6 +380,8 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False) -> Dict:
         _drop_float_weights(wrapper, new, entries, keep)
     if fused_linear:
         _switch_to_fused(wrapper, report)
+    if batched_linear:
+        _switch_to_batched(wrapper, report)
     return report
 
 
@@ -356,6 +402,7 @@ def _drop_float_weights(wrapper, new, entries, keep):
     state = wrapper.__dict__.get('_packed')
     wrapper._packed = PackedState(entries)
     wrapper._packed.fused = state is not None and state.fused
+    wrapper._packed.batched = state is not None and state.batched
 
 
 def _switch_to_fused(wrapper, report):
@@ -371,13 +418,24 @@ def _switch_to_fused(wrapper, report):
         r['fused'], r['fused_reason'] = ok, reason
 
 
+def _switch_to_batched(wrapper, report):
+    ok, reason = batched_linear_eligibility(wrapper)
+    state = wrapper.__dict__.get('_packed')
+    if ok:
+        state.batched, state._lin = True, None
+    for r in report.values():
+        r['batched'], r['batched_reason'] = ok, reason
+
+
 def _bits(t):
     return t.view(torch.int32) if t.element_size() == 4 else t.view(torch.int16)
 
 
-def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False) -> Dict[str, Dict]:
-    """pack_weights(fused_linear) on every PytorchQuantizationWrapper of `model`: {wrapper module name: {weight name: report
-    entry}}."""
+def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batched_linear: bool = False) -> Dict[str, Dict]:
+    """pack_weights(fused_linear, batched_linear) on every PytorchQuantizationWrapper of `model`: {wrapper module name:
+    {weight name: report entry}}."""
+    if batched_linear and not fused_linear:
+        raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
-    return {mod_name: pack_wrapper_weights(mod, fused_linear) for mod_name, mod in model.named_modules()
+    return {mod_name: pack_wrapper_weights(mod, fused_linear, batched_linear) for mod_name, mod in model.named_modules()
             if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization}
