@@ -331,7 +331,7 @@ int mctq_fq_lut_prepared_multi(const void* plan_host, void* stream);
 /* ------------------------------------------------------------------------------------------------------
  * Host-buffer entry points: the same operators for tensors that live in HOST memory (pinned memory
  * overlaps; pageable memory works but serialises).  The data is streamed through `staging_dev`
- * (device scratch owned by the caller, >= mctq_host_staging_min_bytes()) in chunks on internal streams:
+ * (device scratch owned by the caller, >= mctq_host_staging_min_bytes() = 304 MiB) in chunks on three internal streams:
  * H2D copy, kernel and D2H copy of neighbouring chunks overlap.  Parameters are HOST arrays (copied
  * before the call returns; at most 384 Ki channels).  By default these calls return after y_host is
  * complete (they synchronise their internal streams only).
@@ -358,26 +358,16 @@ int mctq_fq_lut_host(const void* x_host, float* y_host, int64_t n, int x_dtype,
  */
 /* launches of this library's kernels since load (what bench.py reports as gpu_launches) */
 int64_t mctq_launch_count(void);
-/* variant selection for experiments: key 0 = unroll (0 = automatic [default], 2, 4, 8), key 1 = force rint path (0/1),
- * key 2 = force IEEE-division LUT path (0/1), key 3 = programmatic dependent launch: 0 off, 1 wait-then-load (default),
+/* process-wide switches.  key 3 = programmatic dependent launch: 0 off, 1 wait-then-load (default),
  *   2 = load-then-wait for launches whose input is not an output of a launch of this library still in flight on the stream,
  *   3 = additionally no wait at all (until a CTA's last instruction) for launches whose buffers are disjoint from those of
- *   every launch still in flight -- 2 and 3 are only legal while the stream carries NO work of other libraries (their
- *   kernels may release dependents before their stores are visible; the allocator may recycle their buffers); opt-in, see
+ *   every launch still in flight (at most three launches in flight together, then a waiting one) -- 2 and 3 are only
+ *   legal while the stream carries NO work of other libraries (their kernels may release dependents before their stores
+ *   are visible; the allocator may recycle their buffers); opt-in, see
  *   mct_quantizers_b200.private_stream(); changing the key makes the next launch on every stream a waiting one,
- * key 4 = warp-shuffle search in the generic LUT kernel for tables of <= 32 entries (default 1),
- * key 5 = wide vectors (8 elements per vector, 256-bit stores) in the kernels that have them (default 1),
- * key 6 = (retired: the multi-tensor LUT launches run one tile per CTA; the key is accepted and ignored),
- * key 7 = xy-record variant of the prepared LUT kernel for per-tensor / long-row launches (default 1),
- * key 8 = kernels stage their prepared parameter tables BEFORE the dependent-launch wait whenever the blob was not written by
- *   a prepare call still in flight on the stream (default 1; the blobs are private to the library, so this is legal whatever
- *   else runs on the stream),
  * key 9 = NVTX ranges (nvtx3, header-only) around every compute entry point, named after the entry point (default 0;
  *   `ncu --nvtx` and timeline tools then attribute kernels to the call of the reference's API they belong to);
- * key 10 = with key 3 = 3: how many launches may be in flight together before one waits again (2..8, default 3);
- * key 11 = data streams (= staging slots) of the host-buffer pipeline (2..6, default 3; mctq_host_staging_min_bytes follows),
- * key 12 = number of chunks a tensor is cut into by the host-buffer pipeline in deferred mode (1..16, default 1: whole staging slots);
- * returns previous value or <0 */
+ * every other key is rejected with MCTQ_E_BADARG.  Returns the previous value or <0 */
 int mctq_set_tuning(int key, int value);
 /* device self-test of the 5-op correctly-rounded division used by the LUT kernels against __fdiv_rn
  * on n_pairs pseudo-random (x, d) pairs; *mismatches_dev (device int64) receives the number that differ */

@@ -145,7 +145,7 @@ def load(build_if_missing=True):
             fn.argtypes = args
         if handle.mctq_abi_version() != 1:
             raise MctqError(f"ABI version mismatch: library reports {handle.mctq_abi_version()}, binding expects 1")
-        # experiments: MCTQ_TUNE="key=value,..." applies mctq_set_tuning at load time (see include/mctq.h)
+        # MCTQ_TUNE="key=value,..." applies mctq_set_tuning at load time: key 3 (dependent launch), key 9 (NVTX); see include/mctq.h
         for kv in filter(None, os.environ.get("MCTQ_TUNE", "").split(",")):
             k, v = kv.split("=")
             if handle.mctq_set_tuning(int(k), int(v)) < 0:

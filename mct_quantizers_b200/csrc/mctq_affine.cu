@@ -689,34 +689,25 @@ int launch_affine_prepared(const AffineArgs& a, int code_mode, cudaStream_t st) 
     }
 }
 
-template <typename T, int CHMODE, int CODE, bool RINT>
-int launch_affine_unroll(const AffineArgs& a, cudaStream_t st) {
-    // the unroll sweep (mctq_set_tuning key 0) exists only for the plain fake-quant variants
-    if (CODE == MCTQ_CODES_NONE && !RINT) {
-        // automatic: 8 KB tiles for per-tensor launches (nothing to stage per tile; tools/stream_probe.cu measures
-        // +2 % over 16 KB tiles), 16 KB tiles when a channel window is staged per tile
-        // (4 KB tiles were measured in round 2 and are slower at every size: 74 MB 5.72 -> 5.16 TB/s queued, 295 MB 6.63 ->
-        // 5.94, 1 GB 6.91 -> 6.16 for bf16; the ~3 us a mid-size launch loses are drain + ramp, not tile granularity)
-        const int u = g_unroll ? g_unroll : (CHMODE == CH_PT ? 2 : 4);
-        if (u == 2) return launch_affine_tiles<T, CHMODE, MCTQ_CODES_NONE, 2, false>(a, st);
-        if (u == 8) return launch_affine_tiles<T, CHMODE, MCTQ_CODES_NONE, 8, false>(a, st);
-    }
-    return launch_affine_tiles<T, CHMODE, CODE, 4, RINT>(a, st);
-}
+// 16-byte vectors in flight per thread: 8 KB tiles for plain per-tensor fake-quant (nothing to stage per tile;
+// tools/stream_probe.cu measures +2 % over 16 KB tiles), 16 KB tiles otherwise.  (4 KB tiles were measured in round 2 and
+// are slower at every size: 74 MB 5.72 -> 5.16 TB/s queued, 295 MB 6.63 -> 5.94, 1 GB 6.91 -> 6.16 for bf16; the ~3 us a
+// mid-size launch loses are drain + ramp, not tile granularity.)
+template <int CHMODE, int CODE, bool RINT> constexpr int affine_unroll() { return CHMODE == CH_PT && CODE == MCTQ_CODES_NONE && !RINT ? 2 : 4; }
 
 template <typename T, int CHMODE, bool RINT>
 int launch_affine_code(const AffineArgs& a, int code_mode, cudaStream_t st) {
     switch (code_mode) {
-        case MCTQ_CODES_INT8: return launch_affine_unroll<T, CHMODE, MCTQ_CODES_INT8, RINT>(a, st);
-        case MCTQ_CODES_INT4: return launch_affine_unroll<T, CHMODE, MCTQ_CODES_INT4, RINT>(a, st);
-        default: return launch_affine_unroll<T, CHMODE, MCTQ_CODES_NONE, RINT>(a, st);
+        case MCTQ_CODES_INT8: return launch_affine_tiles<T, CHMODE, MCTQ_CODES_INT8, affine_unroll<CHMODE, MCTQ_CODES_INT8, RINT>(), RINT>(a, st);
+        case MCTQ_CODES_INT4: return launch_affine_tiles<T, CHMODE, MCTQ_CODES_INT4, affine_unroll<CHMODE, MCTQ_CODES_INT4, RINT>(), RINT>(a, st);
+        default: return launch_affine_tiles<T, CHMODE, MCTQ_CODES_NONE, affine_unroll<CHMODE, MCTQ_CODES_NONE, RINT>(), RINT>(a, st);
     }
 }
 
 template <typename T>
 int launch_affine_typed(const AffineArgs& a, int code_mode, cudaStream_t st) {
     constexpr int V = 16 / sizeof(T);
-    const bool rint_path = g_force_rint || !(a.qmax - (int64_t)a.qmin < kFastRangeLimit);
+    const bool rint_path = !(a.qmax - (int64_t)a.qmin < kFastRangeLimit);
     // vector path needs 16-byte aligned x / y and suitably aligned codes
     bool vec_ok = aligned16(a.x) && (!a.y || aligned16(a.y));
     if (code_mode != MCTQ_CODES_NONE) vec_ok = vec_ok && (reinterpret_cast<uintptr_t>(a.codes) & 7u) == 0;
@@ -744,7 +735,7 @@ int launch_affine_typed(const AffineArgs& a, int code_mode, cudaStream_t st) {
             if (period <= 4096) { chmode = CH_LAST; a2.period = (uint32_t)period; }
         }
     }
-    if (a.prep_rec && !rint_path && (g_unroll == 0 || g_unroll == 4)) {
+    if (a.prep_rec && !rint_path) {
         // prepared blob: bulk-copy staging needs 16-byte granules (CH_LAST: whole arrays of C floats)
         if (chmode == CH_VEC) return launch_affine_prepared<T, CH_VEC>(a2, code_mode, st);
         if (chmode == CH_ELEM) return launch_affine_prepared<T, CH_ELEM>(a2, code_mode, st);
@@ -847,21 +838,17 @@ int mctq_dequant_affine(const void* codes, int code_mode, int is_signed, float* 
         const int mode = C == 1 ? 0 : ((inner % 4 == 0 && elem_offset % 4 == 0) ? 1 : 2);
         // 8 codes per vector (32-byte aligned y, the vector inside one channel) only where it measured faster on the B200:
         // per-channel int4 (5.63 -> 6.14 TB/s; the channel look-up per vector halves).  Per-tensor and int8 variants are
-        // at 6.3-6.4 TB/s with 4-code vectors and lose ~3 % with 8 (key 5 = 2 forces 8 everywhere for experiments).
-        const bool fits8 = mode != 2 && aligned32(y) && (code_mode != MCTQ_CODES_INT8 || (reinterpret_cast<uintptr_t>(codes) & 7u) == 0) &&
-                           (mode == 0 || (inner % 8 == 0 && elem_offset % 8 == 0));
-        const bool v8 = fits8 && ((g_wide && mode == 1 && code_mode == MCTQ_CODES_INT4) || g_wide == 2);
+        // at 6.3-6.4 TB/s with 4-code vectors and lose ~3 % with 8.
+        const bool v8 = mode == 1 && code_mode == MCTQ_CODES_INT4 && aligned32(y) && inner % 8 == 0 && elem_offset % 8 == 0;
         const int64_t tile = (int64_t)kThreads * 4 * (v8 ? 8 : 4);
         const int64_t tiles = (n + tile - 1) / tile;
         if (tiles > 0x7fffffffLL) return MCTQ_E_BADARG;
         const uint32_t C32 = (uint32_t)C, in32 = (uint32_t)(C == 1 ? 1 : inner);
         const FastDiv di = make_fastdiv(in32), dc = make_fastdiv(C32);
 #define MCTQ_DQ(CM, MD, VV) launch_streaming(dequant_affine_vec_kernel<CM, MD, VV>, (unsigned)tiles, 0, st, codes, is_signed, y, n, scale, zp, C32, in32, elem_offset, di, dc)
-        if (code_mode == MCTQ_CODES_INT8) {
-            if (v8) return mode == 0 ? MCTQ_DQ(MCTQ_CODES_INT8, 0, 8) : MCTQ_DQ(MCTQ_CODES_INT8, 1, 8);
+        if (code_mode == MCTQ_CODES_INT8)
             return mode == 0 ? MCTQ_DQ(MCTQ_CODES_INT8, 0, 4) : mode == 1 ? MCTQ_DQ(MCTQ_CODES_INT8, 1, 4) : MCTQ_DQ(MCTQ_CODES_INT8, 2, 4);
-        }
-        if (v8) return mode == 0 ? MCTQ_DQ(MCTQ_CODES_INT4, 0, 8) : MCTQ_DQ(MCTQ_CODES_INT4, 1, 8);
+        if (v8) return MCTQ_DQ(MCTQ_CODES_INT4, 1, 8);
         return mode == 0 ? MCTQ_DQ(MCTQ_CODES_INT4, 0, 4) : mode == 1 ? MCTQ_DQ(MCTQ_CODES_INT4, 1, 4) : MCTQ_DQ(MCTQ_CODES_INT4, 2, 4);
 #undef MCTQ_DQ
     }

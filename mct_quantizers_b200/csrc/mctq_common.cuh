@@ -26,16 +26,7 @@ constexpr int kThreads = 256;
 
 // process-wide state (defined in mctq_host.cu)
 extern std::atomic<int64_t> g_launches;
-extern int g_unroll;
-extern int g_force_rint;
-extern int g_force_ieee_div;
-extern int g_lut_shfl;      // warp-shuffle search in the generic LUT kernel for tables of <= 32 entries (key 4)
-extern int g_wide;          // wide (8-element / 256-bit) vector variants (mctq_set_tuning key 5)
-extern int g_multi_span;    // tiles per CTA of the multi-tensor LUT launch (mctq_set_tuning key 6)
-extern int g_lut_xy;        // xy-record variant of the prepared LUT kernel where it applies (mctq_set_tuning key 7)
 extern int g_pdl;           // programmatic dependent launch for the streaming kernels (mctq_set_tuning key 3)
-extern int g_tab_early;     // parameter tables staged before the dependent-launch wait when legal (mctq_set_tuning key 8)
-extern int g_chain_max;     // launches that may overlap under the "free" order before one waits again (mctq_set_tuning key 10)
 extern int g_nvtx;          // NVTX ranges around the C-ABI compute entry points (mctq_set_tuning key 9 / MCTQ_TUNE=9=1; off by default)
 
 enum ChMode { CH_PT = 0, CH_VEC = 1, CH_ELEM = 2, CH_LAST = 3 };
@@ -421,7 +412,7 @@ __device__ __forceinline__ void locate(uint32_t l, const Window& w, const Args& 
 //   2 free  : trigger -> loads -> math -> stores -> wait         the launch does not wait for anything until its CTAs are
 //             done: consecutive launches overlap completely, there is no drain / ramp between them.  The wait at the end
 //             keeps the stream's completion order (a kernel finishes only after its predecessor has).  Needs: inputs AND
-//             outputs are disjoint from the inputs and outputs of every launch still in flight; at most g_chain_max - 1
+//             outputs are disjoint from the inputs and outputs of every launch still in flight; at most two
 //             such launches in a row, then a late one.
 // Orders 1 and 2 are OPT-IN (mctq_set_tuning key 3 = 2 / 3; Python: `with mct_quantizers_b200.private_stream():`): the library
 // cannot see kernels other libraries enqueue between two of its launches -- such a kernel may itself release its dependents

@@ -7,19 +7,8 @@
 
 namespace mctq {
 std::atomic<int64_t> g_launches{0};
-int g_unroll = 0;           // 0 = automatic (per-tensor tiles: 2 vectors per thread, per-channel tiles: 4)
-int g_force_rint = 0;
-int g_force_ieee_div = 0;
 int g_pdl = 1;              // 0 off, 1 programmatic dependent launch (wait first), opt-in: 2 + loads before the wait, 3 + no wait at all for launches independent of everything still in flight
-int g_lut_shfl = 1;
-int g_wide = 1;             // 8-element vectors / 256-bit stores where a kernel has them (key 5)
-int g_lut_xy = 1;           // key 7
-int g_tab_early = 1;        // key 8
 int g_nvtx = 0;             // key 9
-int g_chain_max = 3;        // key 10
-int g_host_streams = 3;     // key 11: data streams (= staging slots) of the host-buffer pipeline
-int g_host_chunk_div_deferred = 1;   // key 12: a tensor is cut into about this many chunks in deferred mode (whole slots: measured best)
-int g_multi_span = 4;       // tiles per CTA in the multi-tensor LUT launch: 1 or 4 (key 6; read when a plan is compiled)
 
 // ---- dependent-launch bookkeeping (see mctq_common.cuh): per (device, stream), the memory ranges of the library's launches
 // since -- and including -- the last one that waited for its predecessor BEFORE touching memory (a "late" launch: when its
@@ -32,7 +21,8 @@ struct ChainLaunch {
     int prepare;            // a mctq_*_prepare kernel: its output is a parameter blob
     Span in[2], out[2];
 };
-constexpr int kChainMax = 8;             // capacity; g_chain_max (key 10) of them are used: a waiting launch + launches that overlap with it, then a waiting one again
+// a waiting launch + launches that overlap with it, then a waiting one again (longer chains measured no faster: DESIGN.md §5)
+constexpr int kChainMax = 3;
 struct StreamChain {
     cudaStream_t st;
     int device;
@@ -94,14 +84,14 @@ static int plan_launch(cudaStream_t st, const IoSpan* in, int n_in, const IoSpan
                 for (int j = 0; j < c.n_in; ++j) other |= overlaps(me.out[i], c.in[j]);
             }
         }
-        if (!unknown && !raw) order = (g_pdl >= 3 && !other && slot->n < g_chain_max) ? 2 : 1;
+        if (!unknown && !raw) order = (g_pdl >= 3 && !other && slot->n < kChainMax) ? 2 : 1;
     }
     // Parameter tables (prepared blobs) are private to the library: only mctq_*_prepare writes them, and it declares the
     // blob as its output here.  Unless such a launch is still in the chain, the tables were complete before the chain's
     // first launch passed its wait, so a kernel may stage them BEFORE its own wait -- whatever other libraries enqueue
     // on the stream (they never touch a blob), hence legal in the default mode too.  "Unknown" launches (multi-tensor
     // plans) write tensors, never blobs.
-    if (tables && tab_early && g_tab_early && slot) {
+    if (tables && tab_early && slot) {
         // tables->p == nullptr: "several blobs" (multi-tensor plans) -- any prepare kernel in the chain counts
         const Span t = {reinterpret_cast<uintptr_t>(tables->p), reinterpret_cast<uintptr_t>(tables->p) + tables->bytes};
         bool fresh = false;
@@ -147,7 +137,7 @@ extern "C" {
 int mctq_abi_version(void) { return MCTQ_ABI_VERSION; }
 
 const char* mctq_build_info(void) {
-    return "libmctq_sm100 abi=1 arch=sm_100a threads=256 vec=16B unroll={auto,2,4,8} fmad=off";
+    return "libmctq_sm100 abi=1 arch=sm_100a threads=256 vec=16B fmad=off";
 }
 
 int64_t mctq_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
@@ -155,19 +145,8 @@ int64_t mctq_launch_count(void) { return g_launches.load(std::memory_order_relax
 int mctq_set_tuning(int key, int value) {
     int prev;
     switch (key) {
-        case 0: prev = g_unroll; if (value != 0 && value != 2 && value != 4 && value != 8) return MCTQ_E_BADARG; g_unroll = value; return prev;
-        case 1: prev = g_force_rint; g_force_rint = value ? 1 : 0; return prev;
-        case 2: prev = g_force_ieee_div; g_force_ieee_div = value ? 1 : 0; return prev;
         case 3: prev = g_pdl; if (value < 0 || value > 3) return MCTQ_E_BADARG; g_pdl = value; pdl_forget_streams(); return prev;
-        case 4: prev = g_lut_shfl; g_lut_shfl = value ? 1 : 0; return prev;
-        case 5: prev = g_wide; if (value < 0 || value > 2) return MCTQ_E_BADARG; g_wide = value; return prev;
-        case 7: prev = g_lut_xy; g_lut_xy = value ? 1 : 0; return prev;
-        case 11: prev = g_host_streams; if (value < 2 || value > 6) return MCTQ_E_BADARG; g_host_streams = value; return prev;
-        case 12: prev = g_host_chunk_div_deferred; if (value < 1 || value > 16) return MCTQ_E_BADARG; g_host_chunk_div_deferred = value; return prev;
-        case 10: prev = g_chain_max; if (value < 2 || value > 8) return MCTQ_E_BADARG; g_chain_max = value; pdl_forget_streams(); return prev;
         case 9: prev = g_nvtx; g_nvtx = value ? 1 : 0; return prev;
-        case 8: prev = g_tab_early; g_tab_early = value ? 1 : 0; pdl_forget_streams(); return prev;
-        case 6: prev = g_multi_span; if (value != 1 && value != 4) return MCTQ_E_BADARG; g_multi_span = value; return prev;
         default: return MCTQ_E_BADARG;
     }
 }
@@ -176,7 +155,7 @@ int mctq_set_tuning(int key, int value) {
 
 // ---------------------------------------------------------------------------------------------- host staging
 namespace {
-constexpr int kHostStreams = 6;                      // capacity; g_host_streams of them are used (key 11)
+constexpr int kHostStreams = 3;                      // data streams (= staging slots) of the pipeline (6: see pick_chunk_elems)
 constexpr size_t kHostChunkBytesIn = 32u << 20;      // largest input chunk (slot size); small tensors use smaller chunks
 constexpr size_t kParamAreaBytes = 16u << 20;        // head of the staging buffer: parameters (device side)
 // The parameter area is a ring of kRing entries so that the uploads of call i + 1 never overwrite what the kernels of
@@ -246,12 +225,12 @@ int sync_all(HostCtx* ctx) {
 // even for tensors of a few tens of MB, between 1 MB of input and the slot size, a multiple of 64 Ki elements
 // (a sixteenth was measured and is slower: 67 MB 76 -> 71 GB/s, the per-transfer latency of the copy engines dominates)
 // In deferred mode the pipeline does not drain between calls, so there is nothing to overlap WITHIN a tensor and whole
-// slots move best (divisor g_host_chunk_div_deferred, key 12, default 1): MobileNetV2 step with host tensors 87.2 GB/s with
-// eighths, 88.8 with halves, 91.6 with whole slots (6 streams instead of 3 on top: 92.2, not worth 300 MB of staging).
+// slots move best: MobileNetV2 step with host tensors 87.2 GB/s with eighths, 88.8 with halves, 91.6 with whole slots
+// (6 streams instead of 3 on top: 92.2, not worth 300 MB of staging).
 int64_t pick_chunk_elems(int64_t n, size_t in_elem_bytes, size_t slot_elem_bytes, bool deferred) {
     const int64_t max_elems = (int64_t)(kHostChunkBytesIn / slot_elem_bytes);
     const int64_t min_elems = (int64_t)((1u << 20) / in_elem_bytes);
-    const int64_t div = deferred ? g_host_chunk_div_deferred : 8;
+    const int64_t div = deferred ? 1 : 8;
     int64_t c = (n / div + 65535) / 65536 * 65536;
     if (c < min_elems) c = min_elems;
     if (c > max_elems) c = max_elems;
@@ -318,7 +297,7 @@ struct HostCall {
         int rc = 0;
         bool used[kHostStreams] = {};
         auto stream_for = [&](uint64_t k) {
-            const int i = (int)(k % (uint64_t)g_host_streams);
+            const int i = (int)(k % (uint64_t)kHostStreams);
             if (!used[i]) {
                 used[i] = true;
                 if (entry >= 0) cudaStreamWaitEvent(ctx->st[i], ctx->params_ready, 0);
@@ -362,7 +341,7 @@ extern "C" {
 
 size_t mctq_host_staging_min_bytes(void) {
     // per stream: one input chunk + one f32-sized output chunk (LUT output of a 2-byte input is 2x larger) + parameter area
-    return (size_t)g_host_streams * (kHostChunkBytesIn + 2 * kHostChunkBytesIn) + kParamAreaBytes;
+    return (size_t)kHostStreams * (kHostChunkBytesIn + 2 * kHostChunkBytesIn) + kParamAreaBytes;
 }
 
 int mctq_host_set_deferred(int device, int on) {

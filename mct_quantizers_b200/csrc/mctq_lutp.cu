@@ -717,7 +717,7 @@ namespace {
 // variant selection shared by the single-tensor and the multi-tensor entry points
 void lutp_variant(const LutPArgs& a, size_t esz, int idx_mode, int* chmode, int* v) {
     // 8-element vectors for 2-byte inputs: 16-byte aligned x, 32-byte aligned y, 8-byte aligned int8 indices, rows a multiple of 8
-    bool v8 = g_wide && esz == 2 && aligned16(a.x) && (!a.y || aligned32(a.y)) &&
+    bool v8 = esz == 2 && aligned16(a.x) && (!a.y || aligned32(a.y)) &&
               (idx_mode != MCTQ_CODES_INT8 || (reinterpret_cast<uintptr_t>(a.idx) & 7u) == 0);
     if (a.C == 1) *chmode = CH_PT;
     else if (a.inner % 4 == 0 && a.elem_offset % 4 == 0) {
@@ -773,7 +773,7 @@ int launch_lutp_tiles(const LutPArgs& a_in, cudaStream_t st) {
 constexpr uint32_t kXyMaxW = 8;
 bool lutx_eligible(const LutPArgs& a, int chmode, int v) {
     (void)v;
-    if (!g_lut_xy || a.off_xy == 0 || a.P > kXyP) return false;
+    if (a.off_xy == 0 || a.P > kXyP) return false;
     if (chmode == CH_PT) return true;
     return chmode == CH_VEC && a.W <= kXyMaxW;
 }

@@ -89,11 +89,16 @@ int launch_unpack_variant(const UnpackParams& c, cudaStream_t st) {
                             0, st, p);
 }
 
+// exactly the (mode, vector width) pairs unpack_make_args selects
 template <int KIND, typename T, int CAP>
 int launch_unpack_typed(const UnpackParams& c, cudaStream_t st) {
-    if (c.mode == 0) return c.v == 8 ? launch_unpack_variant<KIND, T, 0, 8, CAP>(c, st) : launch_unpack_variant<KIND, T, 0, 4, CAP>(c, st);
-    if (c.mode == 1) return c.v == 8 ? launch_unpack_variant<KIND, T, 1, 8, CAP>(c, st) : launch_unpack_variant<KIND, T, 1, 4, CAP>(c, st);
-    return launch_unpack_variant<KIND, T, 2, 4, CAP>(c, st);
+    constexpr int V0 = sizeof(T) == 2 ? 8 : 4;                                              // per tensor
+    constexpr bool WIDE1 = sizeof(T) == 2 || KIND == MCTQ_PACK_AFFINE_I4 || KIND == MCTQ_PACK_LUT_I4;   // per channel
+    if (c.mode == 0 && c.v == V0) return launch_unpack_variant<KIND, T, 0, V0, CAP>(c, st);
+    if (c.mode == 1 && c.v == 4) return launch_unpack_variant<KIND, T, 1, 4, CAP>(c, st);
+    if constexpr (WIDE1) if (c.mode == 1 && c.v == 8) return launch_unpack_variant<KIND, T, 1, 8, CAP>(c, st);
+    if (c.mode == 2 && c.v == 4) return launch_unpack_variant<KIND, T, 2, 4, CAP>(c, st);
+    return MCTQ_E_BADARG;
 }
 
 template <int KIND, int CAP>
@@ -151,7 +156,7 @@ int unpack_make_args(const MctqPackedDesc& d, UnpackArgs* a, int* mode, int* v, 
     // outputs (16-byte instead of 8-byte stores); for f32 where dequant_affine measured it faster, packed nibbles per channel
     const bool int4 = d.kind == MCTQ_PACK_AFFINE_I4 || d.kind == MCTQ_PACK_LUT_I4;
     const bool fits8 = *mode != 2 && (*mode == 0 || d.inner % 8 == 0) && (d.y_dtype != MCTQ_F32 || aligned32(d.y));
-    *v = fits8 && ((g_wide && (d.y_dtype != MCTQ_F32 || (*mode == 1 && int4))) || g_wide == 2) ? 8 : 4;
+    *v = fits8 && (d.y_dtype != MCTQ_F32 || (*mode == 1 && int4)) ? 8 : 4;
     return 0;
 }
 

@@ -203,7 +203,7 @@ _staging = {}
 
 def _staging_buffer(device_index):
     buf = _staging.get(device_index)
-    nbytes = _native.load().mctq_host_staging_min_bytes()        # depends on the number of pipeline streams (tuning key 11)
+    nbytes = _native.load().mctq_host_staging_min_bytes()        # three staging slots + the parameter area (304 MiB)
     if buf is None or buf.numel() < nbytes:
         buf = torch.empty(nbytes, dtype=torch.uint8, device=torch.device("cuda", device_index))
         _staging[device_index] = buf

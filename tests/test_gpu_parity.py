@@ -254,10 +254,10 @@ def test_lut_ragged_sizes(dtype, lib):
             assert G.bits_equal(y.cpu().numpy(), want), (n, C, inner, G.mismatch_report(y.cpu().numpy(), want))
 
 
-@pytest.mark.parametrize("shuffle_search", [1, 0])
-def test_lut_all_table_sizes_and_ieee_variant(shuffle_search, lib):
-    """K = 1 .. 256 centroids (every padded search depth), fast division vs the IEEE-division variant, warp-shuffle
-    search (tables of <= 32 entries) vs the shared-memory search."""
+@pytest.mark.parametrize("search", ["shuffle", "shared"])
+def test_lut_all_table_sizes_and_searches(search, lib):
+    """K = 1 .. 256 centroids (every padded search depth), values and indices: tables of <= 32 entries take the
+    warp-shuffle search, larger ones the shared-memory search."""
     from mct_quantizers_b200.pytorch.quantizer_utils import lut_search_table
     rng = np.random.default_rng(9)
     n = 50000
@@ -265,23 +265,16 @@ def test_lut_all_table_sizes_and_ieee_variant(shuffle_search, lib):
     xd = x.to(DEV)
     thr = np.array([0.9, 0.013, 2.0], dtype=np.float32)
     td = torch.from_numpy(thr).to(DEV)
-    for K in (1, 2, 3, 5, 16, 17, 64, 100, 256):
+    for K in ((1, 2, 3, 5, 16, 17) if search == "shuffle" else (64, 100, 256)):
         lut = rng.choice(np.arange(-128, 128), size=K, replace=False).astype(np.float32)   # unsorted on purpose
         table = lut_search_table(lut, 8, True).to(DEV)
         want, want_idx = oracle.fq_lut(x.numpy(), oracle.F32, lut, thr, 3, 5, 8, True, 1e-8, want_idx=True)
-        for ieee in (0, 1):
-            lib.mctq_set_tuning(2, ieee)
-            lib.mctq_set_tuning(4, shuffle_search)
-            y = torch.empty(n, dtype=torch.float32, device=DEV)
-            idx = torch.empty(n, dtype=torch.uint8, device=DEV)
-            rc = lib.mctq_fq_lut(_vp(xd), _vp(y), _vp(idx) if not ieee else None, n, 0, _vp(table), K,
-                                 _vp(td), 3, 5, 0, float(np.float32(1e-8)), 0 if ieee else 1, _stream())
-            lib.mctq_set_tuning(2, 0)
-            lib.mctq_set_tuning(4, 1)
-            assert rc == 0
-            assert G.bits_equal(y.cpu().numpy(), want), (K, ieee)
-            if not ieee:
-                assert np.array_equal(idx.cpu().numpy().astype(np.int32), want_idx)
+        y = torch.empty(n, dtype=torch.float32, device=DEV)
+        idx = torch.empty(n, dtype=torch.uint8, device=DEV)
+        rc = lib.mctq_fq_lut(_vp(xd), _vp(y), _vp(idx), n, 0, _vp(table), K, _vp(td), 3, 5, 0, float(np.float32(1e-8)), 1, _stream())
+        assert rc == 0
+        assert G.bits_equal(y.cpu().numpy(), want), K
+        assert np.array_equal(idx.cpu().numpy().astype(np.int32), want_idx), K
 
 
 def test_division_selftest(lib):
@@ -293,37 +286,21 @@ def test_division_selftest(lib):
 
 
 def test_rint_variant_and_wide_ranges(lib):
-    """16-bit and 24-bit ranges; the rint-based variant (forced, and auto-selected beyond 2^21) == oracle."""
+    """8- to 24-bit ranges == oracle.  Ranges of 2^21 codes and more take the rint-based variant: 21 and 22 bits pin the
+    switch (kFastRangeLimit) from both sides."""
     rng = np.random.default_rng(3)
     n = 70001
     x = _rand_x(rng, n, "float32", 3.0)
     xd = x.to(DEV)
-    for bits, force in ((8, 1), (16, 0), (16, 1), (24, 0)):
+    for bits in (8, 16, 21, 22, 24):
         qmin, qmax = -(2 ** (bits - 1)), 2 ** (bits - 1) - 1
         scale = np.array([8.0 / 2 ** (bits - 1)], dtype=np.float32)
         zp = np.zeros(1, np.int32)
-        lib.mctq_set_tuning(1, force)
         y = torch.empty_like(xd)
         rc = lib.mctq_fq_affine_scalar(_vp(xd), _vp(y), None, n, 0, float(scale[0]), 0, qmin, qmax, 0, _stream())
-        lib.mctq_set_tuning(1, 0)
         assert rc == 0
         want = oracle.fq_affine(x.numpy(), 0, scale, zp, 1, 1, qmin, qmax)
-        assert G.bits_equal(y.cpu().numpy(), want), (bits, force)
-
-
-def test_unroll_variants_agree(lib):
-    rng = np.random.default_rng(4)
-    n = 1 << 20
-    for dtype in ("float32", "bfloat16"):
-        x = _rand_x(rng, n + 13, dtype, 2.0).to(DEV)
-        outs = []
-        for u in (2, 4, 8):
-            lib.mctq_set_tuning(0, u)
-            y = torch.empty_like(x)
-            assert lib.mctq_fq_affine_scalar(_vp(x), _vp(y), None, x.numel(), G.DT_TAG[dtype], 0.03125, 0, -128, 127, 0, _stream()) == 0
-            outs.append(y)
-        lib.mctq_set_tuning(0, 0)
-        assert torch.equal(outs[0], outs[1]) and torch.equal(outs[1], outs[2])
+        assert G.bits_equal(y.cpu().numpy(), want), bits
 
 
 def test_dequant_roundtrip(lib):
@@ -348,40 +325,60 @@ def test_dequant_roundtrip(lib):
         assert torch.equal(codes, codes2)
 
 
-@pytest.mark.parametrize("wide", [0, 1, 2])
-def test_dequant_vector_variants(wide, lib):
+def _dequant_vec_widths(fn):
+    """Vector widths (template argument V) of the dequant_affine_vec_kernel launches fn() makes, from the profiler."""
+    import re
+    from torch.profiler import profile, ProfilerActivity
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    widths = set()
+    for e in prof.key_averages():
+        m = (re.search(r"dequant_affine_vec_kernel<\s*\d+\s*,\s*\d+\s*,\s*(\d+)\s*>", e.key)
+             or re.search(r"dequant_affine_vec_kernelILi\d+ELi\d+ELi(\d+)E", e.key))
+        if m:
+            widths.add(int(m.group(1)))
+    return widths
+
+
+@pytest.mark.parametrize("bits,signed", [(8, True), (8, False), (4, True), (4, False)])
+def test_dequant_vector_variants(bits, signed, lib):
     """The streaming dequant kernel in every (code mode, channel mode, vector width) combination, ragged sizes included:
-    per-tensor, rows that are multiples of 8 / 4, odd rows; 4-code vectors (key 5 = 0), the default mix (1) and 8-code
-    vectors with 256-bit stores everywhere (2).  codes -> dequant == fake-quant values bit for bit."""
-    rng = np.random.default_rng(77 + wide)
-    prev = lib.mctq_set_tuning(5, wide)
-    try:
-        for (C, inner, outer, tail) in ((1, 1, 70001, 0), (13, 64, 37, 0), (7, 12, 211, 0), (5, 9, 333, 0), (3, 4096, 3, 0), (6, 8, 1000, 5),
-                                     (11, 3, 500, 0), (4, 1, 1000, 0), (3, 5, 2001, 2), (9, 4097, 2, 0)):
-            n_full = C * inner * outer
-            n = n_full - tail                                     # a flat prefix (ragged last vector)
-            x = _rand_x(rng, n, "float32", 1.0).to(DEV)
-            for bits, signed, mode in ((8, True, 1), (8, False, 1), (4, True, 2), (4, False, 2)):
-                qmin, qmax = (-(2 ** (bits - 1)), 2 ** (bits - 1) - 1) if signed else (0, 2 ** bits - 1)
-                scale = torch.from_numpy((np.abs(rng.standard_normal(C)) * 0.1 + 0.01).astype(np.float32)).to(DEV)
-                zp = torch.from_numpy((np.zeros(C) if signed else rng.integers(0, qmax + 1, size=C)).astype(np.int32)).to(DEV)
-                y = torch.empty_like(x)
-                codes = torch.empty(n if mode == 1 else (n + 1) // 2, dtype=torch.uint8, device=DEV)
-                assert lib.mctq_fq_affine(_vp(x), _vp(y), _vp(codes), n, 0, _vp(scale), _vp(zp), C, inner, 0, qmin, qmax, mode, _stream()) == 0
-                back = torch.full((n + 16,), 7.0, device=DEV)
-                assert lib.mctq_dequant_affine(_vp(codes), mode, int(signed), _vp(back), n, _vp(scale), _vp(zp), C, inner, 0, _stream()) == 0
-                assert torch.equal(back[:n].view(torch.int32), y.view(torch.int32)), (wide, C, inner, bits, signed)
-                assert (back[n:] == 7.0).all()
-    finally:
-        lib.mctq_set_tuning(5, prev)
+    per-tensor, rows that are multiples of 8 / 4, odd rows.  Per-channel int4 rows of 8 take 8-code vectors with 256-bit
+    stores, everything else 4-code vectors; the shapes reach both.  codes -> dequant == fake-quant values bit for bit."""
+    rng = np.random.default_rng(77 + bits + int(signed))
+    mode = 1 if bits == 8 else 2
+    qmin, qmax = (-(2 ** (bits - 1)), 2 ** (bits - 1) - 1) if signed else (0, 2 ** bits - 1)
+    launches = []
+    for (C, inner, outer, tail) in ((1, 1, 70001, 0), (13, 64, 37, 0), (7, 12, 211, 0), (5, 9, 333, 0), (3, 4096, 3, 0), (6, 8, 1000, 5),
+                                 (11, 3, 500, 0), (4, 1, 1000, 0), (3, 5, 2001, 2), (9, 4097, 2, 0)):
+        n_full = C * inner * outer
+        n = n_full - tail                                     # a flat prefix (ragged last vector)
+        x = _rand_x(rng, n, "float32", 1.0).to(DEV)
+        scale = torch.from_numpy((np.abs(rng.standard_normal(C)) * 0.1 + 0.01).astype(np.float32)).to(DEV)
+        zp = torch.from_numpy((np.zeros(C) if signed else rng.integers(0, qmax + 1, size=C)).astype(np.int32)).to(DEV)
+        y = torch.empty_like(x)
+        codes = torch.empty(n if mode == 1 else (n + 1) // 2, dtype=torch.uint8, device=DEV)
+        assert lib.mctq_fq_affine(_vp(x), _vp(y), _vp(codes), n, 0, _vp(scale), _vp(zp), C, inner, 0, qmin, qmax, mode, _stream()) == 0
+        back = torch.full((n + 16,), 7.0, device=DEV)
+        launches.append(lambda codes=codes, back=back, n=n, scale=scale, zp=zp, C=C, inner=inner:
+                        lib.mctq_dequant_affine(_vp(codes), mode, int(signed), _vp(back), n, _vp(scale), _vp(zp), C, inner, 0, _stream()))
+        assert launches[-1]() == 0
+        assert torch.equal(back[:n].view(torch.int32), y.view(torch.int32)), (C, inner)
+        assert (back[n:] == 7.0).all()
+    assert _dequant_vec_widths(lambda: [f() for f in launches]) == ({4, 8} if bits == 4 else {4})
 
 
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16])
 def test_prepared_lut_wide_vectors_match_narrow(dtype, Q, lib):
-    """2-byte inputs: the 8-element / 256-bit-store variant of the prepared LUT kernel == the 4-element variant == the
-    oracle, values and indices (int8, packed int4), ragged tails, per-channel and per-tensor."""
+    """2-byte inputs: the 8-element / 256-bit-store variant of the prepared LUT kernel == the 4-element variant (taken for
+    an output 16 bytes past a 32-byte boundary) == the oracle, values and indices (int8, packed int4), ragged tails,
+    per-channel and per-tensor."""
+    from mct_quantizers_b200.pytorch.quantizer_utils import lut_search_table
     rng = np.random.default_rng(5)
     lut = [float(v) for v in sorted(rng.choice(np.arange(-128, 128), size=16, replace=False))]
+    table = lut_search_table(np.asarray(lut, np.float32), 8, True)
+    tag = 1 if dtype == torch.bfloat16 else 2
     for shape, per_channel in (((37, 264), True), ((3, 8200), True), ((70003,), False)):
         x = torch.from_numpy((rng.standard_normal(shape) * 0.03).astype(np.float32)).to(dtype).to(DEV)
         if per_channel:
@@ -390,24 +387,27 @@ def test_prepared_lut_wide_vectors_match_narrow(dtype, Q, lib):
         else:
             thr = [0.11]
             q = Q.WeightsLUTSymmetricInferableQuantizer(4, lut, thr, False)
-        from mct_quantizers_b200.pytorch.quantizer_utils import lut_search_table
-        table = lut_search_table(np.asarray(lut, np.float32), 8, True)
         thr_t = torch.tensor(thr, dtype=torch.float32, device=DEV)
-        outs = []
-        for wide in (0, 1):
-            prev = lib.mctq_set_tuning(5, wide)
-            try:
-                y = q(x.clone())
-                i8 = torch.ops.mctq.lut_indices(x, table, 16, thr_t, per_channel, 0, 1e-8, 1)
-                i4 = torch.ops.mctq.lut_indices(x, table, 16, thr_t, per_channel, 0, 1e-8, 2)
-                torch.cuda.synchronize()
-            finally:
-                lib.mctq_set_tuning(5, prev)
-            outs.append((y, i8, i4))
+        n = x.numel()
+        C, inner = (shape[0], shape[1]) if per_channel else (1, 1)
+        wide = (q(x.clone()), torch.ops.mctq.lut_indices(x, table, 16, thr_t, per_channel, 0, 1e-8, 1),
+                torch.ops.mctq.lut_indices(x, table, 16, thr_t, per_channel, 0, 1e-8, 2))
+        nb = lib.mctq_lut_prepared_bytes(16, 8, 1, C)
+        blob = torch.empty(nb, dtype=torch.uint8, device=DEV)
+        assert lib.mctq_lut_prepare(_vp(table), 16, _vp(thr_t), C, float(np.float32(1e-8)), 0, 1.0, 1.0, 0, _vp(blob), nb, _stream()) == 0
+        narrow = []
+        for idx_mode in (1, 2):
+            y = torch.empty(n + 8, dtype=torch.float32, device=DEV)[4:4 + n]
+            assert y.data_ptr() % 32 == 16
+            idx = torch.empty(n if idx_mode == 1 else (n + 1) // 2, dtype=torch.uint8, device=DEV)
+            assert lib.mctq_fq_lut_prepared(_vp(x), _vp(y), _vp(idx), n, tag, _vp(blob), 16, 8, 1, C, inner, 0, idx_mode, _stream()) == 0
+            narrow.append((y.reshape(shape), idx))
+        torch.cuda.synchronize()
+        assert torch.equal(narrow[0][0], narrow[1][0])
+        outs = [wide, (narrow[0][0], narrow[0][1].reshape(shape), narrow[1][1])]
         for a, b in zip(outs[0], outs[1]):
             assert torch.equal(a, b)
         xb = x.cpu().contiguous().view(torch.int16).numpy().view(np.uint16)
-        C, inner = (shape[0], shape[1]) if per_channel else (1, 1)
         want, want_idx = oracle.fq_lut(xb, oracle.BF16 if dtype == torch.bfloat16 else oracle.F16, np.asarray(lut, np.float32),
                                        np.asarray(thr, np.float64).astype(np.float32), C, inner, 8, True, 1e-8, want_idx=True)
         assert np.array_equal(outs[1][0].cpu().numpy().view(np.uint32), np.asarray(want).reshape(shape).view(np.uint32))

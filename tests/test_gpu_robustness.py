@@ -343,7 +343,7 @@ def test_activation_quantizers_cut_the_autograd_graph_like_the_reference(Q):
 @pytest.mark.parametrize("pdl_mode", [1, 2, 3])
 def test_tables_staged_before_the_wait_never_see_a_blob_being_prepared(Q, pdl_mode):
     """Kernels stage their prepared parameter tables BEFORE the dependent-launch wait unless the blob was written by a
-    prepare call still in flight on the stream (mctq_set_tuning key 8).  Worst case for that rule: a long launch keeps
+    prepare call still in flight on the stream (mctq_host.cu, plan_launch).  Worst case for that rule: a long launch keeps
     the GPU busy, a NEW quantizer is prepared (the allocator tends to hand out the address of the blob freed one
     iteration earlier) and used at once -- a kernel that read the blob too early would see the previous iteration's
     thresholds."""

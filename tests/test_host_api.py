@@ -273,6 +273,24 @@ def test_shared_library_exports_every_declared_symbol():
     assert os.path.getsize(_native.LIB_PATH) > 100000
 
 
+def test_tuning_keys_and_staging_size():
+    """mctq_set_tuning keeps key 3 (dependent-launch order) and key 9 (NVTX ranges) and rejects every other key; the
+    host-buffer staging size is fixed: three slots of a 32 MiB input and a 64 MiB output chunk, plus 16 MiB of parameters."""
+    lib = _native.load()
+    for key in (-1, 0, 1, 2, 4, 5, 6, 7, 8, 10, 11, 12, 13):
+        for value in (0, 1, 2, 3):
+            assert lib.mctq_set_tuning(key, value) == -1, (key, value)          # MCTQ_E_BADARG
+    prev = lib.mctq_set_tuning(3, 2)
+    assert prev in (0, 1, 2, 3)
+    assert lib.mctq_set_tuning(3, 3) == 2
+    assert lib.mctq_set_tuning(3, 4) == -1
+    assert lib.mctq_set_tuning(3, prev) == 3
+    prev = lib.mctq_set_tuning(9, 1)
+    assert prev in (0, 1)
+    assert lib.mctq_set_tuning(9, prev) == 1
+    assert lib.mctq_host_staging_min_bytes() == 3 * (32 + 64) * 2 ** 20 + 16 * 2 ** 20
+
+
 def test_multi_plan_host_helper():
     lib = _native.load()
     descs = (_native.MctqTensorDesc * 3)()

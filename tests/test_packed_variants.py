@@ -28,7 +28,6 @@ DT = {torch.float32: _native.F32, torch.bfloat16: _native.BF16, torch.float16: _
 KIND_DTYPES = [(k, dt) for k in (I8, I4) for dt in (torch.float32, torch.bfloat16, torch.float16)] + [(k, torch.float32) for k in LUT_KINDS]
 U_OUT = {torch.float32: 2.0 ** -24, torch.bfloat16: 2.0 ** -8, torch.float16: 2.0 ** -11}
 HALF_SUBNORMAL = {torch.float32: 2.0 ** -150, torch.bfloat16: 2.0 ** -134, torch.float16: 2.0 ** -25}
-KEY_WIDE = 5                      # mctq_set_tuning key: vector width of the unpack kernels (0: 4 elements, 1: default, 2: 8)
 
 
 # --------------------------------------------------------------------------------------------- reference decoder
@@ -185,7 +184,7 @@ def _kind_k(kind, i):
 
 
 def coverage_plans():
-    """Plans (lists of Spec) that together launch every (variant, argument capacity) pair under each key-5 setting: per
+    """Plans (lists of Spec) that together launch every (variant, argument capacity) pair: per
     layout a plan with <= 4 tensors per variant, and one plan with all layouts (> 4 tensors per variant), tile counts
     from 1 to 19 in one variant (a launch holds tensors within 16x of its largest), and more than 64 tensors of one variant.  f32 outputs alternate between
     32-byte and 16-byte (not 32-byte) aligned starts."""
@@ -233,29 +232,18 @@ def _plan_variants(blob, nbytes):
 
 
 def _all_variant_pairs():
+    """The (kind, out dtype, mode, V, capacity) launches that mctq_unpack.cu instantiates, no more and no fewer: per tensor
+    (mode 0) 4-element vectors for f32 and 8 for 2-byte outputs; rows of a multiple of 4 (mode 1) 4, and 8 for 2-byte
+    outputs and f32 int4 codes; other rows (mode 2) 4."""
     want = set()
     for kind, dtype in KIND_DTYPES:
-        for mode, v in ((0, 4), (0, 8), (1, 4), (1, 8), (2, 4)):
+        two_byte = dtype != torch.float32
+        modes = [(0, 8 if two_byte else 4), (1, 4), (2, 4)] + ([(1, 8)] if two_byte or kind in INT4_KINDS else [])
+        for mode, v in modes:
             for cap in (4, 64):
                 want.add((kind, DT[dtype], mode, v, cap))
-    assert len(want) == 80
+    assert len(want) == 60
     return want
-
-
-class _wide:
-    """mctq_set_tuning(5, value) for the block; the plan reads it when it is built."""
-
-    def __init__(self, value):
-        self.value = value
-
-    def __enter__(self):
-        self.prev = _native.load().mctq_set_tuning(KEY_WIDE, self.value)
-        assert self.prev >= 0
-        return self
-
-    def __exit__(self, *exc):
-        _native.load().mctq_set_tuning(KEY_WIDE, self.prev)
-        return False
 
 
 def _fake_descs(specs):
@@ -272,33 +260,30 @@ def _fake_descs(specs):
 
 
 def test_unpack_variant_selection_covers_every_kernel():
-    """Host half of the coverage check (no GPU): the plans of coverage_plans(), compiled under key 5 = 0, 1, 2 from
-    descriptors with fake device pointers, launch all 80 (variant, capacity) pairs; a 16-byte but not 32-byte aligned f32
-    output never takes 8-element vectors."""
+    """Host half of the coverage check (no GPU): the plans of coverage_plans(), compiled from descriptors with fake device
+    pointers, launch exactly the 60 (variant, capacity) pairs the library instantiates; a 16-byte but not 32-byte aligned
+    f32 output never takes 8-element vectors."""
     lib = _native.load()
+
+    def plan_variants(specs):
+        ds = _fake_descs(specs)
+        arr = (_native.MctqPackedDesc * len(ds))(*ds)
+        p = ctypes.cast(arr, ctypes.c_void_p)
+        nb = lib.mctq_unpack_plan_bytes(p, len(ds))
+        assert nb > 0
+        buf = (ctypes.c_uint8 * nb)()
+        assert lib.mctq_unpack_plan(p, len(ds), ctypes.cast(buf, ctypes.c_void_p), nb) > 0
+        return _plan_variants(buf, nb)
+
     seen = set()
-    for wide in (0, 1, 2):
-        with _wide(wide):
-            for specs in coverage_plans():
-                ds = _fake_descs(specs)
-                arr = (_native.MctqPackedDesc * len(ds))(*ds)
-                p = ctypes.cast(arr, ctypes.c_void_p)
-                nb = lib.mctq_unpack_plan_bytes(p, len(ds))
-                assert nb > 0
-                buf = (ctypes.c_uint8 * nb)()
-                assert lib.mctq_unpack_plan(p, len(ds), ctypes.cast(buf, ctypes.c_void_p), nb) > 0
-                seen |= set(_plan_variants(buf, nb))
-            # a misaligned f32 output alone: 4-element vectors even when 8 are forced
-            mis = [Spec(k, torch.float32, C, inner, 8200, True) for k in (I8, LI4) for C, inner in ((1, 1), (5, 8))]
-            ds = _fake_descs(mis)
-            arr = (_native.MctqPackedDesc * len(ds))(*ds)
-            p = ctypes.cast(arr, ctypes.c_void_p)
-            nb = lib.mctq_unpack_plan_bytes(p, len(ds))
-            buf = (ctypes.c_uint8 * nb)()
-            assert lib.mctq_unpack_plan(p, len(ds), ctypes.cast(buf, ctypes.c_void_p), nb) > 0
-            assert all(v == 4 for _, _, _, v, _ in _plan_variants(buf, nb))
-    missing = _all_variant_pairs() - seen
-    assert not missing, sorted(missing)
+    for specs in coverage_plans():
+        seen |= set(plan_variants(specs))
+    # a misaligned f32 output alone: 4-element vectors, also for per-channel int4 rows of 8
+    mis = plan_variants([Spec(k, torch.float32, C, inner, 8200, True) for k in (I8, LI4) for C, inner in ((1, 1), (5, 8))])
+    assert all(v == 4 for _, _, _, v, _ in mis)
+    seen |= set(mis)
+    want = _all_variant_pairs()
+    assert seen == want, (sorted(want - seen), sorted(seen - want))
 
 
 def _unpack_data(spec, rng, idx):
@@ -376,26 +361,24 @@ def _run_guarded_unpack(specs, rng):
 
 @pytest.mark.gpu
 def test_unpack_every_variant_against_the_decoder():
-    """All 40 kernel variants, each launched with <= 4 and with > 4 tensors, at every size class and channel layout, with
-    outputs in guarded views; the launched (variant, capacity) pairs are read from the plan blobs and all 80 must occur."""
+    """All 30 kernel variants, each launched with <= 4 and with > 4 tensors, at every size class and channel layout, with
+    outputs in guarded views; the launched (variant, capacity) pairs are read from the plan blobs and must be exactly the
+    60 the library instantiates."""
     rng = np.random.default_rng(2024)
-    seen = {}
-    for wide in (0, 1, 2):
-        with _wide(wide):
-            for specs in coverage_plans():
-                for pair in _run_guarded_unpack(specs, rng):
-                    seen.setdefault(pair, wide)
+    seen = set()
+    for specs in coverage_plans():
+        seen |= set(_run_guarded_unpack(specs, rng))
     names = {I8: "affine_i8", I4: "affine_i4", LU8: "lut_u8", LI4: "lut_i4"}
     dnames = {0: "f32", 1: "bf16", 2: "f16"}
-    print("\nlaunched unpack variants (kind, out, mode, V, capacity; key 5 of the first launch):")
+    print("\nlaunched unpack variants (kind, out, mode, V, capacity):")
     for kind, dt, mode, v, cap in sorted(seen):
-        print(f"  {names[kind]:9s} {dnames[dt]:4s} mode {mode} V={v} cap {cap:2d}  (key 5 = {seen[(kind, dt, mode, v, cap)]})")
-    missing = _all_variant_pairs() - set(seen)
-    assert not missing, sorted(missing)
+        print(f"  {names[kind]:9s} {dnames[dt]:4s} mode {mode} V={v} cap {cap:2d}")
+    want = _all_variant_pairs()
+    assert seen == want, (sorted(want - seen), sorted(seen - want))
 
 
 # --------------------------------------------------------------------------------------------- B: beyond 2^31 elements
-def _big_unpack(kind, C, inner, n, wide):
+def _big_unpack(kind, C, inner, n):
     g = torch.Generator(device="cuda").manual_seed(n % 1000)
     nb = (n + 1) // 2
     codes = torch.randint(0, 256, (nb,), dtype=torch.uint8, device="cuda", generator=g)
@@ -403,8 +386,7 @@ def _big_unpack(kind, C, inner, n, wide):
     scale = (rng.uniform(0.5, 2.0, C) * 2.0 ** -3).astype(np.float32)
     zp = np.arange(-3, -3 + C, dtype=np.int32)
     item = (codes, kind, True, torch.bfloat16, (n,), None, C, inner, torch.from_numpy(scale).cuda(), torch.from_numpy(zp).cuda(), None)
-    with _wide(wide):
-        plan = ops.UnpackPlan([item])
+    plan = ops.UnpackPlan([item])
     y = plan.run()[0]
     torch.cuda.synchronize()
     windows = [(0, 4096), ((1 << 31) - 5000, 10001), (n - 6001, 6001)]
@@ -423,8 +405,8 @@ def _big_unpack(kind, C, inner, n, wide):
 def test_unpack_beyond_2_31_elements():
     """int4 per-channel weights of more than 2^31 elements take the 64-bit channel walk: any row length (inner 3, odd n)
     and rows of a multiple of 8, bf16 out; windows at the start, around element 2^31 and at the end."""
-    _big_unpack(I4, 7, 3, 21 * 102261127, 1)                       # 2147483667 elements, mode 2
-    _big_unpack(I4, 5, 8, 40 * 53687092, 1)                        # 2147483680 elements, mode 1, 8-element vectors
+    _big_unpack(I4, 7, 3, 21 * 102261127)                          # 2147483667 elements, mode 2
+    _big_unpack(I4, 5, 8, 40 * 53687092)                           # 2147483680 elements, mode 1, 8-element vectors
 
 
 # --------------------------------------------------------------------------------------------- C: packed linear

@@ -2,7 +2,7 @@
 """Kernel micro-benchmark (GPU box): achieved algorithmic GB/s of each kernel family through the raw C ABI.
 CUDA events on the launch stream, buffers rotated so that nothing is L2-resident, median of reps.
 
-    python tools/kbench.py [--mb 1024] [--reps 20] [--what affine,lut,codes] [--unroll 2,4,8]
+    python tools/kbench.py [--mb 1024] [--reps 20] [--what affine,lut,codes]
 """
 import argparse
 import ctypes
@@ -59,10 +59,9 @@ def main():
     ap.add_argument("--mb", type=float, default=1024.0, help="input megabytes per launch")
     ap.add_argument("--reps", type=int, default=20)
     ap.add_argument("--what", default="affine,channel,fused,codes,lut,copy")
-    ap.add_argument("--unroll", default="0", help="0 = the library default (automatic)")
     ap.add_argument("--dtypes", default="f32,bf16")
     ap.add_argument("--json", default=None)
-    ap.add_argument("--tune", default="", help="comma separated key=value pairs for mctq_set_tuning (experiments)")
+    ap.add_argument("--tune", default="", help="comma separated key=value pairs for mctq_set_tuning (keys 3, 9)")
     args = ap.parse_args()
     lib = _native.load()
     for kv in filter(None, args.tune.split(",")):
@@ -97,34 +96,30 @@ def main():
         if "copy" in what:
             med, best = timeit(lambda i: ys[i].copy_(xs[i]), args.reps, nbuf)
             report("torch copy_ (reference point)", dt, 2 * n * es, med, best)
-        for u in [int(v) for v in args.unroll.split(",")]:
-            lib.mctq_set_tuning(0, u)
-            if "affine" in what:
-                med, best = timeit(lambda i: lib.mctq_fq_affine_scalar(vp(xs[i]), vp(ys[i]), None, n, tag, 0.03125, 0, -128, 127, 0, stream()),
+        if "affine" in what:
+            med, best = timeit(lambda i: lib.mctq_fq_affine_scalar(vp(xs[i]), vp(ys[i]), None, n, tag, 0.03125, 0, -128, 127, 0, stream()),
+                               args.reps, nbuf)
+            report("affine per-tensor scalar", dt, 2 * n * es, med, best)
+            med, best = timeit(lambda i: lib.mctq_fq_affine_scalar(vp(xs[i]), vp(ys[i]), None, n, tag, 0.0129, 77, 0, 255, 0, stream()),
+                               args.reps, nbuf)
+            report("affine per-tensor uniform zp", dt, 2 * n * es, med, best)
+        if "channel" in what:
+            for (C, inner, label) in ((4096, 11008, "rows 11008"), (11008, 4096, "rows 4096"), (512, 4608, "conv 512x512x3x3"),
+                                      (960, 9, "depthwise inner 9"), (1024, 64, "rows 64"), (256, 16, "convT 4x4 inner 16"),
+                                      (768, 1, "channel-last C=768"), (3, 1, "channel-last C=3")):
+                sc = torch.rand(C, device=dev) * 0.05 + 0.01
+                zp = torch.zeros(C, dtype=torch.int32, device=dev)
+                med, best = timeit(lambda i: lib.mctq_fq_affine(vp(xs[i]), vp(ys[i]), None, n, tag, vp(sc), vp(zp), C, inner, 0, -128, 127, 0, stream()),
                                    args.reps, nbuf)
-                report(f"affine per-tensor scalar u{u}", dt, 2 * n * es, med, best)
-                med, best = timeit(lambda i: lib.mctq_fq_affine_scalar(vp(xs[i]), vp(ys[i]), None, n, tag, 0.0129, 77, 0, 255, 0, stream()),
-                                   args.reps, nbuf)
-                report(f"affine per-tensor uniform zp u{u}", dt, 2 * n * es, med, best)
-            if "channel" in what:
-                for (C, inner, label) in ((4096, 11008, "rows 11008"), (11008, 4096, "rows 4096"), (512, 4608, "conv 512x512x3x3"),
-                                          (960, 9, "depthwise inner 9"), (1024, 64, "rows 64"), (256, 16, "convT 4x4 inner 16"),
-                                          (768, 1, "channel-last C=768"), (3, 1, "channel-last C=3")):
-                    sc = torch.rand(C, device=dev) * 0.05 + 0.01
-                    zp = torch.zeros(C, dtype=torch.int32, device=dev)
-                    med, best = timeit(lambda i: lib.mctq_fq_affine(vp(xs[i]), vp(ys[i]), None, n, tag, vp(sc), vp(zp), C, inner, 0, -128, 127, 0, stream()),
-                                       args.reps, nbuf)
-                    report(f"affine per-channel {label} u{u}", dt, 2 * n * es, med, best)
-                    if u in (0, 4):
-                        nb = lib.mctq_affine_prepared_bytes(C)
-                        blob = torch.empty(nb, dtype=torch.uint8, device=dev)
-                        assert lib.mctq_affine_prepare(vp(sc), vp(zp), C, vp(blob), nb, stream()) == 0
-                        torch.cuda.synchronize()
-                        fn = lambda i: lib.mctq_fq_affine_prepared(vp(xs[i]), vp(ys[i]), None, n, tag, vp(blob), C, inner, 0, -128, 127, 0, stream())
-                        assert fn(0) == 0
-                        med, best = timeit(fn, args.reps, nbuf)
-                        report(f"affine-prepared per-channel {label}", dt, 2 * n * es, med, best)
-        lib.mctq_set_tuning(0, 0)
+                report(f"affine per-channel {label}", dt, 2 * n * es, med, best)
+                nb = lib.mctq_affine_prepared_bytes(C)
+                blob = torch.empty(nb, dtype=torch.uint8, device=dev)
+                assert lib.mctq_affine_prepare(vp(sc), vp(zp), C, vp(blob), nb, stream()) == 0
+                torch.cuda.synchronize()
+                fn = lambda i: lib.mctq_fq_affine_prepared(vp(xs[i]), vp(ys[i]), None, n, tag, vp(blob), C, inner, 0, -128, 127, 0, stream())
+                assert fn(0) == 0
+                med, best = timeit(fn, args.reps, nbuf)
+                report(f"affine-prepared per-channel {label}", dt, 2 * n * es, med, best)
         if "fused" in what:
             for pre, label, streams in ((1, "relu", 2), (2, "relu6", 2), (3, "add", 3), (4, "add+relu", 3)):
                 fn = lambda i: lib.mctq_fq_affine_scalar_pre(vp(xs[i]), vp(xs[(i + 1) % nbuf]), vp(ys[i]), n, tag, pre, 0.0129, 77, 0, 255, stream())
@@ -158,17 +153,14 @@ def main():
             table = lut_search_table(lut, 8, True).to(dev)
             for x in xs:
                 x.normal_(0, 0.02)
-            for u in [int(v) for v in args.unroll.split(",") if int(v) in (0, 4, 8)] or [0]:
-                lib.mctq_set_tuning(0, u)
-                for (C, inner, label) in ((4096, 11008, "rows 11008"), (11008, 4096, "rows 4096"), (1, 1, "per-tensor")):
-                    thr = torch.rand(C, device=dev) * 0.05 + 0.06
-                    med, best = timeit(lambda i: lib.mctq_fq_lut(vp(xs[i]), vp(yf[i]), None, n, tag, vp(table), 16, vp(thr), C, inner, 0,
-                                                                 1e-8, 0, stream()), args.reps, nbuf)
-                    report(f"lut K=16 weights {label} u{u}", dt, n * (es + 4), med, best)
-                med, best = timeit(lambda i: lib.mctq_fq_lut_scalar(vp(xs[i]), vp(yf[i]), None, n, tag, vp(table), 16, 0.125, 0.125, int(es == 2), 0, stream()),
-                                   args.reps, nbuf)
-                report(f"lut K=16 activation scalar u{u}", dt, n * (es + 4), med, best)
-            lib.mctq_set_tuning(0, 0)
+            for (C, inner, label) in ((4096, 11008, "rows 11008"), (11008, 4096, "rows 4096"), (1, 1, "per-tensor")):
+                thr = torch.rand(C, device=dev) * 0.05 + 0.06
+                med, best = timeit(lambda i: lib.mctq_fq_lut(vp(xs[i]), vp(yf[i]), None, n, tag, vp(table), 16, vp(thr), C, inner, 0,
+                                                             1e-8, 0, stream()), args.reps, nbuf)
+                report(f"lut K=16 weights {label}", dt, n * (es + 4), med, best)
+            med, best = timeit(lambda i: lib.mctq_fq_lut_scalar(vp(xs[i]), vp(yf[i]), None, n, tag, vp(table), 16, 0.125, 0.125, int(es == 2), 0, stream()),
+                               args.reps, nbuf)
+            report("lut K=16 activation scalar", dt, n * (es + 4), med, best)
             # prepared path: per-channel decision tables in the x domain (built once, outside the timed region)
             table_host = lut_search_table(lut, 8, True)
             for (C, inner, label) in ((4096, 11008, "rows 11008"), (11008, 4096, "rows 4096"), (1, 1, "per-tensor"), (65536, 64, "rows 64")):
@@ -184,18 +176,6 @@ def main():
                     assert fn(0) == 0
                     med, best = timeit(fn, args.reps, nbuf)
                     report(f"lut-prepared K=16 weights {label}{lab}", dt, n * (es + 4 + (0.5 if mode else 0)), med, best)
-            lib.mctq_set_tuning(4, 0)
-            thr = torch.rand(4096, device=dev) * 0.05 + 0.06
-            med, best = timeit(lambda i: lib.mctq_fq_lut(vp(xs[i]), vp(yf[i]), None, n, tag, vp(table), 16, vp(thr), 4096, 11008, 0, 1e-8, 0, stream()),
-                               args.reps, nbuf)
-            report("lut K=16 weights rows 11008 shared-memory search (no shuffles)", dt, n * (es + 4), med, best)
-            lib.mctq_set_tuning(4, 1)
-            lib.mctq_set_tuning(2, 1)
-            thr = torch.rand(4096, device=dev) * 0.05 + 0.06
-            med, best = timeit(lambda i: lib.mctq_fq_lut(vp(xs[i]), vp(yf[i]), None, n, tag, vp(table), 16, vp(thr), 4096, 11008, 0, 1e-8, 0, stream()),
-                               args.reps, nbuf)
-            report("lut K=16 weights rows 11008 IEEE-div variant", dt, n * (es + 4), med, best)
-            lib.mctq_set_tuning(2, 0)
             del yf
         del xs
         torch.cuda.empty_cache()
