@@ -15,6 +15,14 @@ F32, BF16, F16 = 0, 1, 2
 CODES_NONE, CODES_INT8, CODES_INT4 = 0, 1, 2
 PRE_RELU, PRE_RELU6, PRE_ADD, PRE_ADD_RELU = 1, 2, 3, 4
 PACK_AFFINE_I8, PACK_AFFINE_I4, PACK_LUT_U8, PACK_LUT_I4 = 1, 2, 3, 4
+PACK_LUT_KINDS = (PACK_LUT_U8, PACK_LUT_I4)
+
+
+def packed_code_bytes(kind, n):
+    """Bytes of the codes of n elements of packed kind `kind`: one per element, or one per two for int4 codes and 4-bit
+    LUT indices."""
+    return n if kind in (PACK_AFFINE_I8, PACK_LUT_U8) else (n + 1) // 2
+
 
 _lock = threading.Lock()
 _lib = None

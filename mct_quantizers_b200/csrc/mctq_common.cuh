@@ -16,6 +16,7 @@
 #include <string.h>
 
 #include <atomic>
+#include <type_traits>
 #include <utility>
 
 #include "mctq.h"
@@ -351,6 +352,13 @@ struct LutCodeOp {
     __device__ __forceinline__ float value(int q, float t) const { return __fmul_rn(level(q), t); }
 };
 
+// facts of a packed-weight kind (MCTQ_PACK_*, include/mctq.h): which op decodes it, its code width, and for the LUT kinds
+// the table size its indices can address (the largest K)
+__host__ __device__ constexpr bool pack_is_lut(int kind) { return kind == MCTQ_PACK_LUT_U8 || kind == MCTQ_PACK_LUT_I4; }
+__host__ __device__ constexpr bool pack_is_int4(int kind) { return kind == MCTQ_PACK_AFFINE_I4 || kind == MCTQ_PACK_LUT_I4; }
+__host__ __device__ constexpr int pack_code_mode(int kind) { return pack_is_int4(kind) ? MCTQ_CODES_INT4 : MCTQ_CODES_INT8; }
+__host__ __device__ constexpr int pack_max_k(int kind) { return pack_is_int4(kind) ? 16 : 256; }
+
 // ------------------------------------------------------------------------------------------ channel window
 // A tile covers logical elements [g0, g0 + tile) of the [outer][C][inner] view.  It touches rows
 // r0 .. r0 + nr - 1 (row = g / inner, channel = row % C).  Slot jj of the window holds channel (r0 + jj) % C,
@@ -531,6 +539,62 @@ int ensure_smem(K kernel, size_t bytes) {
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 inline bool aligned32(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 31u) == 0; }
+
+// ------------------------------------------------------------------------------------------ packed-weight descriptors
+// The checks of every entry point that reads an MctqPackedDesc.  Their order fixes the error code of a descriptor with
+// several faults: kind and dtype (pack_check_kind), then the entry point's shape and pointer checks, then the parameters.
+// kind in range (MCTQ_E_BADARG); dtype a valid tag, f32 for the LUT kinds (MCTQ_E_DTYPE)
+inline int pack_check_kind(int kind, int dtype) {
+    if (kind < MCTQ_PACK_AFFINE_I8 || kind > MCTQ_PACK_LUT_I4) return MCTQ_E_BADARG;
+    if (dtype != MCTQ_F32 && dtype != MCTQ_BF16 && dtype != MCTQ_F16) return MCTQ_E_DTYPE;
+    if (pack_is_lut(kind) && dtype != MCTQ_F32) return MCTQ_E_DTYPE;          // LUT weights rebuild as f32, like the reference
+    return 0;
+}
+// LUT kinds: quotients and 1 <= K <= pack_max_k (MCTQ_E_LUT); affine kinds: zero points (MCTQ_E_BADARG)
+inline int pack_check_params(const MctqPackedDesc& d) {
+    if (pack_is_lut(d.kind)) {
+        if (!d.lut_quotients || d.K < 1 || d.K > pack_max_k(d.kind)) return MCTQ_E_LUT;
+    } else if (!d.zp) {
+        return MCTQ_E_BADARG;
+    }
+    return 0;
+}
+// the checks shared by mctq_packed_linear and mctq_packed_linear_batched: w is a row-major [out][in] weight with parameters
+// per tensor or per output row, x and y have its dtype
+inline int packed_linear_check(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x, int x_dtype,
+                               int64_t M, const void* y) {
+    if (!w) return MCTQ_E_BADARG;
+    if (const int rc = pack_check_kind(w->kind, x_dtype)) return rc;
+    if (w->y_dtype != x_dtype) return MCTQ_E_DTYPE;
+    if (out_features < 1 || in_features < 1 || out_features >= (1LL << 31) || in_features >= (1LL << 31) || M < 0)
+        return MCTQ_E_BADARG;
+    if (w->n != out_features * in_features) return MCTQ_E_BADARG;
+    if (w->C != 1 && !(w->C == out_features && w->inner == in_features)) return MCTQ_E_BADARG;
+    if (!w->codes || !w->scale || !x || !y) return MCTQ_E_BADARG;
+    return pack_check_params(*w);
+}
+
+// f(kind, type) with kind a std::integral_constant<int, MCTQ_PACK_*> and type a PackType<T>, for the (kind, dtype) of a
+// checked descriptor: only the pairs the packed-weight kernels are built for, affine x {f32, bf16, f16} and LUT x f32
+template <typename T> struct PackType { using type = T; };
+template <class F>
+int dispatch_packed(int kind, int dtype, F&& f) {
+    auto typed = [&](auto k) {
+        if constexpr (pack_is_lut(decltype(k)::value)) {
+            return f(k, PackType<float>{});
+        } else {
+            if (dtype == MCTQ_F32) return f(k, PackType<float>{});
+            if (dtype == MCTQ_BF16) return f(k, PackType<__nv_bfloat16>{});
+            return f(k, PackType<__half>{});
+        }
+    };
+    switch (kind) {
+        case MCTQ_PACK_AFFINE_I8: return typed(std::integral_constant<int, MCTQ_PACK_AFFINE_I8>{});
+        case MCTQ_PACK_AFFINE_I4: return typed(std::integral_constant<int, MCTQ_PACK_AFFINE_I4>{});
+        case MCTQ_PACK_LUT_U8: return typed(std::integral_constant<int, MCTQ_PACK_LUT_U8>{});
+        default: return typed(std::integral_constant<int, MCTQ_PACK_LUT_I4>{});
+    }
+}
 
 // geometry of the channel window for a tile of `tile` elements
 template <class Args>

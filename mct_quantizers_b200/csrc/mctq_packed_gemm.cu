@@ -89,8 +89,8 @@ __device__ __forceinline__ void split3(float x, float& x0, float& x1, float& x2)
 
 template <int KIND, typename T>
 __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_constant__ GemmArgs a) {
-    constexpr bool LUT = KIND == MCTQ_PACK_LUT_U8 || KIND == MCTQ_PACK_LUT_I4;
-    constexpr int CODE = (KIND == MCTQ_PACK_AFFINE_I4 || KIND == MCTQ_PACK_LUT_I4) ? MCTQ_CODES_INT4 : MCTQ_CODES_INT8;
+    constexpr bool LUT = pack_is_lut(KIND);
+    constexpr int CODE = pack_code_mode(KIND);
     constexpr int RAW = CodeVec<CODE, 8>::kWords;                        // 32-bit code words per 8 elements
     constexpr bool F32X = std::is_same<T, float>::value;
     constexpr bool FACTOR = LUT || F32X;
@@ -412,30 +412,18 @@ extern "C" {
 int mctq_packed_linear_batched(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x, int x_dtype,
                                int64_t M, const void* bias, void* y, const float* lut_quotients_host, void* stream) {
     MCTQ_NVTX("mctq_packed_linear_batched");
-    if (!w) return MCTQ_E_BADARG;
-    if (w->kind < MCTQ_PACK_AFFINE_I8 || w->kind > MCTQ_PACK_LUT_I4) return MCTQ_E_BADARG;
-    if (x_dtype != MCTQ_F32 && x_dtype != MCTQ_BF16 && x_dtype != MCTQ_F16) return MCTQ_E_DTYPE;
-    if (w->y_dtype != x_dtype) return MCTQ_E_DTYPE;
-    const bool lut = w->kind == MCTQ_PACK_LUT_U8 || w->kind == MCTQ_PACK_LUT_I4;
-    if (lut && x_dtype != MCTQ_F32) return MCTQ_E_DTYPE;
-    if (out_features < 1 || in_features < 1 || out_features >= (1LL << 31) || in_features >= (1LL << 31) || M < 0)
-        return MCTQ_E_BADARG;
-    if (w->n != out_features * in_features) return MCTQ_E_BADARG;
-    if (w->C != 1 && !(w->C == out_features && w->inner == in_features)) return MCTQ_E_BADARG;
-    if (!w->codes || !w->scale || !x || !y) return MCTQ_E_BADARG;
+    if (const int rc = packed_linear_check(w, out_features, in_features, x, x_dtype, M, y)) return rc;
+    const bool lut = pack_is_lut(w->kind);
     GemmArgs a;
     memset(&a, 0, sizeof(a));
     if (lut) {
-        if (!w->lut_quotients || !lut_quotients_host || w->K < 1 || w->K > (w->kind == MCTQ_PACK_LUT_I4 ? 16 : 256))
-            return MCTQ_E_LUT;
+        if (!lut_quotients_host) return MCTQ_E_LUT;
         for (int k = 0; k < w->K; ++k) {
             uint32_t bits;
             memcpy(&bits, lut_quotients_host + k, 4);
             if (bits & 0xFFFFu) return MCTQ_E_LUT;                            // not exact in bf16
             a.quot[k] = lut_quotients_host[k];
         }
-    } else if (!w->zp) {
-        return MCTQ_E_BADARG;
     }
     if (M == 0) return 0;
     a.codes = reinterpret_cast<const uint8_t*>(w->codes);
@@ -449,23 +437,13 @@ int mctq_packed_linear_batched(const MctqPackedDesc* w, int64_t out_features, in
     a.K = (int32_t)in_features;
     a.per_channel = w->C != 1;
     a.is_signed = lut ? 0 : (w->is_signed ? 1 : 0);
-    const bool int4 = w->kind == MCTQ_PACK_AFFINE_I4 || w->kind == MCTQ_PACK_LUT_I4;
     const uintptr_t cp = reinterpret_cast<uintptr_t>(w->codes);
-    a.fast_codes = in_features % 8 == 0 && (cp & (int4 ? 3u : 7u)) == 0;
+    a.fast_codes = in_features % 8 == 0 && (cp & (pack_is_int4(w->kind) ? 3u : 7u)) == 0;
     a.fast_x = in_features % 8 == 0 && aligned16(x);
     cudaStream_t st = (cudaStream_t)stream;
-    switch (w->kind) {
-        case MCTQ_PACK_AFFINE_I8:
-            if (x_dtype == MCTQ_F32) return launch_gemm<MCTQ_PACK_AFFINE_I8, float>(a, st);
-            if (x_dtype == MCTQ_BF16) return launch_gemm<MCTQ_PACK_AFFINE_I8, __nv_bfloat16>(a, st);
-            return launch_gemm<MCTQ_PACK_AFFINE_I8, __half>(a, st);
-        case MCTQ_PACK_AFFINE_I4:
-            if (x_dtype == MCTQ_F32) return launch_gemm<MCTQ_PACK_AFFINE_I4, float>(a, st);
-            if (x_dtype == MCTQ_BF16) return launch_gemm<MCTQ_PACK_AFFINE_I4, __nv_bfloat16>(a, st);
-            return launch_gemm<MCTQ_PACK_AFFINE_I4, __half>(a, st);
-        case MCTQ_PACK_LUT_U8: return launch_gemm<MCTQ_PACK_LUT_U8, float>(a, st);
-        default: return launch_gemm<MCTQ_PACK_LUT_I4, float>(a, st);
-    }
+    return dispatch_packed(w->kind, x_dtype, [&](auto kind, auto type) {
+        return launch_gemm<decltype(kind)::value, typename decltype(type)::type>(a, st);
+    });
 }
 
 }  // extern "C"

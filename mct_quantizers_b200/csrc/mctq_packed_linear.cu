@@ -44,11 +44,11 @@ constexpr int kLinGroups = kLinWarps / kLinSplit;
 
 template <int KIND, typename T, int MT, bool FAST>
 __global__ void __launch_bounds__(kThreads, MT >= 8 ? 1 : 2) packed_linear_kernel(const __grid_constant__ LinearArgs a) {
-    constexpr bool LUT = KIND == MCTQ_PACK_LUT_U8 || KIND == MCTQ_PACK_LUT_I4;
-    constexpr int CODE = (KIND == MCTQ_PACK_AFFINE_I4 || KIND == MCTQ_PACK_LUT_I4) ? MCTQ_CODES_INT4 : MCTQ_CODES_INT8;
+    constexpr bool LUT = pack_is_lut(KIND);
+    constexpr int CODE = pack_code_mode(KIND);
     constexpr int EPW = CODE == MCTQ_CODES_INT4 ? 8 : 4;        // elements per 32-bit word of codes
     constexpr int EPV = 2 * EPW;                                 // elements per 8-byte vector
-    constexpr int NQ = CODE == MCTQ_CODES_INT4 ? 16 : 256;
+    constexpr int NQ = pack_max_k(KIND);
     constexpr bool FACTOR = LUT || std::is_same<T, float>::value;
     constexpr int R = LinRows<MT>::value;
     __shared__ float sm_q[LUT ? NQ : 1];
@@ -197,17 +197,6 @@ int launch_linear_typed(const LinearArgs& a, bool fast, cudaStream_t st) {
     return launch_linear_mt<KIND, T, 8>(a, fast, st);
 }
 
-template <int KIND>
-int launch_linear_kind(const LinearArgs& a, int dtype, bool fast, cudaStream_t st) {
-    if constexpr (KIND == MCTQ_PACK_LUT_U8 || KIND == MCTQ_PACK_LUT_I4) {
-        return launch_linear_typed<KIND, float>(a, fast, st);
-    } else {
-        if (dtype == MCTQ_F32) return launch_linear_typed<KIND, float>(a, fast, st);
-        if (dtype == MCTQ_BF16) return launch_linear_typed<KIND, __nv_bfloat16>(a, fast, st);
-        return launch_linear_typed<KIND, __half>(a, fast, st);
-    }
-}
-
 }  // namespace
 
 extern "C" {
@@ -215,23 +204,9 @@ extern "C" {
 int mctq_packed_linear(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x, int x_dtype,
                        int64_t M, const void* bias, void* y, void* stream) {
     MCTQ_NVTX("mctq_packed_linear");
-    if (!w) return MCTQ_E_BADARG;
-    if (w->kind < MCTQ_PACK_AFFINE_I8 || w->kind > MCTQ_PACK_LUT_I4) return MCTQ_E_BADARG;
-    if (x_dtype != MCTQ_F32 && x_dtype != MCTQ_BF16 && x_dtype != MCTQ_F16) return MCTQ_E_DTYPE;
-    if (w->y_dtype != x_dtype) return MCTQ_E_DTYPE;                             // x and y have the rebuilt weight's dtype
-    const bool lut = w->kind == MCTQ_PACK_LUT_U8 || w->kind == MCTQ_PACK_LUT_I4;
-    if (lut && x_dtype != MCTQ_F32) return MCTQ_E_DTYPE;                         // LUT weights rebuild as f32
-    if (out_features < 1 || in_features < 1 || out_features >= (1LL << 31) || in_features >= (1LL << 31) || M < 0)
-        return MCTQ_E_BADARG;
-    if (w->n != out_features * in_features) return MCTQ_E_BADARG;
-    if (w->C != 1 && !(w->C == out_features && w->inner == in_features)) return MCTQ_E_BADARG;   // per tensor or per output row
-    if (!w->codes || !w->scale || !x || !y) return MCTQ_E_BADARG;
-    if (lut) {
-        if (!w->lut_quotients || w->K < 1 || w->K > (w->kind == MCTQ_PACK_LUT_I4 ? 16 : 256)) return MCTQ_E_LUT;
-    } else if (!w->zp) {
-        return MCTQ_E_BADARG;
-    }
+    if (const int rc = packed_linear_check(w, out_features, in_features, x, x_dtype, M, y)) return rc;
     if (M == 0) return 0;
+    const bool lut = pack_is_lut(w->kind);
     LinearArgs a;
     memset(&a, 0, sizeof(a));
     a.codes = reinterpret_cast<const uint8_t*>(w->codes);
@@ -247,15 +222,12 @@ int mctq_packed_linear(const MctqPackedDesc* w, int64_t out_features, int64_t in
     a.per_channel = w->C != 1;
     a.is_signed = lut ? 0 : (w->is_signed ? 1 : 0);
     a.nq = lut ? w->K : 0;
-    const int64_t epv = (w->kind == MCTQ_PACK_AFFINE_I4 || w->kind == MCTQ_PACK_LUT_I4) ? 16 : 8;
+    const int64_t epv = pack_is_int4(w->kind) ? 16 : 8;
     const bool fast = in_features % epv == 0 && aligned16(w->codes) && aligned16(x);
     cudaStream_t st = (cudaStream_t)stream;
-    switch (w->kind) {
-        case MCTQ_PACK_AFFINE_I8: return launch_linear_kind<MCTQ_PACK_AFFINE_I8>(a, x_dtype, fast, st);
-        case MCTQ_PACK_AFFINE_I4: return launch_linear_kind<MCTQ_PACK_AFFINE_I4>(a, x_dtype, fast, st);
-        case MCTQ_PACK_LUT_U8: return launch_linear_kind<MCTQ_PACK_LUT_U8>(a, x_dtype, fast, st);
-        default: return launch_linear_kind<MCTQ_PACK_LUT_I4>(a, x_dtype, fast, st);
-    }
+    return dispatch_packed(w->kind, x_dtype, [&](auto kind, auto type) {
+        return launch_linear_typed<decltype(kind)::value, typename decltype(type)::type>(a, fast, st);
+    });
 }
 
 }  // extern "C"

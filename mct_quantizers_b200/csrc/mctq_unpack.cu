@@ -40,9 +40,9 @@ constexpr int kUnpackUnroll = 4;
 
 template <int KIND, typename T, int MODE, int V, int CAP>
 __global__ void __launch_bounds__(kThreads) unpack_multi_kernel(const __grid_constant__ UnpackParamsT<CAP> p) {
-    constexpr bool LUT = KIND == MCTQ_PACK_LUT_U8 || KIND == MCTQ_PACK_LUT_I4;
-    constexpr int CODE = (KIND == MCTQ_PACK_AFFINE_I4 || KIND == MCTQ_PACK_LUT_I4) ? MCTQ_CODES_INT4 : MCTQ_CODES_INT8;
-    constexpr int NQ = CODE == MCTQ_CODES_INT4 ? 16 : 256;
+    constexpr bool LUT = pack_is_lut(KIND);
+    constexpr int CODE = pack_code_mode(KIND);
+    constexpr int NQ = pack_max_k(KIND);
     constexpr int64_t TILE = (int64_t)kThreads * kUnpackUnroll * V;
     __shared__ float sm_q[LUT ? NQ : 1];
     const uint32_t k = blockIdx.y;
@@ -93,7 +93,7 @@ int launch_unpack_variant(const UnpackParams& c, cudaStream_t st) {
 template <int KIND, typename T, int CAP>
 int launch_unpack_typed(const UnpackParams& c, cudaStream_t st) {
     constexpr int V0 = sizeof(T) == 2 ? 8 : 4;                                              // per tensor
-    constexpr bool WIDE1 = sizeof(T) == 2 || KIND == MCTQ_PACK_AFFINE_I4 || KIND == MCTQ_PACK_LUT_I4;   // per channel
+    constexpr bool WIDE1 = sizeof(T) == 2 || pack_is_int4(KIND);                             // per channel
     if (c.mode == 0 && c.v == V0) return launch_unpack_variant<KIND, T, 0, V0, CAP>(c, st);
     if (c.mode == 1 && c.v == 4) return launch_unpack_variant<KIND, T, 1, 4, CAP>(c, st);
     if constexpr (WIDE1) if (c.mode == 1 && c.v == 8) return launch_unpack_variant<KIND, T, 1, 8, CAP>(c, st);
@@ -101,43 +101,23 @@ int launch_unpack_typed(const UnpackParams& c, cudaStream_t st) {
     return MCTQ_E_BADARG;
 }
 
-template <int KIND, int CAP>
-int launch_unpack_kind(const UnpackParams& c, cudaStream_t st) {
-    if constexpr (KIND == MCTQ_PACK_LUT_U8 || KIND == MCTQ_PACK_LUT_I4) {
-        return launch_unpack_typed<KIND, float, CAP>(c, st);
-    } else {
-        if (c.dtype == MCTQ_F32) return launch_unpack_typed<KIND, float, CAP>(c, st);
-        if (c.dtype == MCTQ_BF16) return launch_unpack_typed<KIND, __nv_bfloat16, CAP>(c, st);
-        return launch_unpack_typed<KIND, __half, CAP>(c, st);
-    }
-}
-
 template <int CAP>
 int launch_unpack_chunk(const UnpackParams& c, cudaStream_t st) {
-    switch (c.kind) {
-        case MCTQ_PACK_AFFINE_I8: return launch_unpack_kind<MCTQ_PACK_AFFINE_I8, CAP>(c, st);
-        case MCTQ_PACK_AFFINE_I4: return launch_unpack_kind<MCTQ_PACK_AFFINE_I4, CAP>(c, st);
-        case MCTQ_PACK_LUT_U8: return launch_unpack_kind<MCTQ_PACK_LUT_U8, CAP>(c, st);
-        default: return launch_unpack_kind<MCTQ_PACK_LUT_I4, CAP>(c, st);
-    }
+    return dispatch_packed(c.kind, c.dtype, [&](auto kind, auto type) {
+        return launch_unpack_typed<decltype(kind)::value, typename decltype(type)::type, CAP>(c, st);
+    });
 }
 
 // argument block and variant of one descriptor; 0 or MCTQ_E_*.  *skip = 1 for an empty tensor (nothing to launch).
 int unpack_make_args(const MctqPackedDesc& d, UnpackArgs* a, int* mode, int* v, int* skip) {
     *skip = 0;
-    if (d.kind < MCTQ_PACK_AFFINE_I8 || d.kind > MCTQ_PACK_LUT_I4) return MCTQ_E_BADARG;
-    if (d.y_dtype != MCTQ_F32 && d.y_dtype != MCTQ_BF16 && d.y_dtype != MCTQ_F16) return MCTQ_E_DTYPE;
-    const bool lut = d.kind == MCTQ_PACK_LUT_U8 || d.kind == MCTQ_PACK_LUT_I4;
-    if (lut && d.y_dtype != MCTQ_F32) return MCTQ_E_DTYPE;                     // LUT outputs are f32, like the reference
+    if (const int rc = pack_check_kind(d.kind, d.y_dtype)) return rc;
     if (d.n < 0 || d.C < 1 || d.inner < 1 || d.C >= (1LL << 31) || d.inner >= (1LL << 31)) return MCTQ_E_BADARG;
     if (d.n % (d.C * d.inner) != 0) return MCTQ_E_BADARG;                      // [outer][C][inner]
     if (d.n == 0) { *skip = 1; return 0; }
     if (!d.codes || !d.y || !d.scale || !aligned16(d.codes) || !aligned16(d.y)) return MCTQ_E_BADARG;
-    if (lut) {
-        if (!d.lut_quotients || d.K < 1 || d.K > (d.kind == MCTQ_PACK_LUT_I4 ? 16 : 256)) return MCTQ_E_LUT;
-    } else if (!d.zp) {
-        return MCTQ_E_BADARG;
-    }
+    if (const int rc = pack_check_params(d)) return rc;
+    const bool lut = pack_is_lut(d.kind);
     memset(a, 0, sizeof(*a));
     a->codes = reinterpret_cast<const uint8_t*>(d.codes);
     a->y = d.y;
@@ -154,19 +134,24 @@ int unpack_make_args(const MctqPackedDesc& d, UnpackArgs* a, int* mode, int* v, 
     *mode = d.C == 1 ? 0 : (d.inner % 4 == 0 ? 1 : 2);
     // 8 codes per vector where the whole vector lies in one channel and (f32) y takes a 32-byte store: always for 2-byte
     // outputs (16-byte instead of 8-byte stores); for f32 where dequant_affine measured it faster, packed nibbles per channel
-    const bool int4 = d.kind == MCTQ_PACK_AFFINE_I4 || d.kind == MCTQ_PACK_LUT_I4;
     const bool fits8 = *mode != 2 && (*mode == 0 || d.inner % 8 == 0) && (d.y_dtype != MCTQ_F32 || aligned32(d.y));
-    *v = fits8 && (d.y_dtype != MCTQ_F32 || (*mode == 1 && int4)) ? 8 : 4;
+    *v = fits8 && (d.y_dtype != MCTQ_F32 || (*mode == 1 && pack_is_int4(d.kind))) ? 8 : 4;
     return 0;
 }
 
 inline int variant_key(int kind, int dtype, int mode, int v) { return (((kind - 1) * 3 + dtype) * 3 + mode) * 2 + (v == 8 ? 1 : 0); }
 constexpr int kUnpackVariants = 4 * 3 * 3 * 2;
 
+// a compiled plan on the host: the header and the chunks of the blob mctq_unpack_plan writes
+struct UnpackPlanHost {
+    UnpackHeader h = {};
+    std::vector<UnpackParams> chunks;
+};
+
 // validates every descriptor and groups the tensors by kernel variant (one chunk = one launch, <= 64 tensors whose tile counts
 // are within a factor of 16: the grid is [largest tile count] x [tensors] and CTAs past a tensor's last tile exit at once);
-// fills the chunks when `blob` is given; returns the number of chunks (or < 0)
-int64_t unpack_compile(const MctqPackedDesc* descs, int n_desc, uint8_t* blob) {
+// 0 or MCTQ_E_*
+int unpack_compile(const MctqPackedDesc* descs, int n_desc, UnpackPlanHost& plan) {
     if (!descs || n_desc < 1) return MCTQ_E_BADARG;
     std::vector<UnpackArgs> args((size_t)n_desc);
     std::vector<int> key((size_t)n_desc, -1), vv((size_t)n_desc), md((size_t)n_desc);
@@ -176,9 +161,6 @@ int64_t unpack_compile(const MctqPackedDesc* descs, int n_desc, uint8_t* blob) {
         if (rc) return rc;
         if (!skip) key[k] = variant_key(descs[k].kind, descs[k].y_dtype, md[k], vv[k]);
     }
-    UnpackHeader* h = reinterpret_cast<UnpackHeader*>(blob);
-    UnpackParams* chunks = blob ? reinterpret_cast<UnpackParams*>(blob + sizeof(UnpackHeader)) : nullptr;
-    int n_chunks = 0;
     int64_t total = 0;
     for (int var = 0; var < kUnpackVariants; ++var) {
         std::vector<std::pair<int64_t, int>> order;               // tensors of this variant, largest first
@@ -198,30 +180,22 @@ int64_t unpack_compile(const MctqPackedDesc* descs, int n_desc, uint8_t* blob) {
             if (in_chunk == kUnpackMaxDesc || (in_chunk && tiles * 16 < first_tiles)) in_chunk = 0;
             if (in_chunk == 0) {
                 first_tiles = tiles;
-                if (chunks) {
-                    UnpackParams& c = chunks[n_chunks];
-                    c.n_desc = 0; c.kind = descs[k].kind; c.dtype = descs[k].y_dtype; c.mode = md[k]; c.v = vv[k];
-                    c.tiles[kUnpackMaxDesc] = (int32_t)tiles;
-                }
-                ++n_chunks;
+                UnpackParams& c = plan.chunks.emplace_back();         // zero-filled
+                c.kind = descs[k].kind; c.dtype = descs[k].y_dtype; c.mode = md[k]; c.v = vv[k];
+                c.tiles[kUnpackMaxDesc] = (int32_t)tiles;
             }
-            if (chunks) {
-                UnpackParams& c = chunks[n_chunks - 1];
-                c.e[in_chunk] = args[k];
-                c.tiles[in_chunk] = (int32_t)tiles;
-                c.n_desc = in_chunk + 1;
-            }
-            ++in_chunk;
+            UnpackParams& c = plan.chunks.back();
+            c.e[in_chunk] = args[k];
+            c.tiles[in_chunk] = (int32_t)tiles;
+            c.n_desc = ++in_chunk;
             total += tiles;
         }
     }
-    if (h) {
-        h->magic = kUnpackMagic;
-        h->n_desc = n_desc;
-        h->n_chunks = n_chunks;
-        h->total_tiles = total;
-    }
-    return n_chunks;
+    plan.h.magic = kUnpackMagic;
+    plan.h.n_desc = n_desc;
+    plan.h.n_chunks = (int32_t)plan.chunks.size();
+    plan.h.total_tiles = total;
+    return 0;
 }
 
 }  // namespace
@@ -229,18 +203,18 @@ int64_t unpack_compile(const MctqPackedDesc* descs, int n_desc, uint8_t* blob) {
 extern "C" {
 
 size_t mctq_unpack_plan_bytes(const MctqPackedDesc* descs, int n_desc) {
-    const int64_t chunks = unpack_compile(descs, n_desc, nullptr);
-    if (chunks < 0) return 0;
-    return unpack_bytes((int)chunks);
+    UnpackPlanHost plan;
+    return unpack_compile(descs, n_desc, plan) ? 0 : unpack_bytes(plan.h.n_chunks);
 }
 
 int64_t mctq_unpack_plan(const MctqPackedDesc* descs, int n_desc, void* plan_host_out, size_t plan_bytes) {
-    const int64_t chunks = unpack_compile(descs, n_desc, nullptr);
-    if (chunks < 0) return chunks;
-    if (!plan_host_out || plan_bytes < unpack_bytes((int)chunks)) return MCTQ_E_BADARG;
-    memset(plan_host_out, 0, unpack_bytes((int)chunks));
-    const int64_t rc = unpack_compile(descs, n_desc, reinterpret_cast<uint8_t*>(plan_host_out));
-    return rc < 0 ? rc : reinterpret_cast<const UnpackHeader*>(plan_host_out)->total_tiles;
+    UnpackPlanHost plan;
+    if (const int rc = unpack_compile(descs, n_desc, plan)) return rc;
+    if (!plan_host_out || plan_bytes < unpack_bytes(plan.h.n_chunks)) return MCTQ_E_BADARG;
+    uint8_t* out = reinterpret_cast<uint8_t*>(plan_host_out);
+    memcpy(out, &plan.h, sizeof(UnpackHeader));
+    if (!plan.chunks.empty()) memcpy(out + sizeof(UnpackHeader), plan.chunks.data(), plan.chunks.size() * sizeof(UnpackParams));
+    return plan.h.total_tiles;
 }
 
 int mctq_unpack_multi(const void* plan_host, void* stream) {

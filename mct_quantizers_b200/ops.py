@@ -17,6 +17,7 @@ host buffer through the GPU (mctq_fq_*_host), and a fake/meta implementation so 
 torch.compile and shape propagation work.  There is no eager / CPU arithmetic fallback anywhere.
 """
 import ctypes
+import functools
 
 import numpy as np
 import torch
@@ -393,7 +394,7 @@ def affine_codes(xd, scale, zero_point, C, inner, quant_min, quant_max, code_mod
     if code_mode == _native.CODES_INT8:
         codes = torch.empty(n, dtype=torch.int8 if quant_min < 0 else torch.uint8, device=xd.device)
     else:
-        codes = torch.empty((n + 1) // 2, dtype=torch.uint8, device=xd.device)
+        codes = torch.empty(_native.packed_code_bytes(_native.PACK_AFFINE_I4, n), dtype=torch.uint8, device=xd.device)
     if n:
         lib = _native.load()
         s, z = _param_on(scale, xd.device), _param_on(zero_point, xd.device)
@@ -434,7 +435,7 @@ def _affine_channel_launch(x, scale, zero_point, axis, quant_min, quant_max, cod
     if code_mode == _native.CODES_INT8:
         codes = torch.empty_like(xd, dtype=torch.int8 if quant_min < 0 else torch.uint8)
     elif code_mode == _native.CODES_INT4:
-        codes = torch.empty((n + 1) // 2, dtype=torch.uint8, device=xd.device)
+        codes = torch.empty(_native.packed_code_bytes(_native.PACK_AFFINE_I4, n), dtype=torch.uint8, device=xd.device)
     if n:
         lib = _native.load()
         s, z = _param_on(scale, xd.device), _param_on(zero_point, xd.device)
@@ -600,7 +601,7 @@ def _lut_tensor_launch(x, table, K, threshold, per_channel, axis, eps, idx_mode,
     if idx_mode == _native.CODES_INT8:
         idx = torch.empty_like(xd, dtype=torch.uint8)
     elif idx_mode == _native.CODES_INT4:
-        idx = torch.empty((n + 1) // 2, dtype=torch.uint8, device=xd.device)
+        idx = torch.empty(_native.packed_code_bytes(_native.PACK_LUT_I4, n), dtype=torch.uint8, device=xd.device)
     if n:
         thr = _param_on(threshold.contiguous(), xd.device)
         _lut_launch(xd, y, idx, idx_mode, table, K, C, inner, thr, eps, False, 1.0, 1.0, False)
@@ -694,12 +695,31 @@ def _dequantize_lut_cuda(idx, idx_mode, shape, lut, lut_values_bitwidth, is_sign
         C, inner = 1, 1
         if threshold.numel() != 1:
             raise RuntimeError("per-tensor LUT dequantization needs a single threshold")
-    need = n if kind == _native.PACK_LUT_U8 else (n + 1) // 2
+    need = _native.packed_code_bytes(kind, n)
     if idx.numel() != need or idx.dtype not in (torch.uint8, torch.int8):
         raise RuntimeError(f"idx must hold {need} bytes for shape {shape} and idx_mode {idx_mode}")
     q = lut_quotients(lut, lut_values_bitwidth, is_signed)
     item = (idx, kind, False, torch.float32, shape if shape else [1], None, C, inner, threshold.reshape(-1), None, q)
     return UnpackPlan([item]).run()[0]
+
+
+def _packed_desc(codes, kind, is_signed, dtype, n, C, inner, scale, zero_point, lut_quotients, device, what):
+    """The MctqPackedDesc of n packed elements (y unset), parameters placed on `device`: (desc, the tensors it points into).
+    `what` names the tensor in the ValueError messages."""
+    if codes.dtype not in (torch.uint8, torch.int8) or codes.numel() != _native.packed_code_bytes(kind, n):
+        raise ValueError(f"{what}: codes ({codes.dtype}, {codes.numel()} bytes) do not hold {n} elements of kind {kind}")
+    codes = codes.contiguous()
+    s = _param_on(scale.detach().reshape(-1).contiguous(), device)
+    z = _param_on(zero_point.detach().reshape(-1).contiguous(), device) if zero_point is not None else None
+    q = _param_on(lut_quotients.detach().reshape(-1).contiguous(), device) if lut_quotients is not None else None
+    if s.dtype != torch.float32 or (z is not None and z.dtype != torch.int32) or (q is not None and q.dtype != torch.float32):
+        raise ValueError(f"{what}: scale / threshold and quotients must be float32, zero points int32")
+    d = _native.MctqPackedDesc()
+    d.codes, d.y, d.n, d.C, d.inner = codes.data_ptr(), None, n, int(C), int(inner)
+    d.kind, d.is_signed, d.y_dtype = int(kind), int(bool(is_signed)), _DT.get(dtype, -1)
+    d.K = q.numel() if q is not None else 0
+    d.scale, d.zp, d.lut_quotients = s.data_ptr(), _ptr(z), _ptr(q)
+    return d, (codes, s, z, q)
 
 
 class PackedLinear:
@@ -720,26 +740,14 @@ class PackedLinear:
         if self.device.type != "cuda":
             raise ValueError("PackedLinear needs CUDA tensors")
         self.out_features, self.in_features, self.dtype = int(out_features), int(in_features), dtype
-        n = self.out_features * self.in_features
-        if codes.dtype not in (torch.uint8, torch.int8) or codes.numel() != (n if kind in (_native.PACK_AFFINE_I8, _native.PACK_LUT_U8) else (n + 1) // 2):
-            raise ValueError(f"codes ({codes.dtype}, {codes.numel()} bytes) do not hold a packed {out_features}x{in_features} weight of kind {kind}")
-        codes = codes.contiguous()
-        s = _param_on(scale.detach().reshape(-1).contiguous(), self.device)
-        z = _param_on(zero_point.detach().reshape(-1).contiguous(), self.device) if zero_point is not None else None
-        q = _param_on(lut_quotients.detach().reshape(-1).contiguous(), self.device) if lut_quotients is not None else None
-        if s.dtype != torch.float32 or (z is not None and z.dtype != torch.int32) or (q is not None and q.dtype != torch.float32):
-            raise ValueError("scale / threshold and quotients must be float32, zero points int32")
+        C, inner = (scale.numel(), self.in_features) if scale.numel() > 1 else (1, 1)
+        self._desc, self._keep = _packed_desc(codes, kind, is_signed, dtype, self.out_features * self.in_features, C, inner,
+                                              scale, zero_point, lut_quotients, self.device, "PackedLinear")
+        s, z = self._keep[1], self._keep[2]
         if s.numel() not in (1, self.out_features) or (z is not None and z.numel() != s.numel()):
             raise ValueError(f"{s.numel()} parameters for {out_features} output channels (per tensor or per output channel)")
         self._quot_src = lut_quotients.detach().reshape(-1) if lut_quotients is not None else None
-        self._keep = (codes, s, z, q)
-        d = self._desc = _native.MctqPackedDesc()
-        d.codes, d.y, d.n = codes.data_ptr(), None, n
-        d.C, d.inner = (s.numel(), self.in_features) if s.numel() > 1 else (1, 1)
-        d.kind, d.is_signed, d.y_dtype = int(kind), int(bool(is_signed)), _DT.get(dtype, -1)
-        d.K = q.numel() if q is not None else 0
-        d.scale, d.zp, d.lut_quotients = s.data_ptr(), _ptr(z), _ptr(q)
-        self._desc_ptr = ctypes.addressof(d)
+        self._desc_ptr = ctypes.addressof(self._desc)
 
     def __call__(self, x, bias=None):
         return self._run(x, bias, False)
@@ -796,21 +804,17 @@ def _quotients_host(q):
     return hit[1]
 
 
-def _packed_linear_cuda(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
+def _packed_linear_cuda(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias, batched=False):
+    """mctq::packed_linear, and mctq::packed_linear_batched with `batched`."""
     _dtype_tag(x)
     if x.dim() == 0:
-        raise RuntimeError("packed_linear: x must have at least one dimension")
-    _native.load()
-    return PackedLinear(codes, kind, is_signed, x.dtype, out_features, x.shape[-1], scale, zero_point, lut_quotients)(x, bias)
-
-
-def _packed_linear_batched_cuda(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
-    _dtype_tag(x)
-    if x.dim() == 0:
-        raise RuntimeError("packed_linear_batched: x must have at least one dimension")
+        raise RuntimeError(f"packed_linear{'_batched' if batched else ''}: x must have at least one dimension")
     _native.load()
     lin = PackedLinear(codes, kind, is_signed, x.dtype, out_features, x.shape[-1], scale, zero_point, lut_quotients)
-    return lin.batched(x, bias)
+    return lin._run(x, bias, batched)
+
+
+_packed_linear_batched_cuda = functools.partial(_packed_linear_cuda, batched=True)
 
 
 def _lut_scalar_cuda(x, table, K, divisor, threshold, round_to_input_dtype, multiply=False):
@@ -1342,27 +1346,14 @@ class UnpackPlan:
         for k, (codes, kind, is_signed, dtype, shape, stride, C, inner, scale, zp, quot) in enumerate(items):
             if codes.device != self.device:
                 raise ValueError("all tensors of an UnpackPlan must live on one CUDA device")
-            if codes.dtype not in (torch.uint8, torch.int8):
-                raise ValueError(f"tensor {k}: codes must be uint8 / int8, found {codes.dtype}")
+            if not codes.is_contiguous() or codes.data_ptr() % 16:      # the kernels load codes in 16-byte aligned vectors
+                codes = codes.clone(memory_format=torch.contiguous_format)
             n = 1
             for s_ in shape:
                 n *= int(s_)
-            need = n if kind in (_native.PACK_AFFINE_I8, _native.PACK_LUT_U8) else (n + 1) // 2
-            if codes.numel() != need:
-                raise ValueError(f"tensor {k}: {codes.numel()} code bytes for {n} elements of kind {kind}")
-            if not codes.is_contiguous() or codes.data_ptr() % 16:      # the kernels load codes in 16-byte aligned vectors
-                codes = codes.clone(memory_format=torch.contiguous_format)
-            s = _param_on(scale.detach().reshape(-1).contiguous(), self.device)
-            z = _param_on(zp.detach().reshape(-1).contiguous(), self.device) if zp is not None else None
-            q = _param_on(quot.detach().reshape(-1).contiguous(), self.device) if quot is not None else None
-            if s.dtype != torch.float32 or (z is not None and z.dtype != torch.int32) or (q is not None and q.dtype != torch.float32):
-                raise ValueError(f"tensor {k}: scale / threshold and quotients must be float32, zero points int32")
-            self._keep.append((codes, s, z, q))
-            d = self._descs[k]
-            d.codes, d.n, d.C, d.inner = codes.data_ptr(), n, int(C), int(inner)
-            d.kind, d.is_signed, d.y_dtype = int(kind), int(bool(is_signed)), _DT[dtype]
-            d.K = q.numel() if q is not None else 0
-            d.scale, d.zp, d.lut_quotients = s.data_ptr(), _ptr(z), _ptr(q)
+            self._descs[k], keep = _packed_desc(codes, kind, is_signed, dtype, n, C, inner, scale, zp, quot, self.device,
+                                                f"tensor {k}")
+            self._keep.append(keep)
             self._out_specs.append((tuple(int(v) for v in shape), None if stride is None else tuple(int(v) for v in stride), dtype))
         self._plan_host, self._plan_nb, self.fresh = None, 0, fresh
         if fresh:

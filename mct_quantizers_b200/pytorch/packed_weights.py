@@ -164,7 +164,7 @@ class PackedWeight:
     def plan_item(self):
         """The UnpackPlan item of this weight, parameters on the codes' device."""
         q, dev = self.quantizer, self.codes.device
-        if self.kind in (_native.PACK_LUT_U8, _native.PACK_LUT_I4):
+        if self.kind in _native.PACK_LUT_KINDS:
             thr, = q._on(dev, q._threshold_torch)
             return (self.codes, self.kind, False, self.dtype_out, self.shape_out, self.stride_out, self.C, self.inner,
                     thr.reshape(-1), None, self.lut_quotients)
@@ -180,7 +180,7 @@ class PackedWeight:
 def _emit_codes(q, w, kind):
     """(codes, is_signed, C, inner) of weight w: the quantizer's kernels in code-emission mode, elements in the memory order
     of quantizer(w)."""
-    if kind in (_native.PACK_LUT_U8, _native.PACK_LUT_I4):
+    if kind in _native.PACK_LUT_KINDS:
         if q.__dict__.get('_search_table') is None:
             from mct_quantizers_b200.pytorch.quantizer_utils import lut_search_table
             q._search_table = lut_search_table(q._lut_values_np, q.lut_values_bitwidth, True)
@@ -228,7 +228,8 @@ def fused_linear_eligibility(wrapper) -> Tuple[bool, str]:
 
 
 def _lut_quotients_host(q):
-    """The f32 quotients of LUT quantizer q, computed on the host (no device synchronisation)."""
+    """The f32 quotients of LUT quantizer q, computed on the host (no device synchronisation): the values a packed wrapper
+    registers and batched_linear_eligibility checks."""
     return ops.lut_quotients(torch.as_tensor(q._lut_values_np), q.lut_values_bitwidth, True)
 
 
@@ -239,7 +240,7 @@ def batched_linear_eligibility(wrapper) -> Tuple[bool, str]:
     if not ok:
         return ok, reason
     e = next(e for e in wrapper.__dict__['_packed'].entries if e.name == 'weight')
-    if e.kind in (_native.PACK_LUT_U8, _native.PACK_LUT_I4):
+    if e.kind in _native.PACK_LUT_KINDS:
         bits = _lut_quotients_host(e.quantizer).view(torch.int32)
         if bool(((bits & 0xFFFF) != 0).any()):
             return False, "a LUT quotient is not exact in bfloat16 (the tensor cores take the quotients as bf16 operands)"
@@ -367,9 +368,8 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
         codes, is_signed, C, inner = _emit_codes(q, w, kind)
         e = PackedWeight(wrapper, name, q, kind, is_signed, y_ref.dtype, y_ref.shape, y_ref.stride(), C, inner)
         wrapper.register_buffer(e.codes_name, codes)
-        if kind in (_native.PACK_LUT_U8, _native.PACK_LUT_I4):
-            quot = ops.lut_quotients(q._lut_values_torch, q.lut_values_bitwidth, True).to(w.device)
-            wrapper.register_buffer(e.quot_name, quot.view(torch.int32))
+        if kind in _native.PACK_LUT_KINDS:
+            wrapper.register_buffer(e.quot_name, _lut_quotients_host(q).to(w.device).view(torch.int32))
         rebuilt = ops.UnpackPlan([e.plan_item()]).run()[0]
         if rebuilt.stride() != y_ref.stride() or not torch.equal(_bits(rebuilt), _bits(y_ref)):
             raise RuntimeError(f"packing weight {name!r}: the rebuilt weight differs from quantizer(weight)")

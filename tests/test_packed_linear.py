@@ -128,6 +128,17 @@ def test_c_abi_rejections():
     assert _call(_lin_desc(kind=_native.PACK_LUT_U8, K=0)) == -4
     assert _call(_lin_desc(), M=-1) == -1
     assert _call(_lin_desc(out_f=0, in_f=33), out_f=0) == -1
+    # several faults: null w -> kind -> dtype -> shape -> pointers -> parameters -> M == 0
+    assert _call(_lin_desc(kind=5, dtype=3)) == -1
+    assert _call(_lin_desc(dtype=3), in_f=34) == -2
+    assert _call(_lin_desc(kind=_native.PACK_LUT_I4, dtype=_native.BF16, K=17)) == -2
+    assert _call(_lin_desc(kind=_native.PACK_LUT_I4, K=17), in_f=34) == -1
+    assert _call(_lin_desc(kind=_native.PACK_LUT_I4, K=17), M=-1) == -1
+    assert _call(_lin_desc(kind=_native.PACK_LUT_I4, K=17), x=None) == -1
+    assert _call(_lin_desc(kind=_native.PACK_LUT_I4, K=17), M=0) == -4
+    d = _lin_desc()
+    d.zp = None
+    assert _call(d, M=0) == -1
 
 
 # --------------------------------------------------------------------------------------------- GPU

@@ -76,6 +76,13 @@ def test_c_abi_rejections():
     bad[5] = np.float32(1.0 + 2.0 ** -9)                                             # needs more than bf16's 8 bits
     assert _call_b(_lin_desc(kind=LI4), quot_host=bad) == -4
     assert _call_b(_lin_desc(kind=LI4), quot_host=bad, M=0) == -4                     # checked before the M == 0 return
+    # several faults: the order of mctq_packed_linear, then the host quotients
+    assert _call_b(_lin_desc(kind=5, dtype=3)) == -1
+    assert _call_b(_lin_desc(kind=LI4, dtype=_native.BF16, K=17)) == -2
+    assert _call_b(_lin_desc(kind=LI4, K=17), in_f=34, quot_host=good) == -1
+    assert _call_b(_lin_desc(kind=LI4), x=None, quot_host=bad) == -1
+    assert _call_b(_lin_desc(kind=LI4, K=17), quot_host=bad) == -4
+    assert _call_b(_lin_desc(kind=LI4), quot_host=None, M=0) == -4
 
 
 def _lut_np(values, bw=8):

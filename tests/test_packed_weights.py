@@ -108,6 +108,18 @@ def test_unpack_plan_host_compiler():
     d.zp = None
     assert _plan([d]) == (-1, None)                                                       # affine needs zero points
     assert _plan([_desc(100, 1, 1), _desc(100, 1, 1, kind=0)]) == (-1, None)              # one bad tensor fails the plan
+    # several faults in one descriptor: kind -> dtype -> LUT dtype -> n / C / inner -> empty -> pointers -> parameters
+    assert _plan([_desc(100, 3, 1, kind=5, dtype=3)]) == (-1, None)
+    assert _plan([_desc(100, 3, 1, dtype=3)]) == (-2, None)
+    assert _plan([_desc(100, 1, 1, kind=_native.PACK_LUT_I4, dtype=_native.BF16, K=17)]) == (-2, None)
+    assert _plan([_desc(100, 3, 1, kind=_native.PACK_LUT_I4, K=17)]) == (-1, None)
+    assert _plan([_desc(100, 1, 1, kind=_native.PACK_LUT_I4, K=17, codes=0x7f0000000004)]) == (-1, None)
+    d = _desc(0, 1, 1, kind=_native.PACK_LUT_I4, K=17, codes=0, y=0)
+    d.lut_quotients = None
+    assert _plan([d]) == (0, 0)                                                           # empty: parameters unchecked
+    d = _desc(0, 1, 1, codes=0, y=0)
+    d.zp = None
+    assert _plan([d, _desc(100, 1, 1)]) == (1, 1)
     lib = _native.load()
     assert lib.mctq_unpack_plan(None, 1, None, 0) == -1 and lib.mctq_unpack_multi(None, None) == -1
 

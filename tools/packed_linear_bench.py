@@ -55,13 +55,12 @@ def make_items(kind, dtype, seed=0):
     """Random codes and per-channel parameters for the 96 matrices: UnpackPlan items (codes, kind, signed, dtype, shape,
     stride, C, inner, scale, zp, quotients)."""
     g = torch.Generator(device="cuda").manual_seed(seed)
-    lut = kind in (_native.PACK_LUT_U8, _native.PACK_LUT_I4)
+    lut = kind in _native.PACK_LUT_KINDS
     quot = ops.lut_quotients(torch.arange(-128, 128, 16, dtype=torch.float32), 8, True).cuda() if lut else None
     items = []
     for out_f, in_f in SHAPES:
         n = out_f * in_f
-        nb = n if kind in (_native.PACK_AFFINE_I8, _native.PACK_LUT_U8) else (n + 1) // 2
-        codes = torch.randint(0, 256, (nb,), dtype=torch.uint8, device="cuda", generator=g)
+        codes = torch.randint(0, 256, (_native.packed_code_bytes(kind, n),), dtype=torch.uint8, device="cuda", generator=g)
         if kind == _native.PACK_AFFINE_I4:                  # symmetric int4: codes in [-8, 7], both nibbles
             codes = codes & 0x77
         scale = torch.rand(out_f, device="cuda", generator=g) * 0.01 + 0.005
