@@ -23,6 +23,12 @@
  *     of x[0], so a caller can hand in any flat slice of a tensor (batch / channel-block shards,
  *     host-staging chunks) without re-deriving parameters.
  *   - dtype tags: MCTQ_F32 / MCTQ_BF16 / MCTQ_F16 describe x (and y for the affine ops).
+ *   - grouped multi-tensor plans (mctq_unpack_plan, mctq_lut_multi_plan) compile a HOST descriptor array into an opaque
+ *     HOST blob that travels as kernel parameters, so there is no device-side copy of the plan.  Grouping rule: the
+ *     tensors are sorted by kernel variant, and within a variant largest first (ties in descriptor order); a launch holds
+ *     one variant and a new launch starts after 64 tensors, or at a tensor with fewer than 1/16 of the tiles of the
+ *     launch's first (largest) tensor.  Each launch runs on a 2-D grid: one row of CTAs per tensor, as many CTAs per
+ *     row as its largest tensor has tiles.
  *   - arithmetic contract (bit-exact with CPU torch 2.11, see DESIGN.md):
  *       affine:  inv = 1.0f / s;  q = clamp(rint(x * inv) + zp, qmin, qmax);  y = (q - zp) * s
  *       lut:     t = clip((x / (thr + eps)) * 2^(bw - signed), lo, hi);  idx = first argmin_k |t - lut_k|;
@@ -131,9 +137,9 @@ int mctq_dequant_affine(const void* codes, int code_mode, int is_signed, float* 
  *                                                       index into the ORIGINAL centroid list (what mctq_fq_lut* emit)
  * mctq_unpack_plan compiles the HOST descriptor array into a HOST plan blob of mctq_unpack_plan_bytes(descs, n_desc) bytes
  * (returns the total number of tiles, or < 0: MCTQ_E_BADARG for a malformed descriptor or a code / output buffer that is not
- * 16-byte aligned, MCTQ_E_DTYPE, MCTQ_E_LUT for K outside 1..256 (1..16 for MCTQ_PACK_LUT_I4)).  Tensors are grouped by kernel
- * variant (kind, output dtype, channel mode, vector width); every group runs as launches of <= 64 tensors whose argument
- * blocks travel as kernel parameters.  Tensors with n == 0 are accepted and skipped.  codes, y and the parameter arrays
+ * 16-byte aligned, MCTQ_E_DTYPE, MCTQ_E_LUT for K outside 1..256 (1..16 for MCTQ_PACK_LUT_I4)).  Tensors are grouped by the
+ * plan grouping rule (Conventions above); the kernel variant is (kind, output dtype, channel mode, vector width).  Tensors
+ * with n == 0 are accepted and skipped.  codes, y and the parameter arrays
  * (device memory) must stay valid while the plan is in use; mctq_unpack_multi enqueues the launches on `stream`. */
 #define MCTQ_PACK_AFFINE_I8 1 /* one byte per element, int8 if is_signed else uint8 */
 #define MCTQ_PACK_AFFINE_I4 2 /* two per byte, element 2j in the low nibble (the MCTQ_CODES_INT4 layout) */
@@ -307,10 +313,9 @@ int mctq_fq_lut_prepared(const void* x, float* y, void* idx, int64_t n, int x_dt
  * weights_lut_pot_inferable_quantizer.py:74-104 calls).  Every tensor brings its own prepared blob (mctq_lut_prepare).
  * mctq_lut_multi_plan compiles the HOST descriptor array into an opaque plan blob of
  * mctq_lut_multi_plan_bytes(descs, n_desc) bytes in HOST memory (returns the number of CTAs of the launch, or < 0:
- * MCTQ_E_RANGE / MCTQ_E_BADARG mean "this tensor needs the single-tensor / generic entry point").  The launch passes the
- * per-tensor argument blocks as kernel parameters, so there is no device-side copy of the plan; the tensors are grouped by
- * kernel variant (dtype, channel mode, vector width, record kind) and every group runs as launches of <= 64 tensors, each
- * specialised for its variant (a model whose LUT weights share one layout is one launch per 64 tensors).
+ * MCTQ_E_RANGE / MCTQ_E_BADARG mean "this tensor needs the single-tensor / generic entry point").  Tensors are grouped by
+ * the plan grouping rule (Conventions above); the kernel variant is (dtype, channel mode, vector width, record kind), so a
+ * model whose LUT weights share one layout and similar sizes is one launch per 64 tensors.
  * x, y and the prepared blobs must stay valid while the plan is in use. */
 typedef struct MctqLutTensorDesc {
     const void* x;            /* device, dtype below, 16-byte aligned */

@@ -18,6 +18,7 @@
 
 #include "mctq_common.cuh"
 #include "mctq_lut_table.cuh"
+#include "mctq_plan.cuh"
 
 namespace mctq {
 
@@ -680,20 +681,12 @@ __global__ void __launch_bounds__(kThreads) fq_lutp_kernel(const __grid_constant
 // groups the tensors by variant.  The first version ran every variant out of one kernel (64 registers, 4 CTAs per SM, four
 // tiles per CTA to amortise the dispatch) and reached 6.3 TB/s on Llama-7B where the single-tensor kernels run at 6.6-6.7;
 // a specialised launch has the single-tensor kernel's registers and one tile per CTA.
-constexpr int kMultiMaxDesc = 64;
-struct alignas(16) LutPMultiEntry {
-    LutPArgs a;
+struct LutPMultiVariant {
+    int32_t dtype, chmode, v, xy, pad[3];
 };
 // The parameter block is copied by every launch, so its capacity is a template parameter: 16 / 64 tensors (2.5 / 10 KB).
 template <int CAP>
-struct LutPMultiParamsT {
-    int32_t n_desc, dtype, chmode, v;
-    int32_t xy, pad[3];
-    int32_t tiles[CAP + 4];                     // tiles[k] = tiles of tensor k; tiles[CAP] = the largest of them (grid x)
-    LutPMultiEntry e[CAP];
-};
-using LutPMultiParams = LutPMultiParamsT<kMultiMaxDesc>;
-static_assert(sizeof(LutPMultiParams) <= 32764, "kernel parameter space");
+using LutPMultiParamsT = PlanChunk<LutPMultiVariant, LutPArgs, CAP>;
 
 // 2-D grid: blockIdx.y = tensor, blockIdx.x = tile of that tensor (CTAs past a tensor's last tile exit at once; the host
 // only puts tensors of similar size into one launch).  No search: a first version found the tensor by a binary search
@@ -703,7 +696,7 @@ template <typename T, int CHMODE, int V, bool XY, int CAP>
 __global__ void __launch_bounds__(kThreads) fq_lut_multi_kernel(const __grid_constant__ LutPMultiParamsT<CAP> p) {
     const uint32_t k = blockIdx.y;
     if ((int32_t)blockIdx.x >= p.tiles[k]) return;
-    const LutPArgs& a = p.e[k].a;
+    const LutPArgs& a = p.e[k];
     if constexpr (XY) lutx_tile<T, CHMODE, MCTQ_CODES_NONE, 4, V>(a, (int64_t)blockIdx.x);
     else lutp_tile<T, CHMODE, MCTQ_CODES_NONE, 4, V>(a, (int64_t)blockIdx.x);
 }
@@ -1000,170 +993,84 @@ int mctq_fq_lut_prepared(const void* x, float* y, void* idx, int64_t n, int x_dt
     }
 }
 
-// ---- multi-tensor plan: a host blob [header][LutPMultiParams x n_chunks]; every chunk is one launch of up to kMultiMaxDesc tensors
 }  // extern "C"
 
 namespace {
-constexpr uint32_t kMultiMagic = 0x4d514c4du;   // 'MQLM'
-struct LutPMultiHeader {     // 64 bytes
-    uint32_t magic;
-    int32_t n_desc, n_chunks, span;
-    int64_t total_spans;
-    uint64_t smem_bytes;
-    int32_t reserved[8];
-};
-static_assert(sizeof(LutPMultiHeader) == 64, "multi header layout");
+
+using LutMultiPlan = Plan<LutPMultiVariant, LutPArgs, 0x4d514c4du>;   // 'MQLM'
 
 template <typename T, int CHMODE, int V, bool XY, int CAP>
-int launch_multi_variant(const LutPMultiParams& c, size_t smem, cudaStream_t st) {
-    static thread_local LutPMultiParamsT<CAP> p;             // up to 10 KB: not on the stack
-    p.n_desc = c.n_desc; p.dtype = c.dtype; p.chmode = c.chmode; p.v = c.v; p.xy = c.xy;
-    memcpy(p.tiles, c.tiles, (size_t)c.n_desc * sizeof(int32_t));
-    memcpy(p.e, c.e, (size_t)c.n_desc * sizeof(LutPMultiEntry));
+int launch_multi_variant(LutPMultiParamsT<CAP>& p, size_t smem, cudaStream_t st) {
     int rc = ensure_smem(fq_lut_multi_kernel<T, CHMODE, V, XY, CAP>, smem);
     if (rc) return rc;
     // ranges "unknown" (late order); the tables of all tensors may be staged before the wait unless a prepare kernel is in flight
     uint32_t te = 0;
     const IoSpan any_blob = {nullptr, 0};
     pdl_plan_launch(st, nullptr, 0, nullptr, 0, &any_blob, &te);
-    for (int i = 0; i < c.n_desc; ++i) p.e[i].a.tab_early = te;
-    return launch_planned(fq_lut_multi_kernel<T, CHMODE, V, XY, CAP>, dim3((unsigned)c.tiles[kMultiMaxDesc], (unsigned)c.n_desc), smem, st, p);
+    for (int i = 0; i < p.n_desc; ++i) p.e[i].tab_early = te;
+    return launch_planned(fq_lut_multi_kernel<T, CHMODE, V, XY, CAP>, dim3((unsigned)p.tiles[CAP], (unsigned)p.n_desc), smem, st, p);
 }
 
 template <typename T, int CAP>
-int launch_multi_typed(const LutPMultiParams& c, size_t smem, cudaStream_t st) {
+int launch_multi_typed(LutPMultiParamsT<CAP>& c, size_t smem, cudaStream_t st) {
     constexpr int V8 = sizeof(T) == 2 ? 8 : 4;
-    const bool wide = c.v == 8 && V8 == 8;
-    if (c.xy) {
-        if (c.chmode == CH_PT) return wide ? launch_multi_variant<T, CH_PT, V8, true, CAP>(c, smem, st) : launch_multi_variant<T, CH_PT, 4, true, CAP>(c, smem, st);
+    const bool wide = c.var.v == 8 && V8 == 8;
+    if (c.var.xy) {
+        if (c.var.chmode == CH_PT) return wide ? launch_multi_variant<T, CH_PT, V8, true, CAP>(c, smem, st) : launch_multi_variant<T, CH_PT, 4, true, CAP>(c, smem, st);
         return wide ? launch_multi_variant<T, CH_VEC, V8, true, CAP>(c, smem, st) : launch_multi_variant<T, CH_VEC, 4, true, CAP>(c, smem, st);
     }
-    if (c.chmode == CH_PT) return wide ? launch_multi_variant<T, CH_PT, V8, false, CAP>(c, smem, st) : launch_multi_variant<T, CH_PT, 4, false, CAP>(c, smem, st);
-    if (c.chmode == CH_VEC) return wide ? launch_multi_variant<T, CH_VEC, V8, false, CAP>(c, smem, st) : launch_multi_variant<T, CH_VEC, 4, false, CAP>(c, smem, st);
+    if (c.var.chmode == CH_PT) return wide ? launch_multi_variant<T, CH_PT, V8, false, CAP>(c, smem, st) : launch_multi_variant<T, CH_PT, 4, false, CAP>(c, smem, st);
+    if (c.var.chmode == CH_VEC) return wide ? launch_multi_variant<T, CH_VEC, V8, false, CAP>(c, smem, st) : launch_multi_variant<T, CH_VEC, 4, false, CAP>(c, smem, st);
     return launch_multi_variant<T, CH_ELEM, 4, false, CAP>(c, smem, st);
 }
 
 template <int CAP>
-int launch_multi_chunk(const LutPMultiParams& c, size_t smem, cudaStream_t st) {
-    if (c.dtype == MCTQ_F32) return launch_multi_typed<float, CAP>(c, smem, st);
-    if (c.dtype == MCTQ_BF16) return launch_multi_typed<__nv_bfloat16, CAP>(c, smem, st);
+int launch_multi_chunk(LutPMultiParamsT<CAP>& c, size_t smem, cudaStream_t st) {
+    if (c.var.dtype == MCTQ_F32) return launch_multi_typed<float, CAP>(c, smem, st);
+    if (c.var.dtype == MCTQ_BF16) return launch_multi_typed<__nv_bfloat16, CAP>(c, smem, st);
     return launch_multi_typed<__half, CAP>(c, smem, st);
 }
 
-constexpr int kMultiVariants = 3 * 3 * 2 * 2;            // dtype x channel mode x vector width x record kind
-inline int variant_key(int dtype, int chmode, int v, int xy) { return ((dtype * 3 + chmode) * 2 + (v == 8 ? 1 : 0)) * 2 + (xy ? 1 : 0); }
-
-size_t multi_bytes(int n_chunks) { return sizeof(LutPMultiHeader) + (size_t)n_chunks * sizeof(LutPMultiParams); }
-
-// validates every tensor and groups the tensors by kernel variant (one chunk = one launch = one variant, <= 64 tensors);
-// fills the chunks when `blob` is given; returns the number of chunks (or < 0)
-int64_t multi_compile(const MctqLutTensorDesc* descs, int n_desc, uint8_t* blob, int64_t* total_tiles_out) {
-    if (!descs || n_desc < 1) return MCTQ_E_BADARG;
-    std::vector<LutPArgs> args((size_t)n_desc);
-    std::vector<int> key((size_t)n_desc), chm((size_t)n_desc), vv((size_t)n_desc), xyv((size_t)n_desc);
-    std::vector<size_t> smem_of((size_t)n_desc);
-    for (int k = 0; k < n_desc; ++k) {
-        const MctqLutTensorDesc& d = descs[k];
-        if (d.n < 1 || !d.y) return MCTQ_E_BADARG;         // empty tensors do not belong in a plan
-        int rc = lutp_make_args(d.x, d.y, nullptr, d.n, d.dtype, d.prepared_dev, d.K, d.lut_values_bitwidth, d.is_signed, d.C, d.inner,
-                                0, MCTQ_CODES_NONE, &args[k]);
-        if (rc) return rc;
-        lutp_variant(args[k], d.dtype == MCTQ_F32 ? 4 : 2, MCTQ_CODES_NONE, &chm[k], &vv[k]);
-        size_t smem = 0;
-        rc = lutp_finish_args(args[k], chm[k], vv[k], &smem);
-        if (rc) return rc;
-        xyv[k] = lutx_eligible(args[k], chm[k], vv[k]) ? 1 : 0;
-        if (xyv[k]) smem = lutx_smem(args[k], chm[k]);
-        smem_of[k] = smem;
-        key[k] = variant_key(d.dtype, chm[k], vv[k], xyv[k]);
-    }
-    LutPMultiHeader* h = reinterpret_cast<LutPMultiHeader*>(blob);
-    LutPMultiParams* chunks = blob ? reinterpret_cast<LutPMultiParams*>(blob + sizeof(LutPMultiHeader)) : nullptr;
-    int n_chunks = 0;
-    int64_t total = 0;
-    size_t smem_max = 0;
-    for (int var = 0; var < kMultiVariants; ++var) {
-        // tensors of this variant, largest first: one launch holds <= 64 tensors whose tile counts are within a factor of 16
-        // (the grid is [largest tile count] x [tensors]; CTAs past a tensor's last tile exit immediately)
-        std::vector<std::pair<int64_t, int>> order;
-        for (int k = 0; k < n_desc; ++k) {
-            if (key[k] != var) continue;
-            const int64_t per_tile = (int64_t)kThreads * 4 * vv[k];
-            const int64_t tiles = (descs[k].n + per_tile - 1) / per_tile;
-            if (tiles > 0x7fffffffLL) return MCTQ_E_BADARG;
-            order.push_back({-tiles, k});
-        }
-        std::sort(order.begin(), order.end());
-        int in_chunk = 0;
-        int64_t first_tiles = 0;
-        for (const auto& it : order) {
-            const int64_t tiles = -it.first;
-            const int k = it.second;
-            if (in_chunk == kMultiMaxDesc || (in_chunk && tiles * 16 < first_tiles)) in_chunk = 0;
-            if (in_chunk == 0) {
-                first_tiles = tiles;
-                if (chunks) {
-                    LutPMultiParams& c = chunks[n_chunks];
-                    c.n_desc = 0; c.dtype = descs[k].dtype; c.chmode = chm[k]; c.v = vv[k]; c.xy = xyv[k];
-                    c.tiles[kMultiMaxDesc] = (int32_t)tiles;
-                }
-                ++n_chunks;
-            }
-            if (chunks) {
-                LutPMultiParams& c = chunks[n_chunks - 1];
-                c.e[in_chunk].a = args[k];
-                c.tiles[in_chunk] = (int32_t)tiles;
-                c.n_desc = in_chunk + 1;
-            }
-            ++in_chunk;
-            total += tiles;
-            if (smem_of[k] > smem_max) smem_max = smem_of[k];
-        }
-    }
-    if (h) {
-        h->magic = kMultiMagic;
-        h->n_desc = n_desc;
-        h->n_chunks = n_chunks;
-        h->span = 1;
-        h->total_spans = total;
-        h->smem_bytes = smem_max;
-    }
-    if (total_tiles_out) *total_tiles_out = total;
-    return n_chunks;
+// argument block, variant, tiles and shared memory of one tensor (validated); 0 or MCTQ_E_*
+int multi_describe(const MctqLutTensorDesc& d, LutMultiPlan::Item& it) {
+    if (d.n < 1 || !d.y) return MCTQ_E_BADARG;         // empty tensors do not belong in a plan
+    LutPArgs& a = it.args;
+    int rc = lutp_make_args(d.x, d.y, nullptr, d.n, d.dtype, d.prepared_dev, d.K, d.lut_values_bitwidth, d.is_signed, d.C, d.inner,
+                            0, MCTQ_CODES_NONE, &a);
+    if (rc) return rc;
+    int chmode, v;
+    lutp_variant(a, d.dtype == MCTQ_F32 ? 4 : 2, MCTQ_CODES_NONE, &chmode, &v);
+    rc = lutp_finish_args(a, chmode, v, &it.smem);
+    if (rc) return rc;
+    const int xy = lutx_eligible(a, chmode, v) ? 1 : 0;
+    if (xy) it.smem = lutx_smem(a, chmode);
+    it.var = {d.dtype, chmode, v, xy, {}};
+    const int64_t per_tile = (int64_t)kThreads * 4 * v;
+    it.tiles = (d.n + per_tile - 1) / per_tile;
+    return 0;
 }
+
 }  // namespace
 
 extern "C" {
 
 size_t mctq_lut_multi_plan_bytes(const MctqLutTensorDesc* descs, int n_desc) {
-    const int64_t chunks = multi_compile(descs, n_desc, nullptr, nullptr);
-    if (chunks < 1) return 0;
-    return multi_bytes((int)chunks);
+    LutMultiPlan plan;
+    return plan.compile(descs, n_desc, multi_describe) ? 0 : plan.bytes();
 }
 
 int64_t mctq_lut_multi_plan(const MctqLutTensorDesc* descs, int n_desc, void* plan_host_out, size_t plan_bytes) {
-    const int64_t chunks = multi_compile(descs, n_desc, nullptr, nullptr);
-    if (chunks < 0) return chunks;
-    if (!plan_host_out || plan_bytes < multi_bytes((int)chunks)) return MCTQ_E_BADARG;
-    memset(plan_host_out, 0, multi_bytes((int)chunks));
-    int64_t total = 0;
-    const int64_t rc = multi_compile(descs, n_desc, reinterpret_cast<uint8_t*>(plan_host_out), &total);
-    return rc < 0 ? rc : total;
+    LutMultiPlan plan;
+    if (const int rc = plan.compile(descs, n_desc, multi_describe)) return rc;
+    plan.h.tiles_per_cta = 1;
+    return plan.write(plan_host_out, plan_bytes);
 }
 
 int mctq_fq_lut_prepared_multi(const void* plan_host, void* stream) {
     MCTQ_NVTX("mctq_fq_lut_prepared_multi");
-    if (!plan_host) return MCTQ_E_BADARG;
-    const LutPMultiHeader* h = reinterpret_cast<const LutPMultiHeader*>(plan_host);
-    if (h->magic != kMultiMagic || h->n_desc < 1 || h->n_chunks < 1) return MCTQ_E_BADARG;
-    const LutPMultiParams* chunks = reinterpret_cast<const LutPMultiParams*>(reinterpret_cast<const uint8_t*>(plan_host) + sizeof(LutPMultiHeader));
-    const size_t smem = (size_t)h->smem_bytes;
-    for (int c = 0; c < h->n_chunks; ++c) {
-        const LutPMultiParams& p = chunks[c];
-        const int rc = p.n_desc <= 16 ? launch_multi_chunk<16>(p, smem, (cudaStream_t)stream) : launch_multi_chunk<kMultiMaxDesc>(p, smem, (cudaStream_t)stream);
-        if (rc) return rc;
-    }
-    return 0;
+    return LutMultiPlan::run<16>(plan_host, 1, [&](auto& p, const PlanHeader& h) {
+        return launch_multi_chunk(p, (size_t)h.smem_bytes, (cudaStream_t)stream);
+    });
 }
 
 }  // extern "C"

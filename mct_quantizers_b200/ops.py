@@ -1226,6 +1226,23 @@ class ScalarSitesPlan:
         return self.outputs
 
 
+def _compile_plan(plan_bytes, plan, descs, n_desc, buf=None):
+    """Compile a descriptor array into a host plan blob with a (`*_plan_bytes`, `*_plan`) pair of the C ABI, reusing `buf`
+    when it is large enough.  Returns (blob, total tiles, launches): launches = n_chunks of the 64-byte blob header, one per
+    kernel variant and 64 tensors."""
+    p = ctypes.cast(descs, c_vp)
+    nb = plan_bytes(p, n_desc)
+    if nb == 0:
+        total = plan(p, n_desc, None, 0)
+    else:
+        if buf is None or len(buf) < nb:
+            buf = (ctypes.c_uint8 * nb)()
+        total = plan(p, n_desc, ctypes.cast(buf, c_vp), len(buf))
+    if total < 0:
+        raise MctqError(f"{plan.__name__}: {_native.ERRORS.get(total, total)}")
+    return buf, int(total), ctypes.c_int32.from_buffer(buf, 8).value
+
+
 class LutMultiPlan:
     """One-launch LUT fake-quant of many weight tensors (C ABI: mctq_lut_multi_plan + mctq_fq_lut_prepared_multi).
 
@@ -1296,16 +1313,9 @@ class LutMultiPlan:
             self.inputs.append(got[1])
             self.outputs.append(y)
             self._keep.append(got[2])
-        nb = lib.mctq_lut_multi_plan_bytes(ctypes.cast(descs, c_vp), len(items))
-        if nb == 0:
-            raise MctqError("mctq_lut_multi_plan_bytes: a tensor of the plan is outside the prepared LUT path")
-        self._plan_host = (ctypes.c_uint8 * nb)()
-        total = lib.mctq_lut_multi_plan(ctypes.cast(descs, c_vp), len(items), ctypes.cast(self._plan_host, c_vp), nb)
-        if total <= 0:
-            raise MctqError(f"mctq_lut_multi_plan: {total}")
-        self.total_tiles = int(total)
         self.n_desc = len(items)
-        self.n_launches = int(np.frombuffer(bytes(self._plan_host[:16]), dtype=np.int32)[2])    # one per kernel variant and 64 tensors
+        self._plan_host, self.total_tiles, self.n_launches = _compile_plan(lib.mctq_lut_multi_plan_bytes, lib.mctq_lut_multi_plan,
+                                                                           descs, self.n_desc)
 
     def run(self):
         lib = _native.load()
@@ -1355,7 +1365,7 @@ class UnpackPlan:
                                                 f"tensor {k}")
             self._keep.append(keep)
             self._out_specs.append((tuple(int(v) for v in shape), None if stride is None else tuple(int(v) for v in stride), dtype))
-        self._plan_host, self._plan_nb, self.fresh = None, 0, fresh
+        self._plan_host, self.fresh = None, fresh
         if fresh:
             if outputs is not None:
                 raise ValueError("a fresh UnpackPlan allocates its outputs on every run")
@@ -1379,17 +1389,9 @@ class UnpackPlan:
     def _install(self, outputs, lib):
         for d, y in zip(self._descs, outputs):
             d.y = y.data_ptr() if y.numel() else None
-        descs = ctypes.cast(self._descs, c_vp)
-        nb = lib.mctq_unpack_plan_bytes(descs, self.n_desc)
-        if nb == 0:
-            raise MctqError(f"mctq_unpack_plan: {_native.ERRORS.get(lib.mctq_unpack_plan(descs, self.n_desc, None, 0), 'rejected')}")
-        if nb > self._plan_nb:
-            self._plan_host, self._plan_nb = (ctypes.c_uint8 * nb)(), nb
-        total = lib.mctq_unpack_plan(descs, self.n_desc, ctypes.cast(self._plan_host, c_vp), self._plan_nb)
-        if total < 0:
-            raise MctqError(f"mctq_unpack_plan: {_native.ERRORS.get(total, total)}")
-        self.total_tiles = int(total)
-        self.n_launches = ctypes.c_int32.from_buffer(self._plan_host, 8).value      # one per kernel variant and 64 tensors
+        self._plan_host, self.total_tiles, self.n_launches = _compile_plan(lib.mctq_unpack_plan_bytes, lib.mctq_unpack_plan,
+                                                                           self._descs, self.n_desc, self._plan_host)
+        self._plan_nb = len(self._plan_host)
         self.outputs = outputs
 
     def run(self):
