@@ -199,6 +199,39 @@ int mctq_packed_linear(const MctqPackedDesc* w, int64_t out_features, int64_t in
 int mctq_packed_linear_batched(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x, int x_dtype,
                                int64_t M, const void* bias, void* y, const float* lut_quotients_host, void* stream);
 
+/* Integer linear mode (packed nn.Linear wrappers whose input comes from a per-tensor 8-bit affine activation quantizer Q).
+ * Both operands of the product are integer codes: x = sx * (qx - zx), W = sw[o] * (qw - zw[o]).
+ *
+ * mctq_quantize_rows_i8: qx [M][K] (row-major, one byte per element: int8 if qmin < 0 else uint8) of x [M][K] (x_dtype,
+ * row-major), by the recipe of mctq_fq_affine_scalar with code_mode MCTQ_CODES_INT8 -- the same codes bit for bit, NaN -> qmin,
+ * +-inf clamped -- and, when rowsum is not NULL, Sx[n] = sum_k qx[n,k] (int32).  scale is Q's scale narrowed to f32.
+ * MCTQ_E_BADARG (null x / codes, M < 0, K < 1), MCTQ_E_DTYPE, MCTQ_E_RANGE (qmin > qmax or a range that does not fit 8-bit
+ * codes) before any CUDA call; M == 0 is a no-op.
+ *
+ * mctq_packed_linear_i8: y[n, o] for n < M, o < out_features, rows of y ldy elements apart (ldy >= out_features; nothing else
+ * of y is written), computed as
+ *   acc = sum_k qx[n,k] * qw[o,k]                                  int32, exact (tcgen05.mma kind::i8)
+ *   c   = acc - zw[o] * Sx[n] - zx * Sw[o] + K * zx * zw[o]       int64, exact;  Sx / Sw: row sums of the codes
+ *   y   = T(fl(fl((float)c * f[o]) + bias[o]))                     T = y_dtype; f[o] = fl32(sx * sw[o]) supplied by the caller
+ *   w          HOST descriptor of an MCTQ_PACK_AFFINE_I8 / _I4 weight [out][in], per tensor or per output row (as for
+ *              mctq_packed_linear); w->y_dtype == y_dtype; codes 16-byte aligned; w->scale is not read (f replaces it)
+ *   x_codes    device qx [M][in_features], 16-byte aligned; x_signed: int8 (1) or uint8 (0) codes; x_zero_point = zx
+ *   x_rowsum   device Sx [M], or NULL when every weight zero point is 0 (the term is then skipped)
+ *   w_rowsum   device Sw [out_features] (int32), needed when zx != 0
+ *   factor     device f [C] (C = w->C); bias: device [out_features] of y_dtype, or NULL
+ * Every output bit is fixed by the formula: the result does not depend on the split of the row length or the tiling, and
+ * two calls give the same bits.  Returns, before any CUDA call: MCTQ_E_BADARG for a LUT kind, a null pointer, a shape or
+ * layout error, in_features not a multiple of 16 (32 for int4 weights), ldy < out_features or unaligned codes;
+ * MCTQ_E_DTYPE; MCTQ_E_RANGE for a zx outside the x codes' range or in_features above
+ * mctq_packed_linear_i8_max_k(w->is_signed, x_signed) (the largest K whose int32 sum cannot overflow: 33025 for uint8 x
+ * uint8, 65793 for one signed operand, 131071 for int8 x int8).  M == 0 is a no-op. */
+int mctq_quantize_rows_i8(const void* x, int x_dtype, int64_t M, int64_t K, float scale, int32_t zp, int32_t qmin,
+                          int32_t qmax, void* codes, int32_t* rowsum, void* stream);
+int64_t mctq_packed_linear_i8_max_k(int w_signed, int x_signed);
+int mctq_packed_linear_i8(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x_codes,
+                          int x_signed, int32_t x_zero_point, int64_t M, const int32_t* x_rowsum, const int32_t* w_rowsum,
+                          const float* factor, const void* bias, int y_dtype, void* y, int64_t ldy, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Whole-model weight quantisation: one launch over a table of tensors (SURVEY 8f rank 1).
  * Replaces the per-layer loop  for name, w, quantizer in self._weights_vars: quantizer(w)

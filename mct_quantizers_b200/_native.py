@@ -18,6 +18,12 @@ PACK_AFFINE_I8, PACK_AFFINE_I4, PACK_LUT_U8, PACK_LUT_I4 = 1, 2, 3, 4
 PACK_LUT_KINDS = (PACK_LUT_U8, PACK_LUT_I4)
 
 
+def integer_linear_max_k(w_signed, x_signed):
+    """Largest in_features of mctq_packed_linear_i8 for the (weight, x) code signedness: the int32 sum of code products
+    cannot overflow (the values of mctq_packed_linear_i8_max_k)."""
+    return 131071 if (w_signed and x_signed) else 65793 if (w_signed or x_signed) else 33025
+
+
 def packed_code_bytes(kind, n):
     """Bytes of the codes of n elements of packed kind `kind`: one per element, or one per two for int4 codes and 4-bit
     LUT indices."""
@@ -73,6 +79,10 @@ SIGNATURES = {
     "mctq_unpack_multi": (c_int, [c_vp, c_vp]),
     "mctq_packed_linear": (c_int, [c_vp, c_i64, c_i64, c_vp, c_int, c_i64, c_vp, c_vp, c_vp]),
     "mctq_packed_linear_batched": (c_int, [c_vp, c_i64, c_i64, c_vp, c_int, c_i64, c_vp, c_vp, c_vp, c_vp]),
+    "mctq_quantize_rows_i8": (c_int, [c_vp, c_int, c_i64, c_i64, c_f32, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp]),
+    "mctq_packed_linear_i8_max_k": (c_i64, [c_int, c_int]),
+    "mctq_packed_linear_i8": (c_int, [c_vp, c_i64, c_i64, c_vp, c_int, c_i32, c_i64, c_vp, c_vp, c_vp, c_vp, c_int, c_vp,
+                                      c_i64, c_vp]),
     "mctq_multi_tile_elems": (c_i64, []),
     "mctq_multi_plan": (c_i64, [c_vp, c_int, c_vp]),
     "mctq_fq_affine_multi": (c_int, [c_vp, c_vp, c_int, c_i64, c_vp]),

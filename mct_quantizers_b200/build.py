@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
-SOURCES = ["mctq_affine.cu", "mctq_lut.cu", "mctq_lutp.cu", "mctq_fused.cu", "mctq_unpack.cu", "mctq_packed_linear.cu", "mctq_packed_gemm.cu", "mctq_host.cu"]
+SOURCES = ["mctq_affine.cu", "mctq_lut.cu", "mctq_lutp.cu", "mctq_fused.cu", "mctq_unpack.cu", "mctq_packed_linear.cu", "mctq_packed_gemm.cu", "mctq_packed_igemm.cu", "mctq_host.cu"]
 OBJ_DIR = os.path.join(HERE, "csrc", "_obj")
 INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(HERE, "libmctq_sm100.so")

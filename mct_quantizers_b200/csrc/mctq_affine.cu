@@ -1,4 +1,6 @@
 // mctq_affine.cu -- affine (round-clip-dequant) fake-quant kernels and their C ABI entry points.
+#include <algorithm>
+
 #include "mctq_common.cuh"
 
 namespace mctq {
@@ -622,6 +624,57 @@ __global__ void __launch_bounds__(kThreads) fq_affine_sites_kernel(const __grid_
     else { if (fast) site_tile<__half, false>(s, t); else site_tile<__half, true>(s, t); }
 }
 
+// ---- 8-bit codes of a [M][K] row-major x and their row sums (integer linear mode, mctq_packed_igemm.cu): one warp per row,
+// the per-tensor recipe of fq_affine_kernel (AffineOp<false>::apply), so the codes are those mctq_fq_affine_scalar emits.
+// VEC: K % 8 == 0 and x 16-byte aligned: 8 elements per lane and step (one or two 16-byte loads, one 8-byte store).
+template <typename T, bool VEC>
+__global__ void __launch_bounds__(kThreads) quantize_rows_kernel(const T* __restrict__ x, uint8_t* __restrict__ codes,
+                                                                  int32_t* __restrict__ rowsum, int64_t M, int64_t K,
+                                                                  float scale, int32_t zp, int32_t qmin, int32_t qmax) {
+    using Op = AffineOp<false>;
+    AffineArgs a;                                   // only the fields AffineOp::make reads
+    a.qmin = qmin;
+    a.qmax = qmax;
+    const Op::ChanParams p = Op::make(scale, zp, a);
+    pdl_wait();
+    pdl_launch_dependents();
+    const int warps = kThreads / 32, lane = threadIdx.x & 31;
+    for (int64_t row = (int64_t)blockIdx.x * warps + (threadIdx.x >> 5); row < M; row += (int64_t)gridDim.x * warps) {
+        const T* xr = x + row * K;
+        uint8_t* cr = codes + row * K;
+        int32_t sum = 0;
+        if (VEC) {
+            constexpr int W = 8 * sizeof(T) / 4;    // 32-bit words of 8 elements
+            for (int64_t k = 8 * lane; k < K; k += 256) {
+                uint32_t w[W];
+                ld_words<4>(xr + k, w);
+                if (W == 8) ld_words<4>(xr + k + 4, w + 4);
+                float f[8];
+                Pack<T, 8>::unpack(w, f);
+                int c[8];
+#pragma unroll
+                for (int e = 0; e < 8; ++e) {
+                    Op::template apply<true>(f[e], p, c[e]);
+                    sum += c[e];
+                }
+                st_codes<8, MCTQ_CODES_INT8>(cr, k, c);
+            }
+        } else {
+            for (int64_t k = lane; k < K; k += 32) {
+                int c;
+                Op::template apply<true>(to_f32<T>(xr[k]), p, c);
+                sum += c;
+                cr[k] = (uint8_t)(c & 0xff);
+            }
+        }
+        if (rowsum) {
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, d);
+            if (lane == 0) rowsum[row] = sum;
+        }
+    }
+}
+
 }  // namespace mctq
 
 using namespace mctq;
@@ -825,6 +878,29 @@ int mctq_fq_affine_scalar(const void* x, void* y, void* codes, int64_t n, int x_
     a.x = x; a.y = y; a.codes = codes; a.n = n; a.scale = nullptr; a.zp = nullptr; a.scale_val = scale; a.zp_val = zp;
     a.C = 1; a.inner = 1; a.elem_offset = 0; a.qmin = qmin; a.qmax = qmax;
     return launch_affine(a, x_dtype, code_mode, (cudaStream_t)stream);
+}
+
+int mctq_quantize_rows_i8(const void* x, int x_dtype, int64_t M, int64_t K, float scale, int32_t zp, int32_t qmin,
+                          int32_t qmax, void* codes, int32_t* rowsum, void* stream) {
+    MCTQ_NVTX("mctq_quantize_rows_i8");
+    if (!x || !codes || M < 0 || K < 1) return MCTQ_E_BADARG;
+    if (x_dtype != MCTQ_F32 && x_dtype != MCTQ_BF16 && x_dtype != MCTQ_F16) return MCTQ_E_DTYPE;
+    if (qmin > qmax) return MCTQ_E_RANGE;
+    if (int rc = check_codes(qmin, qmax, MCTQ_CODES_INT8, codes)) return rc;
+    if (M == 0) return 0;
+    const int64_t blocks = std::min<int64_t>((M + kThreads / 32 - 1) / (kThreads / 32), 148 * 16);
+    const bool vec = K % 8 == 0 && aligned16(x) && (reinterpret_cast<uintptr_t>(codes) & 7u) == 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    auto run = [&](auto type) {
+        using T = typename decltype(type)::type;
+        const T* xt = reinterpret_cast<const T*>(x);
+        uint8_t* c = reinterpret_cast<uint8_t*>(codes);
+        if (vec) return launch_streaming(quantize_rows_kernel<T, true>, (unsigned)blocks, 0, st, xt, c, rowsum, M, K, scale, zp, qmin, qmax);
+        return launch_streaming(quantize_rows_kernel<T, false>, (unsigned)blocks, 0, st, xt, c, rowsum, M, K, scale, zp, qmin, qmax);
+    };
+    if (x_dtype == MCTQ_F32) return run(PackType<float>{});
+    if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});
+    return run(PackType<__half>{});
 }
 
 int mctq_dequant_affine(const void* codes, int code_mode, int is_signed, float* y, int64_t n, const float* scale,

@@ -19,9 +19,10 @@
 // leave their partial sums in their shared memory and rank 0 adds them to its own in rank order (distributed shared
 // memory), so the result is deterministic with no workspace.  The epilogue (tcgen05.ld) gives each thread one output feature,
 // so stores of consecutive lanes coalesce.
+#include <algorithm>
 #include <type_traits>
 
-#include "mctq_common.cuh"
+#include "mctq_tcgen05.cuh"
 
 namespace mctq {
 
@@ -46,37 +47,6 @@ struct GemmArgs {
     int32_t fast_codes, fast_x;  // vector loads (K % 8 == 0 and aligned bases)
     float quot[256];             // LUT quotients (bf16-exact; entries past the table's K are 0)
 };
-
-__device__ __forceinline__ uint32_t cluster_rank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ uint32_t cluster_size() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t peer_addr(uint32_t local_addr, uint32_t rank) {
-    uint32_t a;
-    asm("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(local_addr), "r"(rank));
-    return a;
-}
-// ordered after the cluster barrier by its acquire (asm volatile keeps it below); no memory clobber, so loads overlap
-__device__ __forceinline__ float ld_peer(uint32_t cluster_addr) {
-    float v;
-    asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(v) : "r"(cluster_addr));
-    return v;
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// shared-memory matrix descriptor: K-major, 128-byte swizzle, 8-row groups 1024 bytes apart (sm_100 descriptor version 1)
-__device__ __forceinline__ uint64_t sw128_desc(uint32_t saddr) {
-    return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) |
-           ((uint64_t)2 << 61);
-}
-// byte offset of the 16-byte group j (8 elements) of row r inside a stage operand: Swizzle<3,4,3> on 1024-byte atoms
-__device__ __forceinline__ uint32_t sw128_off(uint32_t r, uint32_t j) { return r * 128u + ((j ^ (r & 7u)) << 4); }
-
-__device__ __forceinline__ void st_shared_v4(uint32_t addr, const uint32_t* w) {
-    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" :: "r"(addr), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]) : "memory");
-}
 
 // x0 + x1 + x2 == x (bf16 terms by truncation; exact for finite x above bf16's subnormal grain), x1 = x2 = 0 for inf / NaN
 __device__ __forceinline__ void split3(float x, float& x0, float& x1, float& x2) {
@@ -296,11 +266,7 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
     auto tmem_block = [&](int cb, float* v) {
         if (have) {
             uint32_t u[16];
-            asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                         : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7]),
-                           "=r"(u[8]), "=r"(u[9]), "=r"(u[10]), "=r"(u[11]), "=r"(u[12]), "=r"(u[13]), "=r"(u[14]), "=r"(u[15])
-                         : "r"(taddr + 16 * cb));
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            tmem_ld16(taddr + 16 * cb, u);
 #pragma unroll
             for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(u[j]);
         } else {
@@ -371,16 +337,11 @@ int launch_gemm(GemmArgs a, cudaStream_t st) {
     const int64_t per = (M + ntiles - 1) / ntiles;
     a.nt = (int32_t)((per + 15) / 16 * 16);
     a.nchunks = (int32_t)((a.K + kChunk - 1) / kChunk);
-    uint32_t cols = 32;
-    while (cols < (uint32_t)a.nt) cols *= 2;
-    a.tmem_cols = cols;
+    a.tmem_cols = tmem_columns(a.nt);
     const int64_t tiles = (a.N + kGemmRows - 1) / kGemmRows;
     const size_t stage = (size_t)kGemmRows * 128 + (size_t)TERMS * a.nt * 128;
     size_t smem = kStages * stage + 1024;                                   // + alignment of the stages to 1024 bytes
-    // co-resident CTAs must fit the SM's 512 TMEM columns: ask for enough shared memory that no more fit
-    const size_t sm_bytes = 228 * 1024, max_ctas = 512 / cols;
-    const size_t floor_smem = sm_bytes / (max_ctas + 1) + 1 - 1024 + 256;
-    if (smem < floor_smem) smem = floor_smem;
+    smem = std::max(smem, tmem_smem_floor(a.tmem_cols));              // co-resident CTAs must fit the SM's TMEM
     auto kernel = packed_gemm_kernel<KIND, T>;
     int rc = ensure_smem(kernel, smem);                                     // per device: set on every launch
     if (rc) return rc;

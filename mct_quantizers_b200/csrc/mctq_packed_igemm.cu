@@ -1,0 +1,389 @@
+// mctq_packed_igemm.cu -- integer linear mode: y = T(((acc - corrections) * f) + b) with acc = sum_k qx[n,k] * qw[o,k] an
+// exact int32 product of 8-bit activation codes and packed int8 / int4 weight codes on the tensor cores
+// (tcgen05.mma kind::i8, s32 accumulator in tensor memory).  Packed nn.Linear wrappers in integer mode
+// (pytorch/packed_weights.py) call it after mctq_quantize_rows_i8 has turned their input into codes.
+//
+// Shape (as in mctq_packed_gemm.cu): output features are the MMA's M (128 per CTA), batch rows its N (nt, a multiple of 16 up
+// to 256; more rows run as further CTAs along grid.y).  A CTA walks its share of the row length in chunks of 128 codes (one
+// 128-byte swizzle row) through a ring of `stages` shared-memory stages with a full and an empty mbarrier each:
+//   warps 0-3  producers: thread 0 arms the stage's full barrier and copies the x codes (and int8 weight codes) with 2-D TMA
+//              (SWIZZLE_128B, zero fill outside the tensor: tail rows and columns are zero codes); for int4 weights the 128
+//              producer threads each load one weight row's nibbles and expand them to bytes into the stage (sign extension
+//              for signed codes) and arrive on the full barrier
+//   warp 4     lane 0 issues the stage's four MMAs (K = 32 each) and commits them onto the stage's empty barrier
+//   all warps  the epilogue: tcgen05.ld, one output feature per thread, corrections and scaling in the fixed formula
+//              c = acc - zw[o] * Sx[n] - zx * Sw[o] + K * zx * zw[o]  (int64),   y = T(fl(fl((float)c * f[o]) + b[o]))
+// There is no CTA-wide barrier in the main loop.  Split-K: the S CTAs of a cluster take consecutive chunk ranges and rank 0
+// adds the int32 partial sums of the others (distributed shared memory); integer sums are exact, so the result does not
+// depend on S or on the tiling.
+#include <cuda.h>               // CUtensorMap and the cuTensorMapEncodeTiled types (the entry point is fetched at run time)
+
+#include <algorithm>
+
+#include "mctq_tcgen05.cuh"
+
+namespace mctq {
+
+constexpr int kIRows = 128;           // output features per CTA (the MMA's M)
+constexpr int kIChunk = 128;          // codes of the row length per stage
+constexpr int kIMinStages = 4, kIMaxStages = 8;
+constexpr int kIMaxSplit = 8;         // portable cluster size
+constexpr int kIProducers = 128;      // warps 0-3
+constexpr int kIMmaWarp = 4;
+
+struct IgemmArgs {
+    CUtensorMap tm_x;                 // x codes [M_total][K], box [nt][128]
+    CUtensorMap tm_w;                 // int8 weight codes [N][K], box [128][128] (int4 weights: unused)
+    const uint8_t* codes;             // int4 weight codes, two per byte
+    const int32_t* w_zp;              // zw[C]
+    const int32_t* x_rowsum;          // Sx[M_total], or null when every zw is 0
+    const int32_t* w_rowsum;          // Sw[N], or null when zx is 0
+    const float* factor;              // f[C]
+    const void* bias;                 // [N] of T, or null
+    void* y;                          // [M_total] rows of ldy elements
+    int64_t ldy;
+    int64_t m0;                       // first row of this launch
+    int64_t M;                        // rows of this launch
+    int32_t N, K;
+    int32_t per_channel, x_zp;
+    int32_t nt, nchunks, stages;
+    uint32_t stage_bytes, tmem_cols, idesc;
+};
+
+__device__ __forceinline__ void tma_2d(const CUtensorMap* map, uint32_t dst, int32_t c0, int32_t c1, uint64_t* bar) {
+    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
+                 :: "r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(smem_u32(bar)) : "memory");
+}
+
+// 8 nibbles (element 2j in the low nibble of byte j) -> 8 bytes, sign-extended when SIGNED
+template <bool SIGNED>
+__device__ __forceinline__ void expand8(uint32_t w, uint32_t& lo, uint32_t& hi) {
+    const uint32_t ev = w & 0x0F0F0F0Fu, od = (w >> 4) & 0x0F0F0F0Fu;
+    lo = __byte_perm(ev, od, 0x5140);
+    hi = __byte_perm(ev, od, 0x7362);
+    if (SIGNED) {
+        lo |= (lo & 0x08080808u) * 0x1Eu;                                // 0x08 * 0x1E = 0xF0: no carry between bytes
+        hi |= (hi & 0x08080808u) * 0x1Eu;
+    }
+}
+
+template <bool INT4, bool WSIGNED, typename T>
+__global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_constant__ IgemmArgs a) {
+    extern __shared__ __align__(1024) uint8_t dsm[];
+    __shared__ uint64_t bar_full[kIMaxStages], bar_empty[kIMaxStages];
+    __shared__ uint64_t bar_done;
+    __shared__ uint32_t tmem_slot;
+
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int nt = a.nt, nst = a.stages;
+    const uint32_t a_bytes = kIRows * 128, stage_bytes = a.stage_bytes;
+    const uint32_t sbase = (smem_u32(dsm) + 1023u) & ~1023u;             // swizzle atoms need 1024-byte alignment
+
+    pdl_wait();                 // x codes may be the output of the previous launch; TMEM is taken only after the wait
+    pdl_launch_dependents();
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(&tmem_slot)), "r"(a.tmem_cols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    if (tid == 0) {
+        for (int s = 0; s < nst; ++s) {
+            mbar_init(&bar_full[s], INT4 ? 1 + kIProducers : 1);
+            mbar_init(&bar_empty[s], 1);
+        }
+        mbar_init(&bar_done, 1);
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = tmem_slot;
+
+    const uint32_t S = cluster_size(), rank = cluster_rank();
+    const int64_t N = a.N, K = a.K;
+    const int64_t o0 = (int64_t)(blockIdx.x / S) * kIRows;
+    const int64_t n0 = (int64_t)blockIdx.y * nt;                         // first row of this CTA inside the launch
+    const int64_t rows = a.M - n0 < nt ? a.M - n0 : nt;
+    const int c_begin = (int)((int64_t)a.nchunks * rank / S), c_end = (int)((int64_t)a.nchunks * (rank + 1) / S);
+    const int nloc = c_end - c_begin;
+
+    if (warp < 4) {
+        // ---- producers
+        if (INT4) {
+            const int64_t o = o0 + tid;
+            const uint8_t* wrow = a.codes + o * (K >> 1);
+            auto load = [&](int c, uint4* v) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {                            // 32 codes per 16 bytes; K % 32 == 0
+                    const int64_t k = (int64_t)c * kIChunk + 32 * j;
+                    v[j] = (o < N && k < K) ? ld_stream(reinterpret_cast<const uint4*>(wrow + (k >> 1))) : make_uint4(0, 0, 0, 0);
+                }
+            };
+            uint4 cur[4], nxt[4];
+            if (nloc > 0) load(c_begin, cur);
+            for (int i = 0; i < nloc; ++i) {
+                const int c = c_begin + i, s = i % nst;
+                const uint32_t st = sbase + (uint32_t)s * stage_bytes;
+                if (i + 1 < nloc) load(c + 1, nxt);                     // in flight while this stage is filled
+                if (i >= nst) mbar_wait(&bar_empty[s], (uint32_t)((i / nst - 1) & 1));
+                if (tid == 0) {
+                    mbar_arrive_expect_tx(&bar_full[s], (uint32_t)nt * 128u);
+                    tma_2d(&a.tm_x, st + a_bytes, c * kIChunk, (int32_t)(a.m0 + n0), &bar_full[s]);
+                }
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const uint32_t words[4] = {cur[j].x, cur[j].y, cur[j].z, cur[j].w};
+                    uint32_t g[8];
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) expand8<WSIGNED>(words[q], g[2 * q], g[2 * q + 1]);
+                    st_shared_v4(st + sw128_off((uint32_t)tid, 2 * j), g);
+                    st_shared_v4(st + sw128_off((uint32_t)tid, 2 * j + 1), g + 4);
+                }
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");    // generic-proxy stores -> tensor-core reads
+                mbar_arrive(&bar_full[s]);
+#pragma unroll
+                for (int j = 0; j < 4; ++j) cur[j] = nxt[j];
+            }
+        } else if (tid == 0) {
+            for (int i = 0; i < nloc; ++i) {
+                const int c = c_begin + i, s = i % nst;
+                const uint32_t st = sbase + (uint32_t)s * stage_bytes;
+                if (i >= nst) mbar_wait(&bar_empty[s], (uint32_t)((i / nst - 1) & 1));
+                mbar_arrive_expect_tx(&bar_full[s], a_bytes + (uint32_t)nt * 128u);
+                tma_2d(&a.tm_w, st, c * kIChunk, (int32_t)o0, &bar_full[s]);
+                tma_2d(&a.tm_x, st + a_bytes, c * kIChunk, (int32_t)(a.m0 + n0), &bar_full[s]);
+            }
+        }
+    } else if (warp == kIMmaWarp && lane == 0) {
+        // ---- MMA issuer
+        for (int i = 0; i < nloc; ++i) {
+            const int s = i % nst;
+            const uint32_t st = sbase + (uint32_t)s * stage_bytes;
+            mbar_wait(&bar_full[s], (uint32_t)((i / nst) & 1));
+            tc_fence_after();
+#pragma unroll
+            for (int ks = 0; ks < kIChunk / 32; ++ks) {
+                const uint64_t ad = sw128_desc(st + 32 * ks), bd = sw128_desc(st + a_bytes + 32 * ks);
+                const uint32_t acc = (i > 0 || ks > 0) ? 1u : 0u;
+                asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+                             "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
+                             :: "r"(tmem), "l"(ad), "l"(bd), "r"(a.idesc), "r"(acc) : "memory");
+            }
+            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
+                         :: "r"(smem_u32(&bar_empty[s])) : "memory");
+        }
+        if (nloc > 0)
+            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
+                         :: "r"(smem_u32(&bar_done)) : "memory");
+    }
+    __syncwarp();
+    const bool have = nloc > 0;
+    if (have) mbar_wait(&bar_done, 0);
+    tc_fence_after();
+
+    // epilogue: warp w reads TMEM lanes 32 (w % 4) .. + 31 (one output feature per thread), column blocks of 16 batch rows
+    // alternate between warps w and w + 4.  Ranks >= 1 park their int32 partial sums in their (now idle) stage memory as
+    // [batch row][feature]; rank 0 adds them after the cluster barrier.
+    const int r = 32 * (warp & 3) + lane;
+    const int64_t o = o0 + r;
+    const uint32_t part = sbase;
+    const uint32_t taddr = tmem + ((uint32_t)(32 * (warp & 3)) << 16);
+    auto tmem_block = [&](int cb, int32_t* v) {
+        uint32_t u[16];
+        if (have) tmem_ld16(taddr + 16 * cb, u);
+#pragma unroll
+        for (int j = 0; j < 16; ++j) v[j] = have ? (int32_t)u[j] : 0;
+    };
+    const int nblocks = nt / 16;
+    if (rank != 0) {
+        for (int cb = warp >> 2; cb < nblocks; cb += 2) {
+            int32_t v[16];
+            tmem_block(cb, v);
+#pragma unroll
+            for (int j = 0; j < 16; ++j)
+                asm volatile("st.shared.s32 [%0], %1;" :: "r"(part + (uint32_t)(((cb * 16 + j) * kIRows + r) * 4)), "r"(v[j]) : "memory");
+        }
+    }
+    __syncwarp();
+    cluster_sync();
+    if (rank == 0) {
+        const bool live = o < N;
+        const int64_t ch = a.per_channel ? o : 0;
+        const float f = live ? __ldg(a.factor + ch) : 0.0f;
+        const int32_t zw = live ? __ldg(a.w_zp + ch) : 0;
+        const int64_t sw = live && a.w_rowsum ? (int64_t)__ldg(a.w_rowsum + o) : 0;
+        const int64_t fixed = K * (int64_t)a.x_zp * zw - (int64_t)a.x_zp * sw;     // K zx zw - zx Sw[o]
+        const float b = a.bias && live ? to_f32<T>(reinterpret_cast<const T*>(a.bias)[o]) : 0.0f;
+        const int64_t g0 = a.m0 + n0;                                      // first global row of this CTA
+        T* y = reinterpret_cast<T*>(a.y);
+        for (int cb = warp >> 2; cb < nblocks; cb += 2) {
+            int32_t v[16];
+            tmem_block(cb, v);
+            for (uint32_t p = 1; p < S; ++p) {
+                const uint32_t base = peer_addr(part + (uint32_t)((cb * 16 * kIRows + r) * 4), p);
+                int32_t pv[16];
+#pragma unroll
+                for (int j = 0; j < 16; ++j) pv[j] = ld_peer_s32(base + j * kIRows * 4);
+#pragma unroll
+                for (int j = 0; j < 16; ++j) v[j] = (int32_t)((uint32_t)v[j] + (uint32_t)pv[j]);
+            }
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+                const int64_t n = cb * 16 + j;
+                if (!live || n >= rows) continue;
+                int64_t c = (int64_t)v[j] + fixed;
+                if (zw != 0 && a.x_rowsum) c -= (int64_t)zw * __ldg(a.x_rowsum + g0 + n);
+                float s = __fmul_rn(__ll2float_rn(c), f);
+                if (a.bias) s = __fadd_rn(s, b);
+                y[(g0 + n) * a.ldy + o] = from_f32<T>(s);
+            }
+        }
+    }
+    __syncwarp();
+    cluster_sync();             // the peers' partial sums stay in place until rank 0 has read them
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(a.tmem_cols) : "memory");
+    }
+}
+
+}  // namespace mctq
+
+using namespace mctq;
+
+namespace {
+
+using EncodeTiled = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                 const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+int encode_fn(EncodeTiled* out) {
+    static EncodeTiled fn = [] {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPointByVersion("cuTensorMapEncodeTiled", &p, 12000, cudaEnableDefault, &q) != cudaSuccess ||
+            q != cudaDriverEntryPointSuccess)
+            p = nullptr;
+        return reinterpret_cast<EncodeTiled>(p);
+    }();
+    *out = fn;
+    return fn ? 0 : (int)cudaErrorSymbolNotFound;
+}
+
+// a [rows][K] uint8 matrix (rows K bytes apart) read in boxes of [box_rows][128] bytes, 128-byte swizzle, zeros outside
+int encode_codes(EncodeTiled fn, CUtensorMap* map, const void* base, int64_t K, int64_t rows, uint32_t box_rows) {
+    const cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
+    const cuuint64_t strides[1] = {(cuuint64_t)K};
+    const cuuint32_t box[2] = {(cuuint32_t)kIChunk, box_rows};
+    const cuuint32_t estr[2] = {1, 1};
+    const CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), dims, strides, box, estr,
+                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
+}
+
+template <bool INT4, bool WSIGNED, typename T>
+int launch_igemm(IgemmArgs& a, int64_t M, cudaStream_t st) {
+    auto kernel = packed_igemm_kernel<INT4, WSIGNED, T>;
+    size_t smem = (size_t)a.stages * a.stage_bytes + 1024;              // + alignment of the stages to 1024 bytes
+    smem = std::max(smem, tmem_smem_floor(a.tmem_cols));
+    int rc = ensure_smem(kernel, smem);
+    if (rc) return rc;
+    const int64_t tiles = (a.N + kIRows - 1) / kIRows;
+    const int64_t ntiles = (M + a.nt - 1) / a.nt;
+    // split-K: as many CTAs as fit the GPU at once (one wave), at least one chunk per CTA.  The ring's shared memory decides
+    // how many CTAs an SM holds: two for small row tiles, one from nt = 96 on (four stages of 28 KB and more)
+    int dev = 0, sms = 0, per_sm = 0;
+    if ((rc = cuda_rc(cudaGetDevice(&dev))) || (rc = cuda_rc(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev))) ||
+        (rc = cuda_rc(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, smem))))
+        return rc;
+    int64_t S = (int64_t)std::max(per_sm, 1) * sms / (tiles * ntiles);
+    S = S < 1 ? 1 : S > kIMaxSplit ? kIMaxSplit : S;
+    if (S > a.nchunks) S = a.nchunks;
+    const int64_t rows_per_launch = (int64_t)65535 * a.nt;
+    for (int64_t m0 = 0; m0 < M; m0 += rows_per_launch) {
+        a.m0 = m0;
+        a.M = M - m0 < rows_per_launch ? M - m0 : rows_per_launch;
+        const dim3 grid((unsigned)(tiles * S), (unsigned)((a.M + a.nt - 1) / a.nt));
+        pdl_plan_launch(st, nullptr, 0, nullptr, 0);                    // ranges "unknown": late order for the successor
+        rc = launch_planned_cluster(kernel, grid, (unsigned)S, smem, st, a);
+        if (rc) return rc;
+    }
+    return 0;
+}
+
+// largest in_features whose int32 sum of code products cannot overflow, per (weight, x) signedness
+int64_t igemm_max_k(bool w_signed, bool x_signed) {
+    if (w_signed && x_signed) return 131071;            // 128 * 128 * K < 2^31
+    if (w_signed || x_signed) return 65793;             // 255 * 128 * K < 2^31
+    return 33025;                                       // 255 * 255 * K < 2^31
+}
+
+}  // namespace
+
+extern "C" {
+
+int64_t mctq_packed_linear_i8_max_k(int w_signed, int x_signed) { return igemm_max_k(w_signed != 0, x_signed != 0); }
+
+int mctq_packed_linear_i8(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x_codes,
+                          int x_signed, int32_t x_zero_point, int64_t M, const int32_t* x_rowsum, const int32_t* w_rowsum,
+                          const float* factor, const void* bias, int y_dtype, void* y, int64_t ldy, void* stream) {
+    MCTQ_NVTX("mctq_packed_linear_i8");
+    if (!w || pack_is_lut(w->kind)) return MCTQ_E_BADARG;
+    if (const int rc = packed_linear_check(w, out_features, in_features, x_codes, y_dtype, M, y)) return rc;
+    const bool int4 = pack_is_int4(w->kind);
+    if (in_features % (int4 ? 32 : 16) != 0 || M >= (1LL << 31) || ldy < out_features) return MCTQ_E_BADARG;
+    if (!factor || (x_zero_point != 0 && !w_rowsum)) return MCTQ_E_BADARG;
+    if (!aligned16(x_codes) || !aligned16(w->codes)) return MCTQ_E_BADARG;
+    if (x_signed ? (x_zero_point < -128 || x_zero_point > 127) : (x_zero_point < 0 || x_zero_point > 255)) return MCTQ_E_RANGE;
+    if (in_features > igemm_max_k(w->is_signed != 0, x_signed != 0)) return MCTQ_E_RANGE;
+    if (M == 0) return 0;
+
+    IgemmArgs a;
+    memset(&a, 0, sizeof(a));
+    const int64_t max_nt = 256;
+    const int64_t ntiles = (M + max_nt - 1) / max_nt;
+    const int64_t per = (M + ntiles - 1) / ntiles;
+    a.nt = (int32_t)((per + 15) / 16 * 16);
+    a.nchunks = (int32_t)((in_features + kIChunk - 1) / kIChunk);
+    a.stage_bytes = (uint32_t)(kIRows * 128 + a.nt * 128);
+    // deep rings for the HBM-bound small-batch shapes, while two CTAs still fit an SM's shared memory where they can
+    a.stages = std::min(kIMaxStages, std::max(kIMinStages, (int)((112 * 1024 - 1024) / a.stage_bytes)));
+    a.tmem_cols = tmem_columns(a.nt);
+    a.idesc = (2u << 4) | ((w->is_signed ? 1u : 0u) << 7) | ((x_signed ? 1u : 0u) << 10) | ((uint32_t)(a.nt >> 3) << 17) |
+              ((uint32_t)(kIRows >> 4) << 24);                           // s32 accumulator, K-major A and B
+    a.codes = reinterpret_cast<const uint8_t*>(w->codes);
+    a.w_zp = w->zp;
+    a.x_rowsum = x_rowsum;
+    a.w_rowsum = x_zero_point != 0 ? w_rowsum : nullptr;
+    a.factor = factor;
+    a.bias = bias;
+    a.y = y;
+    a.ldy = ldy;
+    a.N = (int32_t)out_features;
+    a.K = (int32_t)in_features;
+    a.per_channel = w->C != 1;
+    a.x_zp = x_zero_point;
+
+    EncodeTiled fn;
+    int rc = encode_fn(&fn);
+    if (!rc) rc = encode_codes(fn, &a.tm_x, x_codes, in_features, M, (uint32_t)a.nt);
+    if (!rc && !int4) rc = encode_codes(fn, &a.tm_w, w->codes, in_features, out_features, kIRows);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    auto typed = [&](auto int4_tag, auto signed_tag) {
+        constexpr bool I4 = decltype(int4_tag)::value, WS = decltype(signed_tag)::value;
+        if (y_dtype == MCTQ_F32) return launch_igemm<I4, WS, float>(a, M, st);
+        if (y_dtype == MCTQ_BF16) return launch_igemm<I4, WS, __nv_bfloat16>(a, M, st);
+        return launch_igemm<I4, WS, __half>(a, M, st);
+    };
+    using True = std::true_type;
+    using False = std::false_type;
+    if (int4) return w->is_signed ? typed(True{}, True{}) : typed(True{}, False{});
+    return typed(False{}, False{});         // int8 weights reach the tensor cores as stored: the signedness is in idesc
+}
+
+}  // extern "C"

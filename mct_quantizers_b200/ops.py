@@ -10,6 +10,8 @@ sm_100a kernels.
     torch.ops.mctq.lut_indices        -> LUT indices;                                    mctq.dequantize_lut
     torch.ops.mctq.packed_linear      <- F.linear(x, <weight rebuilt from packed codes>, bias)   (small row counts)
     torch.ops.mctq.packed_linear_batched   the same product on the tensor cores                  (batched row counts)
+    torch.ops.mctq.quantize_rows_i8   -> 8-bit codes of x (fq_affine_scalar's codes) and their row sums
+    torch.ops.mctq.packed_linear_i8   <- the integer product of those codes and packed int8 / int4 weight codes
 
 (reference call sites: see include/mctq.h).  Each op has a CUDA implementation (device pointers + the
 caller's current stream into the C ABI, no synchronisation), a CPU-tensor implementation that streams the
@@ -46,6 +48,10 @@ _LIB.define("packed_linear(Tensor x, Tensor codes, int kind, bool is_signed, int
             "Tensor? zero_point, Tensor? lut_quotients, Tensor? bias) -> Tensor")
 _LIB.define("packed_linear_batched(Tensor x, Tensor codes, int kind, bool is_signed, int out_features, Tensor scale, "
             "Tensor? zero_point, Tensor? lut_quotients, Tensor? bias) -> Tensor")
+_LIB.define("quantize_rows_i8(Tensor x, float scale, int zero_point, int quant_min, int quant_max, bool want_rowsum) "
+            "-> (Tensor, Tensor)")
+_LIB.define("packed_linear_i8(Tensor x_codes, int x_zero_point, Tensor? x_rowsum, Tensor codes, int kind, bool is_signed, "
+            "int out_features, Tensor zero_point, Tensor w_rowsum, Tensor factor, Tensor? bias, ScalarType dtype) -> Tensor")
 
 
 # --------------------------------------------------------------------------------------------- helpers
@@ -817,6 +823,172 @@ def _packed_linear_cuda(x, codes, kind, is_signed, out_features, scale, zero_poi
 _packed_linear_batched_cuda = functools.partial(_packed_linear_cuda, batched=True)
 
 
+def quantize_rows_i8(x, scale_f32, zero_point, quant_min, quant_max, want_rowsum):
+    """(codes, rowsum) of a CUDA tensor x [..., K] under a per-tensor 8-bit affine quantizer (mctq_quantize_rows_i8): codes of
+    x's shape, int8 when quant_min < 0 else uint8, exactly the codes mctq_fq_affine_scalar emits; rowsum int32 [M] (M = the
+    product of the leading dimensions), or an empty tensor unless `want_rowsum`.  `scale_f32` is already narrowed to f32."""
+    tag = _dtype_tag(x)
+    if x.dim() == 0:
+        raise RuntimeError("quantize_rows_i8: x must have at least one dimension")
+    xd = x.contiguous()
+    K = xd.shape[-1]
+    M = xd.numel() // K if K else 0
+    codes = torch.empty(xd.shape, dtype=torch.int8 if quant_min < 0 else torch.uint8, device=xd.device)
+    rowsum = torch.empty((M if want_rowsum else 0,), dtype=torch.int32, device=xd.device)
+    if M:
+        with _on_device(xd.device):
+            rc = _native.load().mctq_quantize_rows_i8(xd.data_ptr(), tag, M, K, scale_f32, zero_point, quant_min, quant_max,
+                                                       codes.data_ptr(), _ptr(rowsum) if want_rowsum else None,
+                                                       _stream(xd.device))
+        _native.check(rc, "mctq_quantize_rows_i8")
+    return codes, rowsum
+
+
+def _quantize_rows_i8_cuda(x, scale, zero_point, quant_min, quant_max, want_rowsum):
+    _check_range(quant_min, quant_max)
+    if not quant_min <= zero_point <= quant_max:
+        raise RuntimeError("`zero_point` must be between `quant_min` and `quant_max`.")
+    return quantize_rows_i8(x, float(np.float32(scale)), int(zero_point), int(quant_min), int(quant_max), bool(want_rowsum))
+
+
+def weight_code_values(codes, kind, is_signed, out_features, in_features):
+    """The integer codes of a packed affine weight as an int32 [out_features, in_features] tensor (one-time set-up of
+    IntegerLinear: the code row sums)."""
+    c = codes.reshape(-1).view(torch.uint8).to(torch.int32)
+    if kind == _native.PACK_AFFINE_I4:
+        c = torch.stack((c & 15, c >> 4), dim=-1).reshape(-1)[:out_features * in_features]
+        return (c - 16 * (c >= 8).to(torch.int32) if is_signed else c).reshape(out_features, in_features)
+    return (c - 256 * (c >= 128).to(torch.int32) if is_signed else c).reshape(out_features, in_features)
+
+
+class IntegerLinear:
+    """Launch state of one packed affine [out_features, in_features] weight in integer linear mode (mctq_quantize_rows_i8 +
+    mctq_packed_linear_i8), built once: the descriptor, the weight code row sums Sw, the factors f = fl32(sx * scale) and the
+    input quantizer's launch constants.
+        codes, kind, is_signed   the packed weight (kind PACK_AFFINE_I8 / PACK_AFFINE_I4), row-major [out][in]
+        dtype                    the rebuilt weight's dtype: x, bias and y have it
+        scale, zero_point        f32 / int32, 1 (per tensor) or out_features entries
+        x_scale, x_zero_point, x_qmin, x_qmax   the input quantizer Q (per tensor, at most 256 levels)
+    `__call__(x, bias)` returns the integer product of Q's codes of x and the weight codes, scaled (include/mctq.h gives the
+    formula), for a CUDA x of `dtype` on the codes' device, enqueued on the current stream.  `quantize` and `gemm` are its two
+    launches."""
+
+    def __init__(self, codes, kind, is_signed, dtype, out_features, in_features, scale, zero_point, x_scale, x_zero_point,
+                 x_qmin, x_qmax):
+        _check_range(x_qmin, x_qmax)
+        if not ((-128 <= x_qmin and x_qmax <= 127) or (0 <= x_qmin and x_qmax <= 255)):
+            raise ValueError(f"IntegerLinear: the input range [{x_qmin}, {x_qmax}] does not fit 8-bit codes")
+        if not x_qmin <= x_zero_point <= x_qmax:
+            raise RuntimeError("`zero_point` must be between `quant_min` and `quant_max`.")
+        self.device = codes.device
+        self.x_scale, self.x_zp = float(np.float32(x_scale)), int(x_zero_point)
+        self.x_qmin, self.x_qmax = int(x_qmin), int(x_qmax)
+        s = _param_on(scale.detach().reshape(-1).contiguous().to(torch.float32), self.device)
+        factor = torch.tensor(self.x_scale, dtype=torch.float32, device=self.device) * s
+        self._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, None, "IntegerLinear")
+
+    @classmethod
+    def from_parts(cls, codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, x_zero_point):
+        """The launch state from a caller-supplied f and Sw (mctq::packed_linear_i8), with the constructor's checks of the
+        weight; only `gemm` is available (the input quantizer's scale and range are not known)."""
+        lin = cls.__new__(cls)
+        lin.device = codes.device
+        lin.x_zp, lin.x_scale, lin.x_qmin, lin.x_qmax = int(x_zero_point), None, None, None
+        lin._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, "packed_linear_i8")
+        return lin
+
+    def _bind(self, codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, what):
+        """Validate the weight, its factors, zero points and code row sums (computed from the codes when None) and build the
+        descriptor."""
+        if self.device.type != "cuda":
+            raise ValueError(f"{what} needs CUDA tensors")
+        if kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
+            raise ValueError(f"{what}: kind {kind} is not an affine int8 / int4 packed weight")
+        if dtype not in _DT:
+            raise ValueError(f"{what}: output dtype {dtype} is not float32 / bfloat16 / float16")
+        if zero_point is None:
+            raise ValueError(f"{what}: affine weights need their zero points")
+        self.out_features, self.in_features, self.dtype = int(out_features), int(in_features), dtype
+        N, K = self.out_features, self.in_features
+        f = _param_on(factor.detach().reshape(-1).contiguous(), self.device)
+        if f.numel() not in (1, N) or zero_point.numel() != f.numel():
+            raise ValueError(f"{what}: {f.numel()} factors and {zero_point.numel()} zero points for {N} output channels "
+                             f"(both per tensor or both per output channel)")
+        C, inner = (f.numel(), K) if f.numel() > 1 else (1, 1)
+        self._desc, self._keep = _packed_desc(codes, kind, is_signed, dtype, N * K, C, inner, f, zero_point, None,
+                                              self.device, what)
+        self.factor, z = self._keep[1], self._keep[2]
+        if w_rowsum is None:
+            w_rowsum = weight_code_values(self._keep[0], kind, is_signed, N, K).sum(1, dtype=torch.int32)
+        self.w_rowsum = _param_on(w_rowsum.detach().reshape(-1).contiguous(), self.device)
+        if self.w_rowsum.dtype != torch.int32 or self.w_rowsum.numel() != N:
+            raise ValueError(f"{what}: w_rowsum must be int32 [{N}]")
+        self.needs_x_rowsum = bool((z != 0).any())
+        self._desc_ptr = ctypes.addressof(self._desc)
+
+    def __call__(self, x, bias=None):
+        if x.dtype != self.dtype or (bias is not None and bias.dtype != self.dtype):
+            raise RuntimeError(f"packed_linear_i8: x and bias must have the weight's dtype {self.dtype}")
+        qx, rowsum = self.quantize(x)
+        return self.gemm(qx, rowsum if self.needs_x_rowsum else None, bias)
+
+    def quantize(self, x):
+        """Q's codes of x and their row sums (empty when no weight zero point needs them)."""
+        if x.dim() == 0 or x.shape[-1] != self.in_features:
+            raise RuntimeError(f"packed_linear_i8: x of shape {list(x.shape)} does not end in in_features = {self.in_features}")
+        if x.device != self.device:
+            raise RuntimeError(f"packed_linear_i8: x must live on {self.device}")
+        return quantize_rows_i8(x, self.x_scale, self.x_zp, self.x_qmin, self.x_qmax, self.needs_x_rowsum)
+
+    def gemm(self, x_codes, x_rowsum=None, bias=None, out=None):
+        """y from x codes [..., in_features] (int8 or uint8, zero point x_zero_point) and their row sums.  `out`: a 2-D
+        [M, out_features] CUDA tensor of `dtype` with unit column stride (its rows may be further apart) to write into."""
+        if x_codes.dtype not in (torch.int8, torch.uint8) or x_codes.dim() == 0 or x_codes.shape[-1] != self.in_features:
+            raise RuntimeError(f"packed_linear_i8: x codes ({x_codes.dtype}, {list(x_codes.shape)}) are not int8 / uint8 "
+                               f"rows of in_features = {self.in_features}")
+        if x_codes.device != self.device or (bias is not None and bias.device != self.device):
+            raise RuntimeError(f"packed_linear_i8: x codes and bias must live on {self.device}")
+        if bias is not None and (bias.numel() != self.out_features or bias.dtype != self.dtype):
+            raise RuntimeError(f"packed_linear_i8: bias must hold {self.out_features} entries of {self.dtype}")
+        if self.needs_x_rowsum and x_rowsum is None:
+            raise RuntimeError("packed_linear_i8: a weight zero point is not 0, so the x code row sums are needed")
+        qx = x_codes.contiguous()
+        M = qx.numel() // self.in_features
+        if out is None:
+            y = torch.empty(tuple(qx.shape[:-1]) + (self.out_features,), dtype=self.dtype, device=self.device)
+            ldy = self.out_features
+        else:
+            if out.dim() != 2 or tuple(out.shape) != (M, self.out_features) or out.stride(1) != 1 or out.dtype != self.dtype \
+                    or out.device != self.device:
+                raise RuntimeError(f"packed_linear_i8: out must be a [{M}, {self.out_features}] {self.dtype} tensor with "
+                                   f"unit column stride on {self.device}")
+            y, ldy = out, max(out.stride(0), self.out_features)
+        if M:
+            rs = x_rowsum.reshape(-1).contiguous() if x_rowsum is not None and self.needs_x_rowsum else None
+            if rs is not None and (rs.dtype != torch.int32 or rs.numel() != M or rs.device != self.device):
+                raise RuntimeError(f"packed_linear_i8: x_rowsum must be int32 [{M}] on {self.device}")
+            b = bias.contiguous() if bias is not None else None
+            with _on_device(self.device):
+                rc = _native.load().mctq_packed_linear_i8(
+                    self._desc_ptr, self.out_features, self.in_features, qx.data_ptr(), int(qx.dtype == torch.int8),
+                    self.x_zp, M, _ptr(rs), self.w_rowsum.data_ptr(), self.factor.data_ptr(), _ptr(b), _DT[self.dtype],
+                    y.data_ptr(), ldy, _stream(self.device))
+            _native.check(rc, "mctq_packed_linear_i8")
+        return y
+
+
+def _packed_linear_i8_cuda(x_codes, x_zero_point, x_rowsum, codes, kind, is_signed, out_features, zero_point, w_rowsum,
+                           factor, bias, dtype):
+    """mctq::packed_linear_i8: the caller supplies Sw and f (IntegerLinear derives them from the weight and Q); x_rowsum may
+    be None only when every weight zero point is 0."""
+    if x_codes.dim() == 0:
+        raise RuntimeError("packed_linear_i8: x codes must have at least one dimension")
+    _native.load()
+    lin = IntegerLinear.from_parts(codes, kind, is_signed, dtype, out_features, x_codes.shape[-1], factor, zero_point,
+                                   w_rowsum, x_zero_point)
+    return lin.gemm(x_codes, x_rowsum, bias)
+
+
 def _lut_scalar_cuda(x, table, K, divisor, threshold, round_to_input_dtype, multiply=False):
     """`multiply`: normalise with x * (float)(1.0 / divisor) -- the reference's CUDA flavour of `tensor / python_number`
     (quantizer_utils.reference_arithmetic) -- instead of the true division x / (float)divisor."""
@@ -1014,6 +1186,8 @@ _LIB.impl("lut_indices", _lut_indices_cuda, "CUDA")
 _LIB.impl("dequantize_lut", _dequantize_lut_cuda, "CUDA")
 _LIB.impl("packed_linear", _packed_linear_cuda, "CUDA")
 _LIB.impl("packed_linear_batched", _packed_linear_batched_cuda, "CUDA")
+_LIB.impl("quantize_rows_i8", _quantize_rows_i8_cuda, "CUDA")
+_LIB.impl("packed_linear_i8", _packed_linear_i8_cuda, "CUDA")
 
 _LIB.impl("fq_affine_scalar_pre", _affine_scalar_pre_cuda, "CUDA")
 _LIB.impl("fq_affine_scalar_pre", _via_device(_affine_scalar_pre_cuda), "CPU")
@@ -1028,6 +1202,8 @@ _LIB.impl("lut_indices", _via_device(_lut_indices_cuda, keep=(1,)), "CPU")
 _LIB.impl("dequantize_lut", _via_device(_dequantize_lut_cuda, keep=(3,)), "CPU")
 _LIB.impl("packed_linear", _via_device(_packed_linear_cuda), "CPU")
 _LIB.impl("packed_linear_batched", _via_device(_packed_linear_batched_cuda), "CPU")
+_LIB.impl("quantize_rows_i8", _via_device(_quantize_rows_i8_cuda), "CPU")
+_LIB.impl("packed_linear_i8", _via_device(_packed_linear_i8_cuda), "CPU")
 
 
 # --------------------------------------------------------------------------------------------- fake / meta impls
@@ -1095,6 +1271,18 @@ def _(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients,
 @torch.library.register_fake("mctq::packed_linear_batched")
 def _(x, codes, kind, is_signed, out_features, scale, zero_point, lut_quotients, bias):
     return x.new_empty(tuple(x.shape[:-1]) + (out_features,))
+
+
+@torch.library.register_fake("mctq::quantize_rows_i8")
+def _(x, scale, zero_point, quant_min, quant_max, want_rowsum):
+    M = x.numel() // x.shape[-1] if x.dim() and x.shape[-1] else 0
+    return (torch.empty_like(x, dtype=torch.int8 if quant_min < 0 else torch.uint8),
+            x.new_empty((M if want_rowsum else 0,), dtype=torch.int32))
+
+
+@torch.library.register_fake("mctq::packed_linear_i8")
+def _(x_codes, x_zero_point, x_rowsum, codes, kind, is_signed, out_features, zero_point, w_rowsum, factor, bias, dtype):
+    return x_codes.new_empty(tuple(x_codes.shape[:-1]) + (out_features,), dtype=dtype)
 
 
 # --------------------------------------------------------------------------------------------- whole-model launch

@@ -27,6 +27,17 @@ inputs of more than FUSED_LINEAR_MAX_ROWS and at most FUSED_BATCHED_MAX_ROWS row
 rebuilt weight, f32 accumulation, one rounding to x's dtype, deterministic.  LUT weights qualify when every quotient of the
 table is exact in bf16 (integer centroids on grids of up to 8 bits).
 
+Integer linear mode (`pack_model_weights(model, integer_linear=True)`, or `wrapper.pack_weights(integer_linear=True,
+input_quantizer=q)` for one wrapper; opt-in): a packed `torch.nn.Linear` wrapper with int8 / int4 affine codes whose input
+comes from a per-tensor 8-bit affine activation quantizer Q computes `layer(Q(x))` with integer arithmetic: Q's codes of x
+(csrc/mctq_affine.cu, mctq_quantize_rows_i8) times the weight codes as an exact int32 sum on the tensor cores
+(csrc/mctq_packed_igemm.cu), then the zero-point corrections and one f32 scaling per output (include/mctq.h gives the formula
+bit for bit).  Q is idempotent on its own outputs, so on a holder -> Linear edge this is the fake-quant model's product summed
+exactly; it differs from the float model by f32 accumulation rounding (and, for bf16 / f16, by the rounding of the holder's
+outputs and of W to that dtype).  It is a numerical contract of its own, so it covers every row count.  The model-level call
+traces the model with torch.fx (holders and wrappers as leaves) and switches each eligible wrapper whose input is a holder's
+output, directly or through flatten / reshape / view / contiguous; integer mode takes precedence over fused / batched mode.
+
 Packing is one-way and for inference only:
   * the rebuild dtype is the weight's dtype at packing time; `.half()` does not change it (the codes are integer buffers);
   * the packed state travels with the module: `state_dict` / `load_state_dict` between packed models of the same structure,
@@ -247,22 +258,94 @@ def batched_linear_eligibility(wrapper) -> Tuple[bool, str]:
     return True, ""
 
 
+def integer_linear_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
+    """(True, '') when `wrapper` can run in integer linear mode with input quantizer `input_quantizer`: fused_linear_eligibility,
+    int8 / int4 affine codes, a per-tensor affine activation quantizer with 8-bit codes, in_features a multiple of 16 (32 for
+    int4 codes) and at most the int32 bound of the code signedness pair.  Host-only."""
+    from mct_quantizers_b200.pytorch.fused_activation_holder import affine_scalar_params
+    ok, reason = fused_linear_eligibility(wrapper)
+    if not ok:
+        return ok, reason
+    e = next(e for e in wrapper.__dict__['_packed'].entries if e.name == 'weight')
+    if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
+        return False, f"the weight is packed as {_KIND_NAMES[e.kind]}, not as int8 / int4 affine codes"
+    if affine_scalar_params(input_quantizer) is None:
+        return False, (f"the input quantizer {type(input_quantizer).__name__} is not a per-tensor affine activation quantizer "
+                       f"(ActivationSymmetric / POT / Uniform)")
+    if input_quantizer.__dict__.get('enable_reuse', False):
+        return False, "the input quantizer reuses its outputs (enable_reuse)"
+    qmin, qmax = int(input_quantizer.min_quantized_domain), int(input_quantizer.max_quantized_domain)
+    if not ((-128 <= qmin and qmax <= 127) or (0 <= qmin and qmax <= 255)):
+        return False, f"the input quantization range [{qmin}, {qmax}] does not fit 8-bit codes"
+    K = wrapper.layer.in_features
+    step = 32 if e.kind == _native.PACK_AFFINE_I4 else 16
+    if K % step:
+        return False, f"in_features = {K} is not a multiple of {step}"
+    bound = _native.integer_linear_max_k(e.is_signed, qmin < 0)
+    if K > bound:
+        return False, f"in_features = {K} exceeds {bound}, the largest row length whose int32 sum of code products cannot overflow"
+    return True, ""
+
+
+_SHAPE_METHODS = ("flatten", "reshape", "view", "contiguous")
+_SHAPE_FUNCS = (torch.flatten, torch.reshape)
+
+
+def integer_linear_edges(model: torch.nn.Module) -> Tuple[Dict[str, Tuple[str, object]], Dict[str, str], str]:
+    """Trace `model` with torch.fx (holders and quantization wrappers as leaves) and find the holder -> wrapper edges of
+    integer linear mode: ({wrapper name: (holder name, holder quantizer)}, {wrapper name: why its input does not qualify},
+    '') -- or ({}, {}, why the model cannot be traced).  An edge may pass through flatten / reshape / view / contiguous."""
+    from mct_quantizers_b200.pytorch.activation_quantization_holder import PytorchActivationQuantizationHolder
+    from mct_quantizers_b200.pytorch.fused_activation_holder import _LeafTracer
+    from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
+    try:
+        graph = _LeafTracer().trace(model)
+    except Exception as err:                                     # noqa: BLE001 - any tracing failure switches nothing
+        return {}, {}, f"the model cannot be traced with torch.fx ({type(err).__name__}: {err})"
+    modules = dict(model.named_modules())
+    edges, why = {}, {}
+    for node in graph.nodes:
+        if node.op != "call_module" or not isinstance(modules.get(node.target), PytorchQuantizationWrapper):
+            continue
+        if len(node.args) != 1 or node.kwargs:
+            why[node.target] = "the wrapper is called with more than one input"
+            continue
+        src = node.args[0]
+        while isinstance(src, torch.fx.Node) and src.args and (
+                (src.op == "call_method" and src.target in _SHAPE_METHODS) or
+                (src.op == "call_function" and src.target in _SHAPE_FUNCS)):
+            src = src.args[0]
+        holder = modules.get(src.target) if isinstance(src, torch.fx.Node) and src.op == "call_module" else None
+        if not isinstance(holder, PytorchActivationQuantizationHolder):
+            why[node.target] = "the input is not the output of an activation quantization holder"
+        elif getattr(holder, "quantization_bypass", False):
+            why[node.target] = f"the input holder {src.target} bypasses quantization"
+        elif node.target in edges and edges[node.target][0] != src.target:
+            why[node.target] = "the wrapper is called on the outputs of different holders"
+        else:
+            edges[node.target] = (src.target, holder.activation_holder_quantizer)
+    return edges, why, ""
+
+
 class PackedState:
     """Per-wrapper packed state (the wrapper's `_packed` attribute): its PackedWeight entries, whether the wrapper runs in
     fused linear mode (and batched linear mode), and the launch state of its forward (the unpack plan / the fused-linear descriptor, built on first use
     and rebuilt when the codes move; not pickled)."""
     fused = False
     batched = False             # class default: states pickled before batched mode existed load with it off
+    integer = False             # integer linear mode (and its input quantizer): off for states pickled before it existed
+    input_quantizer = None
 
     def __init__(self, entries: List[PackedWeight]):
         self.entries = entries
         self.fused = False
         self.batched = False
-        self._plan, self._sig, self._lin = None, None, None
+        self.integer, self.input_quantizer = False, None
+        self._plan, self._sig, self._lin, self._ilin = None, None, None, None
 
     def __getstate__(self):
-        return {'entries': self.entries, 'fused': self.fused, 'batched': self.batched, '_plan': None, '_sig': None,
-                '_lin': None}
+        return {'entries': self.entries, 'fused': self.fused, 'batched': self.batched, 'integer': self.integer,
+                'input_quantizer': self.input_quantizer, '_plan': None, '_sig': None, '_lin': None, '_ilin': None}
 
     def bind(self, wrapper):
         """Point the entries at `wrapper` (after a copy or unpickling they point nowhere)."""
@@ -322,11 +405,47 @@ class PackedState:
             return lin[1].batched(x, bias)
         return lin[1](x, bias)
 
+    def integer_forward(self, wrapper, x):
+        """layer(Q(x)) in integer arithmetic (ops.IntegerLinear), or None when this call must take the packed path of the
+        wrapper's other modes: the conditions of fused_forward, without its row limit."""
+        e = self.entries[0]
+        if e._owner is None or e._owner() is not wrapper:
+            self.bind(wrapper)
+        if type(x) not in ops._PLAIN_TENSOR_TYPES or not x.is_cuda or x.dtype != e.dtype_out or x.dim() == 0:
+            return None
+        layer = wrapper.__dict__['_modules'][LAYER]
+        bias = layer.bias
+        if x.shape[-1] != layer.in_features or (bias is not None and (bias.dtype != x.dtype or bias.device != x.device)):
+            return None
+        if torch.is_grad_enabled() and (x.requires_grad or (bias is not None and bias.requires_grad)):
+            return None
+        if layer._forward_hooks or layer._forward_pre_hooks or _nn_module._global_forward_hooks or \
+                _nn_module._global_forward_pre_hooks or torch.compiler.is_compiling():
+            return None
+        codes = e.codes
+        if x.device != codes.device:
+            return None
+        lin = self.__dict__.get('_ilin')
+        if lin is None or lin[0] != codes.data_ptr():
+            q = self.input_quantizer
+            from mct_quantizers_b200.pytorch.fused_activation_holder import affine_scalar_params
+            scale, zp, _, _ = affine_scalar_params(q)
+            x_scale, x_zp, qmin, qmax = q._validated_launch_args(scale, zp)[1]      # what the holder's kernel receives
+            item = e.plan_item()
+            lin = (codes.data_ptr(), ops.IntegerLinear(codes, e.kind, e.is_signed, e.dtype_out, layer.out_features,
+                                                       layer.in_features, item[8], item[9], x_scale, x_zp, qmin, qmax))
+            self._ilin = lin
+        return lin[1](x, bias)
+
     def forward(self, wrapper, args, kwargs):
         if torch.jit.is_tracing():
             raise RuntimeError("this PytorchQuantizationWrapper holds packed weights (pack_weights / pack_model_weights): "
                                "they cannot be traced or exported to ONNX, which needs the float weights; export the "
                                "model before packing it")
+        if self.__dict__.get('integer', False) and len(args) == 1 and not kwargs:
+            y = self.integer_forward(wrapper, args[0])
+            if y is not None:
+                return y
         if self.fused and len(args) == 1 and not kwargs:
             y = self.fused_forward(wrapper, args[0])
             if y is not None:
@@ -344,15 +463,21 @@ class PackedState:
             wrapper.set_quantize_weights({})               # drop the rebuilt weights: only the codes stay resident
 
 
-def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bool = False) -> Dict:
+def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bool = False, integer_linear: bool = False,
+                         input_quantizer=None) -> Dict:
     """Pack every weight of `wrapper` that can be packed (see the module docstring).  Returns
     {name: {'packed': bool, 'kind': str | None, 'reason': str, 'code_bytes': int, 'float_bytes': int}}.
     `fused_linear=True` also switches the wrapper to fused linear mode when fused_linear_eligibility allows it (on a wrapper
     packed earlier it only switches the mode), and every report entry gains 'fused': bool and 'fused_reason': str.
     `batched_linear=True` (needs fused_linear=True) also switches it to batched linear mode when batched_linear_eligibility
-    allows it, and every report entry gains 'batched': bool and 'batched_reason': str."""
+    allows it, and every report entry gains 'batched': bool and 'batched_reason': str.
+    `integer_linear=True` (needs `input_quantizer`, the quantizer of the activation holder whose output the wrapper reads)
+    also switches it to integer linear mode when integer_linear_eligibility allows it, and every report entry gains
+    'integer': bool, 'integer_reason': str and 'input_holder' (the holder's module name for pack_model_weights, else None)."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
+    if integer_linear and input_quantizer is None:
+        raise ValueError("integer_linear=True needs the input_quantizer of the activation holder that feeds the wrapper")
     report = {}
     state = wrapper.__dict__.get('_packed')
     entries = list(state.entries) if state is not None else []
@@ -382,6 +507,8 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
         _switch_to_fused(wrapper, report)
     if batched_linear:
         _switch_to_batched(wrapper, report)
+    if integer_linear:
+        _switch_to_integer(wrapper, report, input_quantizer, None)
     return report
 
 
@@ -403,6 +530,8 @@ def _drop_float_weights(wrapper, new, entries, keep):
     wrapper._packed = PackedState(entries)
     wrapper._packed.fused = state is not None and state.fused
     wrapper._packed.batched = state is not None and state.batched
+    if state is not None and state.__dict__.get('integer', False):
+        wrapper._packed.integer, wrapper._packed.input_quantizer = True, state.input_quantizer
 
 
 def _switch_to_fused(wrapper, report):
@@ -410,10 +539,7 @@ def _switch_to_fused(wrapper, report):
     state = wrapper.__dict__.get('_packed')
     if ok:
         state.fused, state._lin = True, None
-    for e in (state.entries if state is not None else []):
-        if e.name not in report:                      # packed by an earlier call
-            report[e.name] = dict(packed=True, kind=_KIND_NAMES[e.kind], reason="already packed",
-                                  code_bytes=e.codes.numel() * e.codes.element_size(), float_bytes=0)
+    _report_packed_entries(wrapper, report)
     for r in report.values():
         r['fused'], r['fused_reason'] = ok, reason
 
@@ -427,15 +553,45 @@ def _switch_to_batched(wrapper, report):
         r['batched'], r['batched_reason'] = ok, reason
 
 
+def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None):
+    ok, why = (False, reason) if reason else integer_linear_eligibility(wrapper, input_quantizer)
+    state = wrapper.__dict__.get('_packed')
+    if ok:
+        state.integer, state.input_quantizer, state._ilin = True, input_quantizer, None
+    _report_packed_entries(wrapper, report)
+    for r in report.values():
+        r['integer'], r['integer_reason'], r['input_holder'] = ok, why, holder_name
+
+
+def _report_packed_entries(wrapper, report):
+    state = wrapper.__dict__.get('_packed')
+    for e in (state.entries if state is not None else []):
+        if e.name not in report:                      # packed by an earlier call
+            report[e.name] = dict(packed=True, kind=_KIND_NAMES[e.kind], reason="already packed",
+                                  code_bytes=e.codes.numel() * e.codes.element_size(), float_bytes=0)
+
+
 def _bits(t):
     return t.view(torch.int32) if t.element_size() == 4 else t.view(torch.int16)
 
 
-def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batched_linear: bool = False) -> Dict[str, Dict]:
+def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batched_linear: bool = False,
+                       integer_linear: bool = False) -> Dict[str, Dict]:
     """pack_weights(fused_linear, batched_linear) on every PytorchQuantizationWrapper of `model`: {wrapper module name:
-    {weight name: report entry}}."""
+    {weight name: report entry}}.  `integer_linear=True` then switches, in place, every eligible wrapper whose input is the
+    output of an activation quantization holder (integer_linear_edges) to integer linear mode; every report entry gains
+    'integer', 'integer_reason' and 'input_holder'.  When the model cannot be traced nothing is switched and the reason is
+    reported."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
-    return {mod_name: pack_wrapper_weights(mod, fused_linear, batched_linear) for mod_name, mod in model.named_modules()
-            if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization}
+    wrappers = {mod_name: mod for mod_name, mod in model.named_modules()
+                if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization}
+    reports = {name: pack_wrapper_weights(mod, fused_linear, batched_linear) for name, mod in wrappers.items()}
+    if integer_linear:
+        edges, why, failure = integer_linear_edges(model)
+        for name, mod in wrappers.items():
+            holder, q = edges.get(name, (None, None)) if name not in why else (None, None)
+            reason = failure or why.get(name) or ("" if holder else "the wrapper is not called in the traced forward")
+            _switch_to_integer(mod, reports[name], q, holder, None if holder else reason)
+    return reports
