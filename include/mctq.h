@@ -232,6 +232,47 @@ int mctq_packed_linear_i8(const MctqPackedDesc* w, int64_t out_features, int64_t
                           int x_signed, int32_t x_zero_point, int64_t M, const int32_t* x_rowsum, const int32_t* w_rowsum,
                           const float* factor, const void* bias, int y_dtype, void* y, int64_t ldy, void* stream);
 
+/* Integer convolution mode (packed nn.Conv2d wrappers, groups 1, zero padding, fed by the same quantizer Q as above).
+ *
+ * mctq_quantize_nhwc_i8: qx [N][H*W][C] (NHWC, one byte per element, int8 if qmin < 0 else uint8) of an NCHW-contiguous
+ * x [N][C][H][W] (x_dtype), codes bit for bit those of mctq_quantize_rows_i8 / mctq_fq_affine_scalar, and, when P is not
+ * NULL, P[(b*H + h)*W + w] = sum_c qx (int32).  A channels_last x needs no transpose: mctq_quantize_rows_i8 with M = N*H*W
+ * rows of K = C codes writes the same codes, and its row sums are P.  MCTQ_E_BADARG (null x / codes, N < 0, C / H / W < 1),
+ * MCTQ_E_DTYPE, MCTQ_E_RANGE as mctq_quantize_rows_i8, before any CUDA call; N == 0 is a no-op.
+ *
+ * mctq_packed_conv2d_i8: y = conv2d(x, W) in the integer arithmetic of mctq_packed_linear_i8, with
+ *   qx[b,c,h,w] = Q's codes of x;  zx for (h, w) outside the image (zero padding of Q(x) is exactly code zx)
+ *   row n = (b, ho, wo), column k = (r, s, c),  K = Cin*kh*kw,  M = N*Ho*Wo
+ *   X[n,k] = qx[b, c, ho*sh - pt + r*dh, wo*sw - pl + s*dw]
+ *   acc    = sum_k X[n,k] * qw[o,k]                               int32, exact (tcgen05.mma kind::i8)
+ *   c      = acc - zw[o] * Sx[n] - zx * Sw[o] + K * zx * zw[o]    int64, exact;  Sx[n] = sum_k X[n,k] (padding counts as zx)
+ *   y[b,o,ho,wo] = T(fl(fl((float)c * f[o]) + bias[o]))          T = y_dtype; f[o] = fl32(sx * sw[o])
+ * Padded taps hold zx and so contribute exactly 0, as in the float model; the sum is exact, so the output does not depend on
+ * the order of k, the tiling or the split of K.
+ *   w          HOST descriptor of an MCTQ_PACK_AFFINE_I8 / _I4 weight [Cout][K] in (r, s, c) order (the memory order of a
+ *              channels_last [Cout, Cin, kh, kw] weight), per tensor or per output channel; codes 16-byte aligned
+ *   g          the geometry; Ho / Wo are the caller's (taps outside the image are never read, whatever they are)
+ *   x_codes    device NHWC codes [N][H][W][Cin], 16-byte aligned; x_signed, x_zero_point as for mctq_packed_linear_i8
+ *   x_rowsum   device Sx [M], or NULL when every weight zero point is 0
+ *   w_rowsum, factor, bias   as for mctq_packed_linear_i8 (Cout entries)
+ *   y_nchw     0: y is [M][Cout] row-major (NHWC / channels_last);  1: y is NCHW, y[(b*Cout + o)*Ho*Wo + ho*Wo + wo]
+ * Returns, before any CUDA call: MCTQ_E_BADARG for a LUT kind, a null pointer, a non-positive extent, stride or dilation, a
+ * negative pad, Cin not a multiple of 16, K not a multiple of 32 for int4 weights, unaligned codes, M >= 2^31, or zx != 0
+ * without w_rowsum; MCTQ_E_DTYPE; MCTQ_E_RANGE for a zx outside the x codes' range or K above
+ * mctq_packed_linear_i8_max_k(w->is_signed, x_signed).  M == 0 is a no-op. */
+typedef struct MctqConv2dGeom {
+    int32_t N, H, W, Cin;           /* input [N][H][W][Cin] */
+    int32_t Ho, Wo;                 /* output extent */
+    int32_t kh, kw;
+    int32_t sh, sw, dh, dw;         /* stride, dilation */
+    int32_t pt, pb, pl, pr;         /* zero padding per side */
+} MctqConv2dGeom;
+int mctq_quantize_nhwc_i8(const void* x, int x_dtype, int64_t N, int64_t C, int64_t H, int64_t W, float scale, int32_t zp,
+                          int32_t qmin, int32_t qmax, void* codes, int32_t* P, void* stream);
+int mctq_packed_conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x_codes, int x_signed,
+                          int32_t x_zero_point, const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor,
+                          const void* bias, int y_dtype, void* y, int y_nchw, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Whole-model weight quantisation: one launch over a table of tensors (SURVEY 8f rank 1).
  * Replaces the per-layer loop  for name, w, quantizer in self._weights_vars: quantizer(w)

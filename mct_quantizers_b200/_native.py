@@ -63,6 +63,12 @@ class MctqPackedDesc(ctypes.Structure):
                 ("scale", c_vp), ("zp", c_vp), ("lut_quotients", c_vp)]
 
 
+class MctqConv2dGeom(ctypes.Structure):
+    """Mirror of `struct MctqConv2dGeom` (include/mctq.h)."""
+    _fields_ = [(f, c_i32) for f in ("N", "H", "W", "Cin", "Ho", "Wo", "kh", "kw", "sh", "sw", "dh", "dw",
+                                     "pt", "pb", "pl", "pr")]
+
+
 # name -> (restype, argtypes): every symbol include/mctq.h declares
 SIGNATURES = {
     "mctq_abi_version": (c_int, []),
@@ -83,6 +89,10 @@ SIGNATURES = {
     "mctq_packed_linear_i8_max_k": (c_i64, [c_int, c_int]),
     "mctq_packed_linear_i8": (c_int, [c_vp, c_i64, c_i64, c_vp, c_int, c_i32, c_i64, c_vp, c_vp, c_vp, c_vp, c_int, c_vp,
                                       c_i64, c_vp]),
+    "mctq_quantize_nhwc_i8": (c_int, [c_vp, c_int, c_i64, c_i64, c_i64, c_i64, c_f32, c_i32, c_i32, c_i32, c_vp, c_vp,
+                                      c_vp]),
+    "mctq_packed_conv2d_i8": (c_int, [c_vp, c_vp, c_i64, c_vp, c_int, c_i32, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_int,
+                                      c_vp]),
     "mctq_multi_tile_elems": (c_i64, []),
     "mctq_multi_plan": (c_i64, [c_vp, c_int, c_vp]),
     "mctq_fq_affine_multi": (c_int, [c_vp, c_vp, c_int, c_i64, c_vp]),

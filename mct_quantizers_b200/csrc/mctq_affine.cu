@@ -675,6 +675,65 @@ __global__ void __launch_bounds__(kThreads) quantize_rows_kernel(const T* __rest
     }
 }
 
+// ---- NHWC codes of an NCHW x [N][C][HW] and their per-pixel channel sums (integer convolution mode): the recipe of
+// quantize_rows_kernel as a tiled transpose through shared memory.  A CTA takes 32 pixels of one image and walks the
+// channels 64 at a time: warp w reads channels w, w + 8, .. of the 32 pixels (coalesced along W), then the CTA writes the
+// 64 channel codes of 4 pixels per pass (coalesced along C).
+template <typename T>
+__global__ void __launch_bounds__(kThreads) quantize_nhwc_kernel(const T* __restrict__ x, uint8_t* __restrict__ codes,
+                                                                  int32_t* __restrict__ psum, int64_t N, int64_t C, int64_t HW,
+                                                                  float scale, int32_t zp, int32_t qmin, int32_t qmax) {
+    using Op = AffineOp<false>;
+    AffineArgs a;                                   // only the fields AffineOp::make reads
+    a.qmin = qmin;
+    a.qmax = qmax;
+    const Op::ChanParams p = Op::make(scale, zp, a);
+    __shared__ uint8_t tile[64][33];                // [channel][pixel]; the odd row length spreads the column reads
+    __shared__ int32_t sums[kThreads / 32][32];
+    pdl_wait();
+    pdl_launch_dependents();
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const int64_t ptiles = (HW + 31) / 32;
+    for (int64_t t = blockIdx.x; t < N * ptiles; t += gridDim.x) {
+        const int64_t b = t / ptiles, p0 = (t - b * ptiles) * 32;
+        const T* xb = x + b * C * HW;
+        uint8_t* cb = codes + b * HW * C;
+        int32_t sum = 0;
+        for (int64_t c0 = 0; c0 < C; c0 += 64) {
+#pragma unroll
+            for (int i = 0; i < 64 / (kThreads / 32); ++i) {
+                const int cl = ty + (kThreads / 32) * i;
+                const int64_t c = c0 + cl, px = p0 + tx;
+                int q = 0;
+                if (c < C && px < HW) {
+                    Op::template apply<true>(to_f32<T>(xb[c * HW + px]), p, q);
+                    sum += q;
+                }
+                tile[cl][tx] = (uint8_t)(q & 0xff);
+            }
+            __syncthreads();
+#pragma unroll
+            for (int i = 0; i < 32 / (kThreads / 64); ++i) {
+                const int pl = (kThreads / 64) * i + (threadIdx.x >> 6), cl = threadIdx.x & 63;
+                const int64_t px = p0 + pl, c = c0 + cl;
+                if (px < HW && c < C) cb[px * C + c] = tile[cl][pl];
+            }
+            __syncthreads();
+        }
+        if (psum) {
+            sums[ty][tx] = sum;
+            __syncthreads();
+            if (ty == 0 && p0 + tx < HW) {
+                int32_t s = 0;
+#pragma unroll
+                for (int j = 0; j < kThreads / 32; ++j) s += sums[j][tx];
+                psum[b * HW + p0 + tx] = s;
+            }
+            __syncthreads();
+        }
+    }
+}
+
 }  // namespace mctq
 
 using namespace mctq;
@@ -897,6 +956,27 @@ int mctq_quantize_rows_i8(const void* x, int x_dtype, int64_t M, int64_t K, floa
         uint8_t* c = reinterpret_cast<uint8_t*>(codes);
         if (vec) return launch_streaming(quantize_rows_kernel<T, true>, (unsigned)blocks, 0, st, xt, c, rowsum, M, K, scale, zp, qmin, qmax);
         return launch_streaming(quantize_rows_kernel<T, false>, (unsigned)blocks, 0, st, xt, c, rowsum, M, K, scale, zp, qmin, qmax);
+    };
+    if (x_dtype == MCTQ_F32) return run(PackType<float>{});
+    if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});
+    return run(PackType<__half>{});
+}
+
+int mctq_quantize_nhwc_i8(const void* x, int x_dtype, int64_t N, int64_t C, int64_t H, int64_t W, float scale, int32_t zp,
+                          int32_t qmin, int32_t qmax, void* codes, int32_t* P, void* stream) {
+    MCTQ_NVTX("mctq_quantize_nhwc_i8");
+    if (!x || !codes || N < 0 || C < 1 || H < 1 || W < 1) return MCTQ_E_BADARG;
+    if (x_dtype != MCTQ_F32 && x_dtype != MCTQ_BF16 && x_dtype != MCTQ_F16) return MCTQ_E_DTYPE;
+    if (qmin > qmax) return MCTQ_E_RANGE;
+    if (int rc = check_codes(qmin, qmax, MCTQ_CODES_INT8, codes)) return rc;
+    if (N == 0) return 0;
+    const int64_t HW = H * W;
+    const int64_t blocks = std::min<int64_t>(N * ((HW + 31) / 32), 148 * 16);
+    cudaStream_t st = (cudaStream_t)stream;
+    auto run = [&](auto type) {
+        using T = typename decltype(type)::type;
+        return launch_streaming(quantize_nhwc_kernel<T>, (unsigned)blocks, 0, st, reinterpret_cast<const T*>(x),
+                                reinterpret_cast<uint8_t*>(codes), P, N, C, HW, scale, zp, qmin, qmax);
     };
     if (x_dtype == MCTQ_F32) return run(PackType<float>{});
     if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});

@@ -16,6 +16,14 @@
 // There is no CTA-wide barrier in the main loop.  Split-K: the S CTAs of a cluster take consecutive chunk ranges and rank 0
 // adds the int32 partial sums of the others (distributed shared memory); integer sums are exact, so the result does not
 // depend on S or on the tiling.
+//
+// Integer convolution mode (packed_iconv_kernel, mctq_packed_conv2d_i8) is the same GEMM with batch rows = output pixels
+// (b, ho, wo) and row length K = (r, s, c) taps of the window.  Only the source of the x operand differs: warps 0-3 gather
+// it from NHWC codes.  Each producer thread owns rows tid and tid + 128 of the CTA and decomposes their window origins
+// once; Cin % 16 == 0, so each 16-byte granule of a stage row is 16 channels of one input pixel, copied with a 16-byte
+// cp.async (a tap outside the image is a splat of zx, rows >= M and columns >= K are zero).  The copies of kIConvAhead
+// stages stay in flight (cp.async groups); a stage's full barrier gets the producers' arrivals once its group has landed.
+// The epilogue writes row-major [M][Cout] (NHWC) or NCHW planes.
 #include <cuda.h>               // CUtensorMap and the cuTensorMapEncodeTiled types (the entry point is fetched at run time)
 
 #include <algorithm>
@@ -30,6 +38,7 @@ constexpr int kIMinStages = 4, kIMaxStages = 8;
 constexpr int kIMaxSplit = 8;         // portable cluster size
 constexpr int kIProducers = 128;      // warps 0-3
 constexpr int kIMmaWarp = 4;
+constexpr int kIConvAhead = 3;        // stages of gathered x in flight per producer (<= kIMinStages - 1)
 
 struct IgemmArgs {
     CUtensorMap tm_x;                 // x codes [M_total][K], box [nt][128]
@@ -48,7 +57,17 @@ struct IgemmArgs {
     int32_t per_channel, x_zp;
     int32_t nt, nchunks, stages;
     uint32_t stage_bytes, tmem_cols, idesc;
+    // integer convolution mode only
+    const uint8_t* x_nhwc;            // x codes [N][H][W][Cin]
+    MctqConv2dGeom g;
+    FastDiv div_howo, div_wo, div_cin, div_kw;
+    int32_t y_nchw;                   // y as NCHW planes instead of [M][Cout]
+    uint32_t zx_splat;                // the byte of zx, four times
 };
+
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" :: "r"(dst), "l"(src) : "memory");
+}
 
 __device__ __forceinline__ void tma_2d(const CUtensorMap* map, uint32_t dst, int32_t c0, int32_t c1, uint64_t* bar) {
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
@@ -70,8 +89,30 @@ __device__ __forceinline__ void expand8(uint32_t w, uint32_t& lo, uint32_t& hi) 
     }
 }
 
-template <bool INT4, bool WSIGNED, typename T>
-__global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_constant__ IgemmArgs a) {
+// int4 weight codes of one row, chunk c (128 codes = 64 bytes), or zeros outside the weight
+__device__ __forceinline__ void load_w4(const uint8_t* wrow, int64_t o, int64_t N, int64_t K, int c, uint4* v) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {                                        // 32 codes per 16 bytes; K % 32 == 0
+        const int64_t k = (int64_t)c * kIChunk + 32 * j;
+        v[j] = (o < N && k < K) ? ld_stream(reinterpret_cast<const uint4*>(wrow + (k >> 1))) : make_uint4(0, 0, 0, 0);
+    }
+}
+// row `row` of the weight operand of a stage: the 128 codes of v expanded to bytes
+template <bool WSIGNED>
+__device__ __forceinline__ void store_w4(uint32_t st, uint32_t row, const uint4* v) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        const uint32_t words[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
+        uint32_t g[8];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) expand8<WSIGNED>(words[q], g[2 * q], g[2 * q + 1]);
+        st_shared_v4(st + sw128_off(row, 2 * j), g);
+        st_shared_v4(st + sw128_off(row, 2 * j + 1), g + 4);
+    }
+}
+
+template <bool INT4, bool WSIGNED, typename T, bool CONV>
+__device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
     extern __shared__ __align__(1024) uint8_t dsm[];
     __shared__ uint64_t bar_full[kIMaxStages], bar_empty[kIMaxStages];
     __shared__ uint64_t bar_done;
@@ -90,7 +131,7 @@ __global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_
     }
     if (tid == 0) {
         for (int s = 0; s < nst; ++s) {
-            mbar_init(&bar_full[s], INT4 ? 1 + kIProducers : 1);
+            mbar_init(&bar_full[s], CONV ? (INT4 ? 0 : 1) + kIProducers : INT4 ? 1 + kIProducers : 1);
             mbar_init(&bar_empty[s], 1);
         }
         mbar_init(&bar_done, 1);
@@ -110,7 +151,73 @@ __global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_
 
     if (warp < 4) {
         // ---- producers
-        if (INT4) {
+        if (CONV) {
+            const MctqConv2dGeom& g = a.g;
+            const int64_t o = o0 + tid;
+            const uint8_t* wrow = a.codes + o * (K >> 1);
+            uint4 cur[4], nxt[4];
+            if (INT4 && nloc > 0) load_w4(wrow, o, N, K, c_begin, cur);
+            // the window origins of this thread's rows tid and tid + 128; `have_row`: the row is in the stage (r < nt),
+            // `live`: it is an output pixel (r < rows)
+            bool have_row[2], live[2];
+            int32_t ih0[2], iw0[2];
+            const uint8_t* img[2];
+#pragma unroll
+            for (int q = 0; q < 2; ++q) {
+                const int r = tid + kIProducers * q;
+                have_row[q] = r < nt;
+                live[q] = r < rows;
+                const uint32_t pix = live[q] ? (uint32_t)(a.m0 + n0 + r) : 0u;             // M < 2^31
+                const uint32_t b = fdiv_u32(pix, a.div_howo), rem = pix - b * (uint32_t)(g.Ho * g.Wo);
+                const uint32_t ho = fdiv_u32(rem, a.div_wo), wo = rem - ho * (uint32_t)g.Wo;
+                ih0[q] = (int32_t)ho * g.sh - g.pt;
+                iw0[q] = (int32_t)wo * g.sw - g.pl;
+                img[q] = a.x_nhwc + (int64_t)b * g.H * g.W * g.Cin;
+            }
+            const uint32_t zero[4] = {0u, 0u, 0u, 0u}, pad[4] = {a.zx_splat, a.zx_splat, a.zx_splat, a.zx_splat};
+            for (int i = 0; i < nloc; ++i) {
+                const int c = c_begin + i, s = i % nst;
+                const uint32_t st = sbase + (uint32_t)s * stage_bytes;
+                if (INT4 && i + 1 < nloc) load_w4(wrow, o, N, K, c + 1, nxt);
+                if (i >= nst) mbar_wait(&bar_empty[s], (uint32_t)((i / nst - 1) & 1));
+                if (!INT4 && tid == 0) {
+                    mbar_arrive_expect_tx(&bar_full[s], a_bytes);
+                    tma_2d(&a.tm_w, st, c * kIChunk, (int32_t)o0, &bar_full[s]);
+                }
+                if (INT4) store_w4<WSIGNED>(st, (uint32_t)tid, cur);
+#pragma unroll
+                for (int j = 0; j < kIChunk / 16; ++j) {
+                    const int32_t k = c * kIChunk + 16 * j;
+                    const bool in_k = k < K;
+                    const uint32_t tap = fdiv_u32((uint32_t)k, a.div_cin), ch = (uint32_t)k - tap * (uint32_t)g.Cin;
+                    const uint32_t rr = fdiv_u32(tap, a.div_kw), ss = tap - rr * (uint32_t)g.kw;
+                    const int32_t dy = (int32_t)rr * g.dh, dx = (int32_t)ss * g.dw;
+#pragma unroll
+                    for (int q = 0; q < 2; ++q) {
+                        if (!have_row[q]) continue;
+                        const uint32_t dst = st + a_bytes + sw128_off((uint32_t)(tid + kIProducers * q), (uint32_t)j);
+                        const int32_t ih = ih0[q] + dy, iw = iw0[q] + dx;
+                        if (live[q] && in_k && ih >= 0 && ih < g.H && iw >= 0 && iw < g.W)
+                            cp_async16(dst, img[q] + ((int64_t)ih * g.W + iw) * g.Cin + ch);
+                        else
+                            st_shared_v4(dst, live[q] && in_k ? pad : zero);
+                    }
+                }
+                asm volatile("cp.async.commit_group;" ::: "memory");
+                if (i >= kIConvAhead) {                                  // stage i - kIConvAhead has landed: publish it
+                    asm volatile("cp.async.wait_group %0;" :: "n"(kIConvAhead) : "memory");
+                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    mbar_arrive(&bar_full[(i - kIConvAhead) % nst]);
+                }
+                if (INT4) {
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) cur[j] = nxt[j];
+                }
+            }
+            asm volatile("cp.async.wait_group 0;" ::: "memory");
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            for (int i = nloc > kIConvAhead ? nloc - kIConvAhead : 0; i < nloc; ++i) mbar_arrive(&bar_full[i % nst]);
+        } else if (INT4) {
             const int64_t o = o0 + tid;
             const uint8_t* wrow = a.codes + o * (K >> 1);
             auto load = [&](int c, uint4* v) {
@@ -131,15 +238,7 @@ __global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_
                     mbar_arrive_expect_tx(&bar_full[s], (uint32_t)nt * 128u);
                     tma_2d(&a.tm_x, st + a_bytes, c * kIChunk, (int32_t)(a.m0 + n0), &bar_full[s]);
                 }
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const uint32_t words[4] = {cur[j].x, cur[j].y, cur[j].z, cur[j].w};
-                    uint32_t g[8];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) expand8<WSIGNED>(words[q], g[2 * q], g[2 * q + 1]);
-                    st_shared_v4(st + sw128_off((uint32_t)tid, 2 * j), g);
-                    st_shared_v4(st + sw128_off((uint32_t)tid, 2 * j + 1), g + 4);
-                }
+                store_w4<WSIGNED>(st, (uint32_t)tid, cur);
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");    // generic-proxy stores -> tensor-core reads
                 mbar_arrive(&bar_full[s]);
 #pragma unroll
@@ -236,7 +335,13 @@ __global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_
                 if (zw != 0 && a.x_rowsum) c -= (int64_t)zw * __ldg(a.x_rowsum + g0 + n);
                 float s = __fmul_rn(__ll2float_rn(c), f);
                 if (a.bias) s = __fadd_rn(s, b);
-                y[(g0 + n) * a.ldy + o] = from_f32<T>(s);
+                if (CONV && a.y_nchw) {                                  // pixel g of image b: plane (b, o)
+                    const uint32_t g = (uint32_t)(g0 + n), howo = (uint32_t)(a.g.Ho * a.g.Wo);
+                    const uint32_t img = fdiv_u32(g, a.div_howo);
+                    y[((int64_t)img * N + o) * howo + (g - img * howo)] = from_f32<T>(s);
+                } else {
+                    y[(g0 + n) * a.ldy + o] = from_f32<T>(s);
+                }
             }
         }
     }
@@ -248,6 +353,16 @@ __global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(a.tmem_cols) : "memory");
     }
+}
+
+template <bool INT4, bool WSIGNED, typename T>
+__global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_constant__ IgemmArgs a) {
+    igemm_body<INT4, WSIGNED, T, false>(a);
+}
+
+template <bool INT4, bool WSIGNED, typename T>
+__global__ void __launch_bounds__(kThreads, 1) packed_iconv_kernel(const __grid_constant__ IgemmArgs a) {
+    igemm_body<INT4, WSIGNED, T, true>(a);
 }
 
 }  // namespace mctq
@@ -285,9 +400,9 @@ int encode_codes(EncodeTiled fn, CUtensorMap* map, const void* base, int64_t K, 
     return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
 }
 
-template <bool INT4, bool WSIGNED, typename T>
+template <bool INT4, bool WSIGNED, typename T, bool CONV>
 int launch_igemm(IgemmArgs& a, int64_t M, cudaStream_t st) {
-    auto kernel = packed_igemm_kernel<INT4, WSIGNED, T>;
+    auto kernel = CONV ? packed_iconv_kernel<INT4, WSIGNED, T> : packed_igemm_kernel<INT4, WSIGNED, T>;
     size_t smem = (size_t)a.stages * a.stage_bytes + 1024;              // + alignment of the stages to 1024 bytes
     smem = std::max(smem, tmem_smem_floor(a.tmem_cols));
     int rc = ensure_smem(kernel, smem);
@@ -322,6 +437,58 @@ int64_t igemm_max_k(bool w_signed, bool x_signed) {
     return 33025;                                       // 255 * 255 * K < 2^31
 }
 
+// the checks both entry points make after their shape checks: factors, Sw when zx != 0, aligned codes, zx and K in range
+int igemm_check(const MctqPackedDesc* w, int64_t K, const void* x_codes, int x_signed, int32_t x_zero_point,
+                const int32_t* w_rowsum, const float* factor) {
+    if (!factor || (x_zero_point != 0 && !w_rowsum)) return MCTQ_E_BADARG;
+    if (!aligned16(x_codes) || !aligned16(w->codes)) return MCTQ_E_BADARG;
+    if (x_signed ? (x_zero_point < -128 || x_zero_point > 127) : (x_zero_point < 0 || x_zero_point > 255)) return MCTQ_E_RANGE;
+    if (K > igemm_max_k(w->is_signed != 0, x_signed != 0)) return MCTQ_E_RANGE;
+    return 0;
+}
+
+// the launch arguments shared by both modes: tiling of M rows, ring, TMEM, instruction descriptor, pointers
+void igemm_prepare(IgemmArgs& a, const MctqPackedDesc* w, int64_t N, int64_t K, int64_t M, int x_signed, int32_t x_zero_point,
+                   const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor, const void* bias, void* y) {
+    memset(&a, 0, sizeof(a));
+    const int64_t max_nt = 256;
+    const int64_t ntiles = (M + max_nt - 1) / max_nt;
+    const int64_t per = (M + ntiles - 1) / ntiles;
+    a.nt = (int32_t)((per + 15) / 16 * 16);
+    a.nchunks = (int32_t)((K + kIChunk - 1) / kIChunk);
+    a.stage_bytes = (uint32_t)(kIRows * 128 + a.nt * 128);
+    // deep rings for the HBM-bound small-batch shapes, while two CTAs still fit an SM's shared memory where they can
+    a.stages = std::min(kIMaxStages, std::max(kIMinStages, (int)((112 * 1024 - 1024) / a.stage_bytes)));
+    a.tmem_cols = tmem_columns(a.nt);
+    a.idesc = (2u << 4) | ((w->is_signed ? 1u : 0u) << 7) | ((x_signed ? 1u : 0u) << 10) | ((uint32_t)(a.nt >> 3) << 17) |
+              ((uint32_t)(kIRows >> 4) << 24);                           // s32 accumulator, K-major A and B
+    a.codes = reinterpret_cast<const uint8_t*>(w->codes);
+    a.w_zp = w->zp;
+    a.x_rowsum = x_rowsum;
+    a.w_rowsum = x_zero_point != 0 ? w_rowsum : nullptr;
+    a.factor = factor;
+    a.bias = bias;
+    a.y = y;
+    a.N = (int32_t)N;
+    a.K = (int32_t)K;
+    a.per_channel = w->C != 1;
+    a.x_zp = x_zero_point;
+}
+
+template <bool CONV>
+int igemm_run(IgemmArgs& a, const MctqPackedDesc* w, int y_dtype, int64_t M, cudaStream_t st) {
+    auto typed = [&](auto int4_tag, auto signed_tag) {
+        constexpr bool I4 = decltype(int4_tag)::value, WS = decltype(signed_tag)::value;
+        if (y_dtype == MCTQ_F32) return launch_igemm<I4, WS, float, CONV>(a, M, st);
+        if (y_dtype == MCTQ_BF16) return launch_igemm<I4, WS, __nv_bfloat16, CONV>(a, M, st);
+        return launch_igemm<I4, WS, __half, CONV>(a, M, st);
+    };
+    using True = std::true_type;
+    using False = std::false_type;
+    if (pack_is_int4(w->kind)) return w->is_signed ? typed(True{}, True{}) : typed(True{}, False{});
+    return typed(False{}, False{});         // int8 weights reach the tensor cores as stored: the signedness is in idesc
+}
+
 }  // namespace
 
 extern "C" {
@@ -336,54 +503,53 @@ int mctq_packed_linear_i8(const MctqPackedDesc* w, int64_t out_features, int64_t
     if (const int rc = packed_linear_check(w, out_features, in_features, x_codes, y_dtype, M, y)) return rc;
     const bool int4 = pack_is_int4(w->kind);
     if (in_features % (int4 ? 32 : 16) != 0 || M >= (1LL << 31) || ldy < out_features) return MCTQ_E_BADARG;
-    if (!factor || (x_zero_point != 0 && !w_rowsum)) return MCTQ_E_BADARG;
-    if (!aligned16(x_codes) || !aligned16(w->codes)) return MCTQ_E_BADARG;
-    if (x_signed ? (x_zero_point < -128 || x_zero_point > 127) : (x_zero_point < 0 || x_zero_point > 255)) return MCTQ_E_RANGE;
-    if (in_features > igemm_max_k(w->is_signed != 0, x_signed != 0)) return MCTQ_E_RANGE;
+    if (const int rc = igemm_check(w, in_features, x_codes, x_signed, x_zero_point, w_rowsum, factor)) return rc;
     if (M == 0) return 0;
 
     IgemmArgs a;
-    memset(&a, 0, sizeof(a));
-    const int64_t max_nt = 256;
-    const int64_t ntiles = (M + max_nt - 1) / max_nt;
-    const int64_t per = (M + ntiles - 1) / ntiles;
-    a.nt = (int32_t)((per + 15) / 16 * 16);
-    a.nchunks = (int32_t)((in_features + kIChunk - 1) / kIChunk);
-    a.stage_bytes = (uint32_t)(kIRows * 128 + a.nt * 128);
-    // deep rings for the HBM-bound small-batch shapes, while two CTAs still fit an SM's shared memory where they can
-    a.stages = std::min(kIMaxStages, std::max(kIMinStages, (int)((112 * 1024 - 1024) / a.stage_bytes)));
-    a.tmem_cols = tmem_columns(a.nt);
-    a.idesc = (2u << 4) | ((w->is_signed ? 1u : 0u) << 7) | ((x_signed ? 1u : 0u) << 10) | ((uint32_t)(a.nt >> 3) << 17) |
-              ((uint32_t)(kIRows >> 4) << 24);                           // s32 accumulator, K-major A and B
-    a.codes = reinterpret_cast<const uint8_t*>(w->codes);
-    a.w_zp = w->zp;
-    a.x_rowsum = x_rowsum;
-    a.w_rowsum = x_zero_point != 0 ? w_rowsum : nullptr;
-    a.factor = factor;
-    a.bias = bias;
-    a.y = y;
+    igemm_prepare(a, w, out_features, in_features, M, x_signed, x_zero_point, x_rowsum, w_rowsum, factor, bias, y);
     a.ldy = ldy;
-    a.N = (int32_t)out_features;
-    a.K = (int32_t)in_features;
-    a.per_channel = w->C != 1;
-    a.x_zp = x_zero_point;
-
     EncodeTiled fn;
     int rc = encode_fn(&fn);
     if (!rc) rc = encode_codes(fn, &a.tm_x, x_codes, in_features, M, (uint32_t)a.nt);
     if (!rc && !int4) rc = encode_codes(fn, &a.tm_w, w->codes, in_features, out_features, kIRows);
     if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    auto typed = [&](auto int4_tag, auto signed_tag) {
-        constexpr bool I4 = decltype(int4_tag)::value, WS = decltype(signed_tag)::value;
-        if (y_dtype == MCTQ_F32) return launch_igemm<I4, WS, float>(a, M, st);
-        if (y_dtype == MCTQ_BF16) return launch_igemm<I4, WS, __nv_bfloat16>(a, M, st);
-        return launch_igemm<I4, WS, __half>(a, M, st);
-    };
-    using True = std::true_type;
-    using False = std::false_type;
-    if (int4) return w->is_signed ? typed(True{}, True{}) : typed(True{}, False{});
-    return typed(False{}, False{});         // int8 weights reach the tensor cores as stored: the signedness is in idesc
+    return igemm_run<false>(a, w, y_dtype, M, (cudaStream_t)stream);
+}
+
+int mctq_packed_conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x_codes, int x_signed,
+                          int32_t x_zero_point, const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor,
+                          const void* bias, int y_dtype, void* y, int y_nchw, void* stream) {
+    MCTQ_NVTX("mctq_packed_conv2d_i8");
+    if (!w || !g || pack_is_lut(w->kind)) return MCTQ_E_BADARG;
+    if (g->N < 0 || g->H < 1 || g->W < 1 || g->Cin < 1 || g->Ho < 1 || g->Wo < 1 || g->kh < 1 || g->kw < 1 || g->sh < 1 ||
+        g->sw < 1 || g->dh < 1 || g->dw < 1 || g->pt < 0 || g->pb < 0 || g->pl < 0 || g->pr < 0 || (y_nchw != 0 && y_nchw != 1))
+        return MCTQ_E_BADARG;
+    const int64_t K = (int64_t)g->Cin * g->kh * g->kw, M = (int64_t)g->N * g->Ho * g->Wo;
+    if (const int rc = packed_linear_check(w, Cout, K, x_codes, y_dtype, M, y)) return rc;
+    const bool int4 = pack_is_int4(w->kind);
+    if (g->Cin % 16 != 0 || (int4 && K % 32 != 0) || M >= (1LL << 31)) return MCTQ_E_BADARG;
+    if (const int rc = igemm_check(w, K, x_codes, x_signed, x_zero_point, w_rowsum, factor)) return rc;
+    if (M == 0) return 0;
+
+    IgemmArgs a;
+    igemm_prepare(a, w, Cout, K, M, x_signed, x_zero_point, x_rowsum, w_rowsum, factor, bias, y);
+    a.ldy = Cout;
+    a.x_nhwc = reinterpret_cast<const uint8_t*>(x_codes);
+    a.g = *g;
+    a.div_howo = make_fastdiv((uint32_t)(g->Ho * g->Wo));
+    a.div_wo = make_fastdiv((uint32_t)g->Wo);
+    a.div_cin = make_fastdiv((uint32_t)g->Cin);
+    a.div_kw = make_fastdiv((uint32_t)g->kw);
+    a.y_nchw = y_nchw;
+    a.zx_splat = ((uint32_t)x_zero_point & 0xFFu) * 0x01010101u;
+    if (!int4) {
+        EncodeTiled fn;
+        int rc = encode_fn(&fn);
+        if (!rc) rc = encode_codes(fn, &a.tm_w, w->codes, K, Cout, kIRows);
+        if (rc) return rc;
+    }
+    return igemm_run<true>(a, w, y_dtype, M, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -12,6 +12,8 @@ sm_100a kernels.
     torch.ops.mctq.packed_linear_batched   the same product on the tensor cores                  (batched row counts)
     torch.ops.mctq.quantize_rows_i8   -> 8-bit codes of x (fq_affine_scalar's codes) and their row sums
     torch.ops.mctq.packed_linear_i8   <- the integer product of those codes and packed int8 / int4 weight codes
+    torch.ops.mctq.quantize_nhwc_i8   -> NHWC 8-bit codes of an NCHW x and their per-pixel channel sums
+    torch.ops.mctq.packed_conv2d_i8   <- the integer convolution of NHWC codes and packed weight codes (implicit GEMM)
 
 (reference call sites: see include/mctq.h).  Each op has a CUDA implementation (device pointers + the
 caller's current stream into the C ABI, no synchronisation), a CPU-tensor implementation that streams the
@@ -52,6 +54,11 @@ _LIB.define("quantize_rows_i8(Tensor x, float scale, int zero_point, int quant_m
             "-> (Tensor, Tensor)")
 _LIB.define("packed_linear_i8(Tensor x_codes, int x_zero_point, Tensor? x_rowsum, Tensor codes, int kind, bool is_signed, "
             "int out_features, Tensor zero_point, Tensor w_rowsum, Tensor factor, Tensor? bias, ScalarType dtype) -> Tensor")
+_LIB.define("quantize_nhwc_i8(Tensor x, float scale, int zero_point, int quant_min, int quant_max, bool want_sums) "
+            "-> (Tensor, Tensor)")
+_LIB.define("packed_conv2d_i8(Tensor x_codes, int x_zero_point, Tensor? x_rowsum, Tensor codes, int kind, bool is_signed, "
+            "int out_channels, int[] kernel_size, int[] stride, int[] dilation, int[] padding, Tensor zero_point, "
+            "Tensor w_rowsum, Tensor factor, Tensor? bias, ScalarType dtype, bool channels_last) -> Tensor")
 
 
 # --------------------------------------------------------------------------------------------- helpers
@@ -989,6 +996,232 @@ def _packed_linear_i8_cuda(x_codes, x_zero_point, x_rowsum, codes, kind, is_sign
     return lin.gemm(x_codes, x_rowsum, bias)
 
 
+def quantize_nhwc_i8(x, scale_f32, zero_point, quant_min, quant_max, want_sums):
+    """(codes, P) of a 4-D CUDA tensor x [N, C, H, W] under a per-tensor 8-bit affine quantizer: codes [N, H, W, C]
+    (contiguous, int8 when quant_min < 0 else uint8), exactly the codes mctq_fq_affine_scalar emits, and P int32 [N*H*W]
+    (the sum of a pixel's channel codes), or an empty tensor unless `want_sums`.  A channels_last x is quantized as rows of
+    pixels (mctq_quantize_rows_i8), any other x as NCHW planes (mctq_quantize_nhwc_i8, after .contiguous() when needed)."""
+    if x.dim() != 4:
+        raise RuntimeError(f"quantize_nhwc_i8: x must be 4-D [N, C, H, W], got shape {list(x.shape)}")
+    N, C, H, W = x.shape
+    if not x.is_contiguous() and x.is_contiguous(memory_format=torch.channels_last):
+        codes, P = quantize_rows_i8(x.permute(0, 2, 3, 1), scale_f32, zero_point, quant_min, quant_max, want_sums)
+        return codes, P
+    tag = _dtype_tag(x)
+    xd = x.contiguous()
+    codes = torch.empty((N, H, W, C), dtype=torch.int8 if quant_min < 0 else torch.uint8, device=xd.device)
+    P = torch.empty((N * H * W if want_sums else 0,), dtype=torch.int32, device=xd.device)
+    if xd.numel():
+        with _on_device(xd.device):
+            rc = _native.load().mctq_quantize_nhwc_i8(xd.data_ptr(), tag, N, C, H, W, scale_f32, zero_point, quant_min,
+                                                       quant_max, codes.data_ptr(), _ptr(P) if want_sums else None,
+                                                       _stream(xd.device))
+        _native.check(rc, "mctq_quantize_nhwc_i8")
+    return codes, P
+
+
+def _quantize_nhwc_i8_cuda(x, scale, zero_point, quant_min, quant_max, want_sums):
+    _check_range(quant_min, quant_max)
+    if not quant_min <= zero_point <= quant_max:
+        raise RuntimeError("`zero_point` must be between `quant_min` and `quant_max`.")
+    return quantize_nhwc_i8(x, float(np.float32(scale)), int(zero_point), int(quant_min), int(quant_max), bool(want_sums))
+
+
+def conv_output_hw(H, W, kernel_size, stride, dilation, padding):
+    """(Ho, Wo) of a convolution of an H x W image; padding = (pt, pb, pl, pr)."""
+    (kh, kw), (sh, sw), (dh, dw), (pt, pb, pl, pr) = kernel_size, stride, dilation, padding
+    return (H + pt + pb - dh * (kh - 1) - 1) // sh + 1, (W + pl + pr - dw * (kw - 1) - 1) // sw + 1
+
+
+def conv_padding(layer):
+    """(pt, pb, pl, pr) of a torch.nn.Conv2d, from `_reversed_padding_repeated_twice` ((left, right, top, bottom)): numeric
+    padding, 'valid' and the asymmetric 'same'."""
+    pl, pr, pt, pb = (int(p) for p in layer._reversed_padding_repeated_twice)
+    return pt, pb, pl, pr
+
+
+def pack_weight_codes(qw, kind, is_signed):
+    """Packed codes (int8 / uint8 bytes, or int4 nibbles two per byte, element 2j in the low nibble) of the integer codes
+    qw, in qw's element order: the inverse of weight_code_values."""
+    q = qw.reshape(-1)
+    if kind == _native.PACK_AFFINE_I4:
+        u = (q & 15).to(torch.uint8)
+        if u.numel() % 2:
+            u = torch.cat((u, u.new_zeros(1)))
+        u = u.reshape(-1, 2)
+        return (u[:, 0] | (u[:, 1] << 4)).contiguous()
+    return q.to(torch.int8 if is_signed else torch.uint8).contiguous()
+
+
+def conv_codes_rsc(codes, kind, is_signed, out_channels, in_channels, kh, kw):
+    """The packed codes of a contiguous [Cout, Cin, kh, kw] weight ((c, r, s) order per output channel) reordered to the
+    (r, s, c) order of mctq_packed_conv2d_i8 (one-time set-up of IntegerConv2d)."""
+    qw = weight_code_values(codes, kind, is_signed, out_channels, in_channels * kh * kw)
+    qw = qw.reshape(out_channels, in_channels, kh, kw).permute(0, 2, 3, 1)
+    out = pack_weight_codes(qw.contiguous(), kind, is_signed)
+    return out.view(codes.dtype) if kind == _native.PACK_AFFINE_I8 else out
+
+
+def conv_window_sums(P, N, H, W, Cin, kernel_size, stride, dilation, padding, x_zero_point):
+    """Sx [N*Ho*Wo] (int32) from the per-pixel channel sums P [N*H*W]: the sum of P over each output pixel's window, a tap
+    outside the image counting Cin * zx.  Exact int32 torch ops (no host synchronisation, capturable)."""
+    (kh, kw), (sh, sw), (dh, dw), (pt, pb, pl, pr) = kernel_size, stride, dilation, padding
+    Ho, Wo = conv_output_hw(H, W, kernel_size, stride, dilation, padding)
+    p = torch.nn.functional.pad(P.reshape(N, H, W), (pl, pr, pt, pb), value=Cin * int(x_zero_point))
+    sx = torch.zeros((N, Ho, Wo), dtype=torch.int32, device=P.device)
+    for r in range(kh):
+        for s in range(kw):
+            sx += p[:, r * dh: r * dh + (Ho - 1) * sh + 1: sh, s * dw: s * dw + (Wo - 1) * sw + 1: sw]
+    return sx.reshape(-1)
+
+
+def _suggests_channels_last(shape, stride):
+    from torch._prims_common import suggest_memory_format
+    return suggest_memory_format(torch.empty_strided(tuple(shape), tuple(stride), device="meta")) == torch.channels_last
+
+
+class IntegerConv2d:
+    """Launch state of one packed affine Conv2d weight [Cout, Cin, kh, kw] (groups 1, zero padding) in integer convolution
+    mode (mctq_quantize_nhwc_i8 + mctq_packed_conv2d_i8), built once, like IntegerLinear: the weight codes in (r, s, c) order,
+    the descriptor, Sw, f = fl32(sx * scale), the geometry and the input quantizer's launch constants.
+        codes, kind, is_signed   the packed weight (PACK_AFFINE_I8 / PACK_AFFINE_I4)
+        weight_stride            the rebuilt weight's strides: contiguous codes are reordered once, channels_last codes
+                                 already have the (r, s, c) order and are used as they are
+        dtype                    the rebuilt weight's dtype: x, bias and y have it
+        kernel_size, stride, dilation   pairs;  padding = (pt, pb, pl, pr)
+        scale, zero_point        f32 / int32, 1 (per tensor) or Cout entries
+        x_scale, x_zero_point, x_qmin, x_qmax   the input quantizer Q (per tensor, at most 256 levels)
+    `__call__(x, bias)` returns the integer convolution of Q's codes of a 4-D CUDA x of `dtype` on the codes' device with the
+    weight codes, scaled (include/mctq.h gives the formula), in the memory format F.conv2d gives for x and the rebuilt
+    weight.  `quantize` and `gemm` are its launches."""
+
+    def __init__(self, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, weight_stride, stride,
+                 dilation, padding, scale, zero_point, x_scale, x_zero_point, x_qmin, x_qmax):
+        _check_range(x_qmin, x_qmax)
+        if not ((-128 <= x_qmin and x_qmax <= 127) or (0 <= x_qmin and x_qmax <= 255)):
+            raise ValueError(f"IntegerConv2d: the input range [{x_qmin}, {x_qmax}] does not fit 8-bit codes")
+        if not x_qmin <= x_zero_point <= x_qmax:
+            raise RuntimeError("`zero_point` must be between `quant_min` and `quant_max`.")
+        self.device = codes.device
+        self.x_scale, self.x_zp = float(np.float32(x_scale)), int(x_zero_point)
+        self.x_qmin, self.x_qmax = int(x_qmin), int(x_qmax)
+        kh, kw = (int(k) for k in kernel_size)
+        shape = (int(out_channels), int(in_channels), kh, kw)
+        self.weight_channels_last = _suggests_channels_last(shape, weight_stride)
+        if tuple(weight_stride) == tuple(torch.empty(shape, device="meta").stride()):
+            codes = conv_codes_rsc(codes, kind, is_signed, *shape)
+        elif tuple(weight_stride) != tuple(torch.empty(shape, device="meta").to(memory_format=torch.channels_last).stride()):
+            raise ValueError(f"IntegerConv2d: weight strides {tuple(weight_stride)} are neither contiguous nor channels_last")
+        s = _param_on(scale.detach().reshape(-1).contiguous().to(torch.float32), self.device)
+        factor = torch.tensor(self.x_scale, dtype=torch.float32, device=self.device) * s
+        self._bind(codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, None,
+                   "IntegerConv2d")
+
+    @classmethod
+    def from_parts(cls, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, stride, dilation, padding,
+                   factor, zero_point, w_rowsum, x_zero_point):
+        """The launch state from caller-supplied (r, s, c)-ordered codes, f and Sw (mctq::packed_conv2d_i8), with the
+        constructor's checks of the weight; only `gemm` is available."""
+        conv = cls.__new__(cls)
+        conv.device = codes.device
+        conv.x_zp, conv.x_scale, conv.x_qmin, conv.x_qmax = int(x_zero_point), None, None, None
+        conv.weight_channels_last = False
+        shape = (int(out_channels), int(in_channels), int(kernel_size[0]), int(kernel_size[1]))
+        conv._bind(codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum,
+                   "packed_conv2d_i8")
+        return conv
+
+    def _bind(self, codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum, what):
+        if len(stride) != 2 or len(dilation) != 2 or len(padding) != 4:
+            raise ValueError(f"{what}: stride and dilation are pairs, padding is (top, bottom, left, right)")
+        self.stride, self.dilation = tuple(int(v) for v in stride), tuple(int(v) for v in dilation)
+        self.padding = tuple(int(v) for v in padding)
+        self.out_channels, self.in_channels = shape[0], shape[1]
+        self.kernel_size = shape[2:]
+        K = shape[1] * shape[2] * shape[3]
+        # the weight as a [Cout][K] matrix: IntegerLinear's checks and launch state
+        self._w = IntegerLinear.__new__(IntegerLinear)
+        self._w.device, self._w.x_zp = self.device, self.x_zp
+        self._w._bind(codes, kind, is_signed, dtype, shape[0], K, factor, zero_point, w_rowsum, what)
+        self.dtype, self.factor, self.w_rowsum = dtype, self._w.factor, self._w.w_rowsum
+        self.needs_x_rowsum = self._w.needs_x_rowsum
+
+    def output_hw(self, H, W):
+        return conv_output_hw(H, W, self.kernel_size, self.stride, self.dilation, self.padding)
+
+    def __call__(self, x, bias=None):
+        if x.dtype != self.dtype or (bias is not None and bias.dtype != self.dtype):
+            raise RuntimeError(f"packed_conv2d_i8: x and bias must have the weight's dtype {self.dtype}")
+        cl = self.weight_channels_last or _suggests_channels_last(x.shape, x.stride())
+        qx, sx = self.quantize(x)
+        return self.gemm(qx, sx, bias, channels_last=cl)
+
+    def quantize(self, x):
+        """Q's NHWC codes of x and Sx (empty when no weight zero point needs it)."""
+        if x.dim() != 4 or x.shape[1] != self.in_channels:
+            raise RuntimeError(f"packed_conv2d_i8: x of shape {list(x.shape)} is not [N, {self.in_channels}, H, W]")
+        if x.device != self.device:
+            raise RuntimeError(f"packed_conv2d_i8: x must live on {self.device}")
+        qx, P = quantize_nhwc_i8(x, self.x_scale, self.x_zp, self.x_qmin, self.x_qmax, self.needs_x_rowsum)
+        if not self.needs_x_rowsum:
+            return qx, None
+        N, _, H, W = x.shape
+        return qx, conv_window_sums(P, N, H, W, self.in_channels, self.kernel_size, self.stride, self.dilation,
+                                    self.padding, self.x_zp)
+
+    def gemm(self, x_codes, x_rowsum=None, bias=None, channels_last=False):
+        """y [N, Cout, Ho, Wo] from NHWC x codes [N, H, W, Cin] (int8 or uint8, zero point x_zero_point) and Sx [N*Ho*Wo];
+        channels_last: y's memory format (the kernel writes it directly)."""
+        if x_codes.dtype not in (torch.int8, torch.uint8) or x_codes.dim() != 4 or x_codes.shape[-1] != self.in_channels:
+            raise RuntimeError(f"packed_conv2d_i8: x codes ({x_codes.dtype}, {list(x_codes.shape)}) are not int8 / uint8 "
+                               f"NHWC codes of {self.in_channels} channels")
+        if x_codes.device != self.device or (bias is not None and bias.device != self.device):
+            raise RuntimeError(f"packed_conv2d_i8: x codes and bias must live on {self.device}")
+        if bias is not None and (bias.numel() != self.out_channels or bias.dtype != self.dtype):
+            raise RuntimeError(f"packed_conv2d_i8: bias must hold {self.out_channels} entries of {self.dtype}")
+        if self.needs_x_rowsum and x_rowsum is None:
+            raise RuntimeError("packed_conv2d_i8: a weight zero point is not 0, so the window code sums Sx are needed")
+        qx = x_codes.contiguous()
+        N, H, W, _ = qx.shape
+        Ho, Wo = self.output_hw(H, W)
+        if Ho < 1 or Wo < 1:
+            raise RuntimeError(f"packed_conv2d_i8: a {H} x {W} input is smaller than the dilated kernel")
+        Cout = self.out_channels
+        if channels_last:
+            y = torch.empty((N, Ho, Wo, Cout), dtype=self.dtype, device=self.device).permute(0, 3, 1, 2)
+        else:
+            y = torch.empty((N, Cout, Ho, Wo), dtype=self.dtype, device=self.device)
+        M = N * Ho * Wo
+        if M:
+            rs = x_rowsum.reshape(-1).contiguous() if x_rowsum is not None and self.needs_x_rowsum else None
+            if rs is not None and (rs.dtype != torch.int32 or rs.numel() != M or rs.device != self.device):
+                raise RuntimeError(f"packed_conv2d_i8: x_rowsum must be int32 [{M}] on {self.device}")
+            b = bias.contiguous() if bias is not None else None
+            g = _native.MctqConv2dGeom(N, H, W, self.in_channels, Ho, Wo, *self.kernel_size, *self.stride, *self.dilation,
+                                       *self.padding)
+            with _on_device(self.device):
+                rc = _native.load().mctq_packed_conv2d_i8(
+                    self._w._desc_ptr, ctypes.addressof(g), Cout, qx.data_ptr(), int(qx.dtype == torch.int8), self.x_zp,
+                    _ptr(rs), self.w_rowsum.data_ptr(), self.factor.data_ptr(), _ptr(b), _DT[self.dtype], y.data_ptr(),
+                    0 if channels_last else 1, _stream(self.device))
+            _native.check(rc, "mctq_packed_conv2d_i8")
+        return y
+
+
+def _packed_conv2d_i8_cuda(x_codes, x_zero_point, x_rowsum, codes, kind, is_signed, out_channels, kernel_size, stride,
+                           dilation, padding, zero_point, w_rowsum, factor, bias, dtype, channels_last):
+    """mctq::packed_conv2d_i8: NHWC x codes, (r, s, c)-ordered weight codes, caller-supplied Sw and f; x_rowsum (Sx) may be
+    None only when every weight zero point is 0."""
+    if x_codes.dim() != 4:
+        raise RuntimeError("packed_conv2d_i8: x codes must be 4-D NHWC")
+    if len(kernel_size) != 2:
+        raise ValueError("packed_conv2d_i8: kernel_size is a pair")
+    _native.load()
+    conv = IntegerConv2d.from_parts(codes, kind, is_signed, dtype, out_channels, x_codes.shape[-1], kernel_size, stride,
+                                    dilation, padding, factor, zero_point, w_rowsum, x_zero_point)
+    return conv.gemm(x_codes, x_rowsum, bias, channels_last)
+
+
 def _lut_scalar_cuda(x, table, K, divisor, threshold, round_to_input_dtype, multiply=False):
     """`multiply`: normalise with x * (float)(1.0 / divisor) -- the reference's CUDA flavour of `tensor / python_number`
     (quantizer_utils.reference_arithmetic) -- instead of the true division x / (float)divisor."""
@@ -1188,6 +1421,8 @@ _LIB.impl("packed_linear", _packed_linear_cuda, "CUDA")
 _LIB.impl("packed_linear_batched", _packed_linear_batched_cuda, "CUDA")
 _LIB.impl("quantize_rows_i8", _quantize_rows_i8_cuda, "CUDA")
 _LIB.impl("packed_linear_i8", _packed_linear_i8_cuda, "CUDA")
+_LIB.impl("quantize_nhwc_i8", _quantize_nhwc_i8_cuda, "CUDA")
+_LIB.impl("packed_conv2d_i8", _packed_conv2d_i8_cuda, "CUDA")
 
 _LIB.impl("fq_affine_scalar_pre", _affine_scalar_pre_cuda, "CUDA")
 _LIB.impl("fq_affine_scalar_pre", _via_device(_affine_scalar_pre_cuda), "CPU")
@@ -1204,6 +1439,8 @@ _LIB.impl("packed_linear", _via_device(_packed_linear_cuda), "CPU")
 _LIB.impl("packed_linear_batched", _via_device(_packed_linear_batched_cuda), "CPU")
 _LIB.impl("quantize_rows_i8", _via_device(_quantize_rows_i8_cuda), "CPU")
 _LIB.impl("packed_linear_i8", _via_device(_packed_linear_i8_cuda), "CPU")
+_LIB.impl("quantize_nhwc_i8", _via_device(_quantize_nhwc_i8_cuda), "CPU")
+_LIB.impl("packed_conv2d_i8", _via_device(_packed_conv2d_i8_cuda), "CPU")
 
 
 # --------------------------------------------------------------------------------------------- fake / meta impls
@@ -1283,6 +1520,23 @@ def _(x, scale, zero_point, quant_min, quant_max, want_rowsum):
 @torch.library.register_fake("mctq::packed_linear_i8")
 def _(x_codes, x_zero_point, x_rowsum, codes, kind, is_signed, out_features, zero_point, w_rowsum, factor, bias, dtype):
     return x_codes.new_empty(tuple(x_codes.shape[:-1]) + (out_features,), dtype=dtype)
+
+
+@torch.library.register_fake("mctq::quantize_nhwc_i8")
+def _(x, scale, zero_point, quant_min, quant_max, want_sums):
+    N, C, H, W = x.shape
+    return (x.new_empty((N, H, W, C), dtype=torch.int8 if quant_min < 0 else torch.uint8),
+            x.new_empty((N * H * W if want_sums else 0,), dtype=torch.int32))
+
+
+@torch.library.register_fake("mctq::packed_conv2d_i8")
+def _(x_codes, x_zero_point, x_rowsum, codes, kind, is_signed, out_channels, kernel_size, stride, dilation, padding,
+      zero_point, w_rowsum, factor, bias, dtype, channels_last):
+    N, H, W, _ = x_codes.shape
+    Ho, Wo = conv_output_hw(H, W, kernel_size, stride, dilation, padding)
+    if channels_last:
+        return x_codes.new_empty((N, Ho, Wo, out_channels), dtype=dtype).permute(0, 3, 1, 2)
+    return x_codes.new_empty((N, out_channels, Ho, Wo), dtype=dtype)
 
 
 # --------------------------------------------------------------------------------------------- whole-model launch

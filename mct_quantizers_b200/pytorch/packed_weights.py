@@ -38,6 +38,14 @@ outputs and of W to that dtype).  It is a numerical contract of its own, so it c
 traces the model with torch.fx (holders and wrappers as leaves) and switches each eligible wrapper whose input is a holder's
 output, directly or through flatten / reshape / view / contiguous; integer mode takes precedence over fused / batched mode.
 
+Integer convolution mode (`pack_model_weights(model, integer_conv=True)`, or `wrapper.pack_weights(integer_conv=True,
+input_quantizer=q)`; opt-in, and it may be combined with integer_linear=True): the same arithmetic for a packed
+`torch.nn.Conv2d` wrapper (groups 1, zero padding, Cin a multiple of 16) fed by such a holder.  Q's codes of x are written
+channels-innermost (NHWC, csrc/mctq_affine.cu, mctq_quantize_nhwc_i8) and the convolution is an implicit GEMM whose x
+operand is gathered from each output pixel's window (csrc/mctq_packed_igemm.cu, mctq_packed_conv2d_i8); a padded tap holds
+Q's zero-point code and contributes exactly 0.  The output has the memory format F.conv2d gives for x and the rebuilt
+weight.  Inputs that are not 4-D (unbatched 3-D inputs included) take the packed path.
+
 Packing is one-way and for inference only:
   * the rebuild dtype is the weight's dtype at packing time; `.half()` does not change it (the codes are integer buffers);
   * the packed state travels with the module: `state_dict` / `load_state_dict` between packed models of the same structure,
@@ -258,17 +266,10 @@ def batched_linear_eligibility(wrapper) -> Tuple[bool, str]:
     return True, ""
 
 
-def integer_linear_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
-    """(True, '') when `wrapper` can run in integer linear mode with input quantizer `input_quantizer`: fused_linear_eligibility,
-    int8 / int4 affine codes, a per-tensor affine activation quantizer with 8-bit codes, in_features a multiple of 16 (32 for
-    int4 codes) and at most the int32 bound of the code signedness pair.  Host-only."""
+def _input_quantizer_eligibility(input_quantizer) -> Tuple[bool, str]:
+    """The conditions integer linear and integer convolution mode put on the input quantizer: per-tensor affine, no reuse
+    of its outputs, 8-bit codes."""
     from mct_quantizers_b200.pytorch.fused_activation_holder import affine_scalar_params
-    ok, reason = fused_linear_eligibility(wrapper)
-    if not ok:
-        return ok, reason
-    e = next(e for e in wrapper.__dict__['_packed'].entries if e.name == 'weight')
-    if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
-        return False, f"the weight is packed as {_KIND_NAMES[e.kind]}, not as int8 / int4 affine codes"
     if affine_scalar_params(input_quantizer) is None:
         return False, (f"the input quantizer {type(input_quantizer).__name__} is not a per-tensor affine activation quantizer "
                        f"(ActivationSymmetric / POT / Uniform)")
@@ -277,6 +278,23 @@ def integer_linear_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
     qmin, qmax = int(input_quantizer.min_quantized_domain), int(input_quantizer.max_quantized_domain)
     if not ((-128 <= qmin and qmax <= 127) or (0 <= qmin and qmax <= 255)):
         return False, f"the input quantization range [{qmin}, {qmax}] does not fit 8-bit codes"
+    return True, ""
+
+
+def integer_linear_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
+    """(True, '') when `wrapper` can run in integer linear mode with input quantizer `input_quantizer`: fused_linear_eligibility,
+    int8 / int4 affine codes, a per-tensor affine activation quantizer with 8-bit codes, in_features a multiple of 16 (32 for
+    int4 codes) and at most the int32 bound of the code signedness pair.  Host-only."""
+    ok, reason = fused_linear_eligibility(wrapper)
+    if not ok:
+        return ok, reason
+    e = next(e for e in wrapper.__dict__['_packed'].entries if e.name == 'weight')
+    if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
+        return False, f"the weight is packed as {_KIND_NAMES[e.kind]}, not as int8 / int4 affine codes"
+    ok, reason = _input_quantizer_eligibility(input_quantizer)
+    if not ok:
+        return ok, reason
+    qmin = int(input_quantizer.min_quantized_domain)
     K = wrapper.layer.in_features
     step = 32 if e.kind == _native.PACK_AFFINE_I4 else 16
     if K % step:
@@ -284,6 +302,53 @@ def integer_linear_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
     bound = _native.integer_linear_max_k(e.is_signed, qmin < 0)
     if K > bound:
         return False, f"in_features = {K} exceeds {bound}, the largest row length whose int32 sum of code products cannot overflow"
+    return True, ""
+
+
+def integer_conv_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
+    """(True, '') when `wrapper` can run in integer convolution mode with input quantizer `input_quantizer`: a
+    torch.nn.Conv2d layer with string-attribute weights, no extra call arguments and 'weight' its only quantized weight,
+    packed as int8 / int4 affine codes, rebuilt as a contiguous or channels_last [Cout, Cin, kh, kw] weight with parameters
+    per tensor or per output channel; groups 1 and zero padding; the input quantizer conditions of integer linear mode;
+    Cin a multiple of 16, K = Cin * kh * kw a multiple of 32 for int4 codes and at most the int32 bound of the code
+    signedness pair.  Host-only."""
+    d = wrapper.__dict__
+    if not d.get('is_str_attr', False):
+        return False, "the weights are positional inputs of a functional op"
+    layer = d['_modules'].get(LAYER)
+    if type(layer) is not torch.nn.Conv2d:
+        return False, f"the layer is {type(layer).__name__}, not torch.nn.Conv2d"
+    if d.get('op_call_args') or d.get('op_call_kwargs') or d.get('is_inputs_as_list'):
+        return False, "the wrapper passes extra call arguments to the layer"
+    if list(wrapper.weights_quantizers) != ['weight']:
+        return False, "the wrapper quantizes weights other than 'weight'"
+    if layer.groups != 1:
+        return False, f"groups = {layer.groups}: a grouped or depthwise convolution is not one matrix product"
+    if layer.padding_mode != 'zeros':
+        return False, f"padding_mode = {layer.padding_mode!r}: only zero padding is a padding with Q's zero-point code"
+    state = d.get('_packed')
+    e = next((e for e in state.entries if e.name == 'weight'), None) if state is not None else None
+    if e is None:
+        return False, "the weight is not packed"
+    if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
+        return False, f"the weight is packed as {_KIND_NAMES[e.kind]}, not as int8 / int4 affine codes"
+    shape = (layer.out_channels, layer.in_channels) + tuple(layer.kernel_size)
+    dense = torch.empty(shape, device="meta")
+    if e.shape_out != shape or e.stride_out not in (dense.stride(), dense.to(memory_format=torch.channels_last).stride()):
+        return False, "the rebuilt weight is not a contiguous or channels_last [Cout, Cin, kh, kw] tensor"
+    K = shape[1] * shape[2] * shape[3]
+    if not (e.C == 1 or (e.C == shape[0] and e.inner == K)):
+        return False, "the parameters are not per tensor or per output channel (channel_axis 0)"
+    ok, reason = _input_quantizer_eligibility(input_quantizer)
+    if not ok:
+        return ok, reason
+    if shape[1] % 16:
+        return False, f"in_channels = {shape[1]} is not a multiple of 16"
+    if e.kind == _native.PACK_AFFINE_I4 and K % 32:
+        return False, f"Cin * kh * kw = {K} is not a multiple of 32 (int4 codes)"
+    bound = _native.integer_linear_max_k(e.is_signed, int(input_quantizer.min_quantized_domain) < 0)
+    if K > bound:
+        return False, f"Cin * kh * kw = {K} exceeds {bound}, the largest row length whose int32 sum of code products cannot overflow"
     return True, ""
 
 
@@ -406,8 +471,9 @@ class PackedState:
         return lin[1](x, bias)
 
     def integer_forward(self, wrapper, x):
-        """layer(Q(x)) in integer arithmetic (ops.IntegerLinear), or None when this call must take the packed path of the
-        wrapper's other modes: the conditions of fused_forward, without its row limit."""
+        """layer(Q(x)) in integer arithmetic (ops.IntegerLinear, or ops.IntegerConv2d for a Conv2d layer), or None when this
+        call must take the packed path of the wrapper's other modes: the conditions of fused_forward, without its row limit;
+        a Conv2d layer also needs a 4-D x."""
         e = self.entries[0]
         if e._owner is None or e._owner() is not wrapper:
             self.bind(wrapper)
@@ -415,7 +481,13 @@ class PackedState:
             return None
         layer = wrapper.__dict__['_modules'][LAYER]
         bias = layer.bias
-        if x.shape[-1] != layer.in_features or (bias is not None and (bias.dtype != x.dtype or bias.device != x.device)):
+        conv = type(layer) is torch.nn.Conv2d
+        if conv:
+            if x.dim() != 4 or x.shape[1] != layer.in_channels:
+                return None
+        elif x.shape[-1] != layer.in_features:
+            return None
+        if bias is not None and (bias.dtype != x.dtype or bias.device != x.device):
             return None
         if torch.is_grad_enabled() and (x.requires_grad or (bias is not None and bias.requires_grad)):
             return None
@@ -432,8 +504,14 @@ class PackedState:
             scale, zp, _, _ = affine_scalar_params(q)
             x_scale, x_zp, qmin, qmax = q._validated_launch_args(scale, zp)[1]      # what the holder's kernel receives
             item = e.plan_item()
-            lin = (codes.data_ptr(), ops.IntegerLinear(codes, e.kind, e.is_signed, e.dtype_out, layer.out_features,
-                                                       layer.in_features, item[8], item[9], x_scale, x_zp, qmin, qmax))
+            if conv:
+                launch = ops.IntegerConv2d(codes, e.kind, e.is_signed, e.dtype_out, layer.out_channels, layer.in_channels,
+                                           layer.kernel_size, e.stride_out, layer.stride, layer.dilation,
+                                           ops.conv_padding(layer), item[8], item[9], x_scale, x_zp, qmin, qmax)
+            else:
+                launch = ops.IntegerLinear(codes, e.kind, e.is_signed, e.dtype_out, layer.out_features, layer.in_features,
+                                           item[8], item[9], x_scale, x_zp, qmin, qmax)
+            lin = (codes.data_ptr(), launch)
             self._ilin = lin
         return lin[1](x, bias)
 
@@ -464,7 +542,7 @@ class PackedState:
 
 
 def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bool = False, integer_linear: bool = False,
-                         input_quantizer=None) -> Dict:
+                         input_quantizer=None, integer_conv: bool = False) -> Dict:
     """Pack every weight of `wrapper` that can be packed (see the module docstring).  Returns
     {name: {'packed': bool, 'kind': str | None, 'reason': str, 'code_bytes': int, 'float_bytes': int}}.
     `fused_linear=True` also switches the wrapper to fused linear mode when fused_linear_eligibility allows it (on a wrapper
@@ -473,11 +551,15 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
     allows it, and every report entry gains 'batched': bool and 'batched_reason': str.
     `integer_linear=True` (needs `input_quantizer`, the quantizer of the activation holder whose output the wrapper reads)
     also switches it to integer linear mode when integer_linear_eligibility allows it, and every report entry gains
-    'integer': bool, 'integer_reason': str and 'input_holder' (the holder's module name for pack_model_weights, else None)."""
+    'integer': bool, 'integer_reason': str and 'input_holder' (the holder's module name for pack_model_weights, else None).
+    `integer_conv=True` (needs `input_quantizer` too) does the same for integer convolution mode (integer_conv_eligibility),
+    and every report entry gains 'integer_conv': bool, 'integer_conv_reason': str and 'input_holder'."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     if integer_linear and input_quantizer is None:
         raise ValueError("integer_linear=True needs the input_quantizer of the activation holder that feeds the wrapper")
+    if integer_conv and input_quantizer is None:
+        raise ValueError("integer_conv=True needs the input_quantizer of the activation holder that feeds the wrapper")
     report = {}
     state = wrapper.__dict__.get('_packed')
     entries = list(state.entries) if state is not None else []
@@ -509,6 +591,8 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
         _switch_to_batched(wrapper, report)
     if integer_linear:
         _switch_to_integer(wrapper, report, input_quantizer, None)
+    if integer_conv:
+        _switch_to_integer(wrapper, report, input_quantizer, None, conv=True)
     return report
 
 
@@ -553,14 +637,16 @@ def _switch_to_batched(wrapper, report):
         r['batched'], r['batched_reason'] = ok, reason
 
 
-def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None):
-    ok, why = (False, reason) if reason else integer_linear_eligibility(wrapper, input_quantizer)
+def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None, conv=False):
+    eligibility = integer_conv_eligibility if conv else integer_linear_eligibility
+    ok, why = (False, reason) if reason else eligibility(wrapper, input_quantizer)
     state = wrapper.__dict__.get('_packed')
     if ok:
         state.integer, state.input_quantizer, state._ilin = True, input_quantizer, None
     _report_packed_entries(wrapper, report)
+    flag, flag_reason = ('integer_conv', 'integer_conv_reason') if conv else ('integer', 'integer_reason')
     for r in report.values():
-        r['integer'], r['integer_reason'], r['input_holder'] = ok, why, holder_name
+        r[flag], r[flag_reason], r['input_holder'] = ok, why, holder_name
 
 
 def _report_packed_entries(wrapper, report):
@@ -576,22 +662,24 @@ def _bits(t):
 
 
 def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batched_linear: bool = False,
-                       integer_linear: bool = False) -> Dict[str, Dict]:
+                       integer_linear: bool = False, integer_conv: bool = False) -> Dict[str, Dict]:
     """pack_weights(fused_linear, batched_linear) on every PytorchQuantizationWrapper of `model`: {wrapper module name:
     {weight name: report entry}}.  `integer_linear=True` then switches, in place, every eligible wrapper whose input is the
     output of an activation quantization holder (integer_linear_edges) to integer linear mode; every report entry gains
-    'integer', 'integer_reason' and 'input_holder'.  When the model cannot be traced nothing is switched and the reason is
-    reported."""
+    'integer', 'integer_reason' and 'input_holder'.  `integer_conv=True` does the same for integer convolution mode on the
+    same edges; every report entry gains 'integer_conv', 'integer_conv_reason' and 'input_holder'.  When the model cannot be
+    traced nothing is switched and the reason is reported."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
     wrappers = {mod_name: mod for mod_name, mod in model.named_modules()
                 if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization}
     reports = {name: pack_wrapper_weights(mod, fused_linear, batched_linear) for name, mod in wrappers.items()}
-    if integer_linear:
+    if integer_linear or integer_conv:
         edges, why, failure = integer_linear_edges(model)
         for name, mod in wrappers.items():
             holder, q = edges.get(name, (None, None)) if name not in why else (None, None)
             reason = failure or why.get(name) or ("" if holder else "the wrapper is not called in the traced forward")
-            _switch_to_integer(mod, reports[name], q, holder, None if holder else reason)
+            for conv in (False, True) if integer_linear and integer_conv else (integer_conv,):
+                _switch_to_integer(mod, reports[name], q, holder, None if holder else reason, conv=conv)
     return reports
