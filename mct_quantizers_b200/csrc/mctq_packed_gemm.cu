@@ -1,4 +1,4 @@
-// mctq_packed_gemm.cu -- y = x @ W^T + b straight from packed codes on the tensor cores (tcgen05.mma, kind::f16), for the
+// mctq_packed_gemm.cu -- y = x @ W^T + b straight from packed codes on the tensor cores (tcgen05 MMA, kind::f16), for the
 // batched row counts (9 to a few hundred) of batched decode, speculative decoding and short prefills.  The batched mode of
 // packed nn.Linear wrappers (pytorch/packed_weights.py) calls it above the row limit of mctq_packed_linear.cu.
 //
@@ -18,15 +18,15 @@
 // Split-K: the S CTAs of a thread-block cluster share one 128-row tile and take consecutive chunk ranges; ranks 1..S-1
 // leave their partial sums in their shared memory and rank 0 adds them to its own in rank order (distributed shared
 // memory), so the result is deterministic with no workspace.  The epilogue (tcgen05.ld) gives each thread one output feature,
-// so stores of consecutive lanes coalesce.
-#include <algorithm>
+// so stores of consecutive lanes coalesce.  TMEM, MMA issue, split-K tile and reduction and the launches over row ranges are
+// the frame of mctq_tcgen05.cuh, shared with mctq_packed_igemm.cu; this file owns the decode loop, the split policy and the
+// epilogue arithmetic.
 #include <type_traits>
 
 #include "mctq_tcgen05.cuh"
 
 namespace mctq {
 
-constexpr int kGemmRows = 128;          // output features per CTA (the MMA's M)
 constexpr int kChunk = 64;              // elements of the row length per stage (one 128-byte swizzle row of bf16 / f16)
 constexpr int kStages = 3;
 constexpr int kMaxSplit = 8;            // portable cluster size
@@ -68,7 +68,7 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
     using OT = typename std::conditional<std::is_same<T, __half>::value, __half, __nv_bfloat16>::type;   // operand type
     constexpr int XW = F32X ? 8 : 4;                                     // 32-bit words of x per 8 elements
     constexpr int XU = (F32X ? 128 : 256) * 8 / kThreads;                // max x units (row, 8-element group) per thread
-    constexpr int WU = kGemmRows * 8 / kThreads;                         // weight units per thread (4)
+    constexpr int WU = kTcRows * 8 / kThreads;                           // weight units per thread (4)
     static_assert(kThreads == 256 && WU == 4, "thread mapping");
 
     extern __shared__ __align__(1024) uint8_t dsm[];
@@ -77,17 +77,14 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
     __shared__ uint32_t tmem_slot;
     __shared__ float sm_q[LUT ? 256 : 1];
 
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int tid = threadIdx.x, warp = tid >> 5;
     const int nt = a.nt;
-    const uint32_t a_bytes = kGemmRows * 128, b_bytes = (uint32_t)nt * 128, stage_bytes = a_bytes + TERMS * b_bytes;
+    const uint32_t a_bytes = kTcRows * 128, b_bytes = (uint32_t)nt * 128, stage_bytes = a_bytes + TERMS * b_bytes;
     const uint32_t sbase = (smem_u32(dsm) + 1023u) & ~1023u;             // swizzle atoms need 1024-byte alignment
 
     pdl_wait();                 // x may be the output of the previous launch; TMEM is taken only after the wait
     pdl_launch_dependents();
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(&tmem_slot)), "r"(a.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    tmem_alloc(warp, &tmem_slot, a.tmem_cols);
     if (tid == 0) {
         for (int s = 0; s < kStages; ++s) mbar_init(&bar_empty[s], 1);
         mbar_init(&bar_done, 1);
@@ -95,18 +92,13 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
     if constexpr (LUT) {
         for (int i = tid; i < 256; i += kThreads) sm_q[i] = a.quot[i];
     }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = tmem_slot;
+    const uint32_t tmem = tmem_address(&tmem_slot);
     const LutCodeOp lut{a.scale, sm_q};
 
-    const uint32_t S = cluster_size(), rank = cluster_rank();
     const int64_t N = a.N, K = a.K;
-    const int64_t o0 = (int64_t)(blockIdx.x / S) * kGemmRows;
-    const int64_t n0 = (int64_t)blockIdx.y * nt;
-    const int64_t rows = a.M - n0 < nt ? a.M - n0 : nt;                 // batch rows of this CTA (>= 1)
-    const int c_begin = (int)((int64_t)a.nchunks * rank / S), c_end = (int)((int64_t)a.nchunks * (rank + 1) / S);
+    const TcTile tile = tc_tile(a, nt);
+    const int64_t o0 = tile.o0, rows = tile.rows;
+    const int c_begin = tile.c_begin, c_end = tile.c_end;
 
     // weight units of this thread: rows wr[u] = tid / 8 + 32 u, 8-element group wj = tid % 8 of every chunk
     const int wj = tid & 7;
@@ -118,7 +110,7 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
         prm[u].s = LUT ? 0.0f : __ldg(a.scale + c);
         prm[u].zp = LUT ? 0 : __ldg(a.zp + c);
     }
-    const T* __restrict__ xg = reinterpret_cast<const T*>(a.x) + n0 * K;
+    const T* __restrict__ xg = reinterpret_cast<const T*>(a.x) + tile.n0 * K;
     const int xunits = nt * 8;
 
     using WRaw = uint32_t[WU][RAW];
@@ -207,9 +199,9 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
         }
     };
 
-    // instruction descriptor: f32 accumulator, A / B bf16 (1) or f16 (0), both K-major, N = nt, M = 128
+    // f32 accumulator, A and B bf16 (1) or f16 (0)
     constexpr uint32_t ab = std::is_same<OT, __half>::value ? 0u : 1u;
-    const uint32_t idesc = (1u << 4) | (ab << 7) | (ab << 10) | ((uint32_t)(nt >> 3) << 17) | ((uint32_t)(kGemmRows >> 4) << 24);
+    const uint32_t idesc = tc_idesc(1u, ab, ab, nt);
 
     // chunk c: wait for its stage, decode it from registers into the stage, issue its MMAs
     auto run_chunk = [&](int c, const WRaw& wraw, const XRaw& xraw) {
@@ -227,17 +219,11 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
 #pragma unroll
                 for (int t = 0; t < TERMS; ++t) {
                     const uint64_t bd = sw128_desc(st + a_bytes + t * b_bytes + 32 * ks);
-                    const uint32_t acc = (i > 0 || ks > 0 || t > 0) ? 1u : 0u;
-                    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                                 "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                                 :: "r"(tmem), "l"(ad), "l"(bd), "r"(idesc), "r"(acc) : "memory");
+                    tc_mma<false>(tmem, ad, bd, idesc, (i > 0 || ks > 0 || t > 0) ? 1u : 0u);
                 }
             }
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
-                         :: "r"(smem_u32(&bar_empty[s])) : "memory");
-            if (c + 1 == c_end)
-                asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
-                             :: "r"(smem_u32(&bar_done)) : "memory");
+            tc_commit(&bar_empty[s]);
+            if (c + 1 == c_end) tc_commit(&bar_done);
         }
     };
     // two register sets: the loads of chunk c + 1 are in flight while chunk c is decoded
@@ -252,55 +238,20 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
             run_chunk(c + 1, w1, x1);
         }
     }
-    const bool have = c_begin < c_end;
-    if (have) mbar_wait(&bar_done, 0);
+    if (c_begin < c_end) mbar_wait(&bar_done, 0);
     tc_fence_after();
 
-    // epilogue: warp w reads TMEM lanes 32 (w % 4) .. + 31 (one output feature per thread), column blocks of 16 batch rows
-    // alternate between warps w and w + 4.  Ranks >= 1 park their partial sums in their (now idle) stage memory as
-    // [batch row][feature]; rank 0 adds them in rank order after the cluster barrier.
-    const int r = 32 * (warp & 3) + lane;
-    const int64_t o = o0 + r;
-    const uint32_t part = sbase;
-    const uint32_t taddr = tmem + ((uint32_t)(32 * (warp & 3)) << 16);
-    auto tmem_block = [&](int cb, float* v) {
-        if (have) {
-            uint32_t u[16];
-            tmem_ld16(taddr + 16 * cb, u);
-#pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(u[j]);
-        } else {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] = 0.0f;
-        }
-    };
-    const int nblocks = nt / 16;
-    if (rank != 0) {
-        for (int cb = warp >> 2; cb < nblocks; cb += 2) {
-            float v[16];
-            tmem_block(cb, v);
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-                asm volatile("st.shared.f32 [%0], %1;" :: "r"(part + (uint32_t)(((cb * 16 + j) * kGemmRows + r) * 4)), "f"(v[j]) : "memory");
-        }
-    }
-    __syncwarp();
-    cluster_sync();
-    if (rank == 0) {
+    // epilogue (one output feature o per thread): the split-K sum in f32, added in rank order, then the factor and the bias
+    const TcEpilogue e = tc_epilogue(tile, nt, tmem, sbase, tid);
+    const int64_t o = o0 + e.r;
+    splitk_park<float>(e, tile);
+    if (tile.rank == 0) {
         const float f = FACTOR && o < N ? __ldg(a.scale + (a.per_channel ? o : 0)) : 1.0f;
         const float b = a.bias && o < N ? to_f32<T>(reinterpret_cast<const T*>(a.bias)[o]) : 0.0f;
-        T* y = reinterpret_cast<T*>(a.y) + n0 * N;
-        for (int cb = warp >> 2; cb < nblocks; cb += 2) {
+        T* y = reinterpret_cast<T*>(a.y) + tile.n0 * N;
+        for (int cb = e.cb0; cb < e.nblocks; cb += 2) {
             float v[16];
-            tmem_block(cb, v);
-            for (uint32_t p = 1; p < S; ++p) {
-                const uint32_t base = peer_addr(part + (uint32_t)((cb * 16 * kGemmRows + r) * 4), p);
-                float pv[16];
-#pragma unroll
-                for (int j = 0; j < 16; ++j) pv[j] = ld_peer(base + j * kGemmRows * 4);
-#pragma unroll
-                for (int j = 0; j < 16; ++j) v[j] = __fadd_rn(v[j], pv[j]);
-            }
+            splitk_sum(e, tile, cb, v);
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
                 const int64_t n = cb * 16 + j;
@@ -312,14 +263,8 @@ __global__ void __launch_bounds__(kThreads, 2) packed_gemm_kernel(const __grid_c
             }
         }
     }
-    __syncwarp();
-    cluster_sync();             // the peers' partial sums stay in place until rank 0 has read them
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(a.tmem_cols) : "memory");
-    }
+    splitk_release();
+    tmem_dealloc(warp, tmem, a.tmem_cols);
 }
 
 }  // namespace mctq
@@ -334,36 +279,25 @@ int launch_gemm(GemmArgs a, cudaStream_t st) {
     const int64_t M = a.M;
     const int max_nt = TERMS == 3 ? 128 : 256;
     const int64_t ntiles = (M + max_nt - 1) / max_nt;
-    const int64_t per = (M + ntiles - 1) / ntiles;
-    a.nt = (int32_t)((per + 15) / 16 * 16);
+    a.nt = tc_row_tile(M, max_nt);
     a.nchunks = (int32_t)((a.K + kChunk - 1) / kChunk);
     a.tmem_cols = tmem_columns(a.nt);
-    const int64_t tiles = (a.N + kGemmRows - 1) / kGemmRows;
-    const size_t stage = (size_t)kGemmRows * 128 + (size_t)TERMS * a.nt * 128;
-    size_t smem = kStages * stage + 1024;                                   // + alignment of the stages to 1024 bytes
-    smem = std::max(smem, tmem_smem_floor(a.tmem_cols));              // co-resident CTAs must fit the SM's TMEM
+    const int64_t tiles = (a.N + kTcRows - 1) / kTcRows;
+    const size_t smem = tc_ring_smem(kStages, (size_t)kTcRows * 128 + (size_t)TERMS * a.nt * 128, a.tmem_cols);
     auto kernel = packed_gemm_kernel<KIND, T>;
     int rc = ensure_smem(kernel, smem);                                     // per device: set on every launch
     if (rc) return rc;
     // split-K: about two CTAs per SM (measured faster than one wave of longer CTAs), at least one chunk per CTA
-    int dev = 0, sms = 0;
-    if ((rc = cuda_rc(cudaGetDevice(&dev))) || (rc = cuda_rc(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev))))
-        return rc;
+    int sms = 0;
+    if ((rc = sm_count(&sms))) return rc;
     int64_t S = (2 * (int64_t)sms + tiles * ntiles - 1) / (tiles * ntiles);
     S = S < 1 ? 1 : S > kMaxSplit ? kMaxSplit : S;
     if (S > a.nchunks) S = a.nchunks;
-    const int64_t rows_per_launch = (int64_t)65535 * a.nt;
-    for (int64_t m0 = 0; m0 < M; m0 += rows_per_launch) {
-        GemmArgs b = a;
-        b.M = M - m0 < rows_per_launch ? M - m0 : rows_per_launch;
+    return tc_launch_rows(kernel, a, M, a.nt, tiles, S, smem, st, [&](GemmArgs& b, int64_t m0, int64_t m) {
+        b.M = m;
         b.x = reinterpret_cast<const T*>(a.x) + m0 * a.K;
         b.y = reinterpret_cast<T*>(a.y) + m0 * a.N;
-        const dim3 grid((unsigned)(tiles * S), (unsigned)((b.M + a.nt - 1) / a.nt));
-        pdl_plan_launch(st, nullptr, 0, nullptr, 0);                        // ranges "unknown": late order for the successor
-        rc = launch_planned_cluster(kernel, grid, (unsigned)S, smem, st, b);
-        if (rc) return rc;
-    }
-    return 0;
+    });
 }
 
 }  // namespace

@@ -1,9 +1,10 @@
 // mctq_packed_igemm.cu -- integer linear mode: y = T(((acc - corrections) * f) + b) with acc = sum_k qx[n,k] * qw[o,k] an
 // exact int32 product of 8-bit activation codes and packed int8 / int4 weight codes on the tensor cores
-// (tcgen05.mma kind::i8, s32 accumulator in tensor memory).  Packed nn.Linear wrappers in integer mode
+// (tcgen05 MMA kind::i8, s32 accumulator in tensor memory).  Packed nn.Linear wrappers in integer mode
 // (pytorch/packed_weights.py) call it after mctq_quantize_rows_i8 has turned their input into codes.
 //
-// Shape (as in mctq_packed_gemm.cu): output features are the MMA's M (128 per CTA), batch rows its N (nt, a multiple of 16 up
+// The tensor-core frame (TMEM, MMA issue and commit, split-K tile and reduction, launches over row ranges) is that of
+// mctq_tcgen05.cuh, shared with mctq_packed_gemm.cu.  Shape: output features are the MMA's M (128 per CTA), batch rows its N (nt, a multiple of 16 up
 // to 256; more rows run as further CTAs along grid.y).  A CTA walks its share of the row length in chunks of 128 codes (one
 // 128-byte swizzle row) through a ring of `stages` shared-memory stages with a full and an empty mbarrier each:
 //   warps 0-3  producers: thread 0 arms the stage's full barrier and copies the x codes (and int8 weight codes) with 2-D TMA
@@ -32,7 +33,6 @@
 
 namespace mctq {
 
-constexpr int kIRows = 128;           // output features per CTA (the MMA's M)
 constexpr int kIChunk = 128;          // codes of the row length per stage
 constexpr int kIMinStages = 4, kIMaxStages = 8;
 constexpr int kIMaxSplit = 8;         // portable cluster size
@@ -120,15 +120,12 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int nt = a.nt, nst = a.stages;
-    const uint32_t a_bytes = kIRows * 128, stage_bytes = a.stage_bytes;
+    const uint32_t a_bytes = kTcRows * 128, stage_bytes = a.stage_bytes;
     const uint32_t sbase = (smem_u32(dsm) + 1023u) & ~1023u;             // swizzle atoms need 1024-byte alignment
 
     pdl_wait();                 // x codes may be the output of the previous launch; TMEM is taken only after the wait
     pdl_launch_dependents();
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(&tmem_slot)), "r"(a.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    tmem_alloc(warp, &tmem_slot, a.tmem_cols);
     if (tid == 0) {
         for (int s = 0; s < nst; ++s) {
             mbar_init(&bar_full[s], CONV ? (INT4 ? 0 : 1) + kIProducers : INT4 ? 1 + kIProducers : 1);
@@ -136,18 +133,12 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
         }
         mbar_init(&bar_done, 1);
     }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = tmem_slot;
+    const uint32_t tmem = tmem_address(&tmem_slot);
 
-    const uint32_t S = cluster_size(), rank = cluster_rank();
     const int64_t N = a.N, K = a.K;
-    const int64_t o0 = (int64_t)(blockIdx.x / S) * kIRows;
-    const int64_t n0 = (int64_t)blockIdx.y * nt;                         // first row of this CTA inside the launch
-    const int64_t rows = a.M - n0 < nt ? a.M - n0 : nt;
-    const int c_begin = (int)((int64_t)a.nchunks * rank / S), c_end = (int)((int64_t)a.nchunks * (rank + 1) / S);
-    const int nloc = c_end - c_begin;
+    const TcTile tile = tc_tile(a, nt);
+    const int64_t o0 = tile.o0, n0 = tile.n0, rows = tile.rows;           // n0: first row of this CTA inside the launch
+    const int c_begin = tile.c_begin, nloc = tile.c_end - tile.c_begin;
 
     if (warp < 4) {
         // ---- producers
@@ -220,19 +211,12 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
         } else if (INT4) {
             const int64_t o = o0 + tid;
             const uint8_t* wrow = a.codes + o * (K >> 1);
-            auto load = [&](int c, uint4* v) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {                            // 32 codes per 16 bytes; K % 32 == 0
-                    const int64_t k = (int64_t)c * kIChunk + 32 * j;
-                    v[j] = (o < N && k < K) ? ld_stream(reinterpret_cast<const uint4*>(wrow + (k >> 1))) : make_uint4(0, 0, 0, 0);
-                }
-            };
             uint4 cur[4], nxt[4];
-            if (nloc > 0) load(c_begin, cur);
+            if (nloc > 0) load_w4(wrow, o, N, K, c_begin, cur);
             for (int i = 0; i < nloc; ++i) {
                 const int c = c_begin + i, s = i % nst;
                 const uint32_t st = sbase + (uint32_t)s * stage_bytes;
-                if (i + 1 < nloc) load(c + 1, nxt);                     // in flight while this stage is filled
+                if (i + 1 < nloc) load_w4(wrow, o, N, K, c + 1, nxt);  // in flight while this stage is filled
                 if (i >= nst) mbar_wait(&bar_empty[s], (uint32_t)((i / nst - 1) & 1));
                 if (tid == 0) {
                     mbar_arrive_expect_tx(&bar_full[s], (uint32_t)nt * 128u);
@@ -264,49 +248,21 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
 #pragma unroll
             for (int ks = 0; ks < kIChunk / 32; ++ks) {
                 const uint64_t ad = sw128_desc(st + 32 * ks), bd = sw128_desc(st + a_bytes + 32 * ks);
-                const uint32_t acc = (i > 0 || ks > 0) ? 1u : 0u;
-                asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                             "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-                             :: "r"(tmem), "l"(ad), "l"(bd), "r"(a.idesc), "r"(acc) : "memory");
+                tc_mma<true>(tmem, ad, bd, a.idesc, (i > 0 || ks > 0) ? 1u : 0u);
             }
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
-                         :: "r"(smem_u32(&bar_empty[s])) : "memory");
+            tc_commit(&bar_empty[s]);
         }
-        if (nloc > 0)
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
-                         :: "r"(smem_u32(&bar_done)) : "memory");
+        if (nloc > 0) tc_commit(&bar_done);
     }
     __syncwarp();
-    const bool have = nloc > 0;
-    if (have) mbar_wait(&bar_done, 0);
+    if (nloc > 0) mbar_wait(&bar_done, 0);
     tc_fence_after();
 
-    // epilogue: warp w reads TMEM lanes 32 (w % 4) .. + 31 (one output feature per thread), column blocks of 16 batch rows
-    // alternate between warps w and w + 4.  Ranks >= 1 park their int32 partial sums in their (now idle) stage memory as
-    // [batch row][feature]; rank 0 adds them after the cluster barrier.
-    const int r = 32 * (warp & 3) + lane;
-    const int64_t o = o0 + r;
-    const uint32_t part = sbase;
-    const uint32_t taddr = tmem + ((uint32_t)(32 * (warp & 3)) << 16);
-    auto tmem_block = [&](int cb, int32_t* v) {
-        uint32_t u[16];
-        if (have) tmem_ld16(taddr + 16 * cb, u);
-#pragma unroll
-        for (int j = 0; j < 16; ++j) v[j] = have ? (int32_t)u[j] : 0;
-    };
-    const int nblocks = nt / 16;
-    if (rank != 0) {
-        for (int cb = warp >> 2; cb < nblocks; cb += 2) {
-            int32_t v[16];
-            tmem_block(cb, v);
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-                asm volatile("st.shared.s32 [%0], %1;" :: "r"(part + (uint32_t)(((cb * 16 + j) * kIRows + r) * 4)), "r"(v[j]) : "memory");
-        }
-    }
-    __syncwarp();
-    cluster_sync();
-    if (rank == 0) {
+    // epilogue (one output feature o per thread): the split-K sum in int32, then the corrections and the scaling
+    const TcEpilogue e = tc_epilogue(tile, nt, tmem, sbase, tid);
+    const int64_t o = o0 + e.r;
+    splitk_park<int32_t>(e, tile);
+    if (tile.rank == 0) {
         const bool live = o < N;
         const int64_t ch = a.per_channel ? o : 0;
         const float f = live ? __ldg(a.factor + ch) : 0.0f;
@@ -316,17 +272,9 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
         const float b = a.bias && live ? to_f32<T>(reinterpret_cast<const T*>(a.bias)[o]) : 0.0f;
         const int64_t g0 = a.m0 + n0;                                      // first global row of this CTA
         T* y = reinterpret_cast<T*>(a.y);
-        for (int cb = warp >> 2; cb < nblocks; cb += 2) {
+        for (int cb = e.cb0; cb < e.nblocks; cb += 2) {
             int32_t v[16];
-            tmem_block(cb, v);
-            for (uint32_t p = 1; p < S; ++p) {
-                const uint32_t base = peer_addr(part + (uint32_t)((cb * 16 * kIRows + r) * 4), p);
-                int32_t pv[16];
-#pragma unroll
-                for (int j = 0; j < 16; ++j) pv[j] = ld_peer_s32(base + j * kIRows * 4);
-#pragma unroll
-                for (int j = 0; j < 16; ++j) v[j] = (int32_t)((uint32_t)v[j] + (uint32_t)pv[j]);
-            }
+            splitk_sum(e, tile, cb, v);
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
                 const int64_t n = cb * 16 + j;
@@ -345,14 +293,8 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
             }
         }
     }
-    __syncwarp();
-    cluster_sync();             // the peers' partial sums stay in place until rank 0 has read them
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(a.tmem_cols) : "memory");
-    }
+    splitk_release();
+    tmem_dealloc(warp, tmem, a.tmem_cols);
 }
 
 template <bool INT4, bool WSIGNED, typename T>
@@ -401,33 +343,26 @@ int encode_codes(EncodeTiled fn, CUtensorMap* map, const void* base, int64_t K, 
 }
 
 template <bool INT4, bool WSIGNED, typename T, bool CONV>
-int launch_igemm(IgemmArgs& a, int64_t M, cudaStream_t st) {
+int launch_igemm(const IgemmArgs& a, int64_t M, cudaStream_t st) {
     auto kernel = CONV ? packed_iconv_kernel<INT4, WSIGNED, T> : packed_igemm_kernel<INT4, WSIGNED, T>;
-    size_t smem = (size_t)a.stages * a.stage_bytes + 1024;              // + alignment of the stages to 1024 bytes
-    smem = std::max(smem, tmem_smem_floor(a.tmem_cols));
+    const size_t smem = tc_ring_smem(a.stages, a.stage_bytes, a.tmem_cols);
     int rc = ensure_smem(kernel, smem);
     if (rc) return rc;
-    const int64_t tiles = (a.N + kIRows - 1) / kIRows;
+    const int64_t tiles = (a.N + kTcRows - 1) / kTcRows;
     const int64_t ntiles = (M + a.nt - 1) / a.nt;
     // split-K: as many CTAs as fit the GPU at once (one wave), at least one chunk per CTA.  The ring's shared memory decides
     // how many CTAs an SM holds: two for small row tiles, one from nt = 96 on (four stages of 28 KB and more)
-    int dev = 0, sms = 0, per_sm = 0;
-    if ((rc = cuda_rc(cudaGetDevice(&dev))) || (rc = cuda_rc(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev))) ||
-        (rc = cuda_rc(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, smem))))
+    int sms = 0, per_sm = 0;
+    if ((rc = sm_count(&sms)) || (rc = cuda_rc(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, smem))))
         return rc;
     int64_t S = (int64_t)std::max(per_sm, 1) * sms / (tiles * ntiles);
     S = S < 1 ? 1 : S > kIMaxSplit ? kIMaxSplit : S;
     if (S > a.nchunks) S = a.nchunks;
-    const int64_t rows_per_launch = (int64_t)65535 * a.nt;
-    for (int64_t m0 = 0; m0 < M; m0 += rows_per_launch) {
-        a.m0 = m0;
-        a.M = M - m0 < rows_per_launch ? M - m0 : rows_per_launch;
-        const dim3 grid((unsigned)(tiles * S), (unsigned)((a.M + a.nt - 1) / a.nt));
-        pdl_plan_launch(st, nullptr, 0, nullptr, 0);                    // ranges "unknown": late order for the successor
-        rc = launch_planned_cluster(kernel, grid, (unsigned)S, smem, st, a);
-        if (rc) return rc;
-    }
-    return 0;
+    // the TMA maps and x_rowsum index global rows: a launch gets its range as m0, M
+    return tc_launch_rows(kernel, a, M, a.nt, tiles, S, smem, st, [](IgemmArgs& b, int64_t m0, int64_t m) {
+        b.m0 = m0;
+        b.M = m;
+    });
 }
 
 // largest in_features whose int32 sum of code products cannot overflow, per (weight, x) signedness
@@ -451,17 +386,13 @@ int igemm_check(const MctqPackedDesc* w, int64_t K, const void* x_codes, int x_s
 void igemm_prepare(IgemmArgs& a, const MctqPackedDesc* w, int64_t N, int64_t K, int64_t M, int x_signed, int32_t x_zero_point,
                    const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor, const void* bias, void* y) {
     memset(&a, 0, sizeof(a));
-    const int64_t max_nt = 256;
-    const int64_t ntiles = (M + max_nt - 1) / max_nt;
-    const int64_t per = (M + ntiles - 1) / ntiles;
-    a.nt = (int32_t)((per + 15) / 16 * 16);
+    a.nt = tc_row_tile(M, 256);
     a.nchunks = (int32_t)((K + kIChunk - 1) / kIChunk);
-    a.stage_bytes = (uint32_t)(kIRows * 128 + a.nt * 128);
+    a.stage_bytes = (uint32_t)(kTcRows * 128 + a.nt * 128);
     // deep rings for the HBM-bound small-batch shapes, while two CTAs still fit an SM's shared memory where they can
     a.stages = std::min(kIMaxStages, std::max(kIMinStages, (int)((112 * 1024 - 1024) / a.stage_bytes)));
     a.tmem_cols = tmem_columns(a.nt);
-    a.idesc = (2u << 4) | ((w->is_signed ? 1u : 0u) << 7) | ((x_signed ? 1u : 0u) << 10) | ((uint32_t)(a.nt >> 3) << 17) |
-              ((uint32_t)(kIRows >> 4) << 24);                           // s32 accumulator, K-major A and B
+    a.idesc = tc_idesc(2u, w->is_signed ? 1u : 0u, x_signed ? 1u : 0u, a.nt);     // s32 accumulator, signed or unsigned codes
     a.codes = reinterpret_cast<const uint8_t*>(w->codes);
     a.w_zp = w->zp;
     a.x_rowsum = x_rowsum;
@@ -512,7 +443,7 @@ int mctq_packed_linear_i8(const MctqPackedDesc* w, int64_t out_features, int64_t
     EncodeTiled fn;
     int rc = encode_fn(&fn);
     if (!rc) rc = encode_codes(fn, &a.tm_x, x_codes, in_features, M, (uint32_t)a.nt);
-    if (!rc && !int4) rc = encode_codes(fn, &a.tm_w, w->codes, in_features, out_features, kIRows);
+    if (!rc && !int4) rc = encode_codes(fn, &a.tm_w, w->codes, in_features, out_features, kTcRows);
     if (rc) return rc;
     return igemm_run<false>(a, w, y_dtype, M, (cudaStream_t)stream);
 }
@@ -546,7 +477,7 @@ int mctq_packed_conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int6
     if (!int4) {
         EncodeTiled fn;
         int rc = encode_fn(&fn);
-        if (!rc) rc = encode_codes(fn, &a.tm_w, w->codes, K, Cout, kIRows);
+        if (!rc) rc = encode_codes(fn, &a.tm_w, w->codes, K, Cout, kTcRows);
         if (rc) return rc;
     }
     return igemm_run<true>(a, w, y_dtype, M, (cudaStream_t)stream);
