@@ -273,6 +273,35 @@ int mctq_packed_conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int6
                           int32_t x_zero_point, const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor,
                           const void* bias, int y_dtype, void* y, int y_nchw, void* stream);
 
+/* Integer linear and convolution modes for LUT weights.  A LUT weight rebuilds as W[o,k] = fl32(q[idx[o,k]] * thr[o]) with
+ * q_k = lut_k / 2^(bw-1) and integer centroids lut_k in [-128, 127]: an int8 code lut_k times sw[o] = fl32(thr[o]) * 2^-(bw-1)
+ * (exact in f32 for the weights the wrappers switch), an affine weight with zero point 0.  The formula of
+ * mctq_packed_linear_i8 / mctq_packed_conv2d_i8 then reads
+ *   qw[o,k] = lut[idx[o,k]]   int8;   zw = 0;   Sw[o] = sum_k qw[o,k];   f[o] = fl32(sx * sw[o])
+ *   acc = sum_k qx[n,k] * lut[idx[o,k]]                              int32, exact (tcgen05.mma kind::i8)
+ *   c   = acc - zx * Sw[o]                                           int64, exact
+ *   y   = T(fl(fl((float)c * f[o]) + bias[o]))                       T = f32 (LUT weights rebuild as f32)
+ * Every output bit is fixed by the formula; it does not depend on the tiling, the split of K or the conv's order of k.
+ * The arguments are those of mctq_packed_linear_i8 / mctq_packed_conv2d_i8, with:
+ *   w              HOST descriptor of an MCTQ_PACK_LUT_I4 / _U8 weight (indices, K = w->K table entries, f32, its
+ *                  quotients present but not read; w->scale is not read, f replaces it)
+ *   x_rowsum       unused (zw = 0)
+ *   lut_codes_host HOST array of w->K int8 centroid codes lut[0 .. K-1]; it travels by value in the kernel arguments, so a
+ *                  call (and a CUDA-graph capture of it) needs no device copy of the table and no synchronisation
+ * The index → code lookup happens in the GEMM's weight producers: 4-bit indices by byte permutations of the 16-byte table
+ * held in registers, 8-bit indices through a shared-memory table.  Returns, before any CUDA call: MCTQ_E_BADARG for an
+ * affine kind, a null table and the other argument errors of the affine entry points (in_features / K a multiple of 32 for
+ * 4-bit and of 16 for 8-bit indices); MCTQ_E_DTYPE; MCTQ_E_LUT for K outside 1..16 (4-bit) / 1..256 (8-bit);
+ * MCTQ_E_RANGE for a zx outside the x codes' range or a row length above mctq_packed_linear_i8_max_k(1, x_signed). */
+int mctq_packed_linear_i8_lut(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x_codes,
+                              int x_signed, int32_t x_zero_point, int64_t M, const int32_t* x_rowsum, const int32_t* w_rowsum,
+                              const float* factor, const void* bias, int y_dtype, void* y, int64_t ldy,
+                              const int8_t* lut_codes_host, void* stream);
+int mctq_packed_conv2d_i8_lut(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x_codes,
+                              int x_signed, int32_t x_zero_point, const int32_t* x_rowsum, const int32_t* w_rowsum,
+                              const float* factor, const void* bias, int y_dtype, void* y, int y_nchw,
+                              const int8_t* lut_codes_host, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Whole-model weight quantisation: one launch over a table of tensors (SURVEY 8f rank 1).
  * Replaces the per-layer loop  for name, w, quantizer in self._weights_vars: quantizer(w)

@@ -93,6 +93,10 @@ SIGNATURES = {
                                       c_vp]),
     "mctq_packed_conv2d_i8": (c_int, [c_vp, c_vp, c_i64, c_vp, c_int, c_i32, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_int,
                                       c_vp]),
+    "mctq_packed_linear_i8_lut": (c_int, [c_vp, c_i64, c_i64, c_vp, c_int, c_i32, c_i64, c_vp, c_vp, c_vp, c_vp, c_int,
+                                          c_vp, c_i64, c_vp, c_vp]),
+    "mctq_packed_conv2d_i8_lut": (c_int, [c_vp, c_vp, c_i64, c_vp, c_int, c_i32, c_vp, c_vp, c_vp, c_vp, c_int, c_vp,
+                                          c_int, c_vp, c_vp]),
     "mctq_multi_tile_elems": (c_i64, []),
     "mctq_multi_plan": (c_i64, [c_vp, c_int, c_vp]),
     "mctq_fq_affine_multi": (c_int, [c_vp, c_vp, c_int, c_i64, c_vp]),

@@ -63,7 +63,15 @@ struct IgemmArgs {
     FastDiv div_howo, div_wo, div_cin, div_kw;
     int32_t y_nchw;                   // y as NCHW planes instead of [M][Cout]
     uint32_t zx_splat;                // the byte of zx, four times
+    // LUT weights only: the int8 codes of the centroids, lut[i] in byte i % 4 of word i / 4 (by value: no device pointer)
+    uint32_t lut[64];
 };
+
+// how the weight operand reaches a stage: int8 affine codes by TMA, int4 affine codes or LUT indices through the producers
+enum class WFmt { I8, I4, LUT4, LUT8 };
+__host__ __device__ constexpr bool producer_written(WFmt f) { return f != WFmt::I8; }
+__host__ __device__ constexpr bool is_lut(WFmt f) { return f == WFmt::LUT4 || f == WFmt::LUT8; }
+constexpr uint32_t kLut8TableBytes = 256 * 32;   // the table of 8-bit indices, one copy per lane
 
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" :: "r"(dst), "l"(src) : "memory");
@@ -89,6 +97,15 @@ __device__ __forceinline__ void expand8(uint32_t w, uint32_t& lo, uint32_t& hi) 
     }
 }
 
+// 8 nibbles (element 2j in the low nibble of byte j) -> the 8 bytes lut[nibble] of a 16-entry table in t[0..3]: the low
+// three bits of a nibble select among entries 0-7 and 8-15 (two byte permutations), its bit 3 picks one of the two bytes
+__device__ __forceinline__ void lut8(uint32_t w, const uint32_t* t, uint32_t& lo, uint32_t& hi) {
+    const uint32_t s_lo = w & 0x7777u, s_hi = (w >> 16) & 0x7777u;
+    const uint32_t pick_lo = 0x3210u | ((w >> 1) & 0x4444u), pick_hi = 0x3210u | ((w >> 17) & 0x4444u);
+    lo = __byte_perm(__byte_perm(t[0], t[1], s_lo), __byte_perm(t[2], t[3], s_lo), pick_lo);
+    hi = __byte_perm(__byte_perm(t[0], t[1], s_hi), __byte_perm(t[2], t[3], s_hi), pick_hi);
+}
+
 // int4 weight codes of one row, chunk c (128 codes = 64 bytes), or zeros outside the weight
 __device__ __forceinline__ void load_w4(const uint8_t* wrow, int64_t o, int64_t N, int64_t K, int c, uint4* v) {
 #pragma unroll
@@ -97,22 +114,69 @@ __device__ __forceinline__ void load_w4(const uint8_t* wrow, int64_t o, int64_t 
         v[j] = (o < N && k < K) ? ld_stream(reinterpret_cast<const uint4*>(wrow + (k >> 1))) : make_uint4(0, 0, 0, 0);
     }
 }
-// row `row` of the weight operand of a stage: the 128 codes of v expanded to bytes
-template <bool WSIGNED>
-__device__ __forceinline__ void store_w4(uint32_t st, uint32_t row, const uint4* v) {
+// row `row` of the weight operand of a stage: the 128 codes of v expanded to bytes (LUT: the table codes t[] of the indices)
+template <bool WSIGNED, bool LUT = false>
+__device__ __forceinline__ void store_w4(uint32_t st, uint32_t row, const uint4* v, const uint32_t* t = nullptr) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
         const uint32_t words[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
         uint32_t g[8];
 #pragma unroll
-        for (int q = 0; q < 4; ++q) expand8<WSIGNED>(words[q], g[2 * q], g[2 * q + 1]);
+        for (int q = 0; q < 4; ++q) {
+            if constexpr (LUT) lut8(words[q], t, g[2 * q], g[2 * q + 1]);
+            else expand8<WSIGNED>(words[q], g[2 * q], g[2 * q + 1]);
+        }
         st_shared_v4(st + sw128_off(row, 2 * j), g);
         st_shared_v4(st + sw128_off(row, 2 * j + 1), g + 4);
     }
 }
 
-template <bool INT4, bool WSIGNED, typename T, bool CONV>
+// 8-bit LUT indices of one row, chunk c (128 indices), or zeros outside the weight
+__device__ __forceinline__ void load_w8(const uint8_t* wrow, int64_t o, int64_t N, int64_t K, int c, uint4* v) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {                                        // 16 indices per 16 bytes; K % 16 == 0
+        const int64_t k = (int64_t)c * kIChunk + 16 * j;
+        v[j] = (o < N && k < K) ? ld_stream(reinterpret_cast<const uint4*>(wrow + k)) : make_uint4(0, 0, 0, 0);
+    }
+}
+// row `row` of the weight operand of a stage: the table codes of the 128 indices of v.  `tab` is this lane's column of the
+// replicated table: entry e at byte (e / 4) * 128 + e % 4, so that the 32 lanes of a warp read 32 different banks
+__device__ __forceinline__ void store_w8(uint32_t st, uint32_t row, const uint4* v, const uint8_t* tab) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const uint32_t words[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
+        uint32_t g[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            uint32_t b[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                const uint32_t e = (words[q] >> (8 * i)) & 0xFFu;
+                b[i] = tab[((e & 0xFCu) << 5) | (e & 3u)];
+            }
+            g[q] = __byte_perm(__byte_perm(b[0], b[1], 0x0040u), __byte_perm(b[2], b[3], 0x0040u), 0x5410u);
+        }
+        st_shared_v4(st + sw128_off(row, (uint32_t)j), g);
+    }
+}
+
+// the weight operand's row `row` of chunk c, by format: load_w into registers (one chunk ahead), store_w into a stage.  t: the
+// 16-entry table in four registers (LUT4); tab: this lane's column of the shared-memory table (LUT8)
+template <WFmt F>
+__device__ __forceinline__ void load_w(const uint8_t* wrow, int64_t o, int64_t N, int64_t K, int c, uint4* v) {
+    if constexpr (F == WFmt::LUT8) load_w8(wrow, o, N, K, c, v);
+    else load_w4(wrow, o, N, K, c, v);
+}
+template <WFmt F, bool WSIGNED>
+__device__ __forceinline__ void store_w(uint32_t st, uint32_t row, const uint4* v, const uint32_t* t, const uint8_t* tab) {
+    if constexpr (F == WFmt::LUT8) store_w8(st, row, v, tab);
+    else if constexpr (F == WFmt::LUT4) store_w4<false, true>(st, row, v, t);
+    else store_w4<WSIGNED>(st, row, v);
+}
+
+template <WFmt F, bool WSIGNED, typename T, bool CONV>
 __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
+    constexpr bool INT4 = producer_written(F);     // the producers write the weight operand (int4 codes, LUT indices)
     extern __shared__ __align__(1024) uint8_t dsm[];
     __shared__ uint64_t bar_full[kIMaxStages], bar_empty[kIMaxStages];
     __shared__ uint64_t bar_done;
@@ -133,6 +197,10 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
         }
         mbar_init(&bar_done, 1);
     }
+    if constexpr (F == WFmt::LUT8) {                 // behind the ring: 32 copies of the table, word e / 4 of copy l at 32 e / 4 + l
+        uint32_t* tab = reinterpret_cast<uint32_t*>(dsm + (sbase - smem_u32(dsm)) + (uint32_t)nst * stage_bytes);
+        for (int i = tid; i < (int)(kLut8TableBytes / 4); i += kThreads) tab[i] = a.lut[i >> 5];
+    }
     const uint32_t tmem = tmem_address(&tmem_slot);
 
     const int64_t N = a.N, K = a.K;
@@ -140,14 +208,21 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
     const int64_t o0 = tile.o0, n0 = tile.n0, rows = tile.rows;           // n0: first row of this CTA inside the launch
     const int c_begin = tile.c_begin, nloc = tile.c_end - tile.c_begin;
 
+    constexpr int NV = F == WFmt::LUT8 ? 8 : 4;     // 16-byte words of weight codes per row and chunk
+    uint32_t t[4];
+    if constexpr (F == WFmt::LUT4) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) t[i] = a.lut[i];
+    }
+    const uint8_t* tab = dsm + (sbase - smem_u32(dsm)) + (uint32_t)nst * stage_bytes + 4 * lane;
     if (warp < 4) {
         // ---- producers
         if (CONV) {
             const MctqConv2dGeom& g = a.g;
             const int64_t o = o0 + tid;
-            const uint8_t* wrow = a.codes + o * (K >> 1);
-            uint4 cur[4], nxt[4];
-            if (INT4 && nloc > 0) load_w4(wrow, o, N, K, c_begin, cur);
+            const uint8_t* wrow = a.codes + o * (F == WFmt::LUT8 ? K : K >> 1);
+            uint4 cur[NV], nxt[NV];
+            if (INT4 && nloc > 0) load_w<F>(wrow, o, N, K, c_begin, cur);
             // the window origins of this thread's rows tid and tid + 128; `have_row`: the row is in the stage (r < nt),
             // `live`: it is an output pixel (r < rows)
             bool have_row[2], live[2];
@@ -169,13 +244,13 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
             for (int i = 0; i < nloc; ++i) {
                 const int c = c_begin + i, s = i % nst;
                 const uint32_t st = sbase + (uint32_t)s * stage_bytes;
-                if (INT4 && i + 1 < nloc) load_w4(wrow, o, N, K, c + 1, nxt);
+                if (INT4 && i + 1 < nloc) load_w<F>(wrow, o, N, K, c + 1, nxt);
                 if (i >= nst) mbar_wait(&bar_empty[s], (uint32_t)((i / nst - 1) & 1));
                 if (!INT4 && tid == 0) {
                     mbar_arrive_expect_tx(&bar_full[s], a_bytes);
                     tma_2d(&a.tm_w, st, c * kIChunk, (int32_t)o0, &bar_full[s]);
                 }
-                if (INT4) store_w4<WSIGNED>(st, (uint32_t)tid, cur);
+                if (INT4) store_w<F, WSIGNED>(st, (uint32_t)tid, cur, t, tab);
 #pragma unroll
                 for (int j = 0; j < kIChunk / 16; ++j) {
                     const int32_t k = c * kIChunk + 16 * j;
@@ -202,7 +277,7 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
                 }
                 if (INT4) {
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) cur[j] = nxt[j];
+                    for (int j = 0; j < NV; ++j) cur[j] = nxt[j];
                 }
             }
             asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -210,23 +285,23 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
             for (int i = nloc > kIConvAhead ? nloc - kIConvAhead : 0; i < nloc; ++i) mbar_arrive(&bar_full[i % nst]);
         } else if (INT4) {
             const int64_t o = o0 + tid;
-            const uint8_t* wrow = a.codes + o * (K >> 1);
-            uint4 cur[4], nxt[4];
-            if (nloc > 0) load_w4(wrow, o, N, K, c_begin, cur);
+            const uint8_t* wrow = a.codes + o * (F == WFmt::LUT8 ? K : K >> 1);
+            uint4 cur[NV], nxt[NV];
+            if (nloc > 0) load_w<F>(wrow, o, N, K, c_begin, cur);
             for (int i = 0; i < nloc; ++i) {
                 const int c = c_begin + i, s = i % nst;
                 const uint32_t st = sbase + (uint32_t)s * stage_bytes;
-                if (i + 1 < nloc) load_w4(wrow, o, N, K, c + 1, nxt);  // in flight while this stage is filled
+                if (i + 1 < nloc) load_w<F>(wrow, o, N, K, c + 1, nxt);  // in flight while this stage is filled
                 if (i >= nst) mbar_wait(&bar_empty[s], (uint32_t)((i / nst - 1) & 1));
                 if (tid == 0) {
                     mbar_arrive_expect_tx(&bar_full[s], (uint32_t)nt * 128u);
                     tma_2d(&a.tm_x, st + a_bytes, c * kIChunk, (int32_t)(a.m0 + n0), &bar_full[s]);
                 }
-                store_w4<WSIGNED>(st, (uint32_t)tid, cur);
+                store_w<F, WSIGNED>(st, (uint32_t)tid, cur, t, tab);
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");    // generic-proxy stores -> tensor-core reads
                 mbar_arrive(&bar_full[s]);
 #pragma unroll
-                for (int j = 0; j < 4; ++j) cur[j] = nxt[j];
+                for (int j = 0; j < NV; ++j) cur[j] = nxt[j];
             }
         } else if (tid == 0) {
             for (int i = 0; i < nloc; ++i) {
@@ -266,7 +341,7 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
         const bool live = o < N;
         const int64_t ch = a.per_channel ? o : 0;
         const float f = live ? __ldg(a.factor + ch) : 0.0f;
-        const int32_t zw = live ? __ldg(a.w_zp + ch) : 0;
+        const int32_t zw = !is_lut(F) && live ? __ldg(a.w_zp + ch) : 0;     // LUT codes: zw = 0
         const int64_t sw = live && a.w_rowsum ? (int64_t)__ldg(a.w_rowsum + o) : 0;
         const int64_t fixed = K * (int64_t)a.x_zp * zw - (int64_t)a.x_zp * sw;     // K zx zw - zx Sw[o]
         const float b = a.bias && live ? to_f32<T>(reinterpret_cast<const T*>(a.bias)[o]) : 0.0f;
@@ -297,14 +372,14 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
     tmem_dealloc(warp, tmem, a.tmem_cols);
 }
 
-template <bool INT4, bool WSIGNED, typename T>
+template <WFmt F, bool WSIGNED, typename T>
 __global__ void __launch_bounds__(kThreads, 1) packed_igemm_kernel(const __grid_constant__ IgemmArgs a) {
-    igemm_body<INT4, WSIGNED, T, false>(a);
+    igemm_body<F, WSIGNED, T, false>(a);
 }
 
-template <bool INT4, bool WSIGNED, typename T>
+template <WFmt F, bool WSIGNED, typename T>
 __global__ void __launch_bounds__(kThreads, 1) packed_iconv_kernel(const __grid_constant__ IgemmArgs a) {
-    igemm_body<INT4, WSIGNED, T, true>(a);
+    igemm_body<F, WSIGNED, T, true>(a);
 }
 
 }  // namespace mctq
@@ -342,10 +417,10 @@ int encode_codes(EncodeTiled fn, CUtensorMap* map, const void* base, int64_t K, 
     return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
 }
 
-template <bool INT4, bool WSIGNED, typename T, bool CONV>
+template <WFmt F, bool WSIGNED, typename T, bool CONV>
 int launch_igemm(const IgemmArgs& a, int64_t M, cudaStream_t st) {
-    auto kernel = CONV ? packed_iconv_kernel<INT4, WSIGNED, T> : packed_igemm_kernel<INT4, WSIGNED, T>;
-    const size_t smem = tc_ring_smem(a.stages, a.stage_bytes, a.tmem_cols);
+    auto kernel = CONV ? packed_iconv_kernel<F, WSIGNED, T> : packed_igemm_kernel<F, WSIGNED, T>;
+    const size_t smem = tc_ring_smem(a.stages, a.stage_bytes, a.tmem_cols) + (F == WFmt::LUT8 ? kLut8TableBytes : 0);
     int rc = ensure_smem(kernel, smem);
     if (rc) return rc;
     const int64_t tiles = (a.N + kTcRows - 1) / kTcRows;
@@ -372,13 +447,14 @@ int64_t igemm_max_k(bool w_signed, bool x_signed) {
     return 33025;                                       // 255 * 255 * K < 2^31
 }
 
-// the checks both entry points make after their shape checks: factors, Sw when zx != 0, aligned codes, zx and K in range
-int igemm_check(const MctqPackedDesc* w, int64_t K, const void* x_codes, int x_signed, int32_t x_zero_point,
+// the checks every entry point makes after its shape checks: factors, Sw when zx != 0, aligned codes, zx and K in range
+// (w_signed: the signedness of the weight codes the tensor cores multiply)
+int igemm_check(const MctqPackedDesc* w, bool w_signed, int64_t K, const void* x_codes, int x_signed, int32_t x_zero_point,
                 const int32_t* w_rowsum, const float* factor) {
     if (!factor || (x_zero_point != 0 && !w_rowsum)) return MCTQ_E_BADARG;
     if (!aligned16(x_codes) || !aligned16(w->codes)) return MCTQ_E_BADARG;
     if (x_signed ? (x_zero_point < -128 || x_zero_point > 127) : (x_zero_point < 0 || x_zero_point > 255)) return MCTQ_E_RANGE;
-    if (K > igemm_max_k(w->is_signed != 0, x_signed != 0)) return MCTQ_E_RANGE;
+    if (K > igemm_max_k(w_signed, x_signed != 0)) return MCTQ_E_RANGE;
     return 0;
 }
 
@@ -386,13 +462,17 @@ int igemm_check(const MctqPackedDesc* w, int64_t K, const void* x_codes, int x_s
 void igemm_prepare(IgemmArgs& a, const MctqPackedDesc* w, int64_t N, int64_t K, int64_t M, int x_signed, int32_t x_zero_point,
                    const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor, const void* bias, void* y) {
     memset(&a, 0, sizeof(a));
-    a.nt = tc_row_tile(M, 256);
+    // the table of 8-bit LUT indices (8 KB) and four stages of 256 rows exceed the 200 KB a launch may take: 240 rows fit
+    a.nt = tc_row_tile(M, w->kind == MCTQ_PACK_LUT_U8 ? 240 : 256);
     a.nchunks = (int32_t)((K + kIChunk - 1) / kIChunk);
     a.stage_bytes = (uint32_t)(kTcRows * 128 + a.nt * 128);
     // deep rings for the HBM-bound small-batch shapes, while two CTAs still fit an SM's shared memory where they can
-    a.stages = std::min(kIMaxStages, std::max(kIMinStages, (int)((112 * 1024 - 1024) / a.stage_bytes)));
+    // (the table of 8-bit LUT indices takes its share of that memory)
+    const int budget = 112 * 1024 - 1024 - (w->kind == MCTQ_PACK_LUT_U8 ? (int)kLut8TableBytes : 0);
+    a.stages = std::min(kIMaxStages, std::max(kIMinStages, budget / (int)a.stage_bytes));
     a.tmem_cols = tmem_columns(a.nt);
-    a.idesc = tc_idesc(2u, w->is_signed ? 1u : 0u, x_signed ? 1u : 0u, a.nt);     // s32 accumulator, signed or unsigned codes
+    // s32 accumulator, signed or unsigned codes (LUT codes are int8)
+    a.idesc = tc_idesc(2u, w->is_signed || pack_is_lut(w->kind) ? 1u : 0u, x_signed ? 1u : 0u, a.nt);
     a.codes = reinterpret_cast<const uint8_t*>(w->codes);
     a.w_zp = w->zp;
     a.x_rowsum = x_rowsum;
@@ -408,16 +488,89 @@ void igemm_prepare(IgemmArgs& a, const MctqPackedDesc* w, int64_t N, int64_t K, 
 
 template <bool CONV>
 int igemm_run(IgemmArgs& a, const MctqPackedDesc* w, int y_dtype, int64_t M, cudaStream_t st) {
-    auto typed = [&](auto int4_tag, auto signed_tag) {
-        constexpr bool I4 = decltype(int4_tag)::value, WS = decltype(signed_tag)::value;
-        if (y_dtype == MCTQ_F32) return launch_igemm<I4, WS, float, CONV>(a, M, st);
-        if (y_dtype == MCTQ_BF16) return launch_igemm<I4, WS, __nv_bfloat16, CONV>(a, M, st);
-        return launch_igemm<I4, WS, __half, CONV>(a, M, st);
+    // LUT weights rebuild as f32 (packed_linear_check): one instantiation per index width
+    if (w->kind == MCTQ_PACK_LUT_I4) return launch_igemm<WFmt::LUT4, true, float, CONV>(a, M, st);
+    if (w->kind == MCTQ_PACK_LUT_U8) return launch_igemm<WFmt::LUT8, true, float, CONV>(a, M, st);
+    auto typed = [&](auto fmt_tag, auto signed_tag) {
+        constexpr WFmt F = decltype(fmt_tag)::value;
+        constexpr bool WS = decltype(signed_tag)::value;
+        if (y_dtype == MCTQ_F32) return launch_igemm<F, WS, float, CONV>(a, M, st);
+        if (y_dtype == MCTQ_BF16) return launch_igemm<F, WS, __nv_bfloat16, CONV>(a, M, st);
+        return launch_igemm<F, WS, __half, CONV>(a, M, st);
     };
+    using I4 = std::integral_constant<WFmt, WFmt::I4>;
     using True = std::true_type;
     using False = std::false_type;
-    if (pack_is_int4(w->kind)) return w->is_signed ? typed(True{}, True{}) : typed(True{}, False{});
-    return typed(False{}, False{});         // int8 weights reach the tensor cores as stored: the signedness is in idesc
+    if (pack_is_int4(w->kind)) return w->is_signed ? typed(I4{}, True{}) : typed(I4{}, False{});
+    // int8 weights reach the tensor cores as stored: the signedness is in idesc
+    return typed(std::integral_constant<WFmt, WFmt::I8>{}, False{});
+}
+
+// the LUT table of `K` int8 codes, by value in the launch arguments (entries K.. are 0: no index reaches them)
+void igemm_set_lut(IgemmArgs& a, const int8_t* codes, int K) {
+    uint8_t b[256] = {};
+    memcpy(b, codes, (size_t)K);
+    memcpy(a.lut, b, sizeof(b));
+}
+
+// mctq_packed_linear_i8 (lut null: affine kinds) and mctq_packed_linear_i8_lut (lut: the table, LUT kinds)
+int linear_i8(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x_codes, int x_signed,
+              int32_t x_zero_point, int64_t M, const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor,
+              const void* bias, int y_dtype, void* y, int64_t ldy, const int8_t* lut, void* stream) {
+    if (const int rc = packed_linear_check(w, out_features, in_features, x_codes, y_dtype, M, y)) return rc;
+    const bool int4 = pack_is_int4(w->kind);
+    if (in_features % (int4 ? 32 : 16) != 0 || M >= (1LL << 31) || ldy < out_features) return MCTQ_E_BADARG;
+    if (const int rc = igemm_check(w, lut || w->is_signed, in_features, x_codes, x_signed, x_zero_point, w_rowsum, factor))
+        return rc;
+    if (M == 0) return 0;
+
+    IgemmArgs a;
+    igemm_prepare(a, w, out_features, in_features, M, x_signed, x_zero_point, lut ? nullptr : x_rowsum, w_rowsum, factor,
+                  bias, y);
+    if (lut) igemm_set_lut(a, lut, w->K);
+    a.ldy = ldy;
+    EncodeTiled fn;
+    int rc = encode_fn(&fn);
+    if (!rc) rc = encode_codes(fn, &a.tm_x, x_codes, in_features, M, (uint32_t)a.nt);
+    if (!rc && w->kind == MCTQ_PACK_AFFINE_I8) rc = encode_codes(fn, &a.tm_w, w->codes, in_features, out_features, kTcRows);
+    if (rc) return rc;
+    return igemm_run<false>(a, w, y_dtype, M, (cudaStream_t)stream);
+}
+
+// mctq_packed_conv2d_i8 and mctq_packed_conv2d_i8_lut, as linear_i8
+int conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x_codes, int x_signed,
+              int32_t x_zero_point, const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor, const void* bias,
+              int y_dtype, void* y, int y_nchw, const int8_t* lut, void* stream) {
+    if (!g) return MCTQ_E_BADARG;
+    if (g->N < 0 || g->H < 1 || g->W < 1 || g->Cin < 1 || g->Ho < 1 || g->Wo < 1 || g->kh < 1 || g->kw < 1 || g->sh < 1 ||
+        g->sw < 1 || g->dh < 1 || g->dw < 1 || g->pt < 0 || g->pb < 0 || g->pl < 0 || g->pr < 0 || (y_nchw != 0 && y_nchw != 1))
+        return MCTQ_E_BADARG;
+    const int64_t K = (int64_t)g->Cin * g->kh * g->kw, M = (int64_t)g->N * g->Ho * g->Wo;
+    if (const int rc = packed_linear_check(w, Cout, K, x_codes, y_dtype, M, y)) return rc;
+    const bool int4 = pack_is_int4(w->kind);
+    if (g->Cin % 16 != 0 || (int4 && K % 32 != 0) || M >= (1LL << 31)) return MCTQ_E_BADARG;
+    if (const int rc = igemm_check(w, lut || w->is_signed, K, x_codes, x_signed, x_zero_point, w_rowsum, factor)) return rc;
+    if (M == 0) return 0;
+
+    IgemmArgs a;
+    igemm_prepare(a, w, Cout, K, M, x_signed, x_zero_point, lut ? nullptr : x_rowsum, w_rowsum, factor, bias, y);
+    if (lut) igemm_set_lut(a, lut, w->K);
+    a.ldy = Cout;
+    a.x_nhwc = reinterpret_cast<const uint8_t*>(x_codes);
+    a.g = *g;
+    a.div_howo = make_fastdiv((uint32_t)(g->Ho * g->Wo));
+    a.div_wo = make_fastdiv((uint32_t)g->Wo);
+    a.div_cin = make_fastdiv((uint32_t)g->Cin);
+    a.div_kw = make_fastdiv((uint32_t)g->kw);
+    a.y_nchw = y_nchw;
+    a.zx_splat = ((uint32_t)x_zero_point & 0xFFu) * 0x01010101u;
+    if (w->kind == MCTQ_PACK_AFFINE_I8) {
+        EncodeTiled fn;
+        int rc = encode_fn(&fn);
+        if (!rc) rc = encode_codes(fn, &a.tm_w, w->codes, K, Cout, kTcRows);
+        if (rc) return rc;
+    }
+    return igemm_run<true>(a, w, y_dtype, M, (cudaStream_t)stream);
 }
 
 }  // namespace
@@ -431,56 +584,37 @@ int mctq_packed_linear_i8(const MctqPackedDesc* w, int64_t out_features, int64_t
                           const float* factor, const void* bias, int y_dtype, void* y, int64_t ldy, void* stream) {
     MCTQ_NVTX("mctq_packed_linear_i8");
     if (!w || pack_is_lut(w->kind)) return MCTQ_E_BADARG;
-    if (const int rc = packed_linear_check(w, out_features, in_features, x_codes, y_dtype, M, y)) return rc;
-    const bool int4 = pack_is_int4(w->kind);
-    if (in_features % (int4 ? 32 : 16) != 0 || M >= (1LL << 31) || ldy < out_features) return MCTQ_E_BADARG;
-    if (const int rc = igemm_check(w, in_features, x_codes, x_signed, x_zero_point, w_rowsum, factor)) return rc;
-    if (M == 0) return 0;
+    return linear_i8(w, out_features, in_features, x_codes, x_signed, x_zero_point, M, x_rowsum, w_rowsum, factor, bias,
+                     y_dtype, y, ldy, nullptr, stream);
+}
 
-    IgemmArgs a;
-    igemm_prepare(a, w, out_features, in_features, M, x_signed, x_zero_point, x_rowsum, w_rowsum, factor, bias, y);
-    a.ldy = ldy;
-    EncodeTiled fn;
-    int rc = encode_fn(&fn);
-    if (!rc) rc = encode_codes(fn, &a.tm_x, x_codes, in_features, M, (uint32_t)a.nt);
-    if (!rc && !int4) rc = encode_codes(fn, &a.tm_w, w->codes, in_features, out_features, kTcRows);
-    if (rc) return rc;
-    return igemm_run<false>(a, w, y_dtype, M, (cudaStream_t)stream);
+int mctq_packed_linear_i8_lut(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, const void* x_codes,
+                              int x_signed, int32_t x_zero_point, int64_t M, const int32_t* x_rowsum, const int32_t* w_rowsum,
+                              const float* factor, const void* bias, int y_dtype, void* y, int64_t ldy,
+                              const int8_t* lut_codes_host, void* stream) {
+    MCTQ_NVTX("mctq_packed_linear_i8_lut");
+    if (!w || !pack_is_lut(w->kind) || !lut_codes_host) return MCTQ_E_BADARG;
+    return linear_i8(w, out_features, in_features, x_codes, x_signed, x_zero_point, M, x_rowsum, w_rowsum, factor, bias,
+                     y_dtype, y, ldy, lut_codes_host, stream);
 }
 
 int mctq_packed_conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x_codes, int x_signed,
                           int32_t x_zero_point, const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor,
                           const void* bias, int y_dtype, void* y, int y_nchw, void* stream) {
     MCTQ_NVTX("mctq_packed_conv2d_i8");
-    if (!w || !g || pack_is_lut(w->kind)) return MCTQ_E_BADARG;
-    if (g->N < 0 || g->H < 1 || g->W < 1 || g->Cin < 1 || g->Ho < 1 || g->Wo < 1 || g->kh < 1 || g->kw < 1 || g->sh < 1 ||
-        g->sw < 1 || g->dh < 1 || g->dw < 1 || g->pt < 0 || g->pb < 0 || g->pl < 0 || g->pr < 0 || (y_nchw != 0 && y_nchw != 1))
-        return MCTQ_E_BADARG;
-    const int64_t K = (int64_t)g->Cin * g->kh * g->kw, M = (int64_t)g->N * g->Ho * g->Wo;
-    if (const int rc = packed_linear_check(w, Cout, K, x_codes, y_dtype, M, y)) return rc;
-    const bool int4 = pack_is_int4(w->kind);
-    if (g->Cin % 16 != 0 || (int4 && K % 32 != 0) || M >= (1LL << 31)) return MCTQ_E_BADARG;
-    if (const int rc = igemm_check(w, K, x_codes, x_signed, x_zero_point, w_rowsum, factor)) return rc;
-    if (M == 0) return 0;
+    if (!w || pack_is_lut(w->kind)) return MCTQ_E_BADARG;
+    return conv2d_i8(w, g, Cout, x_codes, x_signed, x_zero_point, x_rowsum, w_rowsum, factor, bias, y_dtype, y, y_nchw,
+                     nullptr, stream);
+}
 
-    IgemmArgs a;
-    igemm_prepare(a, w, Cout, K, M, x_signed, x_zero_point, x_rowsum, w_rowsum, factor, bias, y);
-    a.ldy = Cout;
-    a.x_nhwc = reinterpret_cast<const uint8_t*>(x_codes);
-    a.g = *g;
-    a.div_howo = make_fastdiv((uint32_t)(g->Ho * g->Wo));
-    a.div_wo = make_fastdiv((uint32_t)g->Wo);
-    a.div_cin = make_fastdiv((uint32_t)g->Cin);
-    a.div_kw = make_fastdiv((uint32_t)g->kw);
-    a.y_nchw = y_nchw;
-    a.zx_splat = ((uint32_t)x_zero_point & 0xFFu) * 0x01010101u;
-    if (!int4) {
-        EncodeTiled fn;
-        int rc = encode_fn(&fn);
-        if (!rc) rc = encode_codes(fn, &a.tm_w, w->codes, K, Cout, kTcRows);
-        if (rc) return rc;
-    }
-    return igemm_run<true>(a, w, y_dtype, M, (cudaStream_t)stream);
+int mctq_packed_conv2d_i8_lut(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x_codes,
+                              int x_signed, int32_t x_zero_point, const int32_t* x_rowsum, const int32_t* w_rowsum,
+                              const float* factor, const void* bias, int y_dtype, void* y, int y_nchw,
+                              const int8_t* lut_codes_host, void* stream) {
+    MCTQ_NVTX("mctq_packed_conv2d_i8_lut");
+    if (!w || !pack_is_lut(w->kind) || !lut_codes_host) return MCTQ_E_BADARG;
+    return conv2d_i8(w, g, Cout, x_codes, x_signed, x_zero_point, x_rowsum, w_rowsum, factor, bias, y_dtype, y, y_nchw,
+                     lut_codes_host, stream);
 }
 
 }  // extern "C"

@@ -14,6 +14,7 @@ sm_100a kernels.
     torch.ops.mctq.packed_linear_i8   <- the integer product of those codes and packed int8 / int4 weight codes
     torch.ops.mctq.quantize_nhwc_i8   -> NHWC 8-bit codes of an NCHW x and their per-pixel channel sums
     torch.ops.mctq.packed_conv2d_i8   <- the integer convolution of NHWC codes and packed weight codes (implicit GEMM)
+    torch.ops.mctq.packed_linear_i8_lut / packed_conv2d_i8_lut   the same with LUT weights: indices looked up as int8 codes
 
 (reference call sites: see include/mctq.h).  Each op has a CUDA implementation (device pointers + the
 caller's current stream into the C ABI, no synchronisation), a CPU-tensor implementation that streams the
@@ -59,6 +60,11 @@ _LIB.define("quantize_nhwc_i8(Tensor x, float scale, int zero_point, int quant_m
 _LIB.define("packed_conv2d_i8(Tensor x_codes, int x_zero_point, Tensor? x_rowsum, Tensor codes, int kind, bool is_signed, "
             "int out_channels, int[] kernel_size, int[] stride, int[] dilation, int[] padding, Tensor zero_point, "
             "Tensor w_rowsum, Tensor factor, Tensor? bias, ScalarType dtype, bool channels_last) -> Tensor")
+_LIB.define("packed_linear_i8_lut(Tensor x_codes, int x_zero_point, Tensor codes, int kind, int out_features, "
+            "int[] lut_values, Tensor w_rowsum, Tensor factor, Tensor? bias) -> Tensor")
+_LIB.define("packed_conv2d_i8_lut(Tensor x_codes, int x_zero_point, Tensor codes, int kind, int out_channels, "
+            "int[] kernel_size, int[] stride, int[] dilation, int[] padding, int[] lut_values, Tensor w_rowsum, "
+            "Tensor factor, Tensor? bias, bool channels_last) -> Tensor")
 
 
 # --------------------------------------------------------------------------------------------- helpers
@@ -859,10 +865,10 @@ def _quantize_rows_i8_cuda(x, scale, zero_point, quant_min, quant_max, want_rows
 
 
 def weight_code_values(codes, kind, is_signed, out_features, in_features):
-    """The integer codes of a packed affine weight as an int32 [out_features, in_features] tensor (one-time set-up of
-    IntegerLinear: the code row sums)."""
+    """The integer codes of a packed affine weight (or the indices of a LUT weight: unsigned, 4-bit ones two per byte like
+    int4 codes) as an int32 [out_features, in_features] tensor (one-time set-up of IntegerLinear: the code row sums)."""
     c = codes.reshape(-1).view(torch.uint8).to(torch.int32)
-    if kind == _native.PACK_AFFINE_I4:
+    if kind in (_native.PACK_AFFINE_I4, _native.PACK_LUT_I4):
         c = torch.stack((c & 15, c >> 4), dim=-1).reshape(-1)[:out_features * in_features]
         return (c - 16 * (c >= 8).to(torch.int32) if is_signed else c).reshape(out_features, in_features)
     return (c - 256 * (c >= 128).to(torch.int32) if is_signed else c).reshape(out_features, in_features)
@@ -876,12 +882,15 @@ class IntegerLinear:
         dtype                    the rebuilt weight's dtype: x, bias and y have it
         scale, zero_point        f32 / int32, 1 (per tensor) or out_features entries
         x_scale, x_zero_point, x_qmin, x_qmax   the input quantizer Q (per tensor, at most 256 levels)
+        lut_values               LUT weights (kind PACK_LUT_I4 / PACK_LUT_U8, indices): their int8 centroid codes, a host
+                                 tensor or list (mctq_packed_linear_i8_lut); scale is then sw = thr * 2^-(bw-1), zero_point
+                                 None (zw = 0), and the codes qw are the table entries of the indices
     `__call__(x, bias)` returns the integer product of Q's codes of x and the weight codes, scaled (include/mctq.h gives the
     formula), for a CUDA x of `dtype` on the codes' device, enqueued on the current stream.  `quantize` and `gemm` are its two
     launches."""
 
     def __init__(self, codes, kind, is_signed, dtype, out_features, in_features, scale, zero_point, x_scale, x_zero_point,
-                 x_qmin, x_qmax):
+                 x_qmin, x_qmax, lut_values=None):
         _check_range(x_qmin, x_qmax)
         if not ((-128 <= x_qmin and x_qmax <= 127) or (0 <= x_qmin and x_qmax <= 255)):
             raise ValueError(f"IntegerLinear: the input range [{x_qmin}, {x_qmax}] does not fit 8-bit codes")
@@ -892,45 +901,58 @@ class IntegerLinear:
         self.x_qmin, self.x_qmax = int(x_qmin), int(x_qmax)
         s = _param_on(scale.detach().reshape(-1).contiguous().to(torch.float32), self.device)
         factor = torch.tensor(self.x_scale, dtype=torch.float32, device=self.device) * s
-        self._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, None, "IntegerLinear")
+        self._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, None, "IntegerLinear",
+                   lut_values)
 
     @classmethod
-    def from_parts(cls, codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, x_zero_point):
-        """The launch state from a caller-supplied f and Sw (mctq::packed_linear_i8), with the constructor's checks of the
-        weight; only `gemm` is available (the input quantizer's scale and range are not known)."""
+    def from_parts(cls, codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, x_zero_point,
+                   lut_values=None):
+        """The launch state from a caller-supplied f and Sw (mctq::packed_linear_i8 / _lut), with the constructor's checks of
+        the weight; only `gemm` is available (the input quantizer's scale and range are not known)."""
         lin = cls.__new__(cls)
         lin.device = codes.device
         lin.x_zp, lin.x_scale, lin.x_qmin, lin.x_qmax = int(x_zero_point), None, None, None
-        lin._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, "packed_linear_i8")
+        lin._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum,
+                  "packed_linear_i8" if lut_values is None else "packed_linear_i8_lut", lut_values)
         return lin
 
-    def _bind(self, codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, what):
-        """Validate the weight, its factors, zero points and code row sums (computed from the codes when None) and build the
-        descriptor."""
+    def _bind(self, codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, what,
+              lut_values=None):
+        """Validate the weight, its factors, zero points (LUT weights: the table) and code row sums (computed from the codes
+        when None) and build the descriptor."""
         if self.device.type != "cuda":
             raise ValueError(f"{what} needs CUDA tensors")
-        if kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
+        lut = lut_code_table(kind, lut_values, what) if lut_values is not None else None
+        if lut is None and kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
             raise ValueError(f"{what}: kind {kind} is not an affine int8 / int4 packed weight")
         if dtype not in _DT:
             raise ValueError(f"{what}: output dtype {dtype} is not float32 / bfloat16 / float16")
-        if zero_point is None:
+        if zero_point is None and lut is None:
             raise ValueError(f"{what}: affine weights need their zero points")
         self.out_features, self.in_features, self.dtype = int(out_features), int(in_features), dtype
         N, K = self.out_features, self.in_features
         f = _param_on(factor.detach().reshape(-1).contiguous(), self.device)
-        if f.numel() not in (1, N) or zero_point.numel() != f.numel():
-            raise ValueError(f"{what}: {f.numel()} factors and {zero_point.numel()} zero points for {N} output channels "
+        nz = f.numel() if lut is not None else zero_point.numel()
+        if f.numel() not in (1, N) or nz != f.numel():
+            raise ValueError(f"{what}: {f.numel()} factors and {nz} zero points for {N} output channels "
                              f"(both per tensor or both per output channel)")
         C, inner = (f.numel(), K) if f.numel() > 1 else (1, 1)
-        self._desc, self._keep = _packed_desc(codes, kind, is_signed, dtype, N * K, C, inner, f, zero_point, None,
+        # a LUT weight's descriptor carries the table size K and a table pointer, here the codes as f32 (never read)
+        self._desc, self._keep = _packed_desc(codes, kind, is_signed, dtype, N * K, C, inner, f,
+                                              None if lut is not None else zero_point,
+                                              torch.from_numpy(lut.astype(np.float32)) if lut is not None else None,
                                               self.device, what)
         self.factor, z = self._keep[1], self._keep[2]
+        self.lut = lut
         if w_rowsum is None:
-            w_rowsum = weight_code_values(self._keep[0], kind, is_signed, N, K).sum(1, dtype=torch.int32)
+            qw = weight_code_values(self._keep[0], kind, is_signed, N, K)
+            if lut is not None:
+                qw = torch.from_numpy(lut.astype(np.int32)).to(self.device)[qw]
+            w_rowsum = qw.sum(1, dtype=torch.int32)
         self.w_rowsum = _param_on(w_rowsum.detach().reshape(-1).contiguous(), self.device)
         if self.w_rowsum.dtype != torch.int32 or self.w_rowsum.numel() != N:
             raise ValueError(f"{what}: w_rowsum must be int32 [{N}]")
-        self.needs_x_rowsum = bool((z != 0).any())
+        self.needs_x_rowsum = lut is None and bool((z != 0).any())
         self._desc_ptr = ctypes.addressof(self._desc)
 
     def __call__(self, x, bias=None):
@@ -975,13 +997,32 @@ class IntegerLinear:
             if rs is not None and (rs.dtype != torch.int32 or rs.numel() != M or rs.device != self.device):
                 raise RuntimeError(f"packed_linear_i8: x_rowsum must be int32 [{M}] on {self.device}")
             b = bias.contiguous() if bias is not None else None
-            with _on_device(self.device):
-                rc = _native.load().mctq_packed_linear_i8(
-                    self._desc_ptr, self.out_features, self.in_features, qx.data_ptr(), int(qx.dtype == torch.int8),
+            args = (self._desc_ptr, self.out_features, self.in_features, qx.data_ptr(), int(qx.dtype == torch.int8),
                     self.x_zp, M, _ptr(rs), self.w_rowsum.data_ptr(), self.factor.data_ptr(), _ptr(b), _DT[self.dtype],
-                    y.data_ptr(), ldy, _stream(self.device))
-            _native.check(rc, "mctq_packed_linear_i8")
+                    y.data_ptr(), ldy)
+            lib = _native.load()
+            with _on_device(self.device):
+                if self.lut is not None:
+                    rc = lib.mctq_packed_linear_i8_lut(*args, self.lut.ctypes.data, _stream(self.device))
+                else:
+                    rc = lib.mctq_packed_linear_i8(*args, _stream(self.device))
+            _native.check(rc, "mctq_packed_linear_i8_lut" if self.lut is not None else "mctq_packed_linear_i8")
         return y
+
+
+def lut_code_table(kind, lut_values, what):
+    """The int8 centroid codes of a LUT weight as a host numpy int8 array (the table mctq_packed_linear_i8_lut /
+    mctq_packed_conv2d_i8_lut take by value): 1..16 entries for 4-bit indices, 1..256 for 8-bit ones, integers in
+    [-128, 127]."""
+    if kind not in _native.PACK_LUT_KINDS:
+        raise ValueError(f"{what}: kind {kind} is not a LUT packed weight, but LUT values were given")
+    v = np.asarray(lut_values.detach().cpu().numpy() if isinstance(lut_values, torch.Tensor) else lut_values,
+                   dtype=np.float64).reshape(-1)
+    if not 1 <= v.size <= (16 if kind == _native.PACK_LUT_I4 else 256):
+        raise ValueError(f"{what}: {v.size} LUT values for kind {kind}")
+    if not (np.all(v == np.round(v)) and np.all(v >= -128) and np.all(v <= 127)):
+        raise ValueError(f"{what}: the LUT values are not integers in [-128, 127]")
+    return np.ascontiguousarray(v.astype(np.int8))
 
 
 def _packed_linear_i8_cuda(x_codes, x_zero_point, x_rowsum, codes, kind, is_signed, out_features, zero_point, w_rowsum,
@@ -994,6 +1035,17 @@ def _packed_linear_i8_cuda(x_codes, x_zero_point, x_rowsum, codes, kind, is_sign
     lin = IntegerLinear.from_parts(codes, kind, is_signed, dtype, out_features, x_codes.shape[-1], factor, zero_point,
                                    w_rowsum, x_zero_point)
     return lin.gemm(x_codes, x_rowsum, bias)
+
+
+def _packed_linear_i8_lut_cuda(x_codes, x_zero_point, codes, kind, out_features, lut_values, w_rowsum, factor, bias):
+    """mctq::packed_linear_i8_lut: packed_linear_i8 for LUT indices `codes` with the int8 centroid codes `lut_values` (f32
+    output, zw = 0: no x row sums)."""
+    if x_codes.dim() == 0:
+        raise RuntimeError("packed_linear_i8_lut: x codes must have at least one dimension")
+    _native.load()
+    lin = IntegerLinear.from_parts(codes, kind, False, torch.float32, out_features, x_codes.shape[-1], factor, None,
+                                   w_rowsum, x_zero_point, lut_values)
+    return lin.gemm(x_codes, None, bias)
 
 
 def quantize_nhwc_i8(x, scale_f32, zero_point, quant_min, quant_max, want_sums):
@@ -1044,7 +1096,7 @@ def pack_weight_codes(qw, kind, is_signed):
     """Packed codes (int8 / uint8 bytes, or int4 nibbles two per byte, element 2j in the low nibble) of the integer codes
     qw, in qw's element order: the inverse of weight_code_values."""
     q = qw.reshape(-1)
-    if kind == _native.PACK_AFFINE_I4:
+    if kind in (_native.PACK_AFFINE_I4, _native.PACK_LUT_I4):
         u = (q & 15).to(torch.uint8)
         if u.numel() % 2:
             u = torch.cat((u, u.new_zeros(1)))
@@ -1054,8 +1106,8 @@ def pack_weight_codes(qw, kind, is_signed):
 
 
 def conv_codes_rsc(codes, kind, is_signed, out_channels, in_channels, kh, kw):
-    """The packed codes of a contiguous [Cout, Cin, kh, kw] weight ((c, r, s) order per output channel) reordered to the
-    (r, s, c) order of mctq_packed_conv2d_i8 (one-time set-up of IntegerConv2d)."""
+    """The packed codes (or LUT indices) of a contiguous [Cout, Cin, kh, kw] weight ((c, r, s) order per output channel)
+    reordered to the (r, s, c) order of mctq_packed_conv2d_i8 (one-time set-up of IntegerConv2d)."""
     qw = weight_code_values(codes, kind, is_signed, out_channels, in_channels * kh * kw)
     qw = qw.reshape(out_channels, in_channels, kh, kw).permute(0, 2, 3, 1)
     out = pack_weight_codes(qw.contiguous(), kind, is_signed)
@@ -1091,12 +1143,14 @@ class IntegerConv2d:
         kernel_size, stride, dilation   pairs;  padding = (pt, pb, pl, pr)
         scale, zero_point        f32 / int32, 1 (per tensor) or Cout entries
         x_scale, x_zero_point, x_qmin, x_qmax   the input quantizer Q (per tensor, at most 256 levels)
+        lut_values               LUT weights (PACK_LUT_I4 / PACK_LUT_U8 indices): their int8 centroid codes, as for
+                                 IntegerLinear (mctq_packed_conv2d_i8_lut)
     `__call__(x, bias)` returns the integer convolution of Q's codes of a 4-D CUDA x of `dtype` on the codes' device with the
     weight codes, scaled (include/mctq.h gives the formula), in the memory format F.conv2d gives for x and the rebuilt
     weight.  `quantize` and `gemm` are its launches."""
 
     def __init__(self, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, weight_stride, stride,
-                 dilation, padding, scale, zero_point, x_scale, x_zero_point, x_qmin, x_qmax):
+                 dilation, padding, scale, zero_point, x_scale, x_zero_point, x_qmin, x_qmax, lut_values=None):
         _check_range(x_qmin, x_qmax)
         if not ((-128 <= x_qmin and x_qmax <= 127) or (0 <= x_qmin and x_qmax <= 255)):
             raise ValueError(f"IntegerConv2d: the input range [{x_qmin}, {x_qmax}] does not fit 8-bit codes")
@@ -1115,11 +1169,11 @@ class IntegerConv2d:
         s = _param_on(scale.detach().reshape(-1).contiguous().to(torch.float32), self.device)
         factor = torch.tensor(self.x_scale, dtype=torch.float32, device=self.device) * s
         self._bind(codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, None,
-                   "IntegerConv2d")
+                   "IntegerConv2d", lut_values)
 
     @classmethod
     def from_parts(cls, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, stride, dilation, padding,
-                   factor, zero_point, w_rowsum, x_zero_point):
+                   factor, zero_point, w_rowsum, x_zero_point, lut_values=None):
         """The launch state from caller-supplied (r, s, c)-ordered codes, f and Sw (mctq::packed_conv2d_i8), with the
         constructor's checks of the weight; only `gemm` is available."""
         conv = cls.__new__(cls)
@@ -1128,10 +1182,11 @@ class IntegerConv2d:
         conv.weight_channels_last = False
         shape = (int(out_channels), int(in_channels), int(kernel_size[0]), int(kernel_size[1]))
         conv._bind(codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum,
-                   "packed_conv2d_i8")
+                   "packed_conv2d_i8" if lut_values is None else "packed_conv2d_i8_lut", lut_values)
         return conv
 
-    def _bind(self, codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum, what):
+    def _bind(self, codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum, what,
+              lut_values=None):
         if len(stride) != 2 or len(dilation) != 2 or len(padding) != 4:
             raise ValueError(f"{what}: stride and dilation are pairs, padding is (top, bottom, left, right)")
         self.stride, self.dilation = tuple(int(v) for v in stride), tuple(int(v) for v in dilation)
@@ -1142,7 +1197,7 @@ class IntegerConv2d:
         # the weight as a [Cout][K] matrix: IntegerLinear's checks and launch state
         self._w = IntegerLinear.__new__(IntegerLinear)
         self._w.device, self._w.x_zp = self.device, self.x_zp
-        self._w._bind(codes, kind, is_signed, dtype, shape[0], K, factor, zero_point, w_rowsum, what)
+        self._w._bind(codes, kind, is_signed, dtype, shape[0], K, factor, zero_point, w_rowsum, what, lut_values)
         self.dtype, self.factor, self.w_rowsum = dtype, self._w.factor, self._w.w_rowsum
         self.needs_x_rowsum = self._w.needs_x_rowsum
 
@@ -1199,12 +1254,17 @@ class IntegerConv2d:
             b = bias.contiguous() if bias is not None else None
             g = _native.MctqConv2dGeom(N, H, W, self.in_channels, Ho, Wo, *self.kernel_size, *self.stride, *self.dilation,
                                        *self.padding)
-            with _on_device(self.device):
-                rc = _native.load().mctq_packed_conv2d_i8(
-                    self._w._desc_ptr, ctypes.addressof(g), Cout, qx.data_ptr(), int(qx.dtype == torch.int8), self.x_zp,
+            args = (self._w._desc_ptr, ctypes.addressof(g), Cout, qx.data_ptr(), int(qx.dtype == torch.int8), self.x_zp,
                     _ptr(rs), self.w_rowsum.data_ptr(), self.factor.data_ptr(), _ptr(b), _DT[self.dtype], y.data_ptr(),
-                    0 if channels_last else 1, _stream(self.device))
-            _native.check(rc, "mctq_packed_conv2d_i8")
+                    0 if channels_last else 1)
+            lut = self._w.lut
+            lib = _native.load()
+            with _on_device(self.device):
+                if lut is not None:
+                    rc = lib.mctq_packed_conv2d_i8_lut(*args, lut.ctypes.data, _stream(self.device))
+                else:
+                    rc = lib.mctq_packed_conv2d_i8(*args, _stream(self.device))
+            _native.check(rc, "mctq_packed_conv2d_i8_lut" if lut is not None else "mctq_packed_conv2d_i8")
         return y
 
 
@@ -1220,6 +1280,20 @@ def _packed_conv2d_i8_cuda(x_codes, x_zero_point, x_rowsum, codes, kind, is_sign
     conv = IntegerConv2d.from_parts(codes, kind, is_signed, dtype, out_channels, x_codes.shape[-1], kernel_size, stride,
                                     dilation, padding, factor, zero_point, w_rowsum, x_zero_point)
     return conv.gemm(x_codes, x_rowsum, bias, channels_last)
+
+
+def _packed_conv2d_i8_lut_cuda(x_codes, x_zero_point, codes, kind, out_channels, kernel_size, stride, dilation, padding,
+                               lut_values, w_rowsum, factor, bias, channels_last):
+    """mctq::packed_conv2d_i8_lut: packed_conv2d_i8 for (r, s, c)-ordered LUT indices with the int8 centroid codes
+    `lut_values` (f32 output, zw = 0: no window code sums)."""
+    if x_codes.dim() != 4:
+        raise RuntimeError("packed_conv2d_i8_lut: x codes must be 4-D NHWC")
+    if len(kernel_size) != 2:
+        raise ValueError("packed_conv2d_i8_lut: kernel_size is a pair")
+    _native.load()
+    conv = IntegerConv2d.from_parts(codes, kind, False, torch.float32, out_channels, x_codes.shape[-1], kernel_size, stride,
+                                    dilation, padding, factor, None, w_rowsum, x_zero_point, lut_values)
+    return conv.gemm(x_codes, None, bias, channels_last)
 
 
 def _lut_scalar_cuda(x, table, K, divisor, threshold, round_to_input_dtype, multiply=False):
@@ -1423,6 +1497,8 @@ _LIB.impl("quantize_rows_i8", _quantize_rows_i8_cuda, "CUDA")
 _LIB.impl("packed_linear_i8", _packed_linear_i8_cuda, "CUDA")
 _LIB.impl("quantize_nhwc_i8", _quantize_nhwc_i8_cuda, "CUDA")
 _LIB.impl("packed_conv2d_i8", _packed_conv2d_i8_cuda, "CUDA")
+_LIB.impl("packed_linear_i8_lut", _packed_linear_i8_lut_cuda, "CUDA")
+_LIB.impl("packed_conv2d_i8_lut", _packed_conv2d_i8_lut_cuda, "CUDA")
 
 _LIB.impl("fq_affine_scalar_pre", _affine_scalar_pre_cuda, "CUDA")
 _LIB.impl("fq_affine_scalar_pre", _via_device(_affine_scalar_pre_cuda), "CPU")
@@ -1441,6 +1517,8 @@ _LIB.impl("quantize_rows_i8", _via_device(_quantize_rows_i8_cuda), "CPU")
 _LIB.impl("packed_linear_i8", _via_device(_packed_linear_i8_cuda), "CPU")
 _LIB.impl("quantize_nhwc_i8", _via_device(_quantize_nhwc_i8_cuda), "CPU")
 _LIB.impl("packed_conv2d_i8", _via_device(_packed_conv2d_i8_cuda), "CPU")
+_LIB.impl("packed_linear_i8_lut", _via_device(_packed_linear_i8_lut_cuda), "CPU")
+_LIB.impl("packed_conv2d_i8_lut", _via_device(_packed_conv2d_i8_lut_cuda), "CPU")
 
 
 # --------------------------------------------------------------------------------------------- fake / meta impls
@@ -1537,6 +1615,21 @@ def _(x_codes, x_zero_point, x_rowsum, codes, kind, is_signed, out_channels, ker
     if channels_last:
         return x_codes.new_empty((N, Ho, Wo, out_channels), dtype=dtype).permute(0, 3, 1, 2)
     return x_codes.new_empty((N, out_channels, Ho, Wo), dtype=dtype)
+
+
+@torch.library.register_fake("mctq::packed_linear_i8_lut")
+def _(x_codes, x_zero_point, codes, kind, out_features, lut_values, w_rowsum, factor, bias):
+    return x_codes.new_empty(tuple(x_codes.shape[:-1]) + (out_features,), dtype=torch.float32)
+
+
+@torch.library.register_fake("mctq::packed_conv2d_i8_lut")
+def _(x_codes, x_zero_point, codes, kind, out_channels, kernel_size, stride, dilation, padding, lut_values, w_rowsum, factor,
+      bias, channels_last):
+    N, H, W, _ = x_codes.shape
+    Ho, Wo = conv_output_hw(H, W, kernel_size, stride, dilation, padding)
+    if channels_last:
+        return x_codes.new_empty((N, Ho, Wo, out_channels), dtype=torch.float32).permute(0, 3, 1, 2)
+    return x_codes.new_empty((N, out_channels, Ho, Wo), dtype=torch.float32)
 
 
 # --------------------------------------------------------------------------------------------- whole-model launch

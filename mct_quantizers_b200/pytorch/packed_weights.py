@@ -46,6 +46,13 @@ operand is gathered from each output pixel's window (csrc/mctq_packed_igemm.cu, 
 Q's zero-point code and contributes exactly 0.  The output has the memory format F.conv2d gives for x and the rebuilt
 weight.  Inputs that are not 4-D (unbatched 3-D inputs included) take the packed path.
 
+Integer modes for LUT weights (`integer_lut=True` together with integer_linear=True and / or integer_conv=True; opt-in): a
+LUT weight rebuilds as fl32(lut_k / 2^(bw-1) * thr[o]) with integer centroids lut_k, i.e. an int8 code lut_k times the scale
+sw[o] = thr[o] * 2^-(bw-1) and zero point 0.  When every centroid is an integer in [-128, 127] and every sw[o] is exact and
+normal in f32, the integer modes take LUT wrappers too: the GEMM's weight producers look each index up in the table (passed
+by value with every launch) and the product is the same exact int32 sum (include/mctq.h).  It differs from the packed path
+by the rounding of W to f32 and by f32 accumulation, so it stays opt-in: without the flag LUT wrappers keep their paths.
+
 Packing is one-way and for inference only:
   * the rebuild dtype is the weight's dtype at packing time; `.half()` does not change it (the codes are integer buffers);
   * the packed state travels with the module: `state_dict` / `load_state_dict` between packed models of the same structure,
@@ -55,6 +62,7 @@ Packing is one-way and for inference only:
 import weakref
 from typing import Dict, List, Optional, Tuple
 
+import numpy as np
 import torch
 from torch.nn.modules import module as _nn_module
 
@@ -281,21 +289,46 @@ def _input_quantizer_eligibility(input_quantizer) -> Tuple[bool, str]:
     return True, ""
 
 
-def integer_linear_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
+def _lut_eligibility(e, K, what, x_signed) -> Tuple[bool, str]:
+    """The conditions the integer modes put on a LUT weight (entry e, row length K named `what`): integer centroids in
+    [-128, 127], every thr[o] * 2^-(bw-1) exact and normal in f32, K a multiple of 32 (4-bit indices) or 16 (8-bit
+    indices) and at most the int32 bound of signed weight codes.  Host-only: reads the quantizer's numpy parameters."""
+    q = e.quantizer
+    v = np.asarray(q._lut_values_np, dtype=np.float64).reshape(-1)
+    if not (np.all(v == np.round(v)) and np.all(v >= -128) and np.all(v <= 127)):
+        return False, "a LUT value is not an integer in [-128, 127] (the integer modes take the centroids as int8 codes)"
+    sw = np.asarray(q._threshold_np, dtype=np.float32).reshape(-1).astype(np.float64) * 2.0 ** -(int(q.lut_values_bitwidth) - 1)
+    if not (np.all(np.isfinite(sw)) and np.all(sw.astype(np.float32) == sw) and
+            np.all(np.abs(sw) >= np.finfo(np.float32).tiny)):
+        return False, "a threshold times 2^-(lut_values_bitwidth - 1) is not exact and normal in float32"
+    step, bits = (32, 4) if e.kind == _native.PACK_LUT_I4 else (16, 8)
+    if K % step:
+        return False, f"{what} = {K} is not a multiple of {step} ({bits}-bit LUT indices)"
+    bound = _native.integer_linear_max_k(True, x_signed)
+    if K > bound:
+        return False, f"{what} = {K} exceeds {bound}, the largest row length whose int32 sum of code products cannot overflow"
+    return True, ""
+
+
+def integer_linear_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
     """(True, '') when `wrapper` can run in integer linear mode with input quantizer `input_quantizer`: fused_linear_eligibility,
     int8 / int4 affine codes, a per-tensor affine activation quantizer with 8-bit codes, in_features a multiple of 16 (32 for
-    int4 codes) and at most the int32 bound of the code signedness pair.  Host-only."""
+    int4 codes) and at most the int32 bound of the code signedness pair.  `lut=True` also accepts LUT weights that meet
+    _lut_eligibility.  Host-only."""
     ok, reason = fused_linear_eligibility(wrapper)
     if not ok:
         return ok, reason
     e = next(e for e in wrapper.__dict__['_packed'].entries if e.name == 'weight')
-    if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
+    is_lut = lut and e.kind in _native.PACK_LUT_KINDS
+    if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4) and not is_lut:
         return False, f"the weight is packed as {_KIND_NAMES[e.kind]}, not as int8 / int4 affine codes"
     ok, reason = _input_quantizer_eligibility(input_quantizer)
     if not ok:
         return ok, reason
     qmin = int(input_quantizer.min_quantized_domain)
     K = wrapper.layer.in_features
+    if is_lut:
+        return _lut_eligibility(e, K, "in_features", qmin < 0)
     step = 32 if e.kind == _native.PACK_AFFINE_I4 else 16
     if K % step:
         return False, f"in_features = {K} is not a multiple of {step}"
@@ -305,13 +338,13 @@ def integer_linear_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
     return True, ""
 
 
-def integer_conv_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
+def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
     """(True, '') when `wrapper` can run in integer convolution mode with input quantizer `input_quantizer`: a
     torch.nn.Conv2d layer with string-attribute weights, no extra call arguments and 'weight' its only quantized weight,
     packed as int8 / int4 affine codes, rebuilt as a contiguous or channels_last [Cout, Cin, kh, kw] weight with parameters
     per tensor or per output channel; groups 1 and zero padding; the input quantizer conditions of integer linear mode;
     Cin a multiple of 16, K = Cin * kh * kw a multiple of 32 for int4 codes and at most the int32 bound of the code
-    signedness pair.  Host-only."""
+    signedness pair.  `lut=True` also accepts LUT weights that meet _lut_eligibility.  Host-only."""
     d = wrapper.__dict__
     if not d.get('is_str_attr', False):
         return False, "the weights are positional inputs of a functional op"
@@ -330,7 +363,8 @@ def integer_conv_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
     e = next((e for e in state.entries if e.name == 'weight'), None) if state is not None else None
     if e is None:
         return False, "the weight is not packed"
-    if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4):
+    is_lut = lut and e.kind in _native.PACK_LUT_KINDS
+    if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4) and not is_lut:
         return False, f"the weight is packed as {_KIND_NAMES[e.kind]}, not as int8 / int4 affine codes"
     shape = (layer.out_channels, layer.in_channels) + tuple(layer.kernel_size)
     dense = torch.empty(shape, device="meta")
@@ -344,6 +378,8 @@ def integer_conv_eligibility(wrapper, input_quantizer) -> Tuple[bool, str]:
         return ok, reason
     if shape[1] % 16:
         return False, f"in_channels = {shape[1]} is not a multiple of 16"
+    if is_lut:
+        return _lut_eligibility(e, K, "Cin * kh * kw", int(input_quantizer.min_quantized_domain) < 0)
     if e.kind == _native.PACK_AFFINE_I4 and K % 32:
         return False, f"Cin * kh * kw = {K} is not a multiple of 32 (int4 codes)"
     bound = _native.integer_linear_max_k(e.is_signed, int(input_quantizer.min_quantized_domain) < 0)
@@ -504,13 +540,17 @@ class PackedState:
             scale, zp, _, _ = affine_scalar_params(q)
             x_scale, x_zp, qmin, qmax = q._validated_launch_args(scale, zp)[1]      # what the holder's kernel receives
             item = e.plan_item()
+            scale, zps, lut = item[8], item[9], None
+            if e.kind in _native.PACK_LUT_KINDS:         # codes lut_k, scale thr * 2^-(bw-1) (exact: _lut_eligibility)
+                wq = e.quantizer
+                scale, lut = scale * 2.0 ** -(int(wq.lut_values_bitwidth) - 1), wq._lut_values_np
             if conv:
                 launch = ops.IntegerConv2d(codes, e.kind, e.is_signed, e.dtype_out, layer.out_channels, layer.in_channels,
                                            layer.kernel_size, e.stride_out, layer.stride, layer.dilation,
-                                           ops.conv_padding(layer), item[8], item[9], x_scale, x_zp, qmin, qmax)
+                                           ops.conv_padding(layer), scale, zps, x_scale, x_zp, qmin, qmax, lut)
             else:
                 launch = ops.IntegerLinear(codes, e.kind, e.is_signed, e.dtype_out, layer.out_features, layer.in_features,
-                                           item[8], item[9], x_scale, x_zp, qmin, qmax)
+                                           scale, zps, x_scale, x_zp, qmin, qmax, lut)
             lin = (codes.data_ptr(), launch)
             self._ilin = lin
         return lin[1](x, bias)
@@ -542,7 +582,7 @@ class PackedState:
 
 
 def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bool = False, integer_linear: bool = False,
-                         input_quantizer=None, integer_conv: bool = False) -> Dict:
+                         input_quantizer=None, integer_conv: bool = False, integer_lut: bool = False) -> Dict:
     """Pack every weight of `wrapper` that can be packed (see the module docstring).  Returns
     {name: {'packed': bool, 'kind': str | None, 'reason': str, 'code_bytes': int, 'float_bytes': int}}.
     `fused_linear=True` also switches the wrapper to fused linear mode when fused_linear_eligibility allows it (on a wrapper
@@ -553,9 +593,11 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
     also switches it to integer linear mode when integer_linear_eligibility allows it, and every report entry gains
     'integer': bool, 'integer_reason': str and 'input_holder' (the holder's module name for pack_model_weights, else None).
     `integer_conv=True` (needs `input_quantizer` too) does the same for integer convolution mode (integer_conv_eligibility),
-    and every report entry gains 'integer_conv': bool, 'integer_conv_reason': str and 'input_holder'."""
+    and every report entry gains 'integer_conv': bool, 'integer_conv_reason': str and 'input_holder'.
+    `integer_lut=True` (needs integer_linear=True and / or integer_conv=True) extends those modes to LUT weights."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
+    _check_integer_lut(integer_lut, integer_linear, integer_conv)
     if integer_linear and input_quantizer is None:
         raise ValueError("integer_linear=True needs the input_quantizer of the activation holder that feeds the wrapper")
     if integer_conv and input_quantizer is None:
@@ -590,10 +632,16 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
     if batched_linear:
         _switch_to_batched(wrapper, report)
     if integer_linear:
-        _switch_to_integer(wrapper, report, input_quantizer, None)
+        _switch_to_integer(wrapper, report, input_quantizer, None, lut=integer_lut)
     if integer_conv:
-        _switch_to_integer(wrapper, report, input_quantizer, None, conv=True)
+        _switch_to_integer(wrapper, report, input_quantizer, None, conv=True, lut=integer_lut)
     return report
+
+
+def _check_integer_lut(integer_lut, integer_linear, integer_conv):
+    if integer_lut and not (integer_linear or integer_conv):
+        raise ValueError("integer_lut=True needs integer_linear=True and / or integer_conv=True (it extends those modes to "
+                         "LUT weights)")
 
 
 def _drop_float_weights(wrapper, new, entries, keep):
@@ -637,9 +685,9 @@ def _switch_to_batched(wrapper, report):
         r['batched'], r['batched_reason'] = ok, reason
 
 
-def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None, conv=False):
+def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None, conv=False, lut=False):
     eligibility = integer_conv_eligibility if conv else integer_linear_eligibility
-    ok, why = (False, reason) if reason else eligibility(wrapper, input_quantizer)
+    ok, why = (False, reason) if reason else eligibility(wrapper, input_quantizer, lut=lut)
     state = wrapper.__dict__.get('_packed')
     if ok:
         state.integer, state.input_quantizer, state._ilin = True, input_quantizer, None
@@ -662,15 +710,16 @@ def _bits(t):
 
 
 def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batched_linear: bool = False,
-                       integer_linear: bool = False, integer_conv: bool = False) -> Dict[str, Dict]:
+                       integer_linear: bool = False, integer_conv: bool = False, integer_lut: bool = False) -> Dict[str, Dict]:
     """pack_weights(fused_linear, batched_linear) on every PytorchQuantizationWrapper of `model`: {wrapper module name:
     {weight name: report entry}}.  `integer_linear=True` then switches, in place, every eligible wrapper whose input is the
     output of an activation quantization holder (integer_linear_edges) to integer linear mode; every report entry gains
     'integer', 'integer_reason' and 'input_holder'.  `integer_conv=True` does the same for integer convolution mode on the
-    same edges; every report entry gains 'integer_conv', 'integer_conv_reason' and 'input_holder'.  When the model cannot be
-    traced nothing is switched and the reason is reported."""
+    same edges; every report entry gains 'integer_conv', 'integer_conv_reason' and 'input_holder'.  `integer_lut=True` extends
+    both to LUT weights.  When the model cannot be traced nothing is switched and the reason is reported."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
+    _check_integer_lut(integer_lut, integer_linear, integer_conv)
     from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
     wrappers = {mod_name: mod for mod_name, mod in model.named_modules()
                 if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization}
@@ -681,5 +730,5 @@ def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batch
             holder, q = edges.get(name, (None, None)) if name not in why else (None, None)
             reason = failure or why.get(name) or ("" if holder else "the wrapper is not called in the traced forward")
             for conv in (False, True) if integer_linear and integer_conv else (integer_conv,):
-                _switch_to_integer(mod, reports[name], q, holder, None if holder else reason, conv=conv)
+                _switch_to_integer(mod, reports[name], q, holder, None if holder else reason, conv=conv, lut=integer_lut)
     return reports
