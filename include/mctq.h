@@ -302,6 +302,35 @@ int mctq_packed_conv2d_i8_lut(const MctqPackedDesc* w, const MctqConv2dGeom* g, 
                               const float* factor, const void* bias, int y_dtype, void* y, int y_nchw,
                               const int8_t* lut_codes_host, void* stream);
 
+/* Integer convolution mode for depthwise Conv2d (groups == Cin, any channel multiplier; DESIGN.md §7e).  The formula of
+ * mctq_packed_conv2d_i8 with one input channel per group, in its centred form:
+ *   m = Cout / Cin (channel multiplier); output channel o reads input channel c(o) = o / m;  K = kh * kw
+ *   qx[b,c,h,w]  = Q's codes of x: the recipe of mctq_quantize_rows_i8, bit for bit the codes mctq_fq_affine_scalar emits
+ *                  (NaN -> qmin, +-inf clamped);  zx outside the image
+ *   c[b,o,ho,wo] = sum_{r,s} (qx[b, c(o), ho*sh - pt + r*dh, wo*sw - pl + s*dw] - zx) * (qw[o,r,s] - zw[o])
+ *                  int32, exact for K <= 33025 (each factor has magnitude <= 255); padded taps contribute exactly 0
+ *   y[b,o,ho,wo] = T(fl(fl((float)c * f[o]) + bias[o])),  f[o] = fl32(sx_f32 * sw[o]),  T = the rebuilt weight's dtype
+ *   LUT weights: qw = lut[idx] (int8), zw = 0, sw = thr * 2^-(bw-1), T = f32 (as for mctq_packed_conv2d_i8_lut)
+ * c is the integer acc - zw Sx - zx Sw + K zx zw of mctq_packed_conv2d_i8, so the output does not depend on the order of
+ * the taps or the tiling.  The kernel reads the float x once and computes Q's codes in registers: no code tensor, no Sx.
+ *   w          HOST descriptor of an MCTQ_PACK_AFFINE_I8 / _I4 / LUT_I4 / LUT_U8 weight [Cout][kh*kw] (the memory order of a
+ *              contiguous or channels_last [Cout, 1, kh, kw] weight), per tensor or per output channel (inner = kh*kw);
+ *              w->y_dtype == x_dtype; w->scale is not read (factor replaces it); codes at any alignment
+ *   g          the geometry (g->Cin = C, x's channels); Ho / Wo are the caller's (taps outside the image are never read)
+ *   x          device x [N][C][H][W] (x_nhwc = 0, NCHW-contiguous) or [N][H][W][C] (x_nhwc = 1, channels_last), x_dtype;
+ *              y [N][Cout][Ho][Wo] in the same layout and dtype
+ *   x_scale, x_zero_point, x_qmin, x_qmax   Q (scale narrowed to f32), as for mctq_quantize_rows_i8
+ *   factor     device f [1 or Cout];  bias: device [Cout] of x_dtype, or NULL
+ *   lut_codes_host   LUT kinds: HOST array of w->K int8 centroid codes (by value in the kernel arguments); NULL otherwise
+ * No host-device copy and no synchronisation: CUDA-graph capture works.  Returns, before any CUDA call: MCTQ_E_BADARG for
+ * a null pointer, a non-positive extent, stride or dilation, a negative pad, x_nhwc not 0 / 1, Cout not a multiple of Cin,
+ * w->n != Cout*kh*kw, a bad parameter layout, or a table present / absent against the kind; MCTQ_E_DTYPE; MCTQ_E_RANGE for
+ * a range that does not fit 8-bit codes, zx outside it, kh*kw > 33025, or a dilated window too wide for shared memory even
+ * for one output of one channel; MCTQ_E_LUT.  N == 0 is a no-op. */
+int mctq_packed_dwconv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x, int x_dtype,
+                            int x_nhwc, float x_scale, int32_t x_zero_point, int32_t x_qmin, int32_t x_qmax,
+                            const float* factor, const void* bias, void* y, const int8_t* lut_codes_host, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Whole-model weight quantisation: one launch over a table of tensors (SURVEY 8f rank 1).
  * Replaces the per-layer loop  for name, w, quantizer in self._weights_vars: quantizer(w)

@@ -734,6 +734,155 @@ __global__ void __launch_bounds__(kThreads) quantize_nhwc_kernel(const T* __rest
     }
 }
 
+// ---- depthwise convolution of Q's codes (integer convolution mode, mctq_packed_dwconv2d_i8): x is read once as floats and
+// quantized in registers by the recipe of quantize_rows_kernel; only qx - zx reaches shared memory (0 for taps outside the
+// image), and the centred sum needs neither Sx nor Sw.  A work unit is S "slots" times a TH x TW tile of output pixels:
+//   NCHW  a slot is one (b, c) plane, S consecutive planes per unit (S > 1 for small planes); loads run along W
+//   NHWC  a slot is one channel of image b, S consecutive channels; loads run along C
+// The window tile [IH][IW][SB] holds the slots innermost (SB: S rounded to an odd number of 32-bit words, so that the
+// transposing stores of the NCHW path spread over the banks).  Each unit then walks the channel multiplier t: the m output
+// channels o = c * m + t of every slot reuse the staged tile, their kh * kw codes decoded once into qw - zw.
+struct DwArgs {
+    const void* x;
+    void* y;
+    const uint8_t* codes;            // weight codes / LUT indices [Cout][K]
+    const int32_t* w_zp;             // affine: zw [1 or Cout]; LUT: null (zw = 0)
+    const float* factor;             // f [1 or Cout]
+    const void* bias;                // [Cout] of T, or null
+    int64_t units, groups, nplanes;  // work units; slot groups; N * C
+    int32_t H, W, C, Cout, Ho, Wo, m, K, kh, kw, sh, sw, dh, dw, pt, pl;
+    int32_t S, SB, TH, TW, IH, IW, tiles_x, tiles_y;
+    int32_t kind, w_signed, per_channel;
+    float x_scale;
+    int32_t x_zp, x_qmin, x_qmax;
+    FastDiv div_S, div_npix, div_IW, div_nout, div_TW;
+    int8_t lut[256];                 // LUT kinds: the centroid codes (by value: no device copy)
+};
+
+// qw - zw of weight element i (LUT kinds: the centroid code of its index, zw = 0)
+__device__ __forceinline__ int dw_weight(const DwArgs& a, int64_t i, int32_t zw) {
+    const bool nib = a.kind == MCTQ_PACK_AFFINE_I4 || a.kind == MCTQ_PACK_LUT_I4;
+    const uint32_t byte = __ldg(a.codes + (nib ? i >> 1 : i));
+    const uint32_t u = nib ? ((i & 1) ? byte >> 4 : byte & 15u) : byte;
+    if (a.kind == MCTQ_PACK_LUT_U8 || a.kind == MCTQ_PACK_LUT_I4) return a.lut[u];
+    const int q = !a.w_signed ? (int)u : nib ? (int)(u ^ 8u) - 8 : (int)(int8_t)u;
+    return q - zw;
+}
+
+// KS: 3 for a 3x3 kernel (taps unrolled, the thread's weights held in registers), 0 for any other kernel.  At most 40
+// registers, so that six CTAs share an SM and hide each other's staging (eight would spill)
+template <typename T, bool NHWC, int KS>
+__global__ void __launch_bounds__(kThreads, 6) packed_dwconv_kernel(const __grid_constant__ DwArgs a) {
+    using Op = AffineOp<false>;
+    AffineArgs aa;                                  // only the fields AffineOp::make reads
+    aa.qmin = a.x_qmin;
+    aa.qmax = a.x_qmax;
+    const Op::ChanParams p = Op::make(a.x_scale, a.x_zp, aa);
+    extern __shared__ __align__(16) uint8_t dw_smem[];
+    int64_t* soff = reinterpret_cast<int64_t*>(dw_smem);      // [S] y offset of slot s's output plane / channel
+    float* sf = reinterpret_cast<float*>(soff + a.S);           // [S] f[o]
+    float* sbias = sf + a.S;                                    // [S] bias[o]
+    int32_t* so = reinterpret_cast<int32_t*>(sbias + a.S);      // [S] o, or -1 for a slot past the last plane / channel
+    int32_t* ws = so + a.S;                                     // [K][S] qw - zw
+    int16_t* xs = reinterpret_cast<int16_t*>(ws + (size_t)a.K * a.S);    // [IH * IW][SB] qx - zx
+    pdl_wait();
+    pdl_launch_dependents();
+    const T* x = reinterpret_cast<const T*>(a.x);
+    T* y = reinterpret_cast<T*>(a.y);
+    const int KH = KS ? KS : a.kh, KW = KS ? KS : a.kw;
+    const uint32_t S = (uint32_t)a.S, npix = (uint32_t)(a.IH * a.IW), nout = (uint32_t)(a.TH * a.TW);
+    const int64_t per_group = (int64_t)a.tiles_y * a.tiles_x, HW = (int64_t)a.H * a.W;
+    for (int64_t u = blockIdx.x; u < a.units; u += gridDim.x) {
+        const int64_t g = u / per_group;
+        const int32_t t2 = (int32_t)(u - g * per_group), ty = t2 / a.tiles_x, tx = t2 - ty * a.tiles_x;
+        const int32_t ho0 = ty * a.TH, wo0 = tx * a.TW;
+        const int64_t h0 = (int64_t)ho0 * a.sh - a.pt, w0 = (int64_t)wo0 * a.sw - a.pl;
+        int64_t b = 0, first;                        // NHWC: image b and its first channel; NCHW: the first plane
+        if (NHWC) {
+            const int64_t cblocks = (a.C + a.S - 1) / a.S;
+            b = g / cblocks;
+            first = (g - b * cblocks) * a.S;
+        } else {
+            first = g * a.S;
+        }
+        const int64_t nslots = min((int64_t)a.S, (NHWC ? (int64_t)a.C : a.nplanes) - first);
+        __syncthreads();                             // the previous unit is done with the shared tiles
+        for (uint32_t e = threadIdx.x; e < npix * S; e += kThreads) {
+            uint32_t s, pix;
+            if (NHWC) { pix = fdiv_u32(e, a.div_S); s = e - pix * S; }           // channels innermost: coalesced along C
+            else { s = fdiv_u32(e, a.div_npix); pix = e - s * npix; }            // columns innermost: coalesced along W
+            const uint32_t iy = fdiv_u32(pix, a.div_IW), ix = pix - iy * (uint32_t)a.IW;
+            const int64_t h = h0 + iy, w = w0 + ix;
+            int v = 0;
+            if ((int64_t)s < nslots && h >= 0 && h < a.H && w >= 0 && w < a.W) {
+                const int64_t off = NHWC ? ((b * a.H + h) * a.W + w) * a.C + first + s : (first + s) * HW + h * a.W + w;
+                int q;
+                Op::template apply<true>(to_f32<T>(x[off]), p, q);
+                v = q - a.x_zp;
+            }
+            xs[pix * a.SB + s] = (int16_t)v;
+        }
+        for (int32_t t = 0; t < a.m; ++t) {
+            if (threadIdx.x < S) {
+                const uint32_t s = threadIdx.x;
+                int32_t o = -1;
+                if ((int64_t)s < nslots) {
+                    const int64_t plane = first + s;
+                    const int64_t bb = NHWC ? b : plane / a.C, c = NHWC ? plane : plane - bb * a.C;
+                    o = (int32_t)(c * a.m + t);
+                    const int ch = a.per_channel ? o : 0;
+                    soff[s] = NHWC ? (int64_t)o : (bb * a.Cout + o) * ((int64_t)a.Ho * a.Wo);
+                    sf[s] = __ldg(a.factor + ch);
+                    sbias[s] = a.bias ? to_f32<T>(reinterpret_cast<const T*>(a.bias)[o]) : 0.0f;
+                }
+                so[s] = o;
+            }
+            __syncthreads();                         // slot parameters set; the tile is staged (t = 0)
+            for (uint32_t e = threadIdx.x; e < (uint32_t)a.K * S; e += kThreads) {
+                const uint32_t k = fdiv_u32(e, a.div_S), s = e - k * S;
+                const int32_t o = so[s];
+                int v = 0;
+                if (o >= 0) v = dw_weight(a, (int64_t)o * a.K + k, a.w_zp ? __ldg(a.w_zp + (a.per_channel ? o : 0)) : 0);
+                ws[e] = v;
+            }
+            __syncthreads();
+            int wr[KS ? KS * KS : 1];
+            uint32_t wslot = 0xffffffffu;
+            for (uint32_t q = threadIdx.x; q < nout * S; q += kThreads) {
+                uint32_t s, pix;
+                if (NHWC) { pix = fdiv_u32(q, a.div_S); s = q - pix * S; }        // lanes along C: coalesced NHWC stores
+                else { s = fdiv_u32(q, a.div_nout); pix = q - s * nout; }          // lanes along W: coalesced plane stores
+                const uint32_t oy = fdiv_u32(pix, a.div_TW), ox = pix - oy * (uint32_t)a.TW;
+                const int32_t ho = ho0 + (int32_t)oy, wo = wo0 + (int32_t)ox;
+                if (so[s] < 0 || ho >= a.Ho || wo >= a.Wo) continue;
+                const int16_t* xw = xs + ((size_t)oy * a.sh * a.IW + (size_t)ox * a.sw) * a.SB + s;
+                int32_t acc = 0;
+                if (KS) {
+                    if (s != wslot) {
+#pragma unroll
+                        for (int k = 0; k < KS * KS; ++k) wr[k] = ws[k * S + s];
+                        wslot = s;
+                    }
+#pragma unroll
+                    for (int r = 0; r < KS; ++r)
+#pragma unroll
+                        for (int c = 0; c < KS; ++c)
+                            acc += (int)xw[((size_t)r * a.dh * a.IW + (size_t)c * a.dw) * a.SB] * wr[r * KS + c];
+                } else {
+                    for (int r = 0; r < KH; ++r)
+                        for (int c = 0; c < KW; ++c)
+                            acc += (int)xw[((size_t)r * a.dh * a.IW + (size_t)c * a.dw) * a.SB] * ws[(r * KW + c) * S + s];
+                }
+                float v = __fmul_rn(__int2float_rn(acc), sf[s]);
+                if (a.bias) v = __fadd_rn(v, sbias[s]);
+                const int64_t pix_off = NHWC ? ((b * a.Ho + ho) * a.Wo + wo) * a.Cout : (int64_t)ho * a.Wo + wo;
+                y[soff[s] + pix_off] = from_f32<T>(v);
+            }
+            __syncthreads();                         // the weights of t are read
+        }
+    }
+}
+
 }  // namespace mctq
 
 using namespace mctq;
@@ -877,6 +1026,41 @@ int launch_affine(const AffineArgs& a, int x_dtype, int code_mode, cudaStream_t 
     }
 }
 
+// shared-memory bytes of packed_dwconv_kernel for the tile in `a`
+size_t dw_smem_bytes(const DwArgs& a) {
+    return (size_t)a.S * (8 + 4 + 4 + 4) + (size_t)a.K * a.S * 4 + (size_t)a.IH * a.IW * a.SB * 2;
+}
+
+// the tile of a work unit: about 2048 outputs, S slots, shrunk until the window tile fits shared memory (0, or MCTQ_E_RANGE
+// for a dilated window too wide even for one output row of one slot)
+int dw_plan(DwArgs& a, bool nhwc) {
+    constexpr int64_t kOut = 2048;
+    const int64_t plane = (int64_t)a.Ho * a.Wo;
+    if (nhwc) {
+        a.S = 32;
+        a.TW = (int32_t)std::min<int64_t>(a.Wo, 16);
+        a.TH = (int32_t)std::min<int64_t>(a.Ho, 8);
+    } else {
+        a.S = (int32_t)std::max<int64_t>(1, std::min<int64_t>({32, kOut / plane, a.nplanes}));
+        a.TW = (int32_t)std::min<int64_t>(a.Wo, 64);
+        a.TH = (int32_t)std::min<int64_t>(a.Ho, std::max<int64_t>(1, kOut / ((int64_t)a.S * a.TW)));
+    }
+    for (;;) {
+        const int64_t ih = (int64_t)(a.TH - 1) * a.sh + (int64_t)(a.kh - 1) * a.dh + 1;
+        const int64_t iw = (int64_t)(a.TW - 1) * a.sw + (int64_t)(a.kw - 1) * a.dw + 1;
+        a.SB = 2 * (((a.S + 1) / 2) | 1);
+        if (ih * iw * a.SB < (1LL << 31)) {
+            a.IH = (int32_t)ih;
+            a.IW = (int32_t)iw;
+            if (dw_smem_bytes(a) <= 200 * 1024) return 0;
+        }
+        if (a.TH > 1) a.TH = (a.TH + 1) / 2;
+        else if (a.S > 1) a.S = (a.S + 1) / 2;
+        else if (a.TW > 1) a.TW = (a.TW + 1) / 2;
+        else return MCTQ_E_RANGE;
+    }
+}
+
 }  // namespace
 
 extern "C" {
@@ -977,6 +1161,65 @@ int mctq_quantize_nhwc_i8(const void* x, int x_dtype, int64_t N, int64_t C, int6
         using T = typename decltype(type)::type;
         return launch_streaming(quantize_nhwc_kernel<T>, (unsigned)blocks, 0, st, reinterpret_cast<const T*>(x),
                                 reinterpret_cast<uint8_t*>(codes), P, N, C, HW, scale, zp, qmin, qmax);
+    };
+    if (x_dtype == MCTQ_F32) return run(PackType<float>{});
+    if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});
+    return run(PackType<__half>{});
+}
+
+int mctq_packed_dwconv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x, int x_dtype,
+                            int x_nhwc, float x_scale, int32_t x_zero_point, int32_t x_qmin, int32_t x_qmax,
+                            const float* factor, const void* bias, void* y, const int8_t* lut_codes_host, void* stream) {
+    MCTQ_NVTX("mctq_packed_dwconv2d_i8");
+    if (!w || !g || !factor) return MCTQ_E_BADARG;
+    if (g->N < 0 || g->H < 1 || g->W < 1 || g->Cin < 1 || g->Ho < 1 || g->Wo < 1 || g->kh < 1 || g->kw < 1 || g->sh < 1 ||
+        g->sw < 1 || g->dh < 1 || g->dw < 1 || g->pt < 0 || g->pb < 0 || g->pl < 0 || g->pr < 0 || (x_nhwc != 0 && x_nhwc != 1))
+        return MCTQ_E_BADARG;
+    if (Cout < 1 || Cout % g->Cin != 0) return MCTQ_E_BADARG;
+    const int64_t K = (int64_t)g->kh * g->kw;
+    // the weight as a [Cout][kh * kw] matrix: kind, dtype, extent, parameter layout, pointers
+    if (const int rc = packed_linear_check(w, Cout, K, x, x_dtype, g->N, y)) return rc;
+    if (pack_is_lut(w->kind) != (lut_codes_host != nullptr)) return MCTQ_E_BADARG;
+    if (x_qmin > x_qmax) return MCTQ_E_RANGE;
+    if (int rc = check_codes(x_qmin, x_qmax, MCTQ_CODES_INT8, x)) return rc;
+    if (x_zero_point < x_qmin || x_zero_point > x_qmax || K > 33025) return MCTQ_E_RANGE;    // |qx - zx|, |qw - zw| <= 255
+    if (g->N == 0) return 0;
+
+    DwArgs a;
+    memset(&a, 0, sizeof(a));
+    a.x = x;
+    a.y = y;
+    a.codes = reinterpret_cast<const uint8_t*>(w->codes);
+    a.w_zp = pack_is_lut(w->kind) ? nullptr : w->zp;
+    a.factor = factor;
+    a.bias = bias;
+    a.nplanes = (int64_t)g->N * g->Cin;
+    a.H = g->H; a.W = g->W; a.C = g->Cin; a.Cout = (int32_t)Cout; a.Ho = g->Ho; a.Wo = g->Wo;
+    a.m = (int32_t)(Cout / g->Cin); a.K = (int32_t)K; a.kh = g->kh; a.kw = g->kw;
+    a.sh = g->sh; a.sw = g->sw; a.dh = g->dh; a.dw = g->dw; a.pt = g->pt; a.pl = g->pl;
+    a.kind = w->kind; a.w_signed = w->is_signed ? 1 : 0; a.per_channel = w->C != 1;
+    a.x_scale = x_scale; a.x_zp = x_zero_point; a.x_qmin = x_qmin; a.x_qmax = x_qmax;
+    if (lut_codes_host) memcpy(a.lut, lut_codes_host, (size_t)w->K);
+    if (const int rc = dw_plan(a, x_nhwc != 0)) return rc;
+    a.tiles_y = (a.Ho + a.TH - 1) / a.TH;
+    a.tiles_x = (a.Wo + a.TW - 1) / a.TW;
+    a.groups = x_nhwc ? (int64_t)g->N * ((a.C + a.S - 1) / a.S) : (a.nplanes + a.S - 1) / a.S;
+    a.units = a.groups * a.tiles_y * a.tiles_x;
+    a.div_S = make_fastdiv((uint32_t)a.S);
+    a.div_npix = make_fastdiv((uint32_t)(a.IH * a.IW));
+    a.div_IW = make_fastdiv((uint32_t)a.IW);
+    a.div_nout = make_fastdiv((uint32_t)(a.TH * a.TW));
+    a.div_TW = make_fastdiv((uint32_t)a.TW);
+    const size_t smem = dw_smem_bytes(a);
+    const unsigned blocks = (unsigned)std::min<int64_t>(a.units, 148 * 8);
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool k3 = g->kh == 3 && g->kw == 3;
+    auto run = [&](auto type) {
+        using T = typename decltype(type)::type;
+        auto kernel = x_nhwc ? (k3 ? packed_dwconv_kernel<T, true, 3> : packed_dwconv_kernel<T, true, 0>)
+                             : (k3 ? packed_dwconv_kernel<T, false, 3> : packed_dwconv_kernel<T, false, 0>);
+        if (const int rc = ensure_smem(kernel, smem)) return rc;
+        return launch_streaming(kernel, blocks, smem, st, a);
     };
     if (x_dtype == MCTQ_F32) return run(PackType<float>{});
     if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});

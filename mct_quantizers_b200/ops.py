@@ -15,6 +15,7 @@ sm_100a kernels.
     torch.ops.mctq.quantize_nhwc_i8   -> NHWC 8-bit codes of an NCHW x and their per-pixel channel sums
     torch.ops.mctq.packed_conv2d_i8   <- the integer convolution of NHWC codes and packed weight codes (implicit GEMM)
     torch.ops.mctq.packed_linear_i8_lut / packed_conv2d_i8_lut   the same with LUT weights: indices looked up as int8 codes
+    torch.ops.mctq.packed_dwconv2d_i8 <- the integer depthwise convolution of Q's codes of x (computed in the kernel)
 
 (reference call sites: see include/mctq.h).  Each op has a CUDA implementation (device pointers + the
 caller's current stream into the C ABI, no synchronisation), a CPU-tensor implementation that streams the
@@ -65,6 +66,9 @@ _LIB.define("packed_linear_i8_lut(Tensor x_codes, int x_zero_point, Tensor codes
 _LIB.define("packed_conv2d_i8_lut(Tensor x_codes, int x_zero_point, Tensor codes, int kind, int out_channels, "
             "int[] kernel_size, int[] stride, int[] dilation, int[] padding, int[] lut_values, Tensor w_rowsum, "
             "Tensor factor, Tensor? bias, bool channels_last) -> Tensor")
+_LIB.define("packed_dwconv2d_i8(Tensor x, float x_scale, int x_zero_point, int x_qmin, int x_qmax, Tensor codes, int kind, "
+            "bool is_signed, int out_channels, int[] kernel_size, int[] stride, int[] dilation, int[] padding, "
+            "Tensor? zero_point, Tensor factor, Tensor? lut_values, Tensor? bias, bool channels_last) -> Tensor")
 
 
 # --------------------------------------------------------------------------------------------- helpers
@@ -1296,6 +1300,119 @@ def _packed_conv2d_i8_lut_cuda(x_codes, x_zero_point, codes, kind, out_channels,
     return conv.gemm(x_codes, None, bias, channels_last)
 
 
+class IntegerDepthwiseConv2d:
+    """Launch state of one packed depthwise Conv2d weight [Cout, 1, kh, kw] (groups = in_channels, Cout a multiple of it) in
+    integer convolution mode (mctq_packed_dwconv2d_i8), built once: the descriptor of the weight as a [Cout][kh*kw] matrix,
+    f = fl32(sx * scale), the geometry and the input quantizer's launch constants.  The arguments are IntegerConv2d's; the
+    codes are used as they are (a contiguous and a channels_last [Cout, 1, kh, kw] weight have the same memory order).
+    `__call__(x, bias)` returns the depthwise convolution of Q's codes of a 4-D CUDA x of `dtype` on the codes' device with
+    the weight codes, scaled (include/mctq.h gives the formula), in the memory format F.conv2d gives for x and the rebuilt
+    weight.  The kernel reads x itself and computes Q's codes in registers: one launch, no code tensor."""
+
+    def __init__(self, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, weight_stride, stride,
+                 dilation, padding, scale, zero_point, x_scale, x_zero_point, x_qmin, x_qmax, lut_values=None):
+        shape = (int(out_channels), 1, int(kernel_size[0]), int(kernel_size[1]))
+        self.weight_channels_last = _suggests_channels_last(shape, weight_stride)
+        dense = torch.empty(shape, device="meta")
+        if tuple(weight_stride) not in (dense.stride(), dense.to(memory_format=torch.channels_last).stride()):
+            raise ValueError(f"IntegerDepthwiseConv2d: weight strides {tuple(weight_stride)} are neither contiguous nor "
+                             f"channels_last")
+        s = _param_on(scale.detach().reshape(-1).contiguous().to(torch.float32), codes.device)
+        factor = torch.tensor(float(np.float32(x_scale)), dtype=torch.float32, device=codes.device) * s
+        self._bind(codes, kind, is_signed, dtype, shape[0], in_channels, shape[2:], stride, dilation, padding, factor,
+                   zero_point, x_scale, x_zero_point, x_qmin, x_qmax, "IntegerDepthwiseConv2d", lut_values)
+
+    @classmethod
+    def from_parts(cls, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, stride, dilation, padding,
+                   factor, zero_point, x_scale, x_zero_point, x_qmin, x_qmax, lut_values=None):
+        """The launch state from caller-supplied [Cout][kh*kw] codes and f (mctq::packed_dwconv2d_i8)."""
+        conv = cls.__new__(cls)
+        conv.weight_channels_last = False
+        conv._bind(codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, stride, dilation, padding, factor,
+                   zero_point, x_scale, x_zero_point, x_qmin, x_qmax, "packed_dwconv2d_i8", lut_values)
+        return conv
+
+    def _bind(self, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, stride, dilation, padding, factor,
+              zero_point, x_scale, x_zero_point, x_qmin, x_qmax, what, lut_values):
+        _check_range(x_qmin, x_qmax)
+        if not ((-128 <= x_qmin and x_qmax <= 127) or (0 <= x_qmin and x_qmax <= 255)):
+            raise ValueError(f"{what}: the input range [{x_qmin}, {x_qmax}] does not fit 8-bit codes")
+        if not x_qmin <= x_zero_point <= x_qmax:
+            raise RuntimeError("`zero_point` must be between `quant_min` and `quant_max`.")
+        if len(kernel_size) != 2 or len(stride) != 2 or len(dilation) != 2 or len(padding) != 4:
+            raise ValueError(f"{what}: kernel_size, stride and dilation are pairs, padding is (top, bottom, left, right)")
+        self.out_channels, self.in_channels = int(out_channels), int(in_channels)
+        if self.in_channels < 1 or self.out_channels % self.in_channels:
+            raise ValueError(f"{what}: out_channels = {out_channels} is not a multiple of in_channels = {in_channels}")
+        self.device = codes.device
+        self.x_scale, self.x_zp = float(np.float32(x_scale)), int(x_zero_point)
+        self.x_qmin, self.x_qmax = int(x_qmin), int(x_qmax)
+        self.kernel_size = tuple(int(k) for k in kernel_size)
+        self.stride, self.dilation = tuple(int(v) for v in stride), tuple(int(v) for v in dilation)
+        self.padding = tuple(int(v) for v in padding)
+        # the weight as a [Cout][kh * kw] matrix: IntegerLinear's checks and descriptor
+        self._w = IntegerLinear.__new__(IntegerLinear)
+        self._w.device, self._w.x_zp = self.device, self.x_zp
+        self._w._bind(codes, kind, is_signed, dtype, self.out_channels, self.kernel_size[0] * self.kernel_size[1], factor,
+                      zero_point, torch.zeros(self.out_channels, dtype=torch.int32), what, lut_values)
+        self.dtype, self.factor = dtype, self._w.factor
+
+    def output_hw(self, H, W):
+        return conv_output_hw(H, W, self.kernel_size, self.stride, self.dilation, self.padding)
+
+    def __call__(self, x, bias=None):
+        return self.conv(x, bias, self.weight_channels_last or _suggests_channels_last(x.shape, x.stride()))
+
+    def conv(self, x, bias=None, channels_last=False):
+        """y [N, Cout, Ho, Wo] of x [N, in_channels, H, W]; channels_last: the layout of y, and of x in the kernel (x is
+        converted when it has another one, which changes no value)."""
+        if x.dtype != self.dtype or (bias is not None and bias.dtype != self.dtype):
+            raise RuntimeError(f"packed_dwconv2d_i8: x and bias must have the weight's dtype {self.dtype}")
+        if x.dim() != 4 or x.shape[1] != self.in_channels:
+            raise RuntimeError(f"packed_dwconv2d_i8: x of shape {list(x.shape)} is not [N, {self.in_channels}, H, W]")
+        if x.device != self.device or (bias is not None and bias.device != self.device):
+            raise RuntimeError(f"packed_dwconv2d_i8: x and bias must live on {self.device}")
+        if bias is not None and bias.numel() != self.out_channels:
+            raise RuntimeError(f"packed_dwconv2d_i8: bias must hold {self.out_channels} entries of {self.dtype}")
+        fmt = torch.channels_last if channels_last else torch.contiguous_format
+        if not x.is_contiguous(memory_format=fmt):
+            x = x.contiguous(memory_format=fmt)
+        N, _, H, W = x.shape
+        Ho, Wo = self.output_hw(H, W)
+        if Ho < 1 or Wo < 1:
+            raise RuntimeError(f"packed_dwconv2d_i8: a {H} x {W} input is smaller than the dilated kernel")
+        Cout = self.out_channels
+        if channels_last:
+            y = torch.empty((N, Ho, Wo, Cout), dtype=self.dtype, device=self.device).permute(0, 3, 1, 2)
+        else:
+            y = torch.empty((N, Cout, Ho, Wo), dtype=self.dtype, device=self.device)
+        if y.numel():
+            b = bias.contiguous() if bias is not None else None
+            g = _native.MctqConv2dGeom(N, H, W, self.in_channels, Ho, Wo, *self.kernel_size, *self.stride, *self.dilation,
+                                       *self.padding)
+            lut = self._w.lut
+            with _on_device(self.device):
+                rc = _native.load().mctq_packed_dwconv2d_i8(
+                    self._w._desc_ptr, ctypes.addressof(g), Cout, x.data_ptr(), _DT[self.dtype], int(bool(channels_last)),
+                    self.x_scale, self.x_zp, self.x_qmin, self.x_qmax, self.factor.data_ptr(), _ptr(b), y.data_ptr(),
+                    lut.ctypes.data if lut is not None else None, _stream(self.device))
+            _native.check(rc, "mctq_packed_dwconv2d_i8")
+        return y
+
+
+def _packed_dwconv2d_i8_cuda(x, x_scale, x_zero_point, x_qmin, x_qmax, codes, kind, is_signed, out_channels, kernel_size,
+                             stride, dilation, padding, zero_point, factor, lut_values, bias, channels_last):
+    """mctq::packed_dwconv2d_i8: the [Cout][kh*kw] weight codes (or LUT indices with their int8 centroid codes
+    `lut_values`) and f supplied by the caller; y in x's dtype, channels_last or NCHW."""
+    if x.dim() != 4:
+        raise RuntimeError("packed_dwconv2d_i8: x must be 4-D [N, C, H, W]")
+    _native.load()
+    conv = IntegerDepthwiseConv2d.from_parts(codes, kind, is_signed, x.dtype, out_channels, x.shape[1], kernel_size, stride,
+                                             dilation, padding, factor, zero_point, x_scale, x_zero_point, x_qmin, x_qmax,
+                                             lut_values)
+    return conv.conv(x, bias, channels_last)
+
+
 def _lut_scalar_cuda(x, table, K, divisor, threshold, round_to_input_dtype, multiply=False):
     """`multiply`: normalise with x * (float)(1.0 / divisor) -- the reference's CUDA flavour of `tensor / python_number`
     (quantizer_utils.reference_arithmetic) -- instead of the true division x / (float)divisor."""
@@ -1499,6 +1616,7 @@ _LIB.impl("quantize_nhwc_i8", _quantize_nhwc_i8_cuda, "CUDA")
 _LIB.impl("packed_conv2d_i8", _packed_conv2d_i8_cuda, "CUDA")
 _LIB.impl("packed_linear_i8_lut", _packed_linear_i8_lut_cuda, "CUDA")
 _LIB.impl("packed_conv2d_i8_lut", _packed_conv2d_i8_lut_cuda, "CUDA")
+_LIB.impl("packed_dwconv2d_i8", _packed_dwconv2d_i8_cuda, "CUDA")
 
 _LIB.impl("fq_affine_scalar_pre", _affine_scalar_pre_cuda, "CUDA")
 _LIB.impl("fq_affine_scalar_pre", _via_device(_affine_scalar_pre_cuda), "CPU")
@@ -1519,6 +1637,7 @@ _LIB.impl("quantize_nhwc_i8", _via_device(_quantize_nhwc_i8_cuda), "CPU")
 _LIB.impl("packed_conv2d_i8", _via_device(_packed_conv2d_i8_cuda), "CPU")
 _LIB.impl("packed_linear_i8_lut", _via_device(_packed_linear_i8_lut_cuda), "CPU")
 _LIB.impl("packed_conv2d_i8_lut", _via_device(_packed_conv2d_i8_lut_cuda), "CPU")
+_LIB.impl("packed_dwconv2d_i8", _via_device(_packed_dwconv2d_i8_cuda, keep=(15,)), "CPU")
 
 
 # --------------------------------------------------------------------------------------------- fake / meta impls
@@ -1630,6 +1749,16 @@ def _(x_codes, x_zero_point, codes, kind, out_channels, kernel_size, stride, dil
     if channels_last:
         return x_codes.new_empty((N, Ho, Wo, out_channels), dtype=torch.float32).permute(0, 3, 1, 2)
     return x_codes.new_empty((N, out_channels, Ho, Wo), dtype=torch.float32)
+
+
+@torch.library.register_fake("mctq::packed_dwconv2d_i8")
+def _(x, x_scale, x_zero_point, x_qmin, x_qmax, codes, kind, is_signed, out_channels, kernel_size, stride, dilation, padding,
+      zero_point, factor, lut_values, bias, channels_last):
+    N, _, H, W = x.shape
+    Ho, Wo = conv_output_hw(H, W, kernel_size, stride, dilation, padding)
+    if channels_last:
+        return x.new_empty((N, Ho, Wo, out_channels)).permute(0, 3, 1, 2)
+    return x.new_empty((N, out_channels, Ho, Wo))
 
 
 # --------------------------------------------------------------------------------------------- whole-model launch

@@ -46,6 +46,12 @@ operand is gathered from each output pixel's window (csrc/mctq_packed_igemm.cu, 
 Q's zero-point code and contributes exactly 0.  The output has the memory format F.conv2d gives for x and the rebuilt
 weight.  Inputs that are not 4-D (unbatched 3-D inputs included) take the packed path.
 
+Integer depthwise convolution (`integer_depthwise=True` together with integer_conv=True; opt-in): integer convolution mode
+for Conv2d layers with groups == in_channels > 1 and any channel multiplier, such as the 3x3 depthwise convs of MobileNetV2.
+A depthwise conv is a stencil, not a matrix product: one kernel (csrc/mctq_affine.cu, mctq_packed_dwconv2d_i8) reads the
+float x once, computes Q's codes in registers and sums (qx - zx) * (qw - zw) exactly in int32 over each window (include/mctq.h
+gives the formula).  With integer_lut=True it takes LUT weights too.
+
 Integer modes for LUT weights (`integer_lut=True` together with integer_linear=True and / or integer_conv=True; opt-in): a
 LUT weight rebuilds as fl32(lut_k / 2^(bw-1) * thr[o]) with integer centroids lut_k, i.e. an int8 code lut_k times the scale
 sw[o] = thr[o] * 2^-(bw-1) and zero point 0.  When every centroid is an integer in [-128, 127] and every sw[o] is exact and
@@ -289,10 +295,9 @@ def _input_quantizer_eligibility(input_quantizer) -> Tuple[bool, str]:
     return True, ""
 
 
-def _lut_eligibility(e, K, what, x_signed) -> Tuple[bool, str]:
-    """The conditions the integer modes put on a LUT weight (entry e, row length K named `what`): integer centroids in
-    [-128, 127], every thr[o] * 2^-(bw-1) exact and normal in f32, K a multiple of 32 (4-bit indices) or 16 (8-bit
-    indices) and at most the int32 bound of signed weight codes.  Host-only: reads the quantizer's numpy parameters."""
+def _lut_code_eligibility(e) -> Tuple[bool, str]:
+    """The conditions every integer mode puts on a LUT weight (entry e): integer centroids in [-128, 127] and every
+    thr[o] * 2^-(bw-1) exact and normal in f32.  Host-only: reads the quantizer's numpy parameters."""
     q = e.quantizer
     v = np.asarray(q._lut_values_np, dtype=np.float64).reshape(-1)
     if not (np.all(v == np.round(v)) and np.all(v >= -128) and np.all(v <= 127)):
@@ -301,6 +306,15 @@ def _lut_eligibility(e, K, what, x_signed) -> Tuple[bool, str]:
     if not (np.all(np.isfinite(sw)) and np.all(sw.astype(np.float32) == sw) and
             np.all(np.abs(sw) >= np.finfo(np.float32).tiny)):
         return False, "a threshold times 2^-(lut_values_bitwidth - 1) is not exact and normal in float32"
+    return True, ""
+
+
+def _lut_eligibility(e, K, what, x_signed) -> Tuple[bool, str]:
+    """The conditions the GEMM integer modes put on a LUT weight (entry e, row length K named `what`): _lut_code_eligibility,
+    K a multiple of 32 (4-bit indices) or 16 (8-bit indices) and at most the int32 bound of signed weight codes."""
+    ok, reason = _lut_code_eligibility(e)
+    if not ok:
+        return ok, reason
     step, bits = (32, 4) if e.kind == _native.PACK_LUT_I4 else (16, 8)
     if K % step:
         return False, f"{what} = {K} is not a multiple of {step} ({bits}-bit LUT indices)"
@@ -338,13 +352,9 @@ def integer_linear_eligibility(wrapper, input_quantizer, lut: bool = False) -> T
     return True, ""
 
 
-def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
-    """(True, '') when `wrapper` can run in integer convolution mode with input quantizer `input_quantizer`: a
-    torch.nn.Conv2d layer with string-attribute weights, no extra call arguments and 'weight' its only quantized weight,
-    packed as int8 / int4 affine codes, rebuilt as a contiguous or channels_last [Cout, Cin, kh, kw] weight with parameters
-    per tensor or per output channel; groups 1 and zero padding; the input quantizer conditions of integer linear mode;
-    Cin a multiple of 16, K = Cin * kh * kw a multiple of 32 for int4 codes and at most the int32 bound of the code
-    signedness pair.  `lut=True` also accepts LUT weights that meet _lut_eligibility.  Host-only."""
+def _conv_eligibility(wrapper, input_quantizer, lut, depthwise):
+    """The checks integer convolution mode makes on a Conv2d wrapper, in their order (depthwise: one input channel per
+    group instead of groups 1): (True, '', entry, weight shape, is_lut) or (False, reason)."""
     d = wrapper.__dict__
     if not d.get('is_str_attr', False):
         return False, "the weights are positional inputs of a functional op"
@@ -355,7 +365,13 @@ def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tup
         return False, "the wrapper passes extra call arguments to the layer"
     if list(wrapper.weights_quantizers) != ['weight']:
         return False, "the wrapper quantizes weights other than 'weight'"
-    if layer.groups != 1:
+    if depthwise:
+        if layer.groups == 1:
+            return False, "groups = 1: not a depthwise convolution"
+        if layer.groups != layer.in_channels:
+            return False, (f"groups = {layer.groups}: a grouped convolution with {layer.in_channels // layer.groups} input "
+                           f"channels per group is not depthwise")
+    elif layer.groups != 1:
         return False, f"groups = {layer.groups}: a grouped or depthwise convolution is not one matrix product"
     if layer.padding_mode != 'zeros':
         return False, f"padding_mode = {layer.padding_mode!r}: only zero padding is a padding with Q's zero-point code"
@@ -366,16 +382,32 @@ def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tup
     is_lut = lut and e.kind in _native.PACK_LUT_KINDS
     if e.kind not in (_native.PACK_AFFINE_I8, _native.PACK_AFFINE_I4) and not is_lut:
         return False, f"the weight is packed as {_KIND_NAMES[e.kind]}, not as int8 / int4 affine codes"
-    shape = (layer.out_channels, layer.in_channels) + tuple(layer.kernel_size)
+    shape = (layer.out_channels, layer.in_channels // layer.groups) + tuple(layer.kernel_size)
     dense = torch.empty(shape, device="meta")
     if e.shape_out != shape or e.stride_out not in (dense.stride(), dense.to(memory_format=torch.channels_last).stride()):
-        return False, "the rebuilt weight is not a contiguous or channels_last [Cout, Cin, kh, kw] tensor"
+        return False, (f"the rebuilt weight is not a contiguous or channels_last [Cout, {'1' if depthwise else 'Cin'}, kh, kw] "
+                       f"tensor")
     K = shape[1] * shape[2] * shape[3]
     if not (e.C == 1 or (e.C == shape[0] and e.inner == K)):
         return False, "the parameters are not per tensor or per output channel (channel_axis 0)"
     ok, reason = _input_quantizer_eligibility(input_quantizer)
     if not ok:
         return ok, reason
+    return True, "", e, shape, is_lut
+
+
+def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
+    """(True, '') when `wrapper` can run in integer convolution mode with input quantizer `input_quantizer`: a
+    torch.nn.Conv2d layer with string-attribute weights, no extra call arguments and 'weight' its only quantized weight,
+    packed as int8 / int4 affine codes, rebuilt as a contiguous or channels_last [Cout, Cin, kh, kw] weight with parameters
+    per tensor or per output channel; groups 1 and zero padding; the input quantizer conditions of integer linear mode;
+    Cin a multiple of 16, K = Cin * kh * kw a multiple of 32 for int4 codes and at most the int32 bound of the code
+    signedness pair.  `lut=True` also accepts LUT weights that meet _lut_eligibility.  Host-only."""
+    r = _conv_eligibility(wrapper, input_quantizer, lut, depthwise=False)
+    if not r[0]:
+        return r
+    _, _, e, shape, is_lut = r
+    K = shape[1] * shape[2] * shape[3]
     if shape[1] % 16:
         return False, f"in_channels = {shape[1]} is not a multiple of 16"
     if is_lut:
@@ -385,6 +417,26 @@ def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tup
     bound = _native.integer_linear_max_k(e.is_signed, int(input_quantizer.min_quantized_domain) < 0)
     if K > bound:
         return False, f"Cin * kh * kw = {K} exceeds {bound}, the largest row length whose int32 sum of code products cannot overflow"
+    return True, ""
+
+
+def integer_depthwise_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
+    """(True, '') when `wrapper` can run in integer convolution mode as a depthwise convolution (mctq_packed_dwconv2d_i8):
+    the layer, wrapper and input-quantizer conditions of integer_conv_eligibility, with groups == in_channels > 1 (any
+    channel multiplier) instead of groups 1, a contiguous or channels_last [Cout, 1, kh, kw] weight, and kh * kw at most
+    33025 (the int32 bound of the centred sum: each factor has magnitude <= 255).  `lut=True` also accepts LUT weights that
+    meet _lut_code_eligibility.  Host-only."""
+    r = _conv_eligibility(wrapper, input_quantizer, lut, depthwise=True)
+    if not r[0]:
+        return r
+    _, _, e, shape, is_lut = r
+    if is_lut:
+        ok, reason = _lut_code_eligibility(e)
+        if not ok:
+            return ok, reason
+    K = shape[2] * shape[3]
+    if K > 33025:
+        return False, f"kh * kw = {K} exceeds 33025, the largest window whose int32 sum of code products cannot overflow"
     return True, ""
 
 
@@ -507,7 +559,8 @@ class PackedState:
         return lin[1](x, bias)
 
     def integer_forward(self, wrapper, x):
-        """layer(Q(x)) in integer arithmetic (ops.IntegerLinear, or ops.IntegerConv2d for a Conv2d layer), or None when this
+        """layer(Q(x)) in integer arithmetic (ops.IntegerLinear, or ops.IntegerConv2d / ops.IntegerDepthwiseConv2d for a
+        Conv2d layer), or None when this
         call must take the packed path of the wrapper's other modes: the conditions of fused_forward, without its row limit;
         a Conv2d layer also needs a 4-D x."""
         e = self.entries[0]
@@ -544,7 +597,12 @@ class PackedState:
             if e.kind in _native.PACK_LUT_KINDS:         # codes lut_k, scale thr * 2^-(bw-1) (exact: _lut_eligibility)
                 wq = e.quantizer
                 scale, lut = scale * 2.0 ** -(int(wq.lut_values_bitwidth) - 1), wq._lut_values_np
-            if conv:
+            if conv and layer.groups > 1:              # switched by integer_depthwise_eligibility
+                launch = ops.IntegerDepthwiseConv2d(codes, e.kind, e.is_signed, e.dtype_out, layer.out_channels,
+                                                    layer.in_channels, layer.kernel_size, e.stride_out, layer.stride,
+                                                    layer.dilation, ops.conv_padding(layer), scale, zps, x_scale, x_zp, qmin,
+                                                    qmax, lut)
+            elif conv:
                 launch = ops.IntegerConv2d(codes, e.kind, e.is_signed, e.dtype_out, layer.out_channels, layer.in_channels,
                                            layer.kernel_size, e.stride_out, layer.stride, layer.dilation,
                                            ops.conv_padding(layer), scale, zps, x_scale, x_zp, qmin, qmax, lut)
@@ -582,7 +640,8 @@ class PackedState:
 
 
 def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bool = False, integer_linear: bool = False,
-                         input_quantizer=None, integer_conv: bool = False, integer_lut: bool = False) -> Dict:
+                         input_quantizer=None, integer_conv: bool = False, integer_lut: bool = False,
+                         integer_depthwise: bool = False) -> Dict:
     """Pack every weight of `wrapper` that can be packed (see the module docstring).  Returns
     {name: {'packed': bool, 'kind': str | None, 'reason': str, 'code_bytes': int, 'float_bytes': int}}.
     `fused_linear=True` also switches the wrapper to fused linear mode when fused_linear_eligibility allows it (on a wrapper
@@ -594,10 +653,13 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
     'integer': bool, 'integer_reason': str and 'input_holder' (the holder's module name for pack_model_weights, else None).
     `integer_conv=True` (needs `input_quantizer` too) does the same for integer convolution mode (integer_conv_eligibility),
     and every report entry gains 'integer_conv': bool, 'integer_conv_reason': str and 'input_holder'.
-    `integer_lut=True` (needs integer_linear=True and / or integer_conv=True) extends those modes to LUT weights."""
+    `integer_lut=True` (needs integer_linear=True and / or integer_conv=True) extends those modes to LUT weights.
+    `integer_depthwise=True` (needs integer_conv=True) extends integer convolution mode to depthwise Conv2d layers
+    (integer_depthwise_eligibility); their report entries keep the keys 'integer_conv' and 'integer_conv_reason'."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     _check_integer_lut(integer_lut, integer_linear, integer_conv)
+    _check_integer_depthwise(integer_depthwise, integer_conv)
     if integer_linear and input_quantizer is None:
         raise ValueError("integer_linear=True needs the input_quantizer of the activation holder that feeds the wrapper")
     if integer_conv and input_quantizer is None:
@@ -634,7 +696,7 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
     if integer_linear:
         _switch_to_integer(wrapper, report, input_quantizer, None, lut=integer_lut)
     if integer_conv:
-        _switch_to_integer(wrapper, report, input_quantizer, None, conv=True, lut=integer_lut)
+        _switch_to_integer(wrapper, report, input_quantizer, None, conv=True, lut=integer_lut, depthwise=integer_depthwise)
     return report
 
 
@@ -642,6 +704,12 @@ def _check_integer_lut(integer_lut, integer_linear, integer_conv):
     if integer_lut and not (integer_linear or integer_conv):
         raise ValueError("integer_lut=True needs integer_linear=True and / or integer_conv=True (it extends those modes to "
                          "LUT weights)")
+
+
+def _check_integer_depthwise(integer_depthwise, integer_conv):
+    if integer_depthwise and not integer_conv:
+        raise ValueError("integer_depthwise=True needs integer_conv=True (it extends integer convolution mode to depthwise "
+                         "Conv2d layers)")
 
 
 def _drop_float_weights(wrapper, new, entries, keep):
@@ -685,8 +753,11 @@ def _switch_to_batched(wrapper, report):
         r['batched'], r['batched_reason'] = ok, reason
 
 
-def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None, conv=False, lut=False):
+def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None, conv=False, lut=False, depthwise=False):
     eligibility = integer_conv_eligibility if conv else integer_linear_eligibility
+    layer = wrapper.__dict__['_modules'].get(LAYER)
+    if conv and depthwise and type(layer) is torch.nn.Conv2d and layer.groups > 1:
+        eligibility = integer_depthwise_eligibility
     ok, why = (False, reason) if reason else eligibility(wrapper, input_quantizer, lut=lut)
     state = wrapper.__dict__.get('_packed')
     if ok:
@@ -710,16 +781,19 @@ def _bits(t):
 
 
 def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batched_linear: bool = False,
-                       integer_linear: bool = False, integer_conv: bool = False, integer_lut: bool = False) -> Dict[str, Dict]:
+                       integer_linear: bool = False, integer_conv: bool = False, integer_lut: bool = False,
+                       integer_depthwise: bool = False) -> Dict[str, Dict]:
     """pack_weights(fused_linear, batched_linear) on every PytorchQuantizationWrapper of `model`: {wrapper module name:
     {weight name: report entry}}.  `integer_linear=True` then switches, in place, every eligible wrapper whose input is the
     output of an activation quantization holder (integer_linear_edges) to integer linear mode; every report entry gains
     'integer', 'integer_reason' and 'input_holder'.  `integer_conv=True` does the same for integer convolution mode on the
     same edges; every report entry gains 'integer_conv', 'integer_conv_reason' and 'input_holder'.  `integer_lut=True` extends
-    both to LUT weights.  When the model cannot be traced nothing is switched and the reason is reported."""
+    both to LUT weights, and `integer_depthwise=True` extends integer convolution mode to depthwise Conv2d layers.  When the
+    model cannot be traced nothing is switched and the reason is reported."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     _check_integer_lut(integer_lut, integer_linear, integer_conv)
+    _check_integer_depthwise(integer_depthwise, integer_conv)
     from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
     wrappers = {mod_name: mod for mod_name, mod in model.named_modules()
                 if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization}
@@ -730,5 +804,6 @@ def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batch
             holder, q = edges.get(name, (None, None)) if name not in why else (None, None)
             reason = failure or why.get(name) or ("" if holder else "the wrapper is not called in the traced forward")
             for conv in (False, True) if integer_linear and integer_conv else (integer_conv,):
-                _switch_to_integer(mod, reports[name], q, holder, None if holder else reason, conv=conv, lut=integer_lut)
+                _switch_to_integer(mod, reports[name], q, holder, None if holder else reason, conv=conv, lut=integer_lut,
+                                   depthwise=integer_depthwise)
     return reports
