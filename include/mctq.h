@@ -331,6 +331,45 @@ int mctq_packed_dwconv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, in
                             int x_nhwc, float x_scale, int32_t x_zero_point, int32_t x_qmin, int32_t x_qmax,
                             const float* factor, const void* bias, void* y, const int8_t* lut_codes_host, void* stream);
 
+/* Integer modes for row lengths and channel counts off the GEMM's granule (DESIGN.md §7f).  The padding contract: every
+ * column the kernel sums beyond the real K belongs to one of two classes --
+ *   channel pad  the x code is zx (in the image and, as before, for taps outside it); the column is counted in K, Sx and
+ *                Sw; its weight code may be anything (a LUT table needs no zero centroid)
+ *   row tail     the x code is 0 and the column is counted in none of K, Sx and Sw (the GEMM's "columns >= K are zero")
+ * A channel pad contributes (zx - zx) * (qw - zw) = 0 to the centred sum, so c, and every output bit, is the formula of
+ * mctq_packed_linear_i8 / mctq_packed_conv2d_i8 / their LUT forms over the real row.
+ *
+ * mctq_quantize_rows_i8_padded: mctq_quantize_rows_i8 writing qx [M][ldc] (ldc >= K, ldc % 4 == 0, codes 4-byte aligned),
+ * columns [K, ldc) holding zp; Sx[n] includes them.  MCTQ_E_BADARG also for ldc < K or ldc % 4 != 0, MCTQ_E_RANGE for zp
+ * outside [qmin, qmax].
+ * mctq_quantize_nhwc_i8_padded: mctq_quantize_nhwc_i8 writing qx [N][H*W][Cp] (Cp = 4, 8 or a multiple of 16, Cp >= C, codes
+ * 16-byte aligned), channels [C, Cp) holding zp; P includes them.  One pixel per thread, whole 4 / 8 / 16-byte stores.
+ * MCTQ_E_BADARG also for a Cp outside that set, MCTQ_E_RANGE for zp outside [qmin, qmax].
+ *
+ * mctq_packed_linear_i8_padded: mctq_packed_linear_i8 (lut_codes_host NULL) or mctq_packed_linear_i8_lut (a table) over
+ * x codes [M][ldc] whose columns [in_features, ldc) are channel pads: w is the [out][ldc] weight, Sw sums its ldc columns,
+ * and the correction counts K = ldc.  MCTQ_E_BADARG also for in_features < 1, ldc < in_features, ldc not a multiple of 16
+ * (32 for 4-bit codes) or a table present / absent against the kind; MCTQ_E_RANGE for ldc above the int32 bound.
+ * mctq_packed_conv2d_i8_padded: mctq_packed_conv2d_i8 / _lut over NHWC codes [N][H][W][Cp] whose channels [g->Cin, Cp) are
+ * channel pads (g->Cin is the real channel count).  Sx counts Cp * zx for a tap outside the image.
+ *   Cp % 16 == 0   w is [Cout][kh*kw*Cp] in (r, s, c) order, c < Cp; K = kh*kw*Cp (a multiple of 32 for 4-bit codes)
+ *   Cp = 4 / 8     the narrow gather: w is [Cout][K] with K = kh*kw*Cp rounded up to 16 (32 for 4-bit codes); its first
+ *                  kh*kw*Cp columns are (r, s, c) with c < Cp, the rest a row tail; the correction counts kh*kw*Cp
+ * Sw[o] sums the counted columns.  MCTQ_E_BADARG also for Cp < g->Cin or Cp outside {4, 8, 16, 32, ...}; every other
+ * return as for mctq_packed_conv2d_i8, the int32 bound applying to the kernel's row length K. */
+int mctq_quantize_rows_i8_padded(const void* x, int x_dtype, int64_t M, int64_t K, int64_t ldc, float scale, int32_t zp,
+                                 int32_t qmin, int32_t qmax, void* codes, int32_t* rowsum, void* stream);
+int mctq_quantize_nhwc_i8_padded(const void* x, int x_dtype, int64_t N, int64_t C, int64_t H, int64_t W, int64_t Cp,
+                                 float scale, int32_t zp, int32_t qmin, int32_t qmax, void* codes, int32_t* P, void* stream);
+int mctq_packed_linear_i8_padded(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, int64_t ldc,
+                                 const void* x_codes, int x_signed, int32_t x_zero_point, int64_t M, const int32_t* x_rowsum,
+                                 const int32_t* w_rowsum, const float* factor, const void* bias, int y_dtype, void* y,
+                                 int64_t ldy, const int8_t* lut_codes_host, void* stream);
+int mctq_packed_conv2d_i8_padded(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cp, int64_t Cout,
+                                 const void* x_codes, int x_signed, int32_t x_zero_point, const int32_t* x_rowsum,
+                                 const int32_t* w_rowsum, const float* factor, const void* bias, int y_dtype, void* y,
+                                 int y_nchw, const int8_t* lut_codes_host, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Whole-model weight quantisation: one launch over a table of tensors (SURVEY 8f rank 1).
  * Replaces the per-layer loop  for name, w, quantizer in self._weights_vars: quantizer(w)

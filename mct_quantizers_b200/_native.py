@@ -99,6 +99,14 @@ SIGNATURES = {
                                           c_int, c_vp, c_vp]),
     "mctq_packed_dwconv2d_i8": (c_int, [c_vp, c_vp, c_i64, c_vp, c_int, c_int, c_f32, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp,
                                         c_vp, c_vp]),
+    "mctq_quantize_rows_i8_padded": (c_int, [c_vp, c_int, c_i64, c_i64, c_i64, c_f32, c_i32, c_i32, c_i32, c_vp, c_vp,
+                                             c_vp]),
+    "mctq_quantize_nhwc_i8_padded": (c_int, [c_vp, c_int, c_i64, c_i64, c_i64, c_i64, c_i64, c_f32, c_i32, c_i32, c_i32,
+                                             c_vp, c_vp, c_vp]),
+    "mctq_packed_linear_i8_padded": (c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_int, c_i32, c_i64, c_vp, c_vp, c_vp, c_vp,
+                                             c_int, c_vp, c_i64, c_vp, c_vp]),
+    "mctq_packed_conv2d_i8_padded": (c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_int, c_i32, c_vp, c_vp, c_vp, c_vp, c_int,
+                                             c_vp, c_int, c_vp, c_vp]),
     "mctq_multi_tile_elems": (c_i64, []),
     "mctq_multi_plan": (c_i64, [c_vp, c_int, c_vp]),
     "mctq_fq_affine_multi": (c_int, [c_vp, c_vp, c_int, c_i64, c_vp]),

@@ -734,6 +734,91 @@ __global__ void __launch_bounds__(kThreads) quantize_nhwc_kernel(const T* __rest
     }
 }
 
+// ---- padded codes (integer modes for row lengths and channel counts off the GEMM's granule, DESIGN §7f): the recipe of
+// quantize_rows_kernel, the pad columns / channels holding the code of zx and counted in the sums.
+// Rows: qx [M][ldc] of x [M][K], ldc % 4 == 0.  G lanes (a power of two <= 32) share a row, each writing whole 32-bit
+// words, so that short rows (a channels_last stem: K = 3, ldc = 4) still give one row per thread and coalesced stores.
+template <typename T>
+__global__ void __launch_bounds__(kThreads) quantize_rows_pad_kernel(const T* __restrict__ x, uint8_t* __restrict__ codes,
+                                                                      int32_t* __restrict__ rowsum, int64_t M, int64_t K,
+                                                                      int64_t ldc, int G, float scale, int32_t zp,
+                                                                      int32_t qmin, int32_t qmax) {
+    using Op = AffineOp<false>;
+    AffineArgs a;                                   // only the fields AffineOp::make reads
+    a.qmin = qmin;
+    a.qmax = qmax;
+    const Op::ChanParams p = Op::make(scale, zp, a);
+    pdl_wait();
+    pdl_launch_dependents();
+    const int sub = threadIdx.x & (G - 1);
+    const int64_t per_cta = kThreads / G, words = ldc / 4;
+    // the row loop is uniform across the CTA: every lane reaches the shuffles
+    for (int64_t base = (int64_t)blockIdx.x * per_cta; base < M; base += (int64_t)gridDim.x * per_cta) {
+        const int64_t row = base + threadIdx.x / G;
+        int32_t sum = 0;
+        if (row < M) {
+            const T* xr = x + row * K;
+            uint32_t* cr = reinterpret_cast<uint32_t*>(codes + row * ldc);
+            for (int64_t w = sub; w < words; w += G) {
+                uint32_t word = 0;
+#pragma unroll
+                for (int e = 0; e < 4; ++e) {
+                    int c = zp;
+                    if (4 * w + e < K) Op::template apply<true>(to_f32<T>(xr[4 * w + e]), p, c);
+                    sum += c;
+                    word |= (uint32_t)(c & 0xff) << (8 * e);
+                }
+                cr[w] = word;
+            }
+        }
+        if (rowsum) {
+            for (int d = G >> 1; d > 0; d >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, d);
+            if (row < M && sub == 0) rowsum[row] = sum;
+        }
+    }
+}
+
+// NHWC codes with a channel pitch Cp of an NCHW x [N][C][HW]: one pixel per thread, V codes per store (V = Cp for Cp 4 / 8,
+// else 16: Cp % 16 == 0).  Each channel's load runs along HW across the warp and each store along the pixels, so both
+// sides stay coalesced for tiny C; P[pixel] is the sum over all Cp codes.
+template <typename T, int V>
+__global__ void __launch_bounds__(kThreads) quantize_nhwc_pad_kernel(const T* __restrict__ x, uint8_t* __restrict__ codes,
+                                                                      int32_t* __restrict__ psum, int64_t N, int64_t C,
+                                                                      int64_t HW, int64_t Cp, float scale, int32_t zp,
+                                                                      int32_t qmin, int32_t qmax) {
+    using Op = AffineOp<false>;
+    AffineArgs a;                                   // only the fields AffineOp::make reads
+    a.qmin = qmin;
+    a.qmax = qmax;
+    const Op::ChanParams p = Op::make(scale, zp, a);
+    pdl_wait();
+    pdl_launch_dependents();
+    const int64_t ptiles = (HW + kThreads - 1) / kThreads;
+    for (int64_t t = blockIdx.x; t < N * ptiles; t += gridDim.x) {
+        const int64_t b = t / ptiles, px = (t - b * ptiles) * kThreads + threadIdx.x;
+        if (px >= HW) continue;
+        const T* xp = x + b * C * HW + px;
+        uint8_t* cp = codes + (b * HW + px) * Cp;
+        int32_t sum = 0;
+        for (int64_t c0 = 0; c0 < Cp; c0 += V) {
+            uint32_t w[V / 4];
+#pragma unroll
+            for (int i = 0; i < V / 4; ++i) w[i] = 0;
+#pragma unroll
+            for (int e = 0; e < V; ++e) {
+                int q = zp;
+                if (c0 + e < C) Op::template apply<true>(to_f32<T>(xp[(c0 + e) * HW]), p, q);
+                sum += q;
+                w[e / 4] |= (uint32_t)(q & 0xff) << (8 * (e % 4));
+            }
+            if constexpr (V == 4) *reinterpret_cast<uint32_t*>(cp + c0) = w[0];
+            else if constexpr (V == 8) *reinterpret_cast<uint2*>(cp + c0) = make_uint2(w[0], w[1]);
+            else *reinterpret_cast<uint4*>(cp + c0) = make_uint4(w[0], w[1], w[2], w[3]);
+        }
+        if (psum) psum[b * HW + px] = sum;
+    }
+}
+
 // ---- depthwise convolution of Q's codes (integer convolution mode, mctq_packed_dwconv2d_i8): x is read once as floats and
 // quantized in registers by the recipe of quantize_rows_kernel; only qx - zx reaches shared memory (0 for taps outside the
 // image), and the centred sum needs neither Sx nor Sw.  A work unit is S "slots" times a TH x TW tile of output pixels:
@@ -1161,6 +1246,56 @@ int mctq_quantize_nhwc_i8(const void* x, int x_dtype, int64_t N, int64_t C, int6
         using T = typename decltype(type)::type;
         return launch_streaming(quantize_nhwc_kernel<T>, (unsigned)blocks, 0, st, reinterpret_cast<const T*>(x),
                                 reinterpret_cast<uint8_t*>(codes), P, N, C, HW, scale, zp, qmin, qmax);
+    };
+    if (x_dtype == MCTQ_F32) return run(PackType<float>{});
+    if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});
+    return run(PackType<__half>{});
+}
+
+int mctq_quantize_rows_i8_padded(const void* x, int x_dtype, int64_t M, int64_t K, int64_t ldc, float scale, int32_t zp,
+                                 int32_t qmin, int32_t qmax, void* codes, int32_t* rowsum, void* stream) {
+    MCTQ_NVTX("mctq_quantize_rows_i8_padded");
+    if (!x || !codes || M < 0 || K < 1 || ldc < K || ldc % 4 != 0 || (reinterpret_cast<uintptr_t>(codes) & 3u) != 0)
+        return MCTQ_E_BADARG;
+    if (x_dtype != MCTQ_F32 && x_dtype != MCTQ_BF16 && x_dtype != MCTQ_F16) return MCTQ_E_DTYPE;
+    if (qmin > qmax) return MCTQ_E_RANGE;
+    if (int rc = check_codes(qmin, qmax, MCTQ_CODES_INT8, codes)) return rc;
+    if (zp < qmin || zp > qmax) return MCTQ_E_RANGE;             // the pad columns hold zp as a code
+    if (M == 0) return 0;
+    int G = 1;
+    while (G < 32 && 4 * G < ldc) G *= 2;
+    const int64_t blocks = std::min<int64_t>((M + kThreads / G - 1) / (kThreads / G), 148 * 16);
+    cudaStream_t st = (cudaStream_t)stream;
+    auto run = [&](auto type) {
+        using T = typename decltype(type)::type;
+        return launch_streaming(quantize_rows_pad_kernel<T>, (unsigned)blocks, 0, st, reinterpret_cast<const T*>(x),
+                                reinterpret_cast<uint8_t*>(codes), rowsum, M, K, ldc, G, scale, zp, qmin, qmax);
+    };
+    if (x_dtype == MCTQ_F32) return run(PackType<float>{});
+    if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});
+    return run(PackType<__half>{});
+}
+
+int mctq_quantize_nhwc_i8_padded(const void* x, int x_dtype, int64_t N, int64_t C, int64_t H, int64_t W, int64_t Cp,
+                                 float scale, int32_t zp, int32_t qmin, int32_t qmax, void* codes, int32_t* P, void* stream) {
+    MCTQ_NVTX("mctq_quantize_nhwc_i8_padded");
+    if (!x || !codes || N < 0 || C < 1 || H < 1 || W < 1 || Cp < C || !aligned16(codes)) return MCTQ_E_BADARG;
+    if (Cp != 4 && Cp != 8 && Cp % 16 != 0) return MCTQ_E_BADARG;
+    if (x_dtype != MCTQ_F32 && x_dtype != MCTQ_BF16 && x_dtype != MCTQ_F16) return MCTQ_E_DTYPE;
+    if (qmin > qmax) return MCTQ_E_RANGE;
+    if (int rc = check_codes(qmin, qmax, MCTQ_CODES_INT8, codes)) return rc;
+    if (zp < qmin || zp > qmax) return MCTQ_E_RANGE;
+    if (N == 0) return 0;
+    const int64_t HW = H * W;
+    const int64_t blocks = std::min<int64_t>(N * ((HW + kThreads - 1) / kThreads), 148 * 16);
+    cudaStream_t st = (cudaStream_t)stream;
+    auto run = [&](auto type) {
+        using T = typename decltype(type)::type;
+        const T* xt = reinterpret_cast<const T*>(x);
+        uint8_t* c = reinterpret_cast<uint8_t*>(codes);
+        if (Cp == 4) return launch_streaming(quantize_nhwc_pad_kernel<T, 4>, (unsigned)blocks, 0, st, xt, c, P, N, C, HW, Cp, scale, zp, qmin, qmax);
+        if (Cp == 8) return launch_streaming(quantize_nhwc_pad_kernel<T, 8>, (unsigned)blocks, 0, st, xt, c, P, N, C, HW, Cp, scale, zp, qmin, qmax);
+        return launch_streaming(quantize_nhwc_pad_kernel<T, 16>, (unsigned)blocks, 0, st, xt, c, P, N, C, HW, Cp, scale, zp, qmin, qmax);
     };
     if (x_dtype == MCTQ_F32) return run(PackType<float>{});
     if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});

@@ -25,6 +25,12 @@
 // cp.async (a tap outside the image is a splat of zx, rows >= M and columns >= K are zero).  The copies of kIConvAhead
 // stages stay in flight (cp.async groups); a stage's full barrier gets the producers' arrivals once its group has landed.
 // The epilogue writes row-major [M][Cout] (NHWC) or NCHW planes.
+//
+// Padded codes (mctq_packed_conv2d_i8_padded, DESIGN §7f): the NHWC codes have a pixel pitch Cp >= Cin whose pad channels
+// hold zx.  Cp % 16 == 0 is the gather above with Cin := Cp.  Cp = 4 / 8 (packed_iconv_narrow_kernel) is the narrow gather:
+// a 16-byte granule holds 16 / Cp consecutive taps, each one cp.async of Cp bytes (a tap outside the image is a Cp-byte
+// store of zx); the row length is kh * kw * Cp rounded up to 16 (32 for 4-bit codes), and taps at or beyond kh * kw form
+// a row tail of zero codes that the correction does not count.
 #include <cuda.h>               // CUtensorMap and the cuTensorMapEncodeTiled types (the entry point is fetched at run time)
 
 #include <algorithm>
@@ -75,6 +81,17 @@ constexpr uint32_t kLut8TableBytes = 256 * 32;   // the table of 8-bit indices, 
 
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" :: "r"(dst), "l"(src) : "memory");
+}
+
+// the Cp = 4 / 8 bytes of one tap of the narrow gather, and its splat of zx (or zeros)
+template <int N>
+__device__ __forceinline__ void cp_async_n(uint32_t dst, const void* src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" :: "r"(dst), "l"(src), "n"(N) : "memory");
+}
+template <int N>
+__device__ __forceinline__ void st_shared_n(uint32_t addr, uint32_t v) {
+    if constexpr (N == 4) asm volatile("st.shared.b32 [%0], %1;" :: "r"(addr), "r"(v) : "memory");
+    else asm volatile("st.shared.v2.b32 [%0], {%1,%2};" :: "r"(addr), "r"(v), "r"(v) : "memory");
 }
 
 __device__ __forceinline__ void tma_2d(const CUtensorMap* map, uint32_t dst, int32_t c0, int32_t c1, uint64_t* bar) {
@@ -174,7 +191,7 @@ __device__ __forceinline__ void store_w(uint32_t st, uint32_t row, const uint4* 
     else store_w4<WSIGNED>(st, row, v);
 }
 
-template <WFmt F, bool WSIGNED, typename T, bool CONV>
+template <WFmt F, bool WSIGNED, typename T, bool CONV, int CP = 0>
 __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
     constexpr bool INT4 = producer_written(F);     // the producers write the weight operand (int4 codes, LUT indices)
     extern __shared__ __align__(1024) uint8_t dsm[];
@@ -254,6 +271,27 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
 #pragma unroll
                 for (int j = 0; j < kIChunk / 16; ++j) {
                     const int32_t k = c * kIChunk + 16 * j;
+                    if constexpr (CP != 0) {                 // narrow gather: taps k / CP .. k / CP + 16 / CP - 1
+#pragma unroll
+                        for (int u = 0; u < 16 / CP; ++u) {
+                            const uint32_t tap = (uint32_t)(k / CP + u);
+                            const bool in_k = tap < (uint32_t)(g.kh * g.kw);
+                            const uint32_t rr = fdiv_u32(tap, a.div_kw), ss = tap - rr * (uint32_t)g.kw;
+                            const int32_t dy = (int32_t)rr * g.dh, dx = (int32_t)ss * g.dw;
+#pragma unroll
+                            for (int q = 0; q < 2; ++q) {
+                                if (!have_row[q]) continue;
+                                const uint32_t dst =
+                                    st + a_bytes + sw128_off((uint32_t)(tid + kIProducers * q), (uint32_t)j) + CP * u;
+                                const int32_t ih = ih0[q] + dy, iw = iw0[q] + dx;
+                                if (live[q] && in_k && ih >= 0 && ih < g.H && iw >= 0 && iw < g.W)
+                                    cp_async_n<CP>(dst, img[q] + ((int64_t)ih * g.W + iw) * CP);
+                                else
+                                    st_shared_n<CP>(dst, live[q] && in_k ? a.zx_splat : 0u);
+                            }
+                        }
+                        continue;
+                    }
                     const bool in_k = k < K;
                     const uint32_t tap = fdiv_u32((uint32_t)k, a.div_cin), ch = (uint32_t)k - tap * (uint32_t)g.Cin;
                     const uint32_t rr = fdiv_u32(tap, a.div_kw), ss = tap - rr * (uint32_t)g.kw;
@@ -343,7 +381,9 @@ __device__ __forceinline__ void igemm_body(const IgemmArgs& a) {
         const float f = live ? __ldg(a.factor + ch) : 0.0f;
         const int32_t zw = !is_lut(F) && live ? __ldg(a.w_zp + ch) : 0;     // LUT codes: zw = 0
         const int64_t sw = live && a.w_rowsum ? (int64_t)__ldg(a.w_rowsum + o) : 0;
-        const int64_t fixed = K * (int64_t)a.x_zp * zw - (int64_t)a.x_zp * sw;     // K zx zw - zx Sw[o]
+        int64_t Kc = K;                                                    // the counted columns
+        if constexpr (CP != 0) Kc = (int64_t)a.g.kh * a.g.kw * CP;         // narrow gather: the row tail is not counted
+        const int64_t fixed = Kc * (int64_t)a.x_zp * zw - (int64_t)a.x_zp * sw;    // K zx zw - zx Sw[o]
         const float b = a.bias && live ? to_f32<T>(reinterpret_cast<const T*>(a.bias)[o]) : 0.0f;
         const int64_t g0 = a.m0 + n0;                                      // first global row of this CTA
         T* y = reinterpret_cast<T*>(a.y);
@@ -382,6 +422,11 @@ __global__ void __launch_bounds__(kThreads, 1) packed_iconv_kernel(const __grid_
     igemm_body<F, WSIGNED, T, true>(a);
 }
 
+template <WFmt F, bool WSIGNED, typename T, int CP>
+__global__ void __launch_bounds__(kThreads, 1) packed_iconv_narrow_kernel(const __grid_constant__ IgemmArgs a) {
+    igemm_body<F, WSIGNED, T, true, CP>(a);
+}
+
 }  // namespace mctq
 
 using namespace mctq;
@@ -417,9 +462,12 @@ int encode_codes(EncodeTiled fn, CUtensorMap* map, const void* base, int64_t K, 
     return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
 }
 
-template <WFmt F, bool WSIGNED, typename T, bool CONV>
+template <WFmt F, bool WSIGNED, typename T, bool CONV, int CP = 0>
 int launch_igemm(const IgemmArgs& a, int64_t M, cudaStream_t st) {
-    auto kernel = CONV ? packed_iconv_kernel<F, WSIGNED, T> : packed_igemm_kernel<F, WSIGNED, T>;
+    auto kernel = [] {
+        if constexpr (CP != 0) return packed_iconv_narrow_kernel<F, WSIGNED, T, CP>;
+        else return CONV ? packed_iconv_kernel<F, WSIGNED, T> : packed_igemm_kernel<F, WSIGNED, T>;
+    }();
     const size_t smem = tc_ring_smem(a.stages, a.stage_bytes, a.tmem_cols) + (F == WFmt::LUT8 ? kLut8TableBytes : 0);
     int rc = ensure_smem(kernel, smem);
     if (rc) return rc;
@@ -486,17 +534,17 @@ void igemm_prepare(IgemmArgs& a, const MctqPackedDesc* w, int64_t N, int64_t K, 
     a.x_zp = x_zero_point;
 }
 
-template <bool CONV>
+template <bool CONV, int CP = 0>
 int igemm_run(IgemmArgs& a, const MctqPackedDesc* w, int y_dtype, int64_t M, cudaStream_t st) {
     // LUT weights rebuild as f32 (packed_linear_check): one instantiation per index width
-    if (w->kind == MCTQ_PACK_LUT_I4) return launch_igemm<WFmt::LUT4, true, float, CONV>(a, M, st);
-    if (w->kind == MCTQ_PACK_LUT_U8) return launch_igemm<WFmt::LUT8, true, float, CONV>(a, M, st);
+    if (w->kind == MCTQ_PACK_LUT_I4) return launch_igemm<WFmt::LUT4, true, float, CONV, CP>(a, M, st);
+    if (w->kind == MCTQ_PACK_LUT_U8) return launch_igemm<WFmt::LUT8, true, float, CONV, CP>(a, M, st);
     auto typed = [&](auto fmt_tag, auto signed_tag) {
         constexpr WFmt F = decltype(fmt_tag)::value;
         constexpr bool WS = decltype(signed_tag)::value;
-        if (y_dtype == MCTQ_F32) return launch_igemm<F, WS, float, CONV>(a, M, st);
-        if (y_dtype == MCTQ_BF16) return launch_igemm<F, WS, __nv_bfloat16, CONV>(a, M, st);
-        return launch_igemm<F, WS, __half, CONV>(a, M, st);
+        if (y_dtype == MCTQ_F32) return launch_igemm<F, WS, float, CONV, CP>(a, M, st);
+        if (y_dtype == MCTQ_BF16) return launch_igemm<F, WS, __nv_bfloat16, CONV, CP>(a, M, st);
+        return launch_igemm<F, WS, __half, CONV, CP>(a, M, st);
     };
     using I4 = std::integral_constant<WFmt, WFmt::I4>;
     using True = std::true_type;
@@ -537,18 +585,20 @@ int linear_i8(const MctqPackedDesc* w, int64_t out_features, int64_t in_features
     return igemm_run<false>(a, w, y_dtype, M, (cudaStream_t)stream);
 }
 
-// mctq_packed_conv2d_i8 and mctq_packed_conv2d_i8_lut, as linear_i8
+// mctq_packed_conv2d_i8 and mctq_packed_conv2d_i8_lut, as linear_i8; narrow: the narrow gather of Cp = g->Cin = 4 / 8
 int conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x_codes, int x_signed,
               int32_t x_zero_point, const int32_t* x_rowsum, const int32_t* w_rowsum, const float* factor, const void* bias,
-              int y_dtype, void* y, int y_nchw, const int8_t* lut, void* stream) {
+              int y_dtype, void* y, int y_nchw, const int8_t* lut, void* stream, bool narrow = false) {
     if (!g) return MCTQ_E_BADARG;
     if (g->N < 0 || g->H < 1 || g->W < 1 || g->Cin < 1 || g->Ho < 1 || g->Wo < 1 || g->kh < 1 || g->kw < 1 || g->sh < 1 ||
         g->sw < 1 || g->dh < 1 || g->dw < 1 || g->pt < 0 || g->pb < 0 || g->pl < 0 || g->pr < 0 || (y_nchw != 0 && y_nchw != 1))
         return MCTQ_E_BADARG;
-    const int64_t K = (int64_t)g->Cin * g->kh * g->kw, M = (int64_t)g->N * g->Ho * g->Wo;
-    if (const int rc = packed_linear_check(w, Cout, K, x_codes, y_dtype, M, y)) return rc;
     const bool int4 = pack_is_int4(w->kind);
-    if (g->Cin % 16 != 0 || (int4 && K % 32 != 0) || M >= (1LL << 31)) return MCTQ_E_BADARG;
+    const int64_t step = int4 ? 32 : 16;                       // narrow: kh * kw * Cp and a row tail up to the granule
+    const int64_t K = narrow ? ((int64_t)g->Cin * g->kh * g->kw + step - 1) / step * step : (int64_t)g->Cin * g->kh * g->kw;
+    const int64_t M = (int64_t)g->N * g->Ho * g->Wo;
+    if (const int rc = packed_linear_check(w, Cout, K, x_codes, y_dtype, M, y)) return rc;
+    if ((!narrow && g->Cin % 16 != 0) || (int4 && K % 32 != 0) || M >= (1LL << 31)) return MCTQ_E_BADARG;
     if (const int rc = igemm_check(w, lut || w->is_signed, K, x_codes, x_signed, x_zero_point, w_rowsum, factor)) return rc;
     if (M == 0) return 0;
 
@@ -569,6 +619,10 @@ int conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, co
         int rc = encode_fn(&fn);
         if (!rc) rc = encode_codes(fn, &a.tm_w, w->codes, K, Cout, kTcRows);
         if (rc) return rc;
+    }
+    if (narrow) {
+        return g->Cin == 4 ? igemm_run<true, 4>(a, w, y_dtype, M, (cudaStream_t)stream)
+                           : igemm_run<true, 8>(a, w, y_dtype, M, (cudaStream_t)stream);
     }
     return igemm_run<true>(a, w, y_dtype, M, (cudaStream_t)stream);
 }
@@ -596,6 +650,31 @@ int mctq_packed_linear_i8_lut(const MctqPackedDesc* w, int64_t out_features, int
     if (!w || !pack_is_lut(w->kind) || !lut_codes_host) return MCTQ_E_BADARG;
     return linear_i8(w, out_features, in_features, x_codes, x_signed, x_zero_point, M, x_rowsum, w_rowsum, factor, bias,
                      y_dtype, y, ldy, lut_codes_host, stream);
+}
+
+int mctq_packed_linear_i8_padded(const MctqPackedDesc* w, int64_t out_features, int64_t in_features, int64_t ldc,
+                                 const void* x_codes, int x_signed, int32_t x_zero_point, int64_t M, const int32_t* x_rowsum,
+                                 const int32_t* w_rowsum, const float* factor, const void* bias, int y_dtype, void* y,
+                                 int64_t ldy, const int8_t* lut_codes_host, void* stream) {
+    MCTQ_NVTX("mctq_packed_linear_i8_padded");
+    if (!w || pack_is_lut(w->kind) != (lut_codes_host != nullptr)) return MCTQ_E_BADARG;
+    if (in_features < 1 || ldc < in_features) return MCTQ_E_BADARG;
+    // the GEMM of mctq_packed_linear_i8 over rows of ldc columns (its checks: ldc % 16 / 32, the int32 bound on ldc)
+    return linear_i8(w, out_features, ldc, x_codes, x_signed, x_zero_point, M, x_rowsum, w_rowsum, factor, bias, y_dtype, y,
+                     ldy, lut_codes_host, stream);
+}
+
+int mctq_packed_conv2d_i8_padded(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cp, int64_t Cout,
+                                 const void* x_codes, int x_signed, int32_t x_zero_point, const int32_t* x_rowsum,
+                                 const int32_t* w_rowsum, const float* factor, const void* bias, int y_dtype, void* y,
+                                 int y_nchw, const int8_t* lut_codes_host, void* stream) {
+    MCTQ_NVTX("mctq_packed_conv2d_i8_padded");
+    if (!w || !g || pack_is_lut(w->kind) != (lut_codes_host != nullptr)) return MCTQ_E_BADARG;
+    if (g->Cin < 1 || Cp < g->Cin || Cp > (1 << 20) || (Cp != 4 && Cp != 8 && Cp % 16 != 0)) return MCTQ_E_BADARG;
+    MctqConv2dGeom gp = *g;                                    // the kernel sees Cin := Cp
+    gp.Cin = (int32_t)Cp;
+    return conv2d_i8(w, &gp, Cout, x_codes, x_signed, x_zero_point, x_rowsum, w_rowsum, factor, bias, y_dtype, y, y_nchw,
+                     lut_codes_host, stream, Cp < 16);
 }
 
 int mctq_packed_conv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, int64_t Cout, const void* x_codes, int x_signed,

@@ -66,6 +66,17 @@ _LIB.define("packed_linear_i8_lut(Tensor x_codes, int x_zero_point, Tensor codes
 _LIB.define("packed_conv2d_i8_lut(Tensor x_codes, int x_zero_point, Tensor codes, int kind, int out_channels, "
             "int[] kernel_size, int[] stride, int[] dilation, int[] padding, int[] lut_values, Tensor w_rowsum, "
             "Tensor factor, Tensor? bias, bool channels_last) -> Tensor")
+_LIB.define("quantize_rows_i8_padded(Tensor x, int ldc, float scale, int zero_point, int quant_min, int quant_max, "
+            "bool want_rowsum) -> (Tensor, Tensor)")
+_LIB.define("quantize_nhwc_i8_padded(Tensor x, int channel_pitch, float scale, int zero_point, int quant_min, int quant_max, "
+            "bool want_sums) -> (Tensor, Tensor)")
+_LIB.define("packed_linear_i8_padded(Tensor x_codes, int in_features, int x_zero_point, Tensor? x_rowsum, Tensor codes, "
+            "int kind, bool is_signed, int out_features, Tensor? zero_point, Tensor w_rowsum, Tensor factor, Tensor? bias, "
+            "ScalarType dtype, int[]? lut_values) -> Tensor")
+_LIB.define("packed_conv2d_i8_padded(Tensor x_codes, int in_channels, int x_zero_point, Tensor? x_rowsum, Tensor codes, "
+            "int kind, bool is_signed, int out_channels, int[] kernel_size, int[] stride, int[] dilation, int[] padding, "
+            "Tensor? zero_point, Tensor w_rowsum, Tensor factor, Tensor? bias, ScalarType dtype, bool channels_last, "
+            "int[]? lut_values) -> Tensor")
 _LIB.define("packed_dwconv2d_i8(Tensor x, float x_scale, int x_zero_point, int x_qmin, int x_qmax, Tensor codes, int kind, "
             "bool is_signed, int out_channels, int[] kernel_size, int[] stride, int[] dilation, int[] padding, "
             "Tensor? zero_point, Tensor factor, Tensor? lut_values, Tensor? bias, bool channels_last) -> Tensor")
@@ -868,6 +879,115 @@ def _quantize_rows_i8_cuda(x, scale, zero_point, quant_min, quant_max, want_rows
     return quantize_rows_i8(x, float(np.float32(scale)), int(zero_point), int(quant_min), int(quant_max), bool(want_rowsum))
 
 
+def quantize_rows_i8_padded(x, ldc, scale_f32, zero_point, quant_min, quant_max, want_rowsum):
+    """quantize_rows_i8 with codes [..., ldc] (ldc >= K, a multiple of 4): the columns [K, ldc) hold zero_point and the row
+    sums include them (mctq_quantize_rows_i8_padded)."""
+    tag = _dtype_tag(x)
+    if x.dim() == 0:
+        raise RuntimeError("quantize_rows_i8_padded: x must have at least one dimension")
+    xd = x.contiguous()
+    K = xd.shape[-1]
+    M = xd.numel() // K if K else 0
+    codes = torch.empty(tuple(xd.shape[:-1]) + (int(ldc),), dtype=torch.int8 if quant_min < 0 else torch.uint8,
+                        device=xd.device)
+    rowsum = torch.empty((M if want_rowsum else 0,), dtype=torch.int32, device=xd.device)
+    if M:
+        with _on_device(xd.device):
+            rc = _native.load().mctq_quantize_rows_i8_padded(xd.data_ptr(), tag, M, K, int(ldc), scale_f32, zero_point,
+                                                              quant_min, quant_max, codes.data_ptr(),
+                                                              _ptr(rowsum) if want_rowsum else None, _stream(xd.device))
+        _native.check(rc, "mctq_quantize_rows_i8_padded")
+    return codes, rowsum
+
+
+def _quantize_rows_i8_padded_cuda(x, ldc, scale, zero_point, quant_min, quant_max, want_rowsum):
+    _check_range(quant_min, quant_max)
+    if not quant_min <= zero_point <= quant_max:
+        raise RuntimeError("`zero_point` must be between `quant_min` and `quant_max`.")
+    return quantize_rows_i8_padded(x, int(ldc), float(np.float32(scale)), int(zero_point), int(quant_min), int(quant_max),
+                                   bool(want_rowsum))
+
+
+def _row_step(kind):
+    """The GEMM's row granule: 32 codes for 4-bit codes / indices, else 16."""
+    return 32 if kind in (_native.PACK_AFFINE_I4, _native.PACK_LUT_I4) else 16
+
+
+def linear_code_pitch(in_features, kind):
+    """The padded row length of integer linear mode: in_features rounded up to the GEMM's granule (every pad column a
+    channel pad: x code zx, counted in K, Sx and Sw)."""
+    step = _row_step(kind)
+    return -(-int(in_features) // step) * step
+
+
+def conv_code_pitch(in_channels, kh, kw, kind):
+    """(Cp, K): the pixel pitch of the padded NHWC codes and the conv's row length.  Cin <= 4 / <= 8 take the narrow gather
+    (Cp = 4 / 8, K = kh*kw*Cp rounded up to the granule: a row tail); wider Cin is rounded up to 16, or to 32 where 4-bit
+    codes need kh*kw*Cp % 32 == 0 (K = kh*kw*Cp)."""
+    cin, taps, step = int(in_channels), int(kh) * int(kw), _row_step(kind)
+    if cin <= 8:
+        cp = 4 if cin <= 4 else 8
+    else:
+        cp = -(-cin // 16) * 16
+        if taps * cp % step:
+            cp = -(-cin // 32) * 32
+    return cp, conv_row_length(cp, kh, kw, kind)
+
+
+def conv_row_length(cp, kh, kw, kind):
+    """The row length mctq_packed_conv2d_i8_padded sums for a pixel pitch cp: kh*kw*cp, rounded up to the granule for the
+    narrow gather (cp = 4 / 8)."""
+    n, step = int(kh) * int(kw) * int(cp), _row_step(kind)
+    return -(-n // step) * step if cp in (4, 8) else n
+
+
+def quantize_nhwc_i8_padded(x, cp, scale_f32, zero_point, quant_min, quant_max, want_sums):
+    """quantize_nhwc_i8 with a channel pitch cp (4, 8 or a multiple of 16, >= C): codes [N, H, W, cp] whose channels
+    [C, cp) hold zero_point, P including them.  A channels_last x is quantized as padded rows of pixels
+    (mctq_quantize_rows_i8_padded), any other x as NCHW planes (mctq_quantize_nhwc_i8_padded)."""
+    if x.dim() != 4:
+        raise RuntimeError(f"quantize_nhwc_i8_padded: x must be 4-D [N, C, H, W], got shape {list(x.shape)}")
+    N, C, H, W = x.shape
+    if not x.is_contiguous() and x.is_contiguous(memory_format=torch.channels_last):
+        return quantize_rows_i8_padded(x.permute(0, 2, 3, 1), cp, scale_f32, zero_point, quant_min, quant_max, want_sums)
+    tag = _dtype_tag(x)
+    xd = x.contiguous()
+    codes = torch.empty((N, H, W, int(cp)), dtype=torch.int8 if quant_min < 0 else torch.uint8, device=xd.device)
+    P = torch.empty((N * H * W if want_sums else 0,), dtype=torch.int32, device=xd.device)
+    if xd.numel():
+        with _on_device(xd.device):
+            rc = _native.load().mctq_quantize_nhwc_i8_padded(xd.data_ptr(), tag, N, C, H, W, int(cp), scale_f32, zero_point,
+                                                              quant_min, quant_max, codes.data_ptr(),
+                                                              _ptr(P) if want_sums else None, _stream(xd.device))
+        _native.check(rc, "mctq_quantize_nhwc_i8_padded")
+    return codes, P
+
+
+def _quantize_nhwc_i8_padded_cuda(x, channel_pitch, scale, zero_point, quant_min, quant_max, want_sums):
+    _check_range(quant_min, quant_max)
+    if not quant_min <= zero_point <= quant_max:
+        raise RuntimeError("`zero_point` must be between `quant_min` and `quant_max`.")
+    return quantize_nhwc_i8_padded(x, int(channel_pitch), float(np.float32(scale)), int(zero_point), int(quant_min),
+                                   int(quant_max), bool(want_sums))
+
+
+def padded_code_rows(codes, kind, is_signed, out_channels, in_channels, kh, kw, channels_last, cp, row):
+    """The int32 codes (or LUT indices) of a packed [Cout, Cin, kh, kw] weight (a Linear weight: kh = kw = 1) in (r, s, c)
+    order with a channel pitch cp >= Cin and a row of `row` >= kh*kw*cp columns: [Cout][row], channel pads and the row
+    tail holding 0.  `channels_last`: the codes are already in (r, s, c) order."""
+    qw = weight_code_values(codes, kind, is_signed, out_channels, in_channels * kh * kw)
+    qw = qw.reshape(out_channels, kh, kw, in_channels) if channels_last else \
+        qw.reshape(out_channels, in_channels, kh, kw).permute(0, 2, 3, 1)
+    qw = torch.nn.functional.pad(qw, (0, cp - in_channels)).reshape(out_channels, kh * kw * cp)
+    return torch.nn.functional.pad(qw, (0, row - kh * kw * cp)).contiguous()
+
+
+def pack_code_rows(qw, kind, is_signed, like):
+    """pack_weight_codes of int32 code rows, int8 codes viewed as the dtype of the packed tensor `like`."""
+    out = pack_weight_codes(qw, kind, is_signed)
+    return out.view(like.dtype) if kind == _native.PACK_AFFINE_I8 else out
+
+
 def weight_code_values(codes, kind, is_signed, out_features, in_features):
     """The integer codes of a packed affine weight (or the indices of a LUT weight: unsigned, 4-bit ones two per byte like
     int4 codes) as an int32 [out_features, in_features] tensor (one-time set-up of IntegerLinear: the code row sums)."""
@@ -891,10 +1011,12 @@ class IntegerLinear:
                                  None (zw = 0), and the codes qw are the table entries of the indices
     `__call__(x, bias)` returns the integer product of Q's codes of x and the weight codes, scaled (include/mctq.h gives the
     formula), for a CUDA x of `dtype` on the codes' device, enqueued on the current stream.  `quantize` and `gemm` are its two
-    launches."""
+    launches.  `pad=True` admits an in_features off the GEMM's granule (DESIGN §7f): the launch state then holds a copy of
+    the codes padded to ldc = linear_code_pitch(in_features, kind) columns, Q's codes have ldc columns whose pads hold zx,
+    and the output is that of the same formula over the real row (mctq_packed_linear_i8_padded)."""
 
     def __init__(self, codes, kind, is_signed, dtype, out_features, in_features, scale, zero_point, x_scale, x_zero_point,
-                 x_qmin, x_qmax, lut_values=None):
+                 x_qmin, x_qmax, lut_values=None, pad=False):
         _check_range(x_qmin, x_qmax)
         if not ((-128 <= x_qmin and x_qmax <= 127) or (0 <= x_qmin and x_qmax <= 255)):
             raise ValueError(f"IntegerLinear: the input range [{x_qmin}, {x_qmax}] does not fit 8-bit codes")
@@ -905,25 +1027,33 @@ class IntegerLinear:
         self.x_qmin, self.x_qmax = int(x_qmin), int(x_qmax)
         s = _param_on(scale.detach().reshape(-1).contiguous().to(torch.float32), self.device)
         factor = torch.tensor(self.x_scale, dtype=torch.float32, device=self.device) * s
+        ldc = linear_code_pitch(in_features, kind) if pad else int(in_features)
+        if ldc != int(in_features):
+            qw = padded_code_rows(codes, kind, is_signed, int(out_features), int(in_features), 1, 1, False, ldc, ldc)
+            codes = pack_code_rows(qw, kind, is_signed, codes)
         self._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, None, "IntegerLinear",
-                   lut_values)
+                   lut_values, ldc)
 
     @classmethod
     def from_parts(cls, codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, x_zero_point,
-                   lut_values=None):
-        """The launch state from a caller-supplied f and Sw (mctq::packed_linear_i8 / _lut), with the constructor's checks of
-        the weight; only `gemm` is available (the input quantizer's scale and range are not known)."""
+                   lut_values=None, ldc=None):
+        """The launch state from a caller-supplied f and Sw (mctq::packed_linear_i8 / _lut; with `ldc`, codes already padded
+        to [out][ldc]: mctq::packed_linear_i8_padded), with the constructor's checks of the weight; only `gemm` is available
+        (the input quantizer's scale and range are not known)."""
         lin = cls.__new__(cls)
         lin.device = codes.device
         lin.x_zp, lin.x_scale, lin.x_qmin, lin.x_qmax = int(x_zero_point), None, None, None
-        lin._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum,
-                  "packed_linear_i8" if lut_values is None else "packed_linear_i8_lut", lut_values)
+        what = "packed_linear_i8_padded" if ldc is not None else \
+            "packed_linear_i8" if lut_values is None else "packed_linear_i8_lut"
+        lin._bind(codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, what, lut_values,
+                  ldc)
         return lin
 
     def _bind(self, codes, kind, is_signed, dtype, out_features, in_features, factor, zero_point, w_rowsum, what,
-              lut_values=None):
+              lut_values=None, ldc=None):
         """Validate the weight, its factors, zero points (LUT weights: the table) and code row sums (computed from the codes
-        when None) and build the descriptor."""
+        when None) and build the descriptor.  `ldc`: the codes are [out][ldc] rows whose columns from in_features on are
+        channel pads (None: ldc = in_features)."""
         if self.device.type != "cuda":
             raise ValueError(f"{what} needs CUDA tensors")
         lut = lut_code_table(kind, lut_values, what) if lut_values is not None else None
@@ -934,7 +1064,10 @@ class IntegerLinear:
         if zero_point is None and lut is None:
             raise ValueError(f"{what}: affine weights need their zero points")
         self.out_features, self.in_features, self.dtype = int(out_features), int(in_features), dtype
-        N, K = self.out_features, self.in_features
+        self.ldc = int(ldc) if ldc is not None else self.in_features
+        if self.ldc < self.in_features:
+            raise ValueError(f"{what}: a row pitch of {self.ldc} is shorter than in_features = {self.in_features}")
+        N, K = self.out_features, self.ldc
         f = _param_on(factor.detach().reshape(-1).contiguous(), self.device)
         nz = f.numel() if lut is not None else zero_point.numel()
         if f.numel() not in (1, N) or nz != f.numel():
@@ -971,14 +1104,18 @@ class IntegerLinear:
             raise RuntimeError(f"packed_linear_i8: x of shape {list(x.shape)} does not end in in_features = {self.in_features}")
         if x.device != self.device:
             raise RuntimeError(f"packed_linear_i8: x must live on {self.device}")
+        if self.ldc != self.in_features:
+            return quantize_rows_i8_padded(x, self.ldc, self.x_scale, self.x_zp, self.x_qmin, self.x_qmax, self.needs_x_rowsum)
         return quantize_rows_i8(x, self.x_scale, self.x_zp, self.x_qmin, self.x_qmax, self.needs_x_rowsum)
 
     def gemm(self, x_codes, x_rowsum=None, bias=None, out=None):
-        """y from x codes [..., in_features] (int8 or uint8, zero point x_zero_point) and their row sums.  `out`: a 2-D
-        [M, out_features] CUDA tensor of `dtype` with unit column stride (its rows may be further apart) to write into."""
-        if x_codes.dtype not in (torch.int8, torch.uint8) or x_codes.dim() == 0 or x_codes.shape[-1] != self.in_features:
+        """y from x codes [..., in_features] (int8 or uint8, zero point x_zero_point; padded: [..., ldc], the pads holding
+        zx) and their row sums.  `out`: a 2-D [M, out_features] CUDA tensor of `dtype` with unit column stride (its rows may
+        be further apart) to write into."""
+        if x_codes.dtype not in (torch.int8, torch.uint8) or x_codes.dim() == 0 or x_codes.shape[-1] != self.ldc:
             raise RuntimeError(f"packed_linear_i8: x codes ({x_codes.dtype}, {list(x_codes.shape)}) are not int8 / uint8 "
-                               f"rows of in_features = {self.in_features}")
+                               f"rows of " + (f"in_features = {self.in_features}" if self.ldc == self.in_features else
+                                              f"ldc = {self.ldc} (in_features = {self.in_features}, padded)"))
         if x_codes.device != self.device or (bias is not None and bias.device != self.device):
             raise RuntimeError(f"packed_linear_i8: x codes and bias must live on {self.device}")
         if bias is not None and (bias.numel() != self.out_features or bias.dtype != self.dtype):
@@ -986,7 +1123,7 @@ class IntegerLinear:
         if self.needs_x_rowsum and x_rowsum is None:
             raise RuntimeError("packed_linear_i8: a weight zero point is not 0, so the x code row sums are needed")
         qx = x_codes.contiguous()
-        M = qx.numel() // self.in_features
+        M = qx.numel() // self.ldc
         if out is None:
             y = torch.empty(tuple(qx.shape[:-1]) + (self.out_features,), dtype=self.dtype, device=self.device)
             ldy = self.out_features
@@ -1005,6 +1142,13 @@ class IntegerLinear:
                     self.x_zp, M, _ptr(rs), self.w_rowsum.data_ptr(), self.factor.data_ptr(), _ptr(b), _DT[self.dtype],
                     y.data_ptr(), ldy)
             lib = _native.load()
+            if self.ldc != self.in_features:
+                with _on_device(self.device):
+                    rc = lib.mctq_packed_linear_i8_padded(*args[:3], self.ldc, *args[3:],
+                                                          self.lut.ctypes.data if self.lut is not None else None,
+                                                          _stream(self.device))
+                _native.check(rc, "mctq_packed_linear_i8_padded")
+                return y
             with _on_device(self.device):
                 if self.lut is not None:
                     rc = lib.mctq_packed_linear_i8_lut(*args, self.lut.ctypes.data, _stream(self.device))
@@ -1149,12 +1293,15 @@ class IntegerConv2d:
         x_scale, x_zero_point, x_qmin, x_qmax   the input quantizer Q (per tensor, at most 256 levels)
         lut_values               LUT weights (PACK_LUT_I4 / PACK_LUT_U8 indices): their int8 centroid codes, as for
                                  IntegerLinear (mctq_packed_conv2d_i8_lut)
+        pad                      admit a Cin off the gather's 16 channels (or a K off 32 for 4-bit codes; DESIGN §7f): the
+                                 codes are then copied in (r, s, c) order with a channel pitch Cp = conv_code_pitch(..), Q's
+                                 NHWC codes get Cp channels whose pads hold zx (mctq_packed_conv2d_i8_padded)
     `__call__(x, bias)` returns the integer convolution of Q's codes of a 4-D CUDA x of `dtype` on the codes' device with the
     weight codes, scaled (include/mctq.h gives the formula), in the memory format F.conv2d gives for x and the rebuilt
     weight.  `quantize` and `gemm` are its launches."""
 
     def __init__(self, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, weight_stride, stride,
-                 dilation, padding, scale, zero_point, x_scale, x_zero_point, x_qmin, x_qmax, lut_values=None):
+                 dilation, padding, scale, zero_point, x_scale, x_zero_point, x_qmin, x_qmax, lut_values=None, pad=False):
         _check_range(x_qmin, x_qmax)
         if not ((-128 <= x_qmin and x_qmax <= 127) or (0 <= x_qmin and x_qmax <= 255)):
             raise ValueError(f"IntegerConv2d: the input range [{x_qmin}, {x_qmax}] does not fit 8-bit codes")
@@ -1166,38 +1313,58 @@ class IntegerConv2d:
         kh, kw = (int(k) for k in kernel_size)
         shape = (int(out_channels), int(in_channels), kh, kw)
         self.weight_channels_last = _suggests_channels_last(shape, weight_stride)
-        if tuple(weight_stride) == tuple(torch.empty(shape, device="meta").stride()):
-            codes = conv_codes_rsc(codes, kind, is_signed, *shape)
-        elif tuple(weight_stride) != tuple(torch.empty(shape, device="meta").to(memory_format=torch.channels_last).stride()):
+        contiguous = tuple(weight_stride) == tuple(torch.empty(shape, device="meta").stride())
+        if not contiguous and \
+                tuple(weight_stride) != tuple(torch.empty(shape, device="meta").to(memory_format=torch.channels_last).stride()):
             raise ValueError(f"IntegerConv2d: weight strides {tuple(weight_stride)} are neither contiguous nor channels_last")
+        cp, row, w_rowsum = None, None, None
+        if pad and (shape[1] % 16 or shape[1] * kh * kw % _row_step(kind)):
+            # the padded copy in (r, s, c) order; Sw over the counted columns (the narrow gather's row tail is not counted)
+            cp, row = conv_code_pitch(shape[1], kh, kw, kind)
+            qw = padded_code_rows(codes, kind, is_signed, shape[0], shape[1], kh, kw, not contiguous, cp, row)
+            counted = qw[:, :kh * kw * cp]
+            if lut_values is not None:
+                table = lut_code_table(kind, lut_values, "IntegerConv2d")
+                counted = torch.from_numpy(table.astype(np.int32)).to(self.device)[counted]
+            w_rowsum = counted.sum(1, dtype=torch.int32)
+            codes = pack_code_rows(qw, kind, is_signed, codes)
+        elif contiguous:
+            codes = conv_codes_rsc(codes, kind, is_signed, *shape)
         s = _param_on(scale.detach().reshape(-1).contiguous().to(torch.float32), self.device)
         factor = torch.tensor(self.x_scale, dtype=torch.float32, device=self.device) * s
-        self._bind(codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, None,
-                   "IntegerConv2d", lut_values)
+        self._bind(codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum,
+                   "IntegerConv2d", lut_values, cp)
 
     @classmethod
     def from_parts(cls, codes, kind, is_signed, dtype, out_channels, in_channels, kernel_size, stride, dilation, padding,
-                   factor, zero_point, w_rowsum, x_zero_point, lut_values=None):
-        """The launch state from caller-supplied (r, s, c)-ordered codes, f and Sw (mctq::packed_conv2d_i8), with the
-        constructor's checks of the weight; only `gemm` is available."""
+                   factor, zero_point, w_rowsum, x_zero_point, lut_values=None, cp=None):
+        """The launch state from caller-supplied (r, s, c)-ordered codes, f and Sw (mctq::packed_conv2d_i8; with `cp`, codes
+        already padded to [Cout][conv_row_length(cp, ..)]: mctq::packed_conv2d_i8_padded), with the constructor's checks of
+        the weight; only `gemm` is available."""
         conv = cls.__new__(cls)
         conv.device = codes.device
         conv.x_zp, conv.x_scale, conv.x_qmin, conv.x_qmax = int(x_zero_point), None, None, None
         conv.weight_channels_last = False
         shape = (int(out_channels), int(in_channels), int(kernel_size[0]), int(kernel_size[1]))
-        conv._bind(codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum,
-                   "packed_conv2d_i8" if lut_values is None else "packed_conv2d_i8_lut", lut_values)
+        what = "packed_conv2d_i8_padded" if cp is not None else \
+            "packed_conv2d_i8" if lut_values is None else "packed_conv2d_i8_lut"
+        conv._bind(codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum, what,
+                   lut_values, cp)
         return conv
 
     def _bind(self, codes, kind, is_signed, dtype, shape, stride, dilation, padding, factor, zero_point, w_rowsum, what,
-              lut_values=None):
+              lut_values=None, cp=None):
         if len(stride) != 2 or len(dilation) != 2 or len(padding) != 4:
             raise ValueError(f"{what}: stride and dilation are pairs, padding is (top, bottom, left, right)")
         self.stride, self.dilation = tuple(int(v) for v in stride), tuple(int(v) for v in dilation)
         self.padding = tuple(int(v) for v in padding)
         self.out_channels, self.in_channels = shape[0], shape[1]
         self.kernel_size = shape[2:]
-        K = shape[1] * shape[2] * shape[3]
+        # cp: the pixel pitch of the x codes (padded: the codes are [Cout][conv_row_length(cp, ..)]; Cin = 4 / 8 keeps
+        # cp == Cin but takes the narrow gather)
+        self.padded = cp is not None
+        self.cp = int(cp) if self.padded else shape[1]
+        K = conv_row_length(self.cp, shape[2], shape[3], kind) if cp is not None else shape[1] * shape[2] * shape[3]
         # the weight as a [Cout][K] matrix: IntegerLinear's checks and launch state
         self._w = IntegerLinear.__new__(IntegerLinear)
         self._w.device, self._w.x_zp = self.device, self.x_zp
@@ -1221,19 +1388,26 @@ class IntegerConv2d:
             raise RuntimeError(f"packed_conv2d_i8: x of shape {list(x.shape)} is not [N, {self.in_channels}, H, W]")
         if x.device != self.device:
             raise RuntimeError(f"packed_conv2d_i8: x must live on {self.device}")
-        qx, P = quantize_nhwc_i8(x, self.x_scale, self.x_zp, self.x_qmin, self.x_qmax, self.needs_x_rowsum)
+        if self.padded:
+            qx, P = quantize_nhwc_i8_padded(x, self.cp, self.x_scale, self.x_zp, self.x_qmin, self.x_qmax,
+                                            self.needs_x_rowsum)
+        else:
+            qx, P = quantize_nhwc_i8(x, self.x_scale, self.x_zp, self.x_qmin, self.x_qmax, self.needs_x_rowsum)
         if not self.needs_x_rowsum:
             return qx, None
         N, _, H, W = x.shape
-        return qx, conv_window_sums(P, N, H, W, self.in_channels, self.kernel_size, self.stride, self.dilation,
-                                    self.padding, self.x_zp)
+        # the pad channels are channel pads: a tap outside the image counts cp * zx
+        return qx, conv_window_sums(P, N, H, W, self.cp, self.kernel_size, self.stride, self.dilation, self.padding,
+                                    self.x_zp)
 
     def gemm(self, x_codes, x_rowsum=None, bias=None, channels_last=False):
-        """y [N, Cout, Ho, Wo] from NHWC x codes [N, H, W, Cin] (int8 or uint8, zero point x_zero_point) and Sx [N*Ho*Wo];
-        channels_last: y's memory format (the kernel writes it directly)."""
-        if x_codes.dtype not in (torch.int8, torch.uint8) or x_codes.dim() != 4 or x_codes.shape[-1] != self.in_channels:
+        """y [N, Cout, Ho, Wo] from NHWC x codes [N, H, W, Cin] (int8 or uint8, zero point x_zero_point; padded:
+        [N, H, W, cp], the pads holding zx) and Sx [N*Ho*Wo]; channels_last: y's memory format (the kernel writes it
+        directly)."""
+        if x_codes.dtype not in (torch.int8, torch.uint8) or x_codes.dim() != 4 or x_codes.shape[-1] != self.cp:
             raise RuntimeError(f"packed_conv2d_i8: x codes ({x_codes.dtype}, {list(x_codes.shape)}) are not int8 / uint8 "
-                               f"NHWC codes of {self.in_channels} channels")
+                               f"NHWC codes of {self.in_channels} channels" +
+                               (f" padded to {self.cp}" if self.padded else ""))
         if x_codes.device != self.device or (bias is not None and bias.device != self.device):
             raise RuntimeError(f"packed_conv2d_i8: x codes and bias must live on {self.device}")
         if bias is not None and (bias.numel() != self.out_channels or bias.dtype != self.dtype):
@@ -1263,6 +1437,12 @@ class IntegerConv2d:
                     0 if channels_last else 1)
             lut = self._w.lut
             lib = _native.load()
+            if self.padded:
+                with _on_device(self.device):
+                    rc = lib.mctq_packed_conv2d_i8_padded(args[0], args[1], self.cp, *args[2:],
+                                                          lut.ctypes.data if lut is not None else None, _stream(self.device))
+                _native.check(rc, "mctq_packed_conv2d_i8_padded")
+                return y
             with _on_device(self.device):
                 if lut is not None:
                     rc = lib.mctq_packed_conv2d_i8_lut(*args, lut.ctypes.data, _stream(self.device))
@@ -1298,6 +1478,38 @@ def _packed_conv2d_i8_lut_cuda(x_codes, x_zero_point, codes, kind, out_channels,
     conv = IntegerConv2d.from_parts(codes, kind, False, torch.float32, out_channels, x_codes.shape[-1], kernel_size, stride,
                                     dilation, padding, factor, None, w_rowsum, x_zero_point, lut_values)
     return conv.gemm(x_codes, None, bias, channels_last)
+
+
+def _packed_linear_i8_padded_cuda(x_codes, in_features, x_zero_point, x_rowsum, codes, kind, is_signed, out_features,
+                                  zero_point, w_rowsum, factor, bias, dtype, lut_values):
+    """mctq::packed_linear_i8_padded: x codes [..., ldc] whose columns from in_features on hold zx, codes [out][ldc] (affine
+    with zero_point, or LUT indices with `lut_values` and f32 output), caller-supplied Sw over the ldc columns and f."""
+    if x_codes.dim() == 0:
+        raise RuntimeError("packed_linear_i8_padded: x codes must have at least one dimension")
+    _native.load()
+    lut = lut_values is not None
+    lin = IntegerLinear.from_parts(codes, kind, False if lut else is_signed, torch.float32 if lut else dtype, out_features,
+                                   in_features, factor, None if lut else zero_point, w_rowsum, x_zero_point, lut_values,
+                                   ldc=x_codes.shape[-1])
+    return lin.gemm(x_codes, None if lut else x_rowsum, bias)
+
+
+def _packed_conv2d_i8_padded_cuda(x_codes, in_channels, x_zero_point, x_rowsum, codes, kind, is_signed, out_channels,
+                                  kernel_size, stride, dilation, padding, zero_point, w_rowsum, factor, bias, dtype,
+                                  channels_last, lut_values):
+    """mctq::packed_conv2d_i8_padded: NHWC x codes [N, H, W, cp] whose channels from in_channels on hold zx, codes
+    [Cout][conv_row_length(cp, ..)] in (r, s, c) order (affine with zero_point, or LUT indices with `lut_values` and f32
+    output), caller-supplied Sw over the counted columns and f."""
+    if x_codes.dim() != 4:
+        raise RuntimeError("packed_conv2d_i8_padded: x codes must be 4-D NHWC")
+    if len(kernel_size) != 2:
+        raise ValueError("packed_conv2d_i8_padded: kernel_size is a pair")
+    _native.load()
+    lut = lut_values is not None
+    conv = IntegerConv2d.from_parts(codes, kind, False if lut else is_signed, torch.float32 if lut else dtype, out_channels,
+                                    in_channels, kernel_size, stride, dilation, padding, factor,
+                                    None if lut else zero_point, w_rowsum, x_zero_point, lut_values, cp=x_codes.shape[-1])
+    return conv.gemm(x_codes, None if lut else x_rowsum, bias, channels_last)
 
 
 class IntegerDepthwiseConv2d:
@@ -1617,6 +1829,10 @@ _LIB.impl("packed_conv2d_i8", _packed_conv2d_i8_cuda, "CUDA")
 _LIB.impl("packed_linear_i8_lut", _packed_linear_i8_lut_cuda, "CUDA")
 _LIB.impl("packed_conv2d_i8_lut", _packed_conv2d_i8_lut_cuda, "CUDA")
 _LIB.impl("packed_dwconv2d_i8", _packed_dwconv2d_i8_cuda, "CUDA")
+_LIB.impl("quantize_rows_i8_padded", _quantize_rows_i8_padded_cuda, "CUDA")
+_LIB.impl("quantize_nhwc_i8_padded", _quantize_nhwc_i8_padded_cuda, "CUDA")
+_LIB.impl("packed_linear_i8_padded", _packed_linear_i8_padded_cuda, "CUDA")
+_LIB.impl("packed_conv2d_i8_padded", _packed_conv2d_i8_padded_cuda, "CUDA")
 
 _LIB.impl("fq_affine_scalar_pre", _affine_scalar_pre_cuda, "CUDA")
 _LIB.impl("fq_affine_scalar_pre", _via_device(_affine_scalar_pre_cuda), "CPU")
@@ -1638,6 +1854,10 @@ _LIB.impl("packed_conv2d_i8", _via_device(_packed_conv2d_i8_cuda), "CPU")
 _LIB.impl("packed_linear_i8_lut", _via_device(_packed_linear_i8_lut_cuda), "CPU")
 _LIB.impl("packed_conv2d_i8_lut", _via_device(_packed_conv2d_i8_lut_cuda), "CPU")
 _LIB.impl("packed_dwconv2d_i8", _via_device(_packed_dwconv2d_i8_cuda, keep=(15,)), "CPU")
+_LIB.impl("quantize_rows_i8_padded", _via_device(_quantize_rows_i8_padded_cuda), "CPU")
+_LIB.impl("quantize_nhwc_i8_padded", _via_device(_quantize_nhwc_i8_padded_cuda), "CPU")
+_LIB.impl("packed_linear_i8_padded", _via_device(_packed_linear_i8_padded_cuda), "CPU")
+_LIB.impl("packed_conv2d_i8_padded", _via_device(_packed_conv2d_i8_padded_cuda), "CPU")
 
 
 # --------------------------------------------------------------------------------------------- fake / meta impls
@@ -1759,6 +1979,38 @@ def _(x, x_scale, x_zero_point, x_qmin, x_qmax, codes, kind, is_signed, out_chan
     if channels_last:
         return x.new_empty((N, Ho, Wo, out_channels)).permute(0, 3, 1, 2)
     return x.new_empty((N, out_channels, Ho, Wo))
+
+
+@torch.library.register_fake("mctq::quantize_rows_i8_padded")
+def _(x, ldc, scale, zero_point, quant_min, quant_max, want_rowsum):
+    M = x.numel() // x.shape[-1] if x.dim() and x.shape[-1] else 0
+    return (x.new_empty(tuple(x.shape[:-1]) + (ldc,), dtype=torch.int8 if quant_min < 0 else torch.uint8),
+            x.new_empty((M if want_rowsum else 0,), dtype=torch.int32))
+
+
+@torch.library.register_fake("mctq::quantize_nhwc_i8_padded")
+def _(x, channel_pitch, scale, zero_point, quant_min, quant_max, want_sums):
+    N, C, H, W = x.shape
+    return (x.new_empty((N, H, W, channel_pitch), dtype=torch.int8 if quant_min < 0 else torch.uint8),
+            x.new_empty((N * H * W if want_sums else 0,), dtype=torch.int32))
+
+
+@torch.library.register_fake("mctq::packed_linear_i8_padded")
+def _(x_codes, in_features, x_zero_point, x_rowsum, codes, kind, is_signed, out_features, zero_point, w_rowsum, factor, bias,
+      dtype, lut_values):
+    return x_codes.new_empty(tuple(x_codes.shape[:-1]) + (out_features,),
+                             dtype=torch.float32 if lut_values is not None else dtype)
+
+
+@torch.library.register_fake("mctq::packed_conv2d_i8_padded")
+def _(x_codes, in_channels, x_zero_point, x_rowsum, codes, kind, is_signed, out_channels, kernel_size, stride, dilation,
+      padding, zero_point, w_rowsum, factor, bias, dtype, channels_last, lut_values):
+    N, H, W, _ = x_codes.shape
+    Ho, Wo = conv_output_hw(H, W, kernel_size, stride, dilation, padding)
+    dt = torch.float32 if lut_values is not None else dtype
+    if channels_last:
+        return x_codes.new_empty((N, Ho, Wo, out_channels), dtype=dt).permute(0, 3, 1, 2)
+    return x_codes.new_empty((N, out_channels, Ho, Wo), dtype=dt)
 
 
 # --------------------------------------------------------------------------------------------- whole-model launch

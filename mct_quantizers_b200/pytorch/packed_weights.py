@@ -59,12 +59,19 @@ normal in f32, the integer modes take LUT wrappers too: the GEMM's weight produc
 by value with every launch) and the product is the same exact int32 sum (include/mctq.h).  It differs from the packed path
 by the rounding of W to f32 and by f32 accumulation, so it stays opt-in: without the flag LUT wrappers keep their paths.
 
+Padded integer modes (`integer_pad=True` together with integer_linear=True and / or integer_conv=True; opt-in): Linear layers
+whose in_features and groups-1 Conv2d layers whose Cin is off the GEMM's granule (16 codes, 32 for 4-bit codes), such as a
+stem with Cin = 3 or the squeeze-excitation convs of EfficientNet.  Q's codes get a padded pitch whose pad columns hold Q's
+zero-point code and are counted in the corrections, so they contribute exactly 0: every output is the formula over the real
+row (include/mctq.h, DESIGN §7f).  Convs with Cin <= 8 take a narrow gather with a pixel pitch of 4 or 8 codes.
+
 Packing is one-way and for inference only:
   * the rebuild dtype is the weight's dtype at packing time; `.half()` does not change it (the codes are integer buffers);
   * the packed state travels with the module: `state_dict` / `load_state_dict` between packed models of the same structure,
     `.to(device)`, `torch.save` + `pytorch_load_quantized_model`;
   * a packed wrapper cannot be traced (ONNX export needs the float weights, which are gone) and cannot be trained.
 """
+import functools
 import weakref
 from typing import Dict, List, Optional, Tuple
 
@@ -309,26 +316,35 @@ def _lut_code_eligibility(e) -> Tuple[bool, str]:
     return True, ""
 
 
-def _lut_eligibility(e, K, what, x_signed) -> Tuple[bool, str]:
+def _lut_eligibility(e, K, what, x_signed, padded=None) -> Tuple[bool, str]:
     """The conditions the GEMM integer modes put on a LUT weight (entry e, row length K named `what`): _lut_code_eligibility,
-    K a multiple of 32 (4-bit indices) or 16 (8-bit indices) and at most the int32 bound of signed weight codes."""
+    K a multiple of 32 (4-bit indices) or 16 (8-bit indices) and at most the int32 bound of signed weight codes.  `padded`:
+    the row length the padded kernel sums instead (integer_pad), which takes the place of the multiple rule."""
     ok, reason = _lut_code_eligibility(e)
     if not ok:
         return ok, reason
     step, bits = (32, 4) if e.kind == _native.PACK_LUT_I4 else (16, 8)
-    if K % step:
+    if padded is None and K % step:
         return False, f"{what} = {K} is not a multiple of {step} ({bits}-bit LUT indices)"
-    bound = _native.integer_linear_max_k(True, x_signed)
+    return _row_bound(K, padded, what, _native.integer_linear_max_k(True, x_signed))
+
+
+def _row_bound(K, padded, what, bound) -> Tuple[bool, str]:
+    """The int32 bound on the row length the kernel sums: K, or `padded` (not None) when the codes are padded."""
     if K > bound:
         return False, f"{what} = {K} exceeds {bound}, the largest row length whose int32 sum of code products cannot overflow"
+    if padded is not None and padded > bound:
+        return False, (f"{what} = {K} padded to a row of {padded} exceeds {bound}, the largest row length whose int32 sum "
+                       f"of code products cannot overflow")
     return True, ""
 
 
-def integer_linear_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
+def integer_linear_eligibility(wrapper, input_quantizer, lut: bool = False, pad: bool = False) -> Tuple[bool, str]:
     """(True, '') when `wrapper` can run in integer linear mode with input quantizer `input_quantizer`: fused_linear_eligibility,
     int8 / int4 affine codes, a per-tensor affine activation quantizer with 8-bit codes, in_features a multiple of 16 (32 for
     int4 codes) and at most the int32 bound of the code signedness pair.  `lut=True` also accepts LUT weights that meet
-    _lut_eligibility.  Host-only."""
+    _lut_eligibility.  `pad=True` drops the multiple rule: such rows are padded to ops.linear_code_pitch, and the bound
+    applies to the padded row.  Host-only."""
     ok, reason = fused_linear_eligibility(wrapper)
     if not ok:
         return ok, reason
@@ -341,15 +357,13 @@ def integer_linear_eligibility(wrapper, input_quantizer, lut: bool = False) -> T
         return ok, reason
     qmin = int(input_quantizer.min_quantized_domain)
     K = wrapper.layer.in_features
+    padded = ops.linear_code_pitch(K, e.kind) if pad and K % ops._row_step(e.kind) else None
     if is_lut:
-        return _lut_eligibility(e, K, "in_features", qmin < 0)
+        return _lut_eligibility(e, K, "in_features", qmin < 0, padded)
     step = 32 if e.kind == _native.PACK_AFFINE_I4 else 16
-    if K % step:
+    if padded is None and K % step:
         return False, f"in_features = {K} is not a multiple of {step}"
-    bound = _native.integer_linear_max_k(e.is_signed, qmin < 0)
-    if K > bound:
-        return False, f"in_features = {K} exceeds {bound}, the largest row length whose int32 sum of code products cannot overflow"
-    return True, ""
+    return _row_bound(K, padded, "in_features", _native.integer_linear_max_k(e.is_signed, qmin < 0))
 
 
 def _conv_eligibility(wrapper, input_quantizer, lut, depthwise):
@@ -396,28 +410,31 @@ def _conv_eligibility(wrapper, input_quantizer, lut, depthwise):
     return True, "", e, shape, is_lut
 
 
-def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
+def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False, pad: bool = False) -> Tuple[bool, str]:
     """(True, '') when `wrapper` can run in integer convolution mode with input quantizer `input_quantizer`: a
     torch.nn.Conv2d layer with string-attribute weights, no extra call arguments and 'weight' its only quantized weight,
     packed as int8 / int4 affine codes, rebuilt as a contiguous or channels_last [Cout, Cin, kh, kw] weight with parameters
     per tensor or per output channel; groups 1 and zero padding; the input quantizer conditions of integer linear mode;
     Cin a multiple of 16, K = Cin * kh * kw a multiple of 32 for int4 codes and at most the int32 bound of the code
-    signedness pair.  `lut=True` also accepts LUT weights that meet _lut_eligibility.  Host-only."""
+    signedness pair.  `lut=True` also accepts LUT weights that meet _lut_eligibility.  `pad=True` drops the channel and
+    multiple rules: such codes get the pixel pitch and row length of ops.conv_code_pitch, and the bound applies to that
+    row.  Host-only."""
     r = _conv_eligibility(wrapper, input_quantizer, lut, depthwise=False)
     if not r[0]:
         return r
     _, _, e, shape, is_lut = r
     K = shape[1] * shape[2] * shape[3]
-    if shape[1] % 16:
+    padded = None
+    if pad and (shape[1] % 16 or K % ops._row_step(e.kind)):
+        padded = ops.conv_code_pitch(shape[1], shape[2], shape[3], e.kind)[1]
+    if padded is None and shape[1] % 16:
         return False, f"in_channels = {shape[1]} is not a multiple of 16"
     if is_lut:
-        return _lut_eligibility(e, K, "Cin * kh * kw", int(input_quantizer.min_quantized_domain) < 0)
-    if e.kind == _native.PACK_AFFINE_I4 and K % 32:
+        return _lut_eligibility(e, K, "Cin * kh * kw", int(input_quantizer.min_quantized_domain) < 0, padded)
+    if padded is None and e.kind == _native.PACK_AFFINE_I4 and K % 32:
         return False, f"Cin * kh * kw = {K} is not a multiple of 32 (int4 codes)"
     bound = _native.integer_linear_max_k(e.is_signed, int(input_quantizer.min_quantized_domain) < 0)
-    if K > bound:
-        return False, f"Cin * kh * kw = {K} exceeds {bound}, the largest row length whose int32 sum of code products cannot overflow"
-    return True, ""
+    return _row_bound(K, padded, "Cin * kh * kw", bound)
 
 
 def integer_depthwise_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
@@ -605,10 +622,10 @@ class PackedState:
             elif conv:
                 launch = ops.IntegerConv2d(codes, e.kind, e.is_signed, e.dtype_out, layer.out_channels, layer.in_channels,
                                            layer.kernel_size, e.stride_out, layer.stride, layer.dilation,
-                                           ops.conv_padding(layer), scale, zps, x_scale, x_zp, qmin, qmax, lut)
+                                           ops.conv_padding(layer), scale, zps, x_scale, x_zp, qmin, qmax, lut, pad=True)
             else:
                 launch = ops.IntegerLinear(codes, e.kind, e.is_signed, e.dtype_out, layer.out_features, layer.in_features,
-                                           scale, zps, x_scale, x_zp, qmin, qmax, lut)
+                                           scale, zps, x_scale, x_zp, qmin, qmax, lut, pad=True)
             lin = (codes.data_ptr(), launch)
             self._ilin = lin
         return lin[1](x, bias)
@@ -641,7 +658,7 @@ class PackedState:
 
 def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bool = False, integer_linear: bool = False,
                          input_quantizer=None, integer_conv: bool = False, integer_lut: bool = False,
-                         integer_depthwise: bool = False) -> Dict:
+                         integer_depthwise: bool = False, integer_pad: bool = False) -> Dict:
     """Pack every weight of `wrapper` that can be packed (see the module docstring).  Returns
     {name: {'packed': bool, 'kind': str | None, 'reason': str, 'code_bytes': int, 'float_bytes': int}}.
     `fused_linear=True` also switches the wrapper to fused linear mode when fused_linear_eligibility allows it (on a wrapper
@@ -655,11 +672,14 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
     and every report entry gains 'integer_conv': bool, 'integer_conv_reason': str and 'input_holder'.
     `integer_lut=True` (needs integer_linear=True and / or integer_conv=True) extends those modes to LUT weights.
     `integer_depthwise=True` (needs integer_conv=True) extends integer convolution mode to depthwise Conv2d layers
-    (integer_depthwise_eligibility); their report entries keep the keys 'integer_conv' and 'integer_conv_reason'."""
+    (integer_depthwise_eligibility); their report entries keep the keys 'integer_conv' and 'integer_conv_reason'.
+    `integer_pad=True` (needs integer_linear=True and / or integer_conv=True) lifts the row-length and channel-count rules
+    of those modes: the codes of such Linear and groups-1 Conv2d layers are padded (DESIGN §7f)."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     _check_integer_lut(integer_lut, integer_linear, integer_conv)
     _check_integer_depthwise(integer_depthwise, integer_conv)
+    _check_integer_pad(integer_pad, integer_linear, integer_conv)
     if integer_linear and input_quantizer is None:
         raise ValueError("integer_linear=True needs the input_quantizer of the activation holder that feeds the wrapper")
     if integer_conv and input_quantizer is None:
@@ -694,9 +714,10 @@ def pack_wrapper_weights(wrapper, fused_linear: bool = False, batched_linear: bo
     if batched_linear:
         _switch_to_batched(wrapper, report)
     if integer_linear:
-        _switch_to_integer(wrapper, report, input_quantizer, None, lut=integer_lut)
+        _switch_to_integer(wrapper, report, input_quantizer, None, lut=integer_lut, pad=integer_pad)
     if integer_conv:
-        _switch_to_integer(wrapper, report, input_quantizer, None, conv=True, lut=integer_lut, depthwise=integer_depthwise)
+        _switch_to_integer(wrapper, report, input_quantizer, None, conv=True, lut=integer_lut, depthwise=integer_depthwise,
+                           pad=integer_pad)
     return report
 
 
@@ -710,6 +731,12 @@ def _check_integer_depthwise(integer_depthwise, integer_conv):
     if integer_depthwise and not integer_conv:
         raise ValueError("integer_depthwise=True needs integer_conv=True (it extends integer convolution mode to depthwise "
                          "Conv2d layers)")
+
+
+def _check_integer_pad(integer_pad, integer_linear, integer_conv):
+    if integer_pad and not (integer_linear or integer_conv):
+        raise ValueError("integer_pad=True needs integer_linear=True and / or integer_conv=True (it extends those modes to "
+                         "row lengths and channel counts off the GEMM's granule)")
 
 
 def _drop_float_weights(wrapper, new, entries, keep):
@@ -753,8 +780,9 @@ def _switch_to_batched(wrapper, report):
         r['batched'], r['batched_reason'] = ok, reason
 
 
-def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None, conv=False, lut=False, depthwise=False):
-    eligibility = integer_conv_eligibility if conv else integer_linear_eligibility
+def _switch_to_integer(wrapper, report, input_quantizer, holder_name, reason=None, conv=False, lut=False, depthwise=False,
+                       pad=False):
+    eligibility = functools.partial(integer_conv_eligibility if conv else integer_linear_eligibility, pad=pad)
     layer = wrapper.__dict__['_modules'].get(LAYER)
     if conv and depthwise and type(layer) is torch.nn.Conv2d and layer.groups > 1:
         eligibility = integer_depthwise_eligibility
@@ -782,18 +810,20 @@ def _bits(t):
 
 def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batched_linear: bool = False,
                        integer_linear: bool = False, integer_conv: bool = False, integer_lut: bool = False,
-                       integer_depthwise: bool = False) -> Dict[str, Dict]:
+                       integer_depthwise: bool = False, integer_pad: bool = False) -> Dict[str, Dict]:
     """pack_weights(fused_linear, batched_linear) on every PytorchQuantizationWrapper of `model`: {wrapper module name:
     {weight name: report entry}}.  `integer_linear=True` then switches, in place, every eligible wrapper whose input is the
     output of an activation quantization holder (integer_linear_edges) to integer linear mode; every report entry gains
     'integer', 'integer_reason' and 'input_holder'.  `integer_conv=True` does the same for integer convolution mode on the
     same edges; every report entry gains 'integer_conv', 'integer_conv_reason' and 'input_holder'.  `integer_lut=True` extends
-    both to LUT weights, and `integer_depthwise=True` extends integer convolution mode to depthwise Conv2d layers.  When the
+    both to LUT weights, and `integer_depthwise=True` extends integer convolution mode to depthwise Conv2d layers.
+    `integer_pad=True` lifts the row-length and channel-count rules of both (padded codes, DESIGN §7f).  When the
     model cannot be traced nothing is switched and the reason is reported."""
     if batched_linear and not fused_linear:
         raise ValueError("batched_linear=True needs fused_linear=True (batched mode extends the fused mode)")
     _check_integer_lut(integer_lut, integer_linear, integer_conv)
     _check_integer_depthwise(integer_depthwise, integer_conv)
+    _check_integer_pad(integer_pad, integer_linear, integer_conv)
     from mct_quantizers_b200.pytorch.quantize_wrapper import PytorchQuantizationWrapper
     wrappers = {mod_name: mod for mod_name, mod in model.named_modules()
                 if isinstance(mod, PytorchQuantizationWrapper) and mod.is_weights_quantization}
@@ -805,5 +835,5 @@ def pack_model_weights(model: torch.nn.Module, fused_linear: bool = False, batch
             reason = failure or why.get(name) or ("" if holder else "the wrapper is not called in the traced forward")
             for conv in (False, True) if integer_linear and integer_conv else (integer_conv,):
                 _switch_to_integer(mod, reports[name], q, holder, None if holder else reason, conv=conv, lut=integer_lut,
-                                   depthwise=integer_depthwise)
+                                   depthwise=integer_depthwise, pad=integer_pad)
     return reports

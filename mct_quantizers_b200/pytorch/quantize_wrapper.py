@@ -190,7 +190,7 @@ class PytorchQuantizationWrapper(nn.Module):
 
     def pack_weights(self, fused_linear: bool = False, batched_linear: bool = False, integer_linear: bool = False,
                      input_quantizer=None, integer_conv: bool = False, integer_lut: bool = False,
-                     integer_depthwise: bool = False) -> Dict[str, Dict]:
+                     integer_depthwise: bool = False, integer_pad: bool = False) -> Dict[str, Dict]:
         """Keep the weights of this wrapper as int8 / int4 codes or LUT indices instead of floats (inference only, one-way;
         see mct_quantizers_b200.pytorch.packed_weights).  Returns, per weight, whether it was packed and why not.
         `fused_linear=True`: a packed nn.Linear wrapper computes small-batch products straight from its codes (opt-in: not
@@ -200,10 +200,11 @@ class PytorchQuantizationWrapper(nn.Module):
         8-bit codes on the tensor cores (see packed_weights).  `integer_conv=True` with `input_quantizer`: the same for a
         Conv2d layer, as an implicit GEMM of the codes.  `integer_lut=True` (with either): LUT weights too, their indices
         looked up as int8 codes in the GEMM.  `integer_depthwise=True` (with integer_conv): depthwise Conv2d layers too,
-        as an exact int32 window sum of the codes."""
+        as an exact int32 window sum of the codes.  `integer_pad=True` (with integer_linear / integer_conv): row lengths and
+        channel counts off the GEMM's granule too, their codes padded with Q's zero-point code."""
         from mct_quantizers_b200.pytorch.packed_weights import pack_wrapper_weights
         return pack_wrapper_weights(self, fused_linear, batched_linear, integer_linear, input_quantizer, integer_conv,
-                                    integer_lut, integer_depthwise)
+                                    integer_lut, integer_depthwise, integer_pad)
 
     def quantize_weights_batched(self) -> Dict[str, torch.Tensor]:
         """get_quantized_weights() with every affine weight quantizer of this wrapper fused into one launch."""
