@@ -331,6 +331,17 @@ int mctq_packed_dwconv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, in
                             int x_nhwc, float x_scale, int32_t x_zero_point, int32_t x_qmin, int32_t x_qmax,
                             const float* factor, const void* bias, void* y, const int8_t* lut_codes_host, void* stream);
 
+/* The tile plan mctq_packed_dwconv2d_i8 launches for a geometry (host only, no CUDA call).  A work unit is S slots (NCHW:
+ * consecutive (b, c) planes; NHWC: consecutive channels of one image) times a TH x TW tile of output pixels, staged from an
+ * IH x IW window tile in smem_bytes of shared memory.  The planner starts from about 2048 outputs per unit and halves TH,
+ * then S, then TW until the tile fits 200 KB.  Returns 0, MCTQ_E_BADARG for the launch's geometry rejections or a null
+ * `out`, or MCTQ_E_RANGE for kh*kw > 33025 or a dilated window that does not fit even at S = TH = TW = 1 (20 + 4 kh kw +
+ * 4 IH IW bytes, IH = (kh-1) dh + 1, IW = (kw-1) dw + 1): the launch returns the same.  `out` is written only on 0. */
+typedef struct MctqDwPlan {
+    int32_t S, TH, TW, IH, IW, smem_bytes;
+} MctqDwPlan;
+int mctq_packed_dwconv2d_i8_plan(const MctqConv2dGeom* g, int64_t Cout, int x_nhwc, MctqDwPlan* out);
+
 /* Integer modes for row lengths and channel counts off the GEMM's granule (DESIGN.md §7f).  The padding contract: every
  * column the kernel sums beyond the real K belongs to one of two classes --
  *   channel pad  the x code is zx (in the image and, as before, for taps outside it); the column is counted in K, Sx and

@@ -69,6 +69,11 @@ class MctqConv2dGeom(ctypes.Structure):
                                      "pt", "pb", "pl", "pr")]
 
 
+class MctqDwPlan(ctypes.Structure):
+    """Mirror of `struct MctqDwPlan` (include/mctq.h)."""
+    _fields_ = [(f, c_i32) for f in ("S", "TH", "TW", "IH", "IW", "smem_bytes")]
+
+
 # name -> (restype, argtypes): every symbol include/mctq.h declares
 SIGNATURES = {
     "mctq_abi_version": (c_int, []),
@@ -99,6 +104,7 @@ SIGNATURES = {
                                           c_int, c_vp, c_vp]),
     "mctq_packed_dwconv2d_i8": (c_int, [c_vp, c_vp, c_i64, c_vp, c_int, c_int, c_f32, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp,
                                         c_vp, c_vp]),
+    "mctq_packed_dwconv2d_i8_plan": (c_int, [c_vp, c_i64, c_int, c_vp]),
     "mctq_quantize_rows_i8_padded": (c_int, [c_vp, c_int, c_i64, c_i64, c_i64, c_f32, c_i32, c_i32, c_i32, c_vp, c_vp,
                                              c_vp]),
     "mctq_quantize_nhwc_i8_padded": (c_int, [c_vp, c_int, c_i64, c_i64, c_i64, c_i64, c_i64, c_f32, c_i32, c_i32, c_i32,

@@ -1146,6 +1146,25 @@ int dw_plan(DwArgs& a, bool nhwc) {
     }
 }
 
+// the geometry checks of mctq_packed_dwconv2d_i8 and its plan query
+int dw_check_geometry(const MctqConv2dGeom* g, int64_t Cout, int x_nhwc) {
+    if (!g) return MCTQ_E_BADARG;
+    if (g->N < 0 || g->H < 1 || g->W < 1 || g->Cin < 1 || g->Ho < 1 || g->Wo < 1 || g->kh < 1 || g->kw < 1 || g->sh < 1 ||
+        g->sw < 1 || g->dh < 1 || g->dw < 1 || g->pt < 0 || g->pb < 0 || g->pl < 0 || g->pr < 0 || (x_nhwc != 0 && x_nhwc != 1))
+        return MCTQ_E_BADARG;
+    if (Cout < 1 || Cout % g->Cin != 0) return MCTQ_E_BADARG;
+    return 0;
+}
+
+// the geometry fields of DwArgs that dw_plan reads, on a zeroed `a`
+void dw_set_geometry(DwArgs& a, const MctqConv2dGeom* g, int64_t Cout) {
+    memset(&a, 0, sizeof(a));
+    a.nplanes = (int64_t)g->N * g->Cin;
+    a.H = g->H; a.W = g->W; a.C = g->Cin; a.Cout = (int32_t)Cout; a.Ho = g->Ho; a.Wo = g->Wo;
+    a.m = (int32_t)(Cout / g->Cin); a.K = (int32_t)((int64_t)g->kh * g->kw); a.kh = g->kh; a.kw = g->kw;   // K <= 33025
+    a.sh = g->sh; a.sw = g->sw; a.dh = g->dh; a.dw = g->dw; a.pt = g->pt; a.pl = g->pl;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1307,10 +1326,7 @@ int mctq_packed_dwconv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, in
                             const float* factor, const void* bias, void* y, const int8_t* lut_codes_host, void* stream) {
     MCTQ_NVTX("mctq_packed_dwconv2d_i8");
     if (!w || !g || !factor) return MCTQ_E_BADARG;
-    if (g->N < 0 || g->H < 1 || g->W < 1 || g->Cin < 1 || g->Ho < 1 || g->Wo < 1 || g->kh < 1 || g->kw < 1 || g->sh < 1 ||
-        g->sw < 1 || g->dh < 1 || g->dw < 1 || g->pt < 0 || g->pb < 0 || g->pl < 0 || g->pr < 0 || (x_nhwc != 0 && x_nhwc != 1))
-        return MCTQ_E_BADARG;
-    if (Cout < 1 || Cout % g->Cin != 0) return MCTQ_E_BADARG;
+    if (const int rc = dw_check_geometry(g, Cout, x_nhwc)) return rc;
     const int64_t K = (int64_t)g->kh * g->kw;
     // the weight as a [Cout][kh * kw] matrix: kind, dtype, extent, parameter layout, pointers
     if (const int rc = packed_linear_check(w, Cout, K, x, x_dtype, g->N, y)) return rc;
@@ -1321,17 +1337,13 @@ int mctq_packed_dwconv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, in
     if (g->N == 0) return 0;
 
     DwArgs a;
-    memset(&a, 0, sizeof(a));
+    dw_set_geometry(a, g, Cout);
     a.x = x;
     a.y = y;
     a.codes = reinterpret_cast<const uint8_t*>(w->codes);
     a.w_zp = pack_is_lut(w->kind) ? nullptr : w->zp;
     a.factor = factor;
     a.bias = bias;
-    a.nplanes = (int64_t)g->N * g->Cin;
-    a.H = g->H; a.W = g->W; a.C = g->Cin; a.Cout = (int32_t)Cout; a.Ho = g->Ho; a.Wo = g->Wo;
-    a.m = (int32_t)(Cout / g->Cin); a.K = (int32_t)K; a.kh = g->kh; a.kw = g->kw;
-    a.sh = g->sh; a.sw = g->sw; a.dh = g->dh; a.dw = g->dw; a.pt = g->pt; a.pl = g->pl;
     a.kind = w->kind; a.w_signed = w->is_signed ? 1 : 0; a.per_channel = w->C != 1;
     a.x_scale = x_scale; a.x_zp = x_zero_point; a.x_qmin = x_qmin; a.x_qmax = x_qmax;
     if (lut_codes_host) memcpy(a.lut, lut_codes_host, (size_t)w->K);
@@ -1359,6 +1371,22 @@ int mctq_packed_dwconv2d_i8(const MctqPackedDesc* w, const MctqConv2dGeom* g, in
     if (x_dtype == MCTQ_F32) return run(PackType<float>{});
     if (x_dtype == MCTQ_BF16) return run(PackType<__nv_bfloat16>{});
     return run(PackType<__half>{});
+}
+
+int mctq_packed_dwconv2d_i8_plan(const MctqConv2dGeom* g, int64_t Cout, int x_nhwc, MctqDwPlan* out) {
+    if (!out) return MCTQ_E_BADARG;
+    if (const int rc = dw_check_geometry(g, Cout, x_nhwc)) return rc;
+    if ((int64_t)g->kh * g->kw > 33025) return MCTQ_E_RANGE;
+    DwArgs a;
+    dw_set_geometry(a, g, Cout);
+    if (const int rc = dw_plan(a, x_nhwc != 0)) return rc;
+    out->S = a.S;
+    out->TH = a.TH;
+    out->TW = a.TW;
+    out->IH = a.IH;
+    out->IW = a.IW;
+    out->smem_bytes = (int32_t)dw_smem_bytes(a);
+    return 0;
 }
 
 int mctq_dequant_affine(const void* codes, int code_mode, int is_signed, float* y, int64_t n, const float* scale,

@@ -1612,6 +1612,21 @@ class IntegerDepthwiseConv2d:
         return y
 
 
+def dwconv_plan(N, C, H, W, out_channels, kernel_size, stride, dilation, padding, channels_last=False):
+    """The tile plan mctq_packed_dwconv2d_i8 launches for x [N, C, H, W] (mctq_packed_dwconv2d_i8_plan, host only): a dict
+    of S (slots per work unit), TH x TW (output tile), IH x IW (window tile) and smem_bytes, or None when the dilated window
+    does not fit the kernel's shared memory even for one output of one channel (the launch returns MCTQ_E_RANGE)."""
+    Ho, Wo = conv_output_hw(H, W, kernel_size, stride, dilation, padding)
+    g = _native.MctqConv2dGeom(N, H, W, C, Ho, Wo, *kernel_size, *stride, *dilation, *padding)
+    plan = _native.MctqDwPlan()
+    rc = _native.load().mctq_packed_dwconv2d_i8_plan(ctypes.addressof(g), out_channels, int(bool(channels_last)),
+                                                     ctypes.addressof(plan))
+    if rc == -3:                                                 # MCTQ_E_RANGE
+        return None
+    _native.check(rc, "mctq_packed_dwconv2d_i8_plan")
+    return {f: getattr(plan, f) for f, _ in _native.MctqDwPlan._fields_}
+
+
 def _packed_dwconv2d_i8_cuda(x, x_scale, x_zero_point, x_qmin, x_qmax, codes, kind, is_signed, out_channels, kernel_size,
                              stride, dilation, padding, zero_point, factor, lut_values, bias, channels_last):
     """mctq::packed_dwconv2d_i8: the [Cout][kh*kw] weight codes (or LUT indices with their int8 centroid codes

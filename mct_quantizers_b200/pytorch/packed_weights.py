@@ -440,9 +440,10 @@ def integer_conv_eligibility(wrapper, input_quantizer, lut: bool = False, pad: b
 def integer_depthwise_eligibility(wrapper, input_quantizer, lut: bool = False) -> Tuple[bool, str]:
     """(True, '') when `wrapper` can run in integer convolution mode as a depthwise convolution (mctq_packed_dwconv2d_i8):
     the layer, wrapper and input-quantizer conditions of integer_conv_eligibility, with groups == in_channels > 1 (any
-    channel multiplier) instead of groups 1, a contiguous or channels_last [Cout, 1, kh, kw] weight, and kh * kw at most
-    33025 (the int32 bound of the centred sum: each factor has magnitude <= 255).  `lut=True` also accepts LUT weights that
-    meet _lut_code_eligibility.  Host-only."""
+    channel multiplier) instead of groups 1, a contiguous or channels_last [Cout, 1, kh, kw] weight, kh * kw at most
+    33025 (the int32 bound of the centred sum: each factor has magnitude <= 255), and a dilated window that the kernel can
+    stage in shared memory (mctq_packed_dwconv2d_i8_plan).  `lut=True` also accepts LUT weights that meet
+    _lut_code_eligibility.  Host-only."""
     r = _conv_eligibility(wrapper, input_quantizer, lut, depthwise=True)
     if not r[0]:
         return r
@@ -451,9 +452,17 @@ def integer_depthwise_eligibility(wrapper, input_quantizer, lut: bool = False) -
         ok, reason = _lut_code_eligibility(e)
         if not ok:
             return ok, reason
-    K = shape[2] * shape[3]
+    kh, kw = shape[2], shape[3]
+    K = kh * kw
     if K > 33025:
         return False, f"kh * kw = {K} exceeds 33025, the largest window whose int32 sum of code products cannot overflow"
+    # the planner fails for every input size exactly when its smallest tile (one output of one channel) does not fit: ask
+    # it for the one output of an input as large as the dilated window
+    dh, dw = (int(d) for d in wrapper.layer.dilation)
+    ih, iw = (kh - 1) * dh + 1, (kw - 1) * dw + 1
+    if ops.dwconv_plan(1, 1, ih, iw, 1, (kh, kw), (1, 1), (dh, dw), (0, 0, 0, 0)) is None:
+        return False, (f"the dilated {kh} x {kw} window ({ih} x {iw} input pixels) does not fit the depthwise kernel's "
+                       f"shared memory")
     return True, ""
 
 

@@ -209,7 +209,79 @@ def test_eligibility():
     big = _fake_packed_conv(_dw_wrapper(c=2, k=(2, 16513)))
     assert integer_depthwise_eligibility(big, q) == \
         (False, "kh * kw = 33026 exceeds 33025, the largest window whose int32 sum of code products cannot overflow")
-    assert integer_depthwise_eligibility(_fake_packed_conv(_dw_wrapper(c=2, k=(5, 6605))), q) == (True, "")
+    # under the int32 bound, but a window the kernel cannot stage in shared memory
+    assert integer_depthwise_eligibility(_fake_packed_conv(_dw_wrapper(c=2, k=(5, 6605))), q) == \
+        (False, "the dilated 5 x 6605 window (5 x 6605 input pixels) does not fit the depthwise kernel's shared memory")
+
+
+@pytest.mark.parametrize("k,dilation,ok", [((3, 3), 112, True), ((3, 3), 113, False), ((1, 25597), 1, True),
+                                           ((1, 25598), 1, False), ((5, 6605), 1, False), ((25597, 1), 1, True),
+                                           ((3, 1), (25596, 1), False), ((3, 1), (25595, 1), True)])
+def test_eligibility_window_bound(k, dilation, ok):
+    """The smallest tile of the kernel (one output of one channel) needs 20 + 4 kh kw + 4 IH IW bytes of the 200 KB: 3x3 at
+    dilation 112 (225 x 225 input pixels) fits, at 113 (227 x 227) it does not; a 1 x 25597 row fits, 1 x 25598 does not."""
+    w = _fake_packed_conv(_dw_wrapper(c=2, k=k, dilation=dilation))
+    got = integer_depthwise_eligibility(w, _act())
+    kh, kw = k
+    dh, dw = (dilation, dilation) if isinstance(dilation, int) else dilation
+    ih, iw = (kh - 1) * dh + 1, (kw - 1) * dw + 1
+    assert (20 + 4 * kh * kw + 4 * ih * iw <= 200 * 1024) == ok
+    if ok:
+        assert got == (True, "")
+    else:
+        assert got == (False, f"the dilated {kh} x {kw} window ({ih} x {iw} input pixels) does not fit the depthwise "
+                              f"kernel's shared memory")
+    # the kernel's own answer for a real input of that window, at N = 0 (a no-op when it plans)
+    # the kernel's own answer for an input of that window and any of its paddings, both layouts
+    for nhwc in (False, True):
+        for pad in ((0, 0, 0, 0), (dh, dh, dw, dw)):
+            assert (ops.dwconv_plan(2, 2, ih, iw, 2, k, (1, 1), (dh, dw), pad, nhwc) is not None) == ok, (nhwc, pad)
+
+
+def _plan(N, C, H, W, m, k, stride, dilation, padding, nhwc):
+    p = ops.dwconv_plan(N, C, H, W, C * m, k, stride, dilation, padding, nhwc)
+    return p and (p["S"], p["TH"], p["TW"])
+
+
+def test_plan_query():
+    # hand-worked from the planner: 3x3, dilation 100, padding 100 on 300 x 300 NCHW planes.  S = 1 (90000 outputs a
+    # plane), TW = 64, TH = 2048 / 64 = 32; the 232 x 264 window tile of 4 bytes a pixel is 245 KB: TH halves to 1
+    # (201 x 264: 212 KB), then TW to 32 (201 x 232: 182 KB)
+    p = ops.dwconv_plan(1, 1, 300, 300, 1, (3, 3), (1, 1), (100, 100), (100, 100, 100, 100))
+    assert p == dict(S=1, TH=1, TW=32, IH=201, IW=232, smem_bytes=20 + 36 + 201 * 232 * 4)
+    # 3x3, dilation 30, padding 30 on 8 x 8 planes, 32 or more of them: S = 32, TH = TW = 8, slots padded to SB = 34; TH
+    # halves to 1 (61 x 68 x 34 x 2 bytes = 282 KB), then S to 16 (SB = 18: 150 KB)
+    for nc in (32, 40, 1000):
+        p = ops.dwconv_plan(1, nc, 8, 8, nc, (3, 3), (1, 1), (30, 30), (30, 30, 30, 30))
+        assert p == dict(S=16, TH=1, TW=8, IH=61, IW=68, smem_bytes=16 * 20 + 9 * 16 * 4 + 61 * 68 * 18 * 2)
+    # fewer planes than 32: S is the number of planes (no shrink)
+    assert _plan(1, 5, 8, 8, 1, (3, 3), (1, 1), (1, 1), (1, 1, 1, 1), False) == (5, 8, 8)
+    # NHWC starts at 32 channels of an 8 x 16 tile, whatever C is
+    assert _plan(2, 3, 112, 112, 1, (3, 3), (2, 2), (1, 1), (0, 1, 0, 1), True) == (32, 8, 16)
+    # a 56 x 56 NCHW plane: one plane per unit, the full width and 2048 / 56 = 36 rows
+    assert _plan(2, 144, 56, 56, 1, (3, 3), (1, 1), (1, 1), (1, 1, 1, 1), False) == (1, 36, 56)
+    # the largest windows that plan, and the first that do not
+    assert _plan(1, 1, 225, 225, 1, (3, 3), (1, 1), (112, 112), (0, 0, 0, 0), False) == (1, 1, 1)
+    assert _plan(1, 1, 227, 227, 1, (3, 3), (1, 1), (113, 113), (0, 0, 0, 0), False) is None
+    assert _plan(1, 1, 1, 25597, 1, (1, 25597), (1, 1), (1, 1), (0, 0, 0, 0), True) == (1, 1, 1)
+    assert _plan(1, 1, 1, 25598, 1, (1, 25598), (1, 1), (1, 1), (0, 0, 0, 0), True) is None
+    # rejections: those of the launch
+    lib = _native.load()
+    out = _native.MctqDwPlan()
+    assert lib.mctq_packed_dwconv2d_i8_plan(ctypes.byref(_geom()), 16, 0, None) == E_BADARG
+    assert lib.mctq_packed_dwconv2d_i8_plan(None, 16, 0, ctypes.byref(out)) == E_BADARG
+    assert lib.mctq_packed_dwconv2d_i8_plan(ctypes.byref(_geom()), 24, 0, ctypes.byref(out)) == E_BADARG
+    assert lib.mctq_packed_dwconv2d_i8_plan(ctypes.byref(_geom(kh=0)), 16, 0, ctypes.byref(out)) == E_BADARG
+    assert lib.mctq_packed_dwconv2d_i8_plan(ctypes.byref(_geom()), 16, 2, ctypes.byref(out)) == E_BADARG
+    assert lib.mctq_packed_dwconv2d_i8_plan(ctypes.byref(_geom(kh=2, kw=16513)), 16, 0, ctypes.byref(out)) == E_RANGE
+    assert lib.mctq_packed_dwconv2d_i8_plan(ctypes.byref(_geom()), 16, 1, ctypes.byref(out)) == 0
+    assert (out.S, out.TH, out.TW, out.IH, out.IW) == (32, 8, 8, 10, 10)
+    # the launch refuses exactly the windows the plan query refuses, before any CUDA call
+    for kh, kw, d in ((5, 6605, 1), (3, 3, 113), (1, 25598, 1)):
+        ih, iw = (kh - 1) * d + 1, (kw - 1) * d + 1
+        g = _geom(N=1, Cin=1, H=ih, W=iw, Ho=1, Wo=1, kh=kh, kw=kw, dh=d, dw=d, pt=0, pb=0, pl=0, pr=0)
+        assert lib.mctq_packed_dwconv2d_i8_plan(ctypes.byref(g), 1, 0, ctypes.byref(out)) == E_RANGE
+        assert _dw_call(_lin_desc(out_f=1, in_f=kh * kw), g=g, Cout=1) == E_RANGE
 
 
 def _lut_dw(kind=LI4, c=32, k=3, **q):
